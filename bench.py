@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- HolE training throughput on B200 (BASELINE.json metric), one JSON line.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--batch B]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--batch B] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of B synthetic triples: Philox
 type-safe corruption, fused gather/clip/score/sigmoid/hinge forward+backward, deterministic
@@ -20,6 +20,11 @@ larger than L2, so no flush is needed between steps.
 
 `--impl reference` times that CPU port alone (TensorFlow 1.2, which holE.py needs, cannot be
 installed offline; see DESIGN.md).
+
+`--dump-outputs DIR` (N = 1) writes what the timed call left to its caller, so that two builds can be
+compared output for output on identical seeded inputs: loss_sums.npy (the per-step loss sums it
+returned) and embeddings.npy (table rows after its last step, float32, at the row ids in
+embedding_rows.npy; see dump_rows).
 """
 import argparse
 import json
@@ -173,6 +178,28 @@ def lr_schedule(n_steps, first_step, batch_count):
                      for s in range(first_step, first_step + n_steps)], dtype=np.float32)
 
 
+DUMP_SAMPLE = 16384      # rows per sampled set: at most 2 * 16384 + relations rows of d=256 floats (~34 MB)
+
+
+def dump_rows(kg, last_batch):
+    """Row ids whose final values --dump-outputs writes: every relation row, a seeded sample of the entity
+    rows the last step's triples use, and a seeded sample of all entity rows.  The table itself (1.2 GB) is
+    too large to write whole."""
+    rng = np.random.default_rng(20170904)
+    used = np.unique(last_batch[:, :2])
+    ents = np.arange(kg.n_relations, kg.n_rows)
+    return np.unique(np.concatenate([np.arange(kg.n_relations),
+                                     rng.choice(used, min(DUMP_SAMPLE, len(used)), replace=False),
+                                     rng.choice(ents, min(DUMP_SAMPLE, len(ents)), replace=False)]))
+
+
+def write_dump(out_dir, loss_sums, rows, table_rows):
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss_sums.npy"), loss_sums)
+    np.save(os.path.join(out_dir, "embedding_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "embeddings.npy"), np.ascontiguousarray(table_rows, dtype=np.float32))
+
+
 def cpu_port_throughput(kg, off, ids, B, min_seconds, max_steps, warmup=1):
     """Time oracle/hole_ref.c train steps (corruption drawn by the NumPy Philox oracle
     outside the timed region); cycles over the generated batches until `min_seconds` of CPU
@@ -212,10 +239,14 @@ def run_reference(args):
     negs = [O.corrupt(kg.triples[s * B:(s + 1) * B], kg.type_of, off, ids, 1, s) for s in range(K + W)]
     for s in range(W):
         R.train_step(E, kg.triples[s * B:(s + 1) * B], negs[s][1], negs[s][0], MARGIN, LR0, sc)
+    sums = np.empty(K, np.float64)
     t0 = time.perf_counter()
     for s in range(W, W + K):
-        R.train_step(E, kg.triples[s * B:(s + 1) * B], negs[s][1], negs[s][0], MARGIN, LR0, sc)
+        sums[s - W], _ = R.train_step(E, kg.triples[s * B:(s + 1) * B], negs[s][1], negs[s][0], MARGIN, LR0, sc)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        rows = dump_rows(kg, kg.triples[(W + K - 1) * B:(W + K) * B])
+        write_dump(args.dump_outputs, sums, rows, E[rows])
     v = K * B / dt
     sample = f"{K} steps of B={B} triples of the {WORKLOAD} workload (corruption ids precomputed)"
     print(json.dumps({
@@ -373,6 +404,8 @@ def run_ours(args):
         raise SystemExit(f"--gpus {args.gpus} but WORLD_SIZE={world}; launch with torch.distributed.run")
     torch.cuda.set_device(local_rank)
     if world > 1:
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the single-GPU timed call's outputs; use --gpus 1")
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
         from graphembeddings_b200 import sharded
         return sharded.bench(args, dist, rank, world, local_rank)
@@ -410,6 +443,11 @@ def run_ours(args):
     ms = ev0.elapsed_time(ev1)
     value = K * B / (ms * 1e-3)
     mean_loss = float(sums.mean().item()) / B
+    if args.dump_outputs:
+        # before the e2e and roofline passes below train the same table further
+        rows = dump_rows(kg, kg.triples[(W + K - 1) * B:(W + K) * B])
+        table_rows = eng.embeddings()[torch.from_numpy(rows).to(eng.device)].cpu().numpy()
+        write_dump(args.dump_outputs, sums.cpu().numpy(), rows, table_rows)
 
     # ---- end to end from pinned host triples ("e2e")
     # (warm-up with a call of the timed call's shape: staging and pinned buffers are sized on first use)
@@ -498,6 +536,8 @@ def main():
     ap.add_argument("--no-ranking", action="store_true")
     ap.add_argument("--no-config4", action="store_true", help="skip the 20M-entity d=512 sub-record")
     ap.add_argument("--no-coverage", action="store_true", help="N = 1: skip the configs[0] / B=512 / variant sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="N = 1: write the timed call's loss sums and a fixed sample of its final table rows as .npy")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3

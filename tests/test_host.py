@@ -204,3 +204,26 @@ def test_bench_warm_up_issues_exactly_w_steps_in_order(W):
         assert lo == nxt * B and hi == (nxt + n) * B and first_step == 7 + nxt and n >= 1
         nxt += n
     assert nxt == W
+
+
+def test_bench_dump_outputs_are_seeded_and_bounded(tmp_path):
+    """bench.py --dump-outputs: the same rows on every run, every relation row among them, under 64 MB at the
+    headline shape (1,200,014 rows x d=256, B=32768), written as float32 / float64 .npy files."""
+    import sys
+    import types
+    sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+    import bench
+
+    kg = types.SimpleNamespace(n_relations=14, n_rows=1_200_014)
+    last = np.random.default_rng(0).integers(14, kg.n_rows, size=(32768, 3))
+    rows = bench.dump_rows(kg, last)
+    assert np.array_equal(rows, bench.dump_rows(kg, last))
+    assert np.array_equal(rows[:14], np.arange(14)) and rows[-1] < kg.n_rows
+    assert np.isin(rows, last[:, :2]).sum() >= bench.DUMP_SAMPLE
+    assert len(rows) * 256 * 4 + 8 * len(rows) < 64 << 20
+    table_rows = np.random.default_rng(1).standard_normal((len(rows), 256)).astype(np.float32)
+    bench.write_dump(str(tmp_path), np.arange(5, dtype=np.float32), rows, table_rows)
+    got = {p.stem: np.load(p) for p in tmp_path.iterdir()}
+    assert sorted(got) == ["embedding_rows", "embeddings", "loss_sums"]
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert np.array_equal(got["embedding_rows"], rows) and np.array_equal(got["embeddings"], table_rows)
