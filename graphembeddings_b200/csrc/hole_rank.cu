@@ -41,6 +41,9 @@ constexpr int MAX_STAGES = 8;     // barrier slots
 constexpr int SMEM_LIMIT = 227 * 1024;
 
 enum { MODE_COUNT = 0, MODE_DIAG = 1 };
+// epilogue of hole_rank_kernel, chosen at compile time: EPI_RANK runs MODE_COUNT / MODE_DIAG, EPI_TOPK keeps
+// each thread's k best candidates (hole_topk)
+enum { EPI_RANK = 0, EPI_TOPK = 1 };
 
 struct RankParams {
   int mode;
@@ -62,6 +65,12 @@ struct RankParams {
   float* true_out;             // [Q]   DIAG: score of the true candidate if it lives in this shard
   const uint32_t* qp_words;    // wide kernel: the packed query operand as 32-bit words, K/2 per row
   int K;                       // wide kernel: operand columns (bf16) per row
+  // top-k epilogue (EPI_TOPK)
+  int topk;                    // k
+  uint64_t* tk_keys;           // [Qpad][n_chunks][2][k] per-thread candidate lists (binary max-heaps)
+  const int64_t* f_off;        // [Q+1] filter CSR, or null
+  const int32_t* f_ids;        //       ids ascending within a query's slice
+  int64_t ent_begin;
 };
 
 // ------------------------------------------------------------------------------------ PTX
@@ -329,6 +338,121 @@ __device__ __forceinline__ int epi_count128(uint32_t taddr0, int j0, float thr, 
   return c0;
 }
 
+// ---- top-k epilogue.  A candidate is the 64-bit key (order-preserving bits of s, local index j): ascending
+// keys are ascending (s, id), the reference heap's pop order (holE.py:434, 446-453).  -0 is folded into +0 so
+// that the float compare and the key order agree.
+constexpr uint64_t TOPK_EMPTY = ~0ull;      // larger than every real key
+__device__ __forceinline__ uint32_t f32_order_bits(float s) {
+  const uint32_t u = __float_as_uint(s + 0.0f);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float f32_from_order_bits(uint32_t b) {
+  return __uint_as_float((b & 0x80000000u) ? (b & 0x7fffffffu) : ~b);
+}
+__device__ __forceinline__ uint64_t topk_key(float s, uint32_t j) {
+  return ((uint64_t)f32_order_bits(s) << 32) | j;
+}
+
+// One thread's list: a binary max-heap of at most k keys in global memory; thr = the float of its root once
+// it is full (+inf before).  Candidates arrive in increasing index order, so a later candidate with the
+// root's score loses the tie and `s < thr` is the whole admission test.
+struct TopkList {
+  uint64_t* heap;
+  int n, k;
+  float thr;
+  int64_t f0, f1;            // the query's filter slice [f0, f1) of f_ids
+};
+
+__device__ __forceinline__ bool in_filter(const int32_t* __restrict__ ids, int64_t lo, int64_t hi, int32_t id) {
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) >> 1;
+    const int32_t v = ids[mid];
+    if (v == id) return true;
+    if (v < id) lo = mid + 1; else hi = mid;
+  }
+  return false;
+}
+
+__device__ __forceinline__ void topk_insert(TopkList& L, uint64_t key) {
+  uint64_t* h = L.heap;
+  if (L.n < L.k) {                                // sift up from the new leaf
+    int i = L.n++;
+    while (i > 0) {
+      const int par = (i - 1) >> 1;
+      const uint64_t pk = h[par];
+      if (pk >= key) break;
+      h[i] = pk;
+      i = par;
+    }
+    h[i] = key;
+  } else {                                        // replace the root (key < root), sift down
+    int i = 0;
+    for (;;) {
+      int c = 2 * i + 1;
+      if (c >= L.k) break;
+      uint64_t ck = h[c];
+      if (c + 1 < L.k) {
+        const uint64_t rk = h[c + 1];
+        if (rk > ck) { ck = rk; ++c; }
+      }
+      if (ck <= key) break;
+      h[i] = ck;
+      i = c;
+    }
+    h[i] = key;
+  }
+  if (L.n == L.k) L.thr = f32_from_order_bits((uint32_t)(h[0] >> 32));
+}
+
+// Hot path: one compare per score of 32 accumulator columns, and a warp vote.
+__device__ __forceinline__ bool epi_topk_vote(const uint32_t (&v)[32], float thr) {
+  bool hit = false;
+#pragma unroll
+  for (int c = 0; c < 32; ++c) hit |= __uint_as_float(v[c]) < thr;
+  return __any_sync(0xffffffffu, hit);
+}
+// Slow path, only for a warp in which some lane admits a candidate of columns j0 .. j0+31: bounds, filter,
+// heap insert.  Runs while no tcgen05.ld is in flight (the loaded registers are final).
+__device__ __forceinline__ void epi_topk_admit(const uint32_t (&v)[32], int j0, TopkList& L, int Nc,
+                                               const int32_t* __restrict__ f_ids, int64_t ent_begin) {
+  uint32_t m = 0;
+#pragma unroll
+  for (int c = 0; c < 32; ++c) m |= (__uint_as_float(v[c]) < L.thr ? 1u : 0u) << c;
+  while (m != 0) {
+    const int c = __ffs(m) - 1;
+    m &= m - 1;
+    float s = 0.f;
+#pragma unroll
+    for (int i = 0; i < 32; ++i) s = (i == c) ? __uint_as_float(v[i]) : s;     // no dynamic register index
+    const int j = j0 + c;
+    if (!(s < L.thr) || j >= Nc) continue;                                     // thr may have dropped
+    if (L.f0 < L.f1 && in_filter(f_ids, L.f0, L.f1, (int32_t)(ent_begin + j))) continue;
+    topk_insert(L, topk_key(s, (uint32_t)j));
+  }
+  __syncwarp();          // reconverge before the next .sync.aligned tcgen05 instruction
+}
+// 128 columns of one accumulator row.  The next chunk's TMEM load is in flight during the vote on the current
+// one; the slow path of a chunk runs after that load has landed.
+__device__ __forceinline__ void epi_topk128(uint32_t taddr0, int j0, TopkList& L, int Nc,
+                                            const int32_t* __restrict__ f_ids, int64_t ent_begin) {
+  uint32_t va[32], vb[32];
+  tmem_ld32_async(taddr0, va);
+  tmem_ld_wait(va);
+  tmem_ld32_async(taddr0 + 32, vb);
+  bool h = epi_topk_vote(va, L.thr);
+  tmem_ld_wait(vb);
+  if (h) epi_topk_admit(va, j0, L, Nc, f_ids, ent_begin);
+  tmem_ld32_async(taddr0 + 64, va);
+  h = epi_topk_vote(vb, L.thr);
+  tmem_ld_wait(va);
+  if (h) epi_topk_admit(vb, j0 + 32, L, Nc, f_ids, ent_begin);
+  tmem_ld32_async(taddr0 + 96, vb);
+  h = epi_topk_vote(va, L.thr);
+  tmem_ld_wait(vb);
+  if (h) epi_topk_admit(va, j0 + 64, L, Nc, f_ids, ent_begin);
+  if (epi_topk_vote(vb, L.thr)) epi_topk_admit(vb, j0 + 96, L, Nc, f_ids, ent_begin);
+}
+
 struct SmemLayout {
   uint64_t full[MAX_STAGES];
   uint64_t empty[MAX_STAGES];
@@ -341,8 +465,9 @@ struct SmemLayout {
 
 // ------------------------------------------------------------------------------------ kernel
 // PARTS = 1 plain bf16, 2 split-bf16 (compile-time, so that the bf16 instantiation's single-thread
-// producer / issue loops carry none of the split mode's bookkeeping)
-template <int PARTS>
+// producer / issue loops carry none of the split mode's bookkeeping); EPI = EPI_RANK / EPI_TOPK (compile-time,
+// so that the counting epilogue carries none of the top-k code)
+template <int PARTS, int EPI>
 __global__ void __launch_bounds__(RANK_THREADS, 1)
 hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const RankParams p) {
@@ -456,6 +581,40 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         }
         umma_commit(&sl->a_empty);                   // query tile may be overwritten
       }
+    }
+  } else if constexpr (EPI == EPI_TOPK) {
+    // ===================== top-k epilogue =====================
+    // Each thread keeps the k best of its 128 columns of every tile of the work item: list
+    // [q][chunk][cgrp] of p.tk_keys, unused slots TOPK_EMPTY.  hole_topk_merge_kernel combines the lists.
+    const int ew = warp - WARP_EPI0;
+    const int quarter = warp & 3;
+    const int cgrp = ew >> 2;
+    const int row_in_tile = quarter * 32 + lane;
+    int acc = 0; uint32_t acc_phase = 0;
+    for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
+      const int m_tile = item / p.n_chunks, chunk = item % p.n_chunks;
+      const int q = m_tile * BM + row_in_tile;
+      const bool qok = q < p.Q;
+      TopkList L;
+      L.heap = p.tk_keys + (((size_t)q * p.n_chunks + chunk) * 2 + cgrp) * p.topk;
+      L.n = 0; L.k = p.topk;
+      L.thr = qok ? INFINITY : -INFINITY;            // rows past Q admit nothing
+      L.f0 = L.f1 = 0;
+      if (qok && p.f_off != nullptr) { L.f0 = p.f_off[q]; L.f1 = p.f_off[q + 1]; }
+      const int t0 = chunk * p.chunk_tiles;
+      const int t1 = min(p.n_tiles, t0 + p.chunk_tiles);
+      for (int t = t0; t < t1; ++t) {
+        mbar_wait(&sl->tmem_full[acc], acc_phase);
+        tc_fence_after();
+        const uint32_t taddr0 = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * BN + cgrp * EPI_COLS);
+        epi_topk128(taddr0, t * BN + cgrp * EPI_COLS, L, p.Nc, p.f_ids, p.ent_begin);
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&sl->tmem_empty[acc]);
+        if (++acc == 2) { acc = 0; acc_phase ^= 1; }
+      }
+      if (qok)
+        for (int i = L.n; i < L.k; ++i) L.heap[i] = TOPK_EMPTY;
     }
   } else {
     // ===================== epilogue =====================
@@ -898,7 +1057,7 @@ __global__ void __launch_bounds__(256)
 hole_rank_pack_query_kernel(const float* __restrict__ table, int stride, int H,
                             const int32_t* __restrict__ queries, int Q, int Qpad, int side,
                             int64_t ent_begin, int K, int parts, __nv_bfloat16* __restrict__ out,
-                            int32_t* __restrict__ true_idx) {
+                            int32_t* __restrict__ true_idx, float* __restrict__ qf) {
   extern __shared__ uint4 pq_smem[];                    // one operand row per warp, written out as 16-byte vectors
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   const int64_t qi = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
@@ -963,6 +1122,12 @@ hole_rank_pack_query_kernel(const float* __restrict__ table, int stride, int H,
         im[i] = a[i] * d[i] + b[i] * c[i];
       }
       const int k0 = 4 * g;
+      if (qf != nullptr) {     // hole_topk: the fp32 query vector before rounding, [Re | Im] of K floats
+        float* qrow = qf + (size_t)qi * K;
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+          if (k0 + i < H) { qrow[k0 + i] = re[i]; qrow[H + k0 + i] = im[i]; }
+      }
       if (k0 + 4 <= H) {       // whole group: the real part is 8-byte aligned in the row
         __nv_bfloat162 p0 = __floats2bfloat162_rn(re[0], re[1]), p1 = __floats2bfloat162_rn(re[2], re[3]);
         uint2 u;
@@ -1002,7 +1167,7 @@ __global__ void __launch_bounds__(256)
 hole_rank_pack_query_ccorr_kernel(const float* __restrict__ table, int stride, int H,
                                   const int32_t* __restrict__ queries, int Q, int Qpad, int side,
                                   int64_t ent_begin, int K, int parts, __nv_bfloat16* __restrict__ out,
-                                  int32_t* __restrict__ true_idx) {
+                                  int32_t* __restrict__ true_idx, float* __restrict__ qf) {
   extern __shared__ float pqc_smem[];                   // per warp: entity row doubled (4H), rho (2H)
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   const int64_t qi = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
@@ -1050,6 +1215,7 @@ hole_rank_pack_query_ccorr_kernel(const float* __restrict__ table, int stride, i
   for (int v = 0; v < NV; ++v) {
     const int k = lane + 32 * v;
     if (k < H) {
+      if (qf != nullptr) { qf[(size_t)qi * K + k] = qv.re[v]; qf[(size_t)qi * K + H + k] = qv.im[v]; }
       const __nv_bfloat16 rh = __float2bfloat16(qv.re[v]), ih = __float2bfloat16(qv.im[v]);
       o[k] = rh;
       o[H + k] = ih;
@@ -1116,6 +1282,110 @@ hole_rank_filter_kernel(const __nv_bfloat16* __restrict__ qp, const __nv_bfloat1
   if (lane == 0 && hits != 0) atomicSub(&filt_cnt[qi], hits);
 }
 
+// hole_topk, after the contraction: one block per output row.
+//  1. the k smallest keys of the row's n_lists partial lists (k keys each, TOPK_EMPTY-padded): an 8-pass
+//     MSB-first radix select finds the k-th smallest key K*, then every key < K* and K* itself are taken
+//     (real keys are unique -- each candidate lives in one list -- so only TOPK_EMPTY repeats);
+//  2. each selected candidate is rescored in fp32: the clipped fp32 table row times the fp32 query vector qf;
+//  3. the row is sorted by (fp32 score, id); slots without a candidate get id -1 and score +inf.
+constexpr int TOPK_MAX = 128;
+constexpr int MERGE_THREADS = 256;
+__global__ void __launch_bounds__(MERGE_THREADS)
+hole_topk_merge_kernel(const uint64_t* __restrict__ keys, int n_lists, int k, const float* __restrict__ table,
+                       int stride, int H, int64_t ent_begin, const float* __restrict__ qf, int K,
+                       int32_t* __restrict__ ids_out, float* __restrict__ scores_out) {
+  __shared__ uint32_t hist[256];
+  __shared__ uint64_t sel[TOPK_MAX];
+  __shared__ float sc[TOPK_MAX];
+  __shared__ uint64_t prefix_s;
+  __shared__ int kk_s, cnt_s;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int64_t q = blockIdx.x;
+  int32_t* ido = ids_out + q * k;
+  float* sco = scores_out + q * k;
+  if (n_lists == 0) {                                  // empty candidate range
+    for (int i = tid; i < k; i += MERGE_THREADS) { ido[i] = -1; sco[i] = INFINITY; }
+    return;
+  }
+  const int64_t L = (int64_t)n_lists * k;              // >= 2k: the k-th smallest key exists
+  const uint64_t* kr = keys + q * L;
+  uint64_t prefix = 0, mask = 0;
+  int kk = k;                                          // rank of K* among the keys matching prefix
+  for (int shift = 56; shift >= 0; shift -= 8) {
+    for (int i = tid; i < 256; i += MERGE_THREADS) hist[i] = 0;
+    __syncthreads();
+    for (int64_t i = tid; i < L; i += MERGE_THREADS) {
+      const uint64_t x = kr[i];
+      if ((x & mask) == prefix) atomicAdd(&hist[(x >> shift) & 255], 1u);
+    }
+    __syncthreads();
+    if (warp == 0) {                                   // digit of K*: lane l scans bins 8l .. 8l+7
+      uint32_t c[8], tot = 0;
+#pragma unroll
+      for (int i = 0; i < 8; ++i) { c[i] = hist[lane * 8 + i]; tot += c[i]; }
+      uint32_t inc = tot;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t y = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= o) inc += y;
+      }
+      uint32_t cum = inc - tot;
+      if (cum < (uint32_t)kk && (uint32_t)kk <= inc) {
+        int d = -1;
+#pragma unroll
+        for (int i = 0; i < 8; ++i)
+          if (d < 0) {
+            if (cum + c[i] >= (uint32_t)kk) d = lane * 8 + i; else cum += c[i];
+          }
+        kk_s = kk - (int)cum;
+        prefix_s = prefix | ((uint64_t)d << shift);
+      }
+    }
+    __syncthreads();
+    kk = kk_s;
+    prefix = prefix_s;
+    mask |= 0xffull << shift;
+  }
+  if (tid == 0) cnt_s = 0;
+  __syncthreads();
+  for (int64_t i = tid; i < L; i += MERGE_THREADS) {
+    const uint64_t x = kr[i];
+    if (x < prefix) sel[atomicAdd(&cnt_s, 1)] = x;     // k - kk keys
+  }
+  __syncthreads();
+  for (int i = k - kk + tid; i < k; i += MERGE_THREADS) sel[i] = prefix;
+  __syncthreads();
+  const float* qrow = qf + q * K;
+  const int Hp = stride / 2;
+  for (int i = warp; i < k; i += MERGE_THREADS / 32) {
+    const uint64_t x = sel[i];
+    if (x == TOPK_EMPTY) continue;
+    const float* row = table + (size_t)(ent_begin + (uint32_t)x) * stride;
+    float ss = 0.f;
+    for (int c = lane; c < H; c += 32) { const float a = row[c], b = row[Hp + c]; ss = fmaf(a, a, fmaf(b, b, ss)); }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
+    const float scl = fminf(__frsqrt_rn(ss), 1.0f);
+    float d = 0.f;
+    for (int c = lane; c < H; c += 32) d = fmaf(row[c] * scl, qrow[c], fmaf(row[Hp + c] * scl, qrow[H + c], d));
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) d += __shfl_xor_sync(0xffffffffu, d, o);
+    if (lane == 0) sc[i] = d;
+  }
+  __syncthreads();
+  uint64_t mine = TOPK_EMPTY;
+  if (tid < k && sel[tid] != TOPK_EMPTY) mine = topk_key(sc[tid], (uint32_t)sel[tid]);
+  __syncthreads();
+  if (tid < k) sel[tid] = mine;
+  __syncthreads();
+  if (tid < k) {
+    int r = 0;
+    for (int i = 0; i < k; ++i) { const uint64_t o = sel[i]; r += (o < mine || (o == mine && i < tid)) ? 1 : 0; }
+    if (mine == TOPK_EMPTY) { ido[r] = -1; sco[r] = INFINITY; }
+    else { ido[r] = (int32_t)(ent_begin + (uint32_t)mine); sco[r] = f32_from_order_bits((uint32_t)(mine >> 32)); }
+  }
+}
+
 // ------------------------------------------------------------------------------------ host
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
@@ -1157,6 +1427,9 @@ struct hole_rank_ws {
   __nv_bfloat16* tq = nullptr;     // [Qpad + BN, K] gathered true rows
   int32_t* true_idx = nullptr;     // [Qpad]
   size_t cand_cap = 0, q_cap = 0;  // elements
+  float* qf = nullptr;             // hole_topk: [Qpad, K] fp32 query vectors
+  uint64_t* tk_keys = nullptr;     // hole_topk: [Qpad][n_chunks][2][k] partial lists
+  size_t qf_cap = 0, tk_cap = 0;   // elements
   bool attr_set = false;
   int64_t last_npad = 0, last_qpad = 0;
   int last_K = 0;
@@ -1174,24 +1447,51 @@ void hole_rank_cache_invalidate(hole_ctx* c) {
 void hole_rank_ws_free(hole_ctx* c) {
   if (c->rank == nullptr) return;
   cudaFree(c->rank->cand); cudaFree(c->rank->qp); cudaFree(c->rank->tq); cudaFree(c->rank->true_idx);
+  cudaFree(c->rank->qf); cudaFree(c->rank->tk_keys);
   delete c->rank;
   c->rank = nullptr;
 }
 
+// Work items of the 128-query kernel: enough to balance the persistent CTAs, chunks of at least 8 candidate tiles.
+static void split_chunks(RankParams& p, int sm_count) {
+  const int want_items = 8 * sm_count;
+  const int chunks = std::max(1, std::min(p.n_tiles / 8, (want_items + p.m_tiles - 1) / p.m_tiles));
+  p.chunk_tiles = (p.n_tiles + chunks - 1) / chunks;
+  p.n_chunks = (p.n_tiles + p.chunk_tiles - 1) / p.chunk_tiles;
+}
+
+struct TopkArgs {
+  int k;
+  int32_t* ids_out;
+  float* scores_out;
+};
+
 // prepare_only: pack (and keep) the candidate operand, nothing else
+// tk != null: hole_topk (the k best candidates per row instead of counts / true scores)
 static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t ent_end,
                      const float* query_table, const int32_t* queries, int64_t Q, int side, int precision,
                      const int64_t* filter_off, const int32_t* filter_ids, float* true_score_io,
                      int compute_true, int32_t* raw_before, int32_t* filt_before, void* stream,
-                     bool prepare_only) {
+                     bool prepare_only, const TopkArgs* tk = nullptr) {
   HOLE_CHECK_ARG(c && Q >= 0 && ent_begin >= 0 && ent_end >= ent_begin && ent_end <= c->n_rows);
   HOLE_CHECK_ARG(side == HOLE_SIDE_TAIL || side == HOLE_SIDE_HEAD || side == HOLE_SIDE_BOTH);
+  const bool topk = tk != nullptr;
+  if (topk && Q > 0 && ent_end == ent_begin) {       // no candidates: every output row is padding
+    HOLE_CHECK_ARG(queries != nullptr);
+    HOLE_CUDA_TRY(cudaSetDevice(c->device));
+    const int64_t rows = (side == HOLE_SIDE_BOTH) ? 2 * Q : Q;
+    HOLE_CHECK_ARG(rows < (int64_t(1) << 30));
+    hole_topk_merge_kernel<<<(unsigned)rows, MERGE_THREADS, 0, (cudaStream_t)stream>>>(
+        nullptr, 0, tk->k, nullptr, 0, 0, 0, nullptr, 0, tk->ids_out, tk->scores_out);
+    HOLE_LAUNCHED();
+    return HOLE_OK;
+  }
   if ((Q == 0 && !prepare_only) || ent_end == ent_begin) return HOLE_OK;
   if (side == HOLE_SIDE_BOTH) Q *= 2;    // output rows: [tail ranks of all queries | head ranks]
   const bool count = raw_before != nullptr;          // without count buffers: true scores only
-  HOLE_CHECK_ARG(table != nullptr && (prepare_only || (queries && true_score_io)));
+  HOLE_CHECK_ARG(table != nullptr && (prepare_only || (queries && (topk || true_score_io))));
   HOLE_CHECK_ARG((raw_before == nullptr) == (filt_before == nullptr));
-  HOLE_CHECK_ARG(prepare_only || count || compute_true);
+  HOLE_CHECK_ARG(prepare_only || topk || count || compute_true);
   if (query_table == nullptr) query_table = table;
   HOLE_CHECK_ARG((filter_off == nullptr) == (filter_ids == nullptr));
   HOLE_CHECK_ARG(precision == HOLE_RANK_BF16 || precision == HOLE_RANK_BF16X3);
@@ -1201,7 +1501,7 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
   cudaStream_t st = (cudaStream_t)stream;
 
   const char* pe_ = getenv("HOLE_RANK_PAIR");      // experimental cta_group::2 kernel (see DESIGN.md)
-  const bool use_pair = pe_ != nullptr && pe_[0] == '1';
+  const bool use_pair = !topk && pe_ != nullptr && pe_[0] == '1';
   const int Nc = (int)(ent_end - ent_begin);
   const int K = (c->dim + BK - 1) / BK * BK;
   const int num_kb = K / BK;
@@ -1209,7 +1509,7 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
   // experimental wide kernel (256 queries per candidate tile, query operand in TMEM; plain bf16, K <= 256):
   // bit-identical counts, half the L2->SM traffic, and no faster because the call is power-bound (DESIGN.md section 9)
   const char* we_ = getenv("HOLE_RANK_WIDE");
-  const bool use_wide = !use_pair && parts == 1 && K <= 256 && we_ != nullptr && we_[0] == '1';
+  const bool use_wide = !topk && !use_pair && parts == 1 && K <= 256 && we_ != nullptr && we_[0] == '1';
   const int qtile = (use_pair || use_wide) ? 2 * BM : BM;
   const int Qpad = (int)((Q + qtile - 1) / qtile * qtile);
   const int Kall = K * parts;                                  // operand columns in memory
@@ -1249,9 +1549,31 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
     }
     w->q_cap = (size_t)Qpad * Kall;
   }
+  RankParams p{};
+  p.m_tiles = use_pair ? Qpad / (2 * BM) : Qpad / BM;      // diagonal pass and the 128-query kernels
+  if (topk) {
+    p.n_tiles = Npad / BN;
+    split_chunks(p, c->sm_count);
+    const size_t n_keys = (size_t)Qpad * p.n_chunks * 2 * tk->k;
+    if ((size_t)Qpad * K > w->qf_cap || n_keys > w->tk_cap) {
+      const size_t qf_n = std::max((size_t)Qpad * K, w->qf_cap), tk_n = std::max(n_keys, w->tk_cap);
+      HOLE_CUDA_TRY(cudaStreamSynchronize(st));
+      cudaFree(w->qf); cudaFree(w->tk_keys);
+      w->qf = nullptr; w->tk_keys = nullptr; w->qf_cap = w->tk_cap = 0;
+      if (cudaMalloc((void**)&w->qf, qf_n * sizeof(float)) != cudaSuccess ||
+          cudaMalloc((void**)&w->tk_keys, tk_n * sizeof(uint64_t)) != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(w->qf); w->qf = nullptr;
+        return hole_set_error(HOLE_ERR_ALLOC, "top-k workspace allocation failed (%zu candidate keys)", tk_n);
+      }
+      w->qf_cap = qf_n; w->tk_cap = tk_n;
+    }
+  }
   if (!w->attr_set) {
-    HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-    HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<1, EPI_RANK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<2, EPI_RANK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<1, EPI_TOPK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<2, EPI_TOPK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     w->attr_set = true;
@@ -1284,7 +1606,7 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));                 \
       hole_rank_pack_query_ccorr_kernel<N><<<grid, 32 * warps, smem, st>>>(query_table, c->row_stride, c->H, queries, \
                                                                            (int)Q, Qpad, side, ent_begin, K, parts,  \
-                                                                           w->qp, w->true_idx);                      \
+                                                                           w->qp, w->true_idx, topk ? w->qf : nullptr); \
     } while (0)
     if (nv <= 1) HOLE_PQC_LAUNCH(1);
     else if (nv <= 2) HOLE_PQC_LAUNCH(2);
@@ -1301,7 +1623,8 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
     const int pq_iters = (c->row_stride / 2 + 127) / 128;
 #define HOLE_PQ_LAUNCH(N)                                                                                          \
     hole_rank_pack_query_kernel<N><<<pq_grid, 256, pq_smem, st>>>(query_table, c->row_stride, c->H, queries, (int)Q, \
-                                                                  Qpad, side, ent_begin, K, parts, w->qp, w->true_idx)
+                                                                  Qpad, side, ent_begin, K, parts, w->qp, w->true_idx, \
+                                                                  topk ? w->qf : nullptr)
     if (pq_iters == 1) HOLE_PQ_LAUNCH(1);
     else if (pq_iters == 2) HOLE_PQ_LAUNCH(2);
     else if (pq_iters == 3) HOLE_PQ_LAUNCH(3);
@@ -1314,15 +1637,33 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
   int rc = make_map(&mapA, w->qp, Qpad, Kall, BM);
   if (rc) return rc;
 
-  RankParams p{};
   p.num_kb = num_kb;
   p.parts = parts;
   p.last_kb_mmas = (c->dim - (num_kb - 1) * BK + UMMA_K - 1) / UMMA_K;
   p.stages = stages;
-  p.m_tiles = use_pair ? Qpad / (2 * BM) : Qpad / BM;      // diagonal pass and the 128-query kernels
   p.Q = (int)Q;
   p.Nc = Nc;
   p.true_idx = w->true_idx;
+
+  if (topk) {
+    rc = make_map(&mapB, w->cand, Npad, Kall, BN);
+    if (rc) return rc;
+    p.mode = MODE_COUNT;
+    p.topk = tk->k;
+    p.tk_keys = w->tk_keys;
+    p.f_off = filter_off;
+    p.f_ids = filter_ids;
+    p.ent_begin = ent_begin;
+    const int grid = std::min(p.m_tiles * p.n_chunks, c->sm_count);
+    if (parts == 2) hole_rank_kernel<2, EPI_TOPK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+    else hole_rank_kernel<1, EPI_TOPK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+    HOLE_LAUNCHED();
+    hole_topk_merge_kernel<<<(unsigned)Q, MERGE_THREADS, 0, st>>>(w->tk_keys, p.n_chunks * 2, tk->k, table,
+                                                                  c->row_stride, c->H, ent_begin, w->qf, K,
+                                                                  tk->ids_out, tk->scores_out);
+    HOLE_LAUNCHED();
+    return HOLE_OK;
+  }
 
   if (compute_true) {
     const int rows = Qpad + BN;
@@ -1339,8 +1680,8 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
       hole_rank_pair_kernel<<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
     } else {
       const int grid = std::min(p.m_tiles, c->sm_count);
-      if (parts == 2) hole_rank_kernel<2><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
-      else hole_rank_kernel<1><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+      if (parts == 2) hole_rank_kernel<2, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+      else hole_rank_kernel<1, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
     }
     HOLE_LAUNCHED();
   }
@@ -1377,13 +1718,7 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
   if (rc) return rc;
   p.mode = MODE_COUNT;
   p.n_tiles = Npad / BN;
-  // work items: enough to balance the persistent CTAs, chunks of at least 8 candidate tiles
-  {
-    int want_items = 8 * c->sm_count;
-    int chunks = std::max(1, std::min(p.n_tiles / 8, (want_items + p.m_tiles - 1) / p.m_tiles));
-    p.chunk_tiles = (p.n_tiles + chunks - 1) / chunks;
-    p.n_chunks = (p.n_tiles + p.chunk_tiles - 1) / p.chunk_tiles;
-  }
+  split_chunks(p, c->sm_count);
   p.true_score = true_score_io;
   p.raw_cnt = raw_before;
   p.filt_cnt = filt_before;
@@ -1394,8 +1729,8 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
       hole_rank_pair_kernel<<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
     } else {
       const int grid = std::min(n_items, c->sm_count);
-      if (parts == 2) hole_rank_kernel<2><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
-      else hole_rank_kernel<1><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+      if (parts == 2) hole_rank_kernel<2, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+      else hole_rank_kernel<1, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
     }
     HOLE_LAUNCHED();
   }
@@ -1420,6 +1755,16 @@ extern "C" int hole_rank_ex(hole_ctx* c, const float* table, int64_t ent_begin, 
                             int compute_true, int32_t* raw_before, int32_t* filt_before, void* stream) {
   return rank_impl(c, table, ent_begin, ent_end, query_table, queries, Q, side, precision, filter_off, filter_ids,
                    true_score_io, compute_true, raw_before, filt_before, stream, false);
+}
+
+extern "C" int hole_topk(hole_ctx* c, const float* table, int64_t ent_begin, int64_t ent_end,
+                         const int32_t* queries, int64_t Q, int side, int precision, int k,
+                         const int64_t* filter_off, const int32_t* filter_ids,
+                         int32_t* ids_out, float* scores_out, void* stream) {
+  HOLE_CHECK_ARG(c && k >= 1 && k <= TOPK_MAX && ids_out != nullptr && scores_out != nullptr);
+  const TopkArgs tk{k, ids_out, scores_out};
+  return rank_impl(c, table, ent_begin, ent_end, nullptr, queries, Q, side, precision, filter_off, filter_ids,
+                   nullptr, 0, nullptr, nullptr, stream, false, &tk);
 }
 
 extern "C" int hole_rank_prepare(hole_ctx* c, const float* table, int64_t ent_begin, int64_t ent_end,

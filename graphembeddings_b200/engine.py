@@ -347,6 +347,34 @@ class HoleEngine:
                                  _stream()))
         return raw_before, filt_before, true_score
 
+    def topk(self, queries, side, ent_begin, ent_end, k, filter_off=None, filter_ids=None,
+             precision=HOLE_RANK_BF16X3):
+        """Top-k link prediction (the pop loop of eval_link_prediction, holE.py:427-472, over all candidates
+        [ent_begin, ent_end)): for every query row the k candidates first in ascending (score, id) order,
+        skipping its filter slice.  Returns (ids int32[Q', k], scores float32[Q', k]) on the device, Q' = Q or
+        2Q for HOLE_SIDE_BOTH; padding is id -1 / score +inf.  Each filter slice must be ascending."""
+        q = self._triples(queries)
+        rows = q.shape[0] * (2 if int(side) == HOLE_SIDE_BOTH else 1)
+        fo = fi = None
+        if filter_off is not None:
+            off = np.asarray(filter_off.cpu() if isinstance(filter_off, torch.Tensor) else filter_off, dtype=np.int64)
+            ids = np.asarray(filter_ids.cpu() if isinstance(filter_ids, torch.Tensor) else filter_ids, dtype=np.int64)
+            if off.shape != (rows + 1,) or off[0] != 0 or off[-1] != len(ids) or np.any(np.diff(off) < 0):
+                raise HoleError(f"filter_off must be a CSR offset array of {rows + 1} entries over {len(ids)} ids")
+            desc = np.diff(ids) < 0                    # descending step inside one slice
+            starts = off[1:-1]
+            desc[starts[(starts > 0) & (starts < len(ids))] - 1] = False
+            if desc.any():
+                raise HoleError("filter ids must be ascending within each query's slice")
+            fo = torch.as_tensor(off).to(self.device).contiguous()
+            fi = torch.as_tensor(ids.astype(np.int32)).to(self.device).contiguous()
+        ids_out = torch.empty((rows, int(k)), dtype=torch.int32, device=self.device)
+        scores = torch.empty((rows, int(k)), dtype=torch.float32, device=self.device)
+        check(self.lib.hole_topk(self._ctx, _ptr(self.table), int(ent_begin), int(ent_end), _ptr(q), q.shape[0],
+                                 int(side), int(precision), int(k), _ptr(fo), _ptr(fi), _ptr(ids_out), _ptr(scores),
+                                 _stream()))
+        return ids_out, scores
+
     def rank_prepare(self, ent_begin, ent_end, precision=HOLE_RANK_BF16):
         """Pack the candidate operand of [ent_begin, ent_end) once; later rank() calls on the same table /
         range reuse it (until a training call on this engine or rank_invalidate())."""

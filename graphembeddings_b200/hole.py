@@ -458,6 +458,42 @@ def eval_link_prediction_typed(eng, heads, candidate, true_triples, test_triples
     return (raw[ok] + 1).tolist(), (filt[ok] + 1).tolist()
 
 
+def predict_top_k(eng, test, known, relation_count, entity_count, k, path, precision=HOLE_RANK_BF16X3,
+                  value=None):
+    """The all-entity generalisation of the reference's `max_triples` cut of the pop loop (holE.py:427-472):
+    the k best NEW tails of every distinct (head, relation) pair of the test file and the k best new heads of
+    every distinct (tail, relation) pair, filtered against the train + valid triples.  Writes one line per
+    prediction to `path`:  side  head  tail  relation  position  score  value  in_test
+    (position 1-based, score = raw s, value = value(s) (sigma by default), in_test = the predicted triple is
+    a test triple: the reference's MATCH vs GUESS).  Returns the number of lines written."""
+    value = value or (lambda s: 1.0 / (1.0 + np.exp(-s)))
+    test = np.asarray(test, dtype=np.int64).reshape(-1, 3)
+    test_set = set(map(tuple, test.tolist()))
+    n = 0
+    with open(path, 'w') as out:
+        for side_name, side, key_col in (("tail", HOLE_SIDE_TAIL, 0), ("head", HOLE_SIDE_HEAD, 1)):
+            pairs = np.unique(test[:, [key_col, 2]], axis=0)
+            if len(pairs) == 0:
+                continue
+            queries = np.zeros((len(pairs), 3), dtype=np.int32)     # the predicted column is ignored
+            queries[:, key_col] = pairs[:, 0]
+            queries[:, 2] = pairs[:, 1]
+            foff, fids = D.build_filter_csr(queries, known, side_name)
+            ids, scores = eng.topk(queries, side, relation_count, entity_count, k, foff, fids, precision=precision)
+            ids, scores = ids.cpu().numpy(), scores.cpu().numpy().astype(np.float64)
+            vals = value(scores)
+            for i, (a, r) in enumerate(pairs.tolist()):
+                for pos in range(k):
+                    c = int(ids[i, pos])
+                    if c < 0:
+                        break
+                    h, t = (a, c) if side == HOLE_SIDE_TAIL else (c, a)
+                    out.write('{}\t{}\t{}\t{}\t{}\t{:.9g}\t{:.6f}\t{}\n'.format(
+                        side_name, h, t, r, pos + 1, scores[i, pos], vals[i, pos], (h, t, r) in test_set))
+                    n += 1
+    return n
+
+
 def infer_triples(flags=None, log=print):
     """holE.py:530-582 with the all-entity filtered protocol."""
     flags = flags or FLAGS
@@ -476,6 +512,13 @@ def infer_triples(flags=None, log=print):
     raw, filt = eval_link_prediction(eng, data.test, data.known, data.relation_count, data.entity_count,
                                      threshold=threshold, results_path='inference_results.tsv',
                                      precision=precision)
+    k = getattr(flags, 'predict_top_k', 0)
+    if k:
+        value = np.tanh if getattr(flags, 'score_variant', 'complex') != 'complex' else None
+        path = os.path.join(flags.output_dir, 'predictions.tsv')
+        n = predict_top_k(eng, data.test, data.known, data.relation_count, data.entity_count, k, path,
+                          precision=precision, value=value)
+        log('Wrote {} predictions to {}'.format(n, path))
     if not raw:
         log('No test triple passed the confidence gate; no ranks recorded.')
         return None
@@ -511,6 +554,9 @@ def build_parser():
                         help='Apply the reference\'s `min sigma < infer_threshold` gate (off: it never fires).')
     parser.add_argument('--rank_precision', choices=['bf16', 'bf16x3'], default='bf16x3',
                         help='Tensor-core operand precision of --infer (bf16x3 = split-bf16, ~fp32 ranks).')
+    parser.add_argument('--predict_top_k', type=int, default=0,
+                        help='With --infer: write the K best new tails of every (head, relation) and heads of every '
+                             '(tail, relation) pair of the test file to <output_dir>/predictions.tsv (0 = off).')
     parser.add_argument('--valid_sample', action='store_true',
                         help='Validate on one sampled batch as holE.py does (default: the whole triples-valid.txt).')
     parser.add_argument('--score_variant', choices=['complex', 'ccorr_tanh'], default='complex',

@@ -50,14 +50,14 @@ typedef struct hole_ctx hole_ctx;
 
 #define HOLE_SIDE_TAIL 0         /* corrupt / rank tails */
 #define HOLE_SIDE_HEAD 1         /* corrupt / rank heads */
-#define HOLE_SIDE_BOTH 2         /* hole_rank only: tails then heads in one pass */
+#define HOLE_SIDE_BOTH 2         /* hole_rank / hole_topk only: tails then heads in one pass */
 
 /* Operand precision of the tensor-core ranking contraction. */
 #define HOLE_RANK_BF16   0       /* bf16 operands, fp32 accumulate                      */
 #define HOLE_RANK_BF16X3 1       /* split-bf16 (hi*hi + lo*hi + hi*lo): ranks match fp32 except within ~3e-5 of a tie; dim <= 320 */
 
 /* ABI version of this header; hole_abi_version() returns the library's. */
-#define HOLE_ABI_VERSION 2
+#define HOLE_ABI_VERSION 3
 HOLE_API int hole_abi_version(void);
 
 /* Thread-local message of the last failing call on this thread ("" if none). */
@@ -305,6 +305,31 @@ HOLE_API int hole_rank_ex(hole_ctx* ctx, const float* table, int64_t ent_begin, 
 HOLE_API int hole_rank_prepare(hole_ctx* ctx, const float* table, int64_t ent_begin, int64_t ent_end,
                       int precision, void* stream);
 HOLE_API int hole_rank_invalidate(hole_ctx* ctx);
+
+/* ---- top-k link prediction: the entities the model puts first for (h, r, ?) or (?, r, t).  Replaces the pop
+ * loop of eval_link_prediction (holE.py:427-472: candidates popped in ascending order, at most
+ * InferenceCandidates.max_triples of them) over ALL candidates [ent_begin, ent_end), on the same tensor-core
+ * contraction as hole_rank (same operand packing, same hole_rank_prepare cache and invalidation rules).
+ * For query q = (h, t, r) the candidate scores s_j are hole_rank's (TAIL / HEAD, or the HOLE_SCORE_CCORR_TANH
+ * query vector in that mode); the id being predicted (t for TAIL, h for HEAD) is ignored.
+ * Row q of the output holds the k candidates first in ascending (s, id) order (lower is better, ties to the
+ * smaller id: the heap's order, holE.py:231, 434, 446-453), skipping the ids of q's filter slice:
+ *   ids_out    int32 [Q', k]  global row ids, sorted by (score, id)
+ *   scores_out float32 [Q', k] raw s of each id
+ * with Q' = Q, or 2Q for HOLE_SIDE_BOTH (rows [0,Q) tails, [Q,2Q) heads, filter_off then has 2Q+1 entries).
+ * filter_off int64[Q'+1] / filter_ids int32[.] may be NULL; the ids of each slice must be ASCENDING (binary
+ * search; data.build_filter_csr produces them so).  Fewer than k remaining candidates: the row is padded with
+ * id -1, score +inf.
+ * Precision: the selection runs at the contraction's operand precision (HOLE_RANK_BF16 / _BF16X3); the
+ * returned scores are recomputed in fp32 from the fp32 table (clipped candidate row . fp32 query vector), so
+ * the id set is the exact top-k except for candidates within the precision's near-tie band of the k-th score.
+ * 1 <= k <= 128, else HOLE_ERR_ARG.  HOLE_ERR_ALLOC when the workspace ([Q'][work items][2][k] 8-byte keys)
+ * cannot be allocated: split Q.  hole_rank_debug_operands returns the operands of the last hole_rank or
+ * hole_topk call. */
+HOLE_API int hole_topk(hole_ctx* ctx, const float* table, int64_t ent_begin, int64_t ent_end,
+                       const int32_t* queries, int64_t Q, int side, int precision, int k,
+                       const int64_t* filter_off, const int32_t* filter_ids,
+                       int32_t* ids_out, float* scores_out, void* stream);
 
 /* Test hook: copy the bf16 operands the last hole_rank call packed (device to device).
  * cand_out [n_pad, K] / query_out [q_pad, K] may be NULL to query the shapes only. */
