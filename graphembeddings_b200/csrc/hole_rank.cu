@@ -15,8 +15,6 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 
-#include <stdlib.h>
-
 #include <algorithm>
 
 #include "hole_common.cuh"
@@ -37,7 +35,7 @@ constexpr int RANK_THREADS = 64 + 32 * EPI_WARPS;
 // that feed the tensor pipe must not be starved by the epilogue warps, so they come last.
 constexpr int WARP_TMA = EPI_WARPS, WARP_MMA = EPI_WARPS + 1, WARP_EPI0 = 0;
 constexpr int EPI_COLS = 256 / (EPI_WARPS / 4);    // columns of the 256-wide tile one warp owns
-constexpr int MAX_STAGES = 8;     // barrier slots
+constexpr int MAX_STAGES = 4;     // candidate k-block ring slots and their barriers; a fifth 32 KB stage measured no gain
 constexpr int SMEM_LIMIT = 227 * 1024;
 
 enum { MODE_COUNT = 0, MODE_DIAG = 1 };
@@ -63,8 +61,6 @@ struct RankParams {
   int32_t* raw_cnt;            // [Q]   COUNT: += count
   int32_t* filt_cnt;           // [Q]   COUNT: += count (filter hits are subtracted afterwards)
   float* true_out;             // [Q]   DIAG: score of the true candidate if it lives in this shard
-  const uint32_t* qp_words;    // wide kernel: the packed query operand as 32-bit words, K/2 per row
-  int K;                       // wide kernel: operand columns (bf16) per row
   // top-k epilogue (EPI_TOPK)
   int topk;                    // k
   uint64_t* tk_keys;           // [Qpad][n_chunks][2][k] per-thread candidate lists (binary max-heaps)
@@ -183,104 +179,6 @@ __device__ __forceinline__ void tmem_ld_wait(uint32_t (&v)[32]) {
         "+r"(v[22]), "+r"(v[23]), "+r"(v[24]), "+r"(v[25]), "+r"(v[26]), "+r"(v[27]), "+r"(v[28]),
         "+r"(v[29]), "+r"(v[30]), "+r"(v[31])
       :
-      : "memory");
-}
-// one lane of a converged warp (warp-uniform control flow around it keeps MMA operands in uniform registers)
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "elect.sync _|p, 0xffffffff;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t"
-      "}" : "=r"(pred));
-  return pred != 0;
-}
-// 32 registers of this thread -> 32 consecutive TMEM columns of its lane
-__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&v)[32]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-      ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]),
-        "r"(v[8]), "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]),
-        "r"(v[16]), "r"(v[17]), "r"(v[18]), "r"(v[19]), "r"(v[20]), "r"(v[21]), "r"(v[22]), "r"(v[23]),
-        "r"(v[24]), "r"(v[25]), "r"(v[26]), "r"(v[27]), "r"(v[28]), "r"(v[29]), "r"(v[30]), "r"(v[31])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() {
-  asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-}
-// D[tmem] (+)= A[tmem] * B[smem]^T: the A operand (128 rows x 16 bf16) is read from TMEM (lane = row,
-// two consecutive K elements per 32-bit column), so shared memory serves the B operand only
-__device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b,
-                                             uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t"
-      "}" ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
-// ---- CTA-pair (cta_group::2) variants
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// TMA load issued by either CTA of the pair; the transaction bytes are credited to the barrier
-// at the same offset in CTA 0 (peer bit of the shared::cluster address cleared)
-__device__ __forceinline__ void tma_load_2d_pair(void* smem_dst, const CUtensorMap* map, uint64_t* bar,
-                                                 int c0, int c1) {
-  uint32_t bar0;   // shared::cluster address of the same barrier in CTA 0
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(bar0) : "r"(smem_u32(bar)), "r"(0));
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(smem_dst)), "l"((uint64_t)map), "r"(bar0), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t* slot, uint32_t cols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)),
-               "r"(cols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t addr, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(cols) : "memory");
-}
-// D[tmem of both CTAs] (+)= A (128 rows per CTA) * B^T (N/2 rows per CTA), issued by CTA 0 only
-__device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b,
-                                               uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
-      "}" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// arrive on the barrier at this offset in BOTH CTAs when the pair's MMAs issued so far retire
-__device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-          smem_u32(bar)),
-      "h"((uint16_t)3)
-      : "memory");
-}
-// arrive on the barrier at this offset in CTA `cta` of the cluster
-__device__ __forceinline__ void mbar_arrive_cluster(uint64_t* bar, uint32_t cta) {
-  asm volatile(
-      "{\n\t"
-      ".reg .b32 ra;\n\t"
-      "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-      "mbarrier.arrive.shared::cluster.b64 _, [ra];\n\t"
-      "}" ::"r"(smem_u32(bar)), "r"(cta)
       : "memory");
 }
 
@@ -466,11 +364,14 @@ struct SmemLayout {
 // ------------------------------------------------------------------------------------ kernel
 // PARTS = 1 plain bf16, 2 split-bf16 (compile-time, so that the bf16 instantiation's single-thread
 // producer / issue loops carry none of the split mode's bookkeeping); EPI = EPI_RANK / EPI_TOPK (compile-time,
-// so that the counting epilogue carries none of the top-k code)
+// so that the counting epilogue carries none of the top-k code).
+// p is __grid_constant__ so that its fields are read in place from parameter space where they are used.  Passed
+// by value, the struct (128 bytes) is loaded into registers at entry, and each top-k instantiation compiles to
+// 112 more instructions.
 template <int PARTS, int EPI>
 __global__ void __launch_bounds__(RANK_THREADS, 1)
 hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                 const RankParams p) {
+                 const __grid_constant__ RankParams p) {
   extern __shared__ uint8_t smem_raw[];
   // 128-byte swizzle atoms repeat every 1024 bytes: align the operand area explicitly
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -669,349 +570,6 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     }
   }
   __syncwarp();          // the single-lane roles rejoin their warps
-  tc_fence_before();
-  __syncthreads();
-  if (warp == WARP_MMA) tmem_dealloc(tmem_base, 512);
-}
-
-// ------------------------------------------------------------------------------------ CTA-pair kernel
-// Same contraction with cta_group::2: a cluster of two CTAs (one SM pair) computes a
-// 256-query x 256-candidate tile per MMA.  Each CTA keeps its own 128 query rows and loads only
-// HALF of every candidate k-block (128 rows), which halves the per-SM operand traffic that
-// bounds the single-CTA kernel; CTA 0 issues the MMAs for both, every CTA runs the epilogue
-// on its own TMEM (its 128 rows x all 256 columns).
-constexpr int B_HALF_BYTES = (BN / 2) * BK * 2;   // 16 KB
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(RANK_THREADS, 1)
-hole_rank_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                      const RankParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  uint8_t* sA = smem;                                       // num_kb x 16 KB (my 128 query rows)
-  uint8_t* sB = smem + (size_t)p.num_kb * A_KB_BYTES;       // stages x 16 KB (my half of the tile)
-  SmemLayout* sl = reinterpret_cast<SmemLayout*>(sB + (size_t)p.stages * B_HALF_BYTES);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t cta = cluster_ctarank();                   // 0 = leader (issues the MMAs)
-  const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-  const int n_items = p.m_tiles * p.n_chunks;               // m_tiles counts 256-row query pairs here
-
-  if (warp == WARP_TMA && lane == 0) {
-    tma_prefetch_desc(&tmA);
-    tma_prefetch_desc(&tmB);
-    for (int s = 0; s < p.stages; ++s) { mbar_init(&sl->full[s], 1); mbar_init(&sl->empty[s], 1); }
-    mbar_init(&sl->a_full, 1);
-    mbar_init(&sl->a_empty, 1);
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(&sl->tmem_full[s], 1);
-      mbar_init(&sl->tmem_empty[s], 2 * EPI_WARPS);         // both CTAs' epilogue warps (used in CTA 0)
-    }
-    fence_barrier_init();
-  }
-  if (warp == WARP_MMA) tmem_alloc_pair(&sl->tmem_base, 512);
-  tc_fence_before();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = sl->tmem_base;
-
-  if (warp == WARP_TMA) {
-    // ===================== TMA producer (both CTAs) =====================
-    if (lane == 0) {
-      int stage = 0; uint32_t phase = 0, a_phase = 0;
-      for (int item = pair; item < n_items; item += n_pairs) {
-        const int m_pair = item / p.n_chunks, chunk = item % p.n_chunks;
-        const int m_tile = m_pair * 2 + (int)cta;
-        mbar_wait(&sl->a_empty, a_phase ^ 1);
-        if (cta == 0) mbar_expect_tx(&sl->a_full, (uint32_t)(2 * p.num_kb * A_KB_BYTES));
-        for (int kb = 0; kb < p.num_kb; ++kb)
-          tma_load_2d_pair(sA + (size_t)kb * A_KB_BYTES, &tmA, &sl->a_full, kb * BK, m_tile * BM);
-        a_phase ^= 1;
-        const int t0 = (p.mode == MODE_DIAG) ? 0 : chunk * p.chunk_tiles;
-        const int t1 = (p.mode == MODE_DIAG) ? 1 : min(p.n_tiles, t0 + p.chunk_tiles);
-        for (int t = t0; t < t1; ++t) {
-          const int row0 = ((p.mode == MODE_DIAG) ? m_pair * BN : t * BN) + (int)cta * (BN / 2);
-          for (int kb = 0; kb < p.num_kb; ++kb) {
-            mbar_wait(&sl->empty[stage], phase ^ 1);
-            if (cta == 0) mbar_expect_tx(&sl->full[stage], 2 * B_HALF_BYTES);
-            tma_load_2d_pair(sB + (size_t)stage * B_HALF_BYTES, &tmB, &sl->full[stage], kb * BK, row0);
-            if (++stage == p.stages) { stage = 0; phase ^= 1; }
-          }
-        }
-      }
-    }
-  } else if (warp == WARP_MMA) {
-    // ===================== MMA issuer (CTA 0 only) =====================
-    if (lane == 0 && cta == 0) {
-      constexpr uint32_t idesc = umma_idesc_bf16(2 * BM, BN);
-      int stage = 0; uint32_t phase = 0, a_phase = 0;
-      int acc = 0; uint32_t acc_phase = 0;
-      for (int item = pair; item < n_items; item += n_pairs) {
-        const int chunk = item % p.n_chunks;
-        mbar_wait(&sl->a_full, a_phase);
-        a_phase ^= 1;
-        tc_fence_after();
-        const int t0 = (p.mode == MODE_DIAG) ? 0 : chunk * p.chunk_tiles;
-        const int t1 = (p.mode == MODE_DIAG) ? 1 : min(p.n_tiles, t0 + p.chunk_tiles);
-        for (int t = t0; t < t1; ++t) {
-          mbar_wait(&sl->tmem_empty[acc], acc_phase ^ 1);
-          tc_fence_after();
-          const uint32_t d_addr = tmem_base + (uint32_t)acc * BN;
-          for (int kb = 0; kb < p.num_kb; ++kb) {
-            mbar_wait(&sl->full[stage], phase);
-            tc_fence_after();
-            const uint32_t a_addr = smem_u32(sA + (size_t)kb * A_KB_BYTES);
-            const uint32_t b_addr = smem_u32(sB + (size_t)stage * B_HALF_BYTES);
-            const int nk = (kb == p.num_kb - 1) ? p.last_kb_mmas : BK / UMMA_K;
-#pragma unroll
-            for (int k = 0; k < BK / UMMA_K; ++k) {
-              if (k < nk) {
-                const uint64_t da = umma_desc_sw128(a_addr + k * UMMA_K * 2);
-                const uint64_t db = umma_desc_sw128(b_addr + k * UMMA_K * 2);
-                umma_bf16_pair(d_addr, da, db, idesc, (kb | k) != 0 ? 1u : 0u);
-              }
-            }
-            umma_commit_pair(&sl->empty[stage]);     // frees the stage in both CTAs
-            if (++stage == p.stages) { stage = 0; phase ^= 1; }
-          }
-          umma_commit_pair(&sl->tmem_full[acc]);     // accumulators of both CTAs ready
-          if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-        }
-        umma_commit_pair(&sl->a_empty);              // query tiles of both CTAs may be overwritten
-      }
-    }
-  } else {
-    // ===================== epilogue (both CTAs, own TMEM) =====================
-    const int ew = warp - WARP_EPI0;
-    const int quarter = warp & 3;
-    const int half = ew >> 2;
-    const int row_in_tile = quarter * 32 + lane;
-    int acc = 0; uint32_t acc_phase = 0;
-    for (int item = pair; item < n_items; item += n_pairs) {
-      const int m_pair = item / p.n_chunks, chunk = item % p.n_chunks;
-      const int q = (m_pair * 2 + (int)cta) * BM + row_in_tile;
-      const bool qok = q < p.Q;
-      float thr = -INFINITY, thr_hi = -INFINITY;
-      int tie = 0;
-      if (p.mode == MODE_COUNT && qok) {
-        thr = p.true_score[q];
-        thr_hi = nextafterf(thr, INFINITY);
-        const int ti = p.true_idx[q];
-        tie = ti < 0 ? 0 : (ti > p.Nc ? p.Nc : ti);
-      }
-      int cnt = 0;
-      const int t0 = (p.mode == MODE_DIAG) ? 0 : chunk * p.chunk_tiles;
-      const int t1 = (p.mode == MODE_DIAG) ? 1 : min(p.n_tiles, t0 + p.chunk_tiles);
-      for (int t = t0; t < t1; ++t) {
-        mbar_wait(&sl->tmem_full[acc], acc_phase);
-        tc_fence_after();
-        const uint32_t taddr0 = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * BN + half * 128);
-        if (p.mode == MODE_COUNT) {
-          cnt += epi_count128(taddr0, t * BN + half * 128, thr, thr_hi, tie, p.Nc);
-        } else if (half == (int)cta) {
-          // DIAG: the tile's columns [cta*128, +128) are the true rows of this CTA's queries
-          uint32_t v[32];
-          tmem_ld32(taddr0 + quarter * 32, v);
-          float sc = 0.f;
-#pragma unroll
-          for (int k = 0; k < 32; ++k) sc = (k == lane) ? __uint_as_float(v[k]) : sc;
-          if (qok) {
-            const int ti = p.true_idx[q];
-            if (ti >= 0 && ti < p.Nc) p.true_out[q] = sc;
-          }
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(&sl->tmem_empty[acc], 0);   // the MMA issuer lives in CTA 0
-        if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-      }
-      if (p.mode == MODE_COUNT && qok && cnt != 0) {
-        atomicAdd(&p.raw_cnt[q], cnt);
-        atomicAdd(&p.filt_cnt[q], cnt);
-      }
-    }
-  }
-  __syncwarp();          // the single-lane roles rejoin their warps
-  tc_fence_before();
-  cluster_sync_all();
-  if (warp == WARP_MMA) tmem_dealloc_pair(tmem_base, 512);
-}
-
-// ------------------------------------------------------------------------------------ wide kernel
-// 256 queries per streamed candidate tile in ONE CTA, the query operand in TMEM.
-// The single-CTA kernel above streams the whole candidate operand for every 128 queries (K/64 bytes
-// of L2->SM traffic per score: 10 TB/s on this chip, its limit) and re-reads the query tile from
-// shared memory for every MMA (4 KB of the 12 KB an M=128 N=256 K=16 MMA reads).  Here the CTA
-// keeps TWO 128-query tiles in TMEM (2 x K/2 columns, written once per work item by the epilogue
-// warps with tcgen05.st) and multiplies each 128-candidate tile by both, one after the other: half
-// the L2->SM bytes per score, and shared memory serves the candidate operand only.  The two passes
-// over a candidate tile write two accumulators; the epilogue of one runs under the MMAs of the other,
-// so neither needs a second buffer.
-// TMEM columns: [0, K/2) queries 0-127, [K/2, K) queries 128-255, then two 128-column accumulators.  K <= 256.
-constexpr int WN = 128;                        // candidates per tile
-constexpr int W_STAGE_BYTES = WN * BK * 2;     // 16 KB
-constexpr int W_MAX_STAGES = 13;
-
-struct WideSmem {
-  uint64_t full[W_MAX_STAGES];
-  uint64_t empty[W_MAX_STAGES];
-  uint64_t a_full;
-  uint64_t a_empty;
-  uint64_t tmem_full[2];        // per query half
-  uint64_t tmem_empty[2];
-  uint32_t tmem_base;
-};
-
-__global__ void __launch_bounds__(RANK_THREADS, 1)
-hole_rank_wide_kernel(const __grid_constant__ CUtensorMap tmB, const RankParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* sB = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  WideSmem* sl = reinterpret_cast<WideSmem*>(sB + (size_t)p.stages * W_STAGE_BYTES);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int n_items = p.m_tiles * p.n_chunks;            // m_tiles counts 256-query pairs here
-  const int a_cols = p.K / 2;                            // TMEM columns of one 128-query tile
-
-  if (warp == WARP_TMA && lane == 0) {
-    tma_prefetch_desc(&tmB);
-    for (int s = 0; s < p.stages; ++s) { mbar_init(&sl->full[s], 1); mbar_init(&sl->empty[s], 1); }
-    mbar_init(&sl->a_full, EPI_WARPS);
-    mbar_init(&sl->a_empty, 1);
-    for (int s = 0; s < 2; ++s) { mbar_init(&sl->tmem_full[s], 1); mbar_init(&sl->tmem_empty[s], EPI_WARPS / 2); }
-    fence_barrier_init();
-  }
-  if (warp == WARP_MMA) tmem_alloc(&sl->tmem_base, 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = sl->tmem_base;
-  const uint32_t acc_base = tmem_base + (uint32_t)p.K;   // after the two query tiles
-
-  if (warp == WARP_TMA) {
-    // ===================== TMA producer: candidate k-blocks only =====================
-    if (lane == 0) {
-      int stage = 0; uint32_t phase = 0;
-      for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-        const int chunk = item % p.n_chunks;
-        const int t0 = chunk * p.chunk_tiles, t1 = min(p.n_tiles, t0 + p.chunk_tiles);
-        for (int t = t0; t < t1; ++t) {
-          for (int kb = 0; kb < p.num_kb; ++kb) {
-            mbar_wait(&sl->empty[stage], phase ^ 1);
-            mbar_expect_tx(&sl->full[stage], W_STAGE_BYTES);
-            tma_load_2d(sB + (size_t)stage * W_STAGE_BYTES, &tmB, &sl->full[stage], kb * BK, t * WN);
-            if (++stage == p.stages) { stage = 0; phase ^= 1; }
-          }
-        }
-      }
-    }
-  } else if (warp == WARP_MMA) {
-    // ===================== MMA issuer =====================
-    // The whole warp walks the loops (warp-uniform control flow, so that addresses and descriptors stay in
-    // uniform registers); one elected lane issues.
-    constexpr uint32_t idesc = umma_idesc_bf16(BM, WN);
-    int stage = 0; uint32_t phase = 0, a_phase = 0, acc_phase = 0;
-    for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-      const int chunk = item % p.n_chunks;
-      mbar_wait(&sl->a_full, a_phase);                   // both query tiles are in TMEM
-      a_phase ^= 1;
-      tc_fence_after();
-      const int t0 = chunk * p.chunk_tiles, t1 = min(p.n_tiles, t0 + p.chunk_tiles);
-      for (int t = t0; t < t1; ++t) {
-        const int stage0 = stage;
-        const uint32_t phase0 = phase;
-#pragma unroll 1
-        for (int mh = 0; mh < 2; ++mh) {                 // the tile against queries 0-127, then against 128-255
-          mbar_wait(&sl->tmem_empty[mh], acc_phase ^ 1);
-          tc_fence_after();
-          const uint32_t d = acc_base + (uint32_t)(mh * WN);
-          const uint32_t a_mh = tmem_base + (uint32_t)(mh * a_cols);
-          stage = stage0; phase = phase0;
-          for (int kb = 0; kb < p.num_kb; ++kb) {
-            if (mh == 0) {                               // the second pass finds the k-block in place
-              mbar_wait(&sl->full[stage], phase);
-              tc_fence_after();
-            }
-            const uint64_t db0 = umma_desc_sw128(smem_u32(sB + (size_t)stage * W_STAGE_BYTES));
-            const uint32_t a_kb = a_mh + (uint32_t)(kb * (BK / UMMA_K) * (UMMA_K / 2));
-            const int nk = (kb == p.num_kb - 1) ? p.last_kb_mmas : BK / UMMA_K;
-            if (elect_one()) {
-#pragma unroll
-              for (int k = 0; k < BK / UMMA_K; ++k) {
-                if (k < nk) {
-                  const uint64_t db = db0 + (uint64_t)(k * UMMA_K * 2 / 16);     // start-address field, 16-byte units
-                  umma_bf16_ts(d, a_kb + (uint32_t)(k * (UMMA_K / 2)), db, idesc, (kb | k) != 0 ? 1u : 0u);
-                }
-              }
-              if (mh == 1) umma_commit(&sl->empty[stage]);          // both passes have read the k-block
-            }
-            __syncwarp();
-            if (++stage == p.stages) { stage = 0; phase ^= 1; }
-          }
-          if (elect_one()) umma_commit(&sl->tmem_full[mh]);
-          __syncwarp();
-        }
-        acc_phase ^= 1;
-      }
-      if (elect_one()) umma_commit(&sl->a_empty);        // the query tiles may be overwritten
-      __syncwarp();
-    }
-  } else {
-    // ===================== epilogue warps: load the query tiles, then count =====================
-    const int quarter = warp & 3;            // TMEM lane quarter this warp may access
-    const int mh = (warp - WARP_EPI0) >> 2;  // which 128-query half
-    const uint32_t lane_base = (uint32_t)(quarter * 32) << 16;
-    uint32_t acc_phase = 0, a_phase = 0;
-    for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-      const int m_pair = item / p.n_chunks, chunk = item % p.n_chunks;
-      const int q = m_pair * (2 * BM) + mh * BM + quarter * 32 + lane;
-      // ---- this thread's query row -> its TMEM lane (K/2 columns), once per work item
-      mbar_wait(&sl->a_empty, a_phase ^ 1);              // the previous item's MMAs have retired
-      a_phase ^= 1;
-      tc_fence_after();
-      {
-        const uint4* src = reinterpret_cast<const uint4*>(p.qp_words + (size_t)q * a_cols);
-        const uint32_t ta = tmem_base + lane_base + (uint32_t)(mh * a_cols);
-        for (int c = 0; c < a_cols / 32; ++c) {
-          uint32_t v[32];
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            const uint4 u = src[c * 8 + i];
-            v[4 * i] = u.x; v[4 * i + 1] = u.y; v[4 * i + 2] = u.z; v[4 * i + 3] = u.w;
-          }
-          tmem_st32(ta + c * 32, v);
-        }
-        tmem_st_wait();
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&sl->a_full);
-      // ---- thresholds of this thread's query
-      const bool qok = q < p.Q;
-      float thr = -INFINITY, thr_hi = -INFINITY;
-      int tie = 0;
-      if (qok) {
-        thr = p.true_score[q];
-        thr_hi = nextafterf(thr, INFINITY);
-        const int ti = p.true_idx[q];
-        tie = ti < 0 ? 0 : (ti > p.Nc ? p.Nc : ti);
-      }
-      int cnt = 0;
-      const int t0 = chunk * p.chunk_tiles, t1 = min(p.n_tiles, t0 + p.chunk_tiles);
-      const uint32_t taddr0 = acc_base + lane_base + (uint32_t)(mh * WN);
-      for (int t = t0; t < t1; ++t) {
-        mbar_wait(&sl->tmem_full[mh], acc_phase);
-        tc_fence_after();
-        cnt += epi_count128(taddr0, t * WN, thr, thr_hi, tie, p.Nc);
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&sl->tmem_empty[mh]);
-        acc_phase ^= 1;
-      }
-      if (qok && cnt != 0) {
-        atomicAdd(&p.raw_cnt[q], cnt);
-        atomicAdd(&p.filt_cnt[q], cnt);
-      }
-    }
-  }
-  __syncwarp();
   tc_fence_before();
   __syncthreads();
   if (warp == WARP_MMA) tmem_dealloc(tmem_base, 512);
@@ -1452,7 +1010,7 @@ void hole_rank_ws_free(hole_ctx* c) {
   c->rank = nullptr;
 }
 
-// Work items of the 128-query kernel: enough to balance the persistent CTAs, chunks of at least 8 candidate tiles.
+// Work items of hole_rank_kernel: enough to balance the persistent CTAs, chunks of at least 8 candidate tiles.
 static void split_chunks(RankParams& p, int sm_count) {
   const int want_items = 8 * sm_count;
   const int chunks = std::max(1, std::min(p.n_tiles / 8, (want_items + p.m_tiles - 1) / p.m_tiles));
@@ -1500,30 +1058,18 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
   HOLE_CUDA_TRY(cudaSetDevice(c->device));
   cudaStream_t st = (cudaStream_t)stream;
 
-  const char* pe_ = getenv("HOLE_RANK_PAIR");      // experimental cta_group::2 kernel (see DESIGN.md)
-  const bool use_pair = !topk && pe_ != nullptr && pe_[0] == '1';
   const int Nc = (int)(ent_end - ent_begin);
   const int K = (c->dim + BK - 1) / BK * BK;
   const int num_kb = K / BK;
   const int Npad = (Nc + BN - 1) / BN * BN;
-  // experimental wide kernel (256 queries per candidate tile, query operand in TMEM; plain bf16, K <= 256):
-  // bit-identical counts, half the L2->SM traffic, and no faster because the call is power-bound (DESIGN.md section 9)
-  const char* we_ = getenv("HOLE_RANK_WIDE");
-  const bool use_wide = !topk && !use_pair && parts == 1 && K <= 256 && we_ != nullptr && we_[0] == '1';
-  const int qtile = (use_pair || use_wide) ? 2 * BM : BM;
-  const int Qpad = (int)((Q + qtile - 1) / qtile * qtile);
+  const int Qpad = (int)((Q + BM - 1) / BM * BM);
   const int Kall = K * parts;                                  // operand columns in memory
   const int a_bytes = num_kb * parts * A_KB_BYTES;
-  const int b_stage_bytes = use_pair ? B_HALF_BYTES : B_KB_BYTES;
-  int stages = (SMEM_LIMIT - a_bytes - 2048) / b_stage_bytes;
-  stages = std::min(stages, use_pair ? MAX_STAGES : 4);   // a fifth 32 KB stage measured no gain
-  if (const char* se_ = getenv("HOLE_RANK_STAGES")) stages = std::min(stages, std::max(2, atoi(se_)));   // tuning knob
+  const int stages = std::min((SMEM_LIMIT - a_bytes - 2048) / B_KB_BYTES, MAX_STAGES);
   if (stages < 2)
     return hole_set_error(HOLE_ERR_UNSUPPORTED, "embedding_dim %d too large for the ranking kernel's smem budget at precision %d",
                           c->dim, precision);
-  if (use_pair && parts == 2)
-    return hole_set_error(HOLE_ERR_UNSUPPORTED, "the experimental CTA-pair kernel has no split-bf16 mode");
-  const int smem_bytes = a_bytes + stages * b_stage_bytes + 2048;   // + alignment slack + barriers
+  const int smem_bytes = a_bytes + stages * B_KB_BYTES + 2048;   // + alignment slack + barriers
 
   if (c->rank == nullptr) c->rank = new hole_rank_ws();
   hole_rank_ws* w = c->rank;
@@ -1550,7 +1096,7 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
     w->q_cap = (size_t)Qpad * Kall;
   }
   RankParams p{};
-  p.m_tiles = use_pair ? Qpad / (2 * BM) : Qpad / BM;      // diagonal pass and the 128-query kernels
+  p.m_tiles = Qpad / BM;
   if (topk) {
     p.n_tiles = Npad / BN;
     split_chunks(p, c->sm_count);
@@ -1574,8 +1120,6 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
     HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<2, EPI_RANK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<1, EPI_TOPK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<2, EPI_TOPK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-    HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-    HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     w->attr_set = true;
   }
 
@@ -1670,51 +1214,19 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
     hole_rank_gather_true_kernel<<<(unsigned)((Qpad + 31) / 32), 256, 0, st>>>(w->cand, w->true_idx, Nc, Qpad, Kall, w->tq);
     HOLE_LAUNCHED();
     HOLE_CUDA_TRY(cudaMemsetAsync(w->tq + (size_t)Qpad * Kall, 0, (size_t)BN * Kall * 2, st));
-    rc = make_map(&mapB, w->tq, rows, Kall, BN / 2);      // DIAG tiles: 128 true rows per CTA in both kernels
+    rc = make_map(&mapB, w->tq, rows, Kall, BN / 2);      // DIAG tiles: the query tile's own 128 true rows
     if (rc) return rc;
     p.mode = MODE_DIAG;
     p.n_tiles = 1; p.chunk_tiles = 1; p.n_chunks = 1;
     p.true_out = true_score_io;
-    if (use_pair) {
-      const int grid = 2 * std::min(p.m_tiles, c->sm_count / 2);
-      hole_rank_pair_kernel<<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
-    } else {
-      const int grid = std::min(p.m_tiles, c->sm_count);
-      if (parts == 2) hole_rank_kernel<2, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
-      else hole_rank_kernel<1, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
-    }
+    const int grid = std::min(p.m_tiles, c->sm_count);
+    if (parts == 2) hole_rank_kernel<2, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+    else hole_rank_kernel<1, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
     HOLE_LAUNCHED();
   }
 
   if (!count) return HOLE_OK;                      // true scores only (first phase of the sharded ranking)
-  if (use_wide) {
-    rc = make_map(&mapB, w->cand, Npad, Kall, WN);
-    if (rc) return rc;
-    p.mode = MODE_COUNT;
-    p.m_tiles = Qpad / (2 * BM);
-    p.n_tiles = Npad / WN;
-    p.stages = std::min(W_MAX_STAGES, (SMEM_LIMIT - 2048) / W_STAGE_BYTES);
-    {
-      const int want_items = 8 * c->sm_count;
-      const int chunks = std::max(1, std::min(p.n_tiles / 32, (want_items + p.m_tiles - 1) / p.m_tiles));
-      p.chunk_tiles = (p.n_tiles + chunks - 1) / chunks;
-      p.n_chunks = (p.n_tiles + p.chunk_tiles - 1) / p.chunk_tiles;
-    }
-    p.true_score = true_score_io;
-    p.raw_cnt = raw_before;
-    p.filt_cnt = filt_before;
-    p.qp_words = reinterpret_cast<const uint32_t*>(w->qp);
-    p.K = K;
-    const int n_items = p.m_tiles * p.n_chunks;
-    hole_rank_wide_kernel<<<std::min(n_items, c->sm_count), RANK_THREADS, p.stages * W_STAGE_BYTES + 2048, st>>>(mapB, p);
-    HOLE_LAUNCHED();
-    if (filter_off != nullptr) {
-      hole_rank_filter_kernel<<<(unsigned)((Q + 7) / 8), 256, 0, st>>>(w->qp, w->cand, K, parts, filter_off, filter_ids, ent_begin, Nc, true_score_io, w->true_idx, (int)Q, filt_before);
-      HOLE_LAUNCHED();
-    }
-    return HOLE_OK;
-  }
-  rc = make_map(&mapB, w->cand, Npad, Kall, use_pair ? BN / 2 : BN);
+  rc = make_map(&mapB, w->cand, Npad, Kall, BN);
   if (rc) return rc;
   p.mode = MODE_COUNT;
   p.n_tiles = Npad / BN;
@@ -1722,18 +1234,10 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
   p.true_score = true_score_io;
   p.raw_cnt = raw_before;
   p.filt_cnt = filt_before;
-  {
-    const int n_items = p.m_tiles * p.n_chunks;
-    if (use_pair) {
-      const int grid = 2 * std::min(n_items, c->sm_count / 2);
-      hole_rank_pair_kernel<<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
-    } else {
-      const int grid = std::min(n_items, c->sm_count);
-      if (parts == 2) hole_rank_kernel<2, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
-      else hole_rank_kernel<1, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
-    }
-    HOLE_LAUNCHED();
-  }
+  const int grid = std::min(p.m_tiles * p.n_chunks, c->sm_count);
+  if (parts == 2) hole_rank_kernel<2, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+  else hole_rank_kernel<1, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+  HOLE_LAUNCHED();
   if (filter_off != nullptr) {
     hole_rank_filter_kernel<<<(unsigned)((Q + 7) / 8), 256, 0, st>>>(w->qp, w->cand, K, parts, filter_off, filter_ids, ent_begin, Nc, true_score_io, w->true_idx, (int)Q, filt_before);
     HOLE_LAUNCHED();

@@ -1,5 +1,7 @@
-"""Ranking kernel probe: times the count kernel of config 2 (FB15k shape) and a reduced config 3
-under the kernel's tuning switches (HOLE_RANK_PAIR, HOLE_RANK_STAGES)."""
+"""Ranking kernel probe: times the ranking call on config 2 (FB15k shape) and a reduced config 3.
+
+PROBE_ZERO=1 ranks all-zero tables, PROBE_Q3 sets the config 3 query count (default 20000) and PROBE_ENV is a
+label printed on the timing line (tools/rank_ab.sh passes the library's name)."""
 import json
 import os
 import sys
@@ -14,7 +16,6 @@ from graphembeddings_b200.rank_bench import time_rank
 
 
 def main():
-    out = {}
     kg2 = D.make_config("rank_fb15k_d150", trained_scale=True)
     e2 = HoleEngine(kg2.n_rows, kg2.dim).set_embeddings(kg2.E)
     kg3 = D.make_config("diffbot_d256", n_triples=100000)
@@ -24,21 +25,13 @@ def main():
         e3.set_embeddings(np.zeros_like(kg3.E))
     rng = np.random.default_rng(1)
     q3 = kg3.triples[rng.integers(0, len(kg3.triples), size=int(os.environ.get("PROBE_Q3", "20000")))]
-    variants = [("0", "4"), ("0", "5"), ("1", "8")]          # (pair kernel?, ring depth cap)
-    if os.environ.get("PROBE_ONLY"):      # e.g. "0:5,1:8"
-        variants = [tuple(v.split(":")) for v in os.environ["PROBE_ONLY"].split(",")]
     extra = os.environ.get("PROBE_ENV", "")
-    for pair, dbg in variants:
-        os.environ["HOLE_RANK_PAIR"] = pair
-        os.environ["HOLE_RANK_STAGES"] = dbg
-        ms2, _, _ = time_rank(e2, kg2.triples, kg2.n_relations, kg2.n_rows, sides=(HOLE_SIDE_BOTH,))
-        ms3, _, _ = time_rank(e3, q3, kg3.n_relations, kg3.n_rows, sides=(HOLE_SIDE_TAIL,), reps=2)
-        tf2 = 2 * len(kg2.triples) * kg2.n_entities * 2 * kg2.dim / ms2 / 1e9
-        tf3 = len(q3) * kg3.n_entities * 2 * kg3.dim / ms3 / 1e9
-        out[f"pair{pair}_stages{dbg}"] = {"cfg2_ms": ms2, "cfg2_tflops": tf2, "cfg3_ms": ms3, "cfg3_tflops": tf3}
-        print(f"pair={pair} stages<={dbg} {extra}: cfg2 {ms2:.3f} ms {tf2:.0f} TF/s | cfg3 {ms3:.3f} ms {tf3:.0f} TF/s",
-              flush=True)
-    print(json.dumps(out))
+    ms2, _, _ = time_rank(e2, kg2.triples, kg2.n_relations, kg2.n_rows, sides=(HOLE_SIDE_BOTH,))
+    ms3, _, _ = time_rank(e3, q3, kg3.n_relations, kg3.n_rows, sides=(HOLE_SIDE_TAIL,), reps=2)
+    tf2 = 2 * len(kg2.triples) * kg2.n_entities * 2 * kg2.dim / ms2 / 1e9
+    tf3 = len(q3) * kg3.n_entities * 2 * kg3.dim / ms3 / 1e9
+    print(f"rank {extra}: cfg2 {ms2:.3f} ms {tf2:.0f} TF/s | cfg3 {ms3:.3f} ms {tf3:.0f} TF/s", flush=True)
+    print(json.dumps({"cfg2_ms": ms2, "cfg2_tflops": tf2, "cfg3_ms": ms3, "cfg3_tflops": tf3}))
 
 
 if __name__ == "__main__":
