@@ -2330,7 +2330,7 @@ static int run_step(hole_ctx* c, hole_plan& pl, float* table, const int32_t* pos
     int rc = k1_launch(c, dm, ka, shard ? *shard : no_shard, st, k1_follows_k3 && !c->profile);
     if (rc) return rc;
   } else {
-    if (c->k1_smem > 227 * 1024)
+    if (c->k1_smem > 227 * 1024)   // (hole_train_step_logloss refuses this at its entry; kept as a guard)
       return hole_set_error(HOLE_ERR_UNSUPPORTED, "embedding_dim %d: the --log_loss kernel needs %d bytes of shared memory",
                             c->dim, c->k1_smem);
     HOLE_DISPATCH_SMEM(c, hole_train_fwd_bwd_ll_kernel, grid_for_groups((B + pl.T - 1) / pl.T, c->gs), 256,
@@ -2453,6 +2453,10 @@ extern "C" int hole_train_step_logloss(hole_ctx* c, float* table, float* delta_w
   HOLE_CHECK_ARG(c && B >= 0 && negative_ratio >= 1 && negative_ratio <= 64);
   if (c->score_mode != HOLE_SCORE_COMPLEX)
     return hole_set_error(HOLE_ERR_UNSUPPORTED, "the archived ccorr/tanh score mode has no log-loss branch");
+  // Refuse before the workspace and the plan: a refused call launches nothing and leaves plan slot 0 as it was.
+  if (c->k1_smem > 227 * 1024)
+    return hole_set_error(HOLE_ERR_UNSUPPORTED, "embedding_dim %d: the --log_loss kernel needs %d bytes of shared memory",
+                          c->dim, c->k1_smem);
   if (B == 0) return HOLE_OK;
   HOLE_CHECK_ARG(table && delta_ws && triples && type_of && csr_off && csr_ids && loss_out);
   HOLE_CHECK_ARG(4 * B < (int64_t(1) << 31));

@@ -25,7 +25,7 @@ def _triples(rng, n_rel, n, B):
                     axis=1).astype(np.int32)
 
 
-@pytest.mark.parametrize("dim", [8, 64, 150, 256, 384])
+@pytest.mark.parametrize("dim", [8, 64, 150, 256, 384, 66, 128, 290, 450, 514, 768])   # NV 1, 2, 3, 4, 6, 8, 12
 def test_ccorr_score_matches_oracle(eng_mod, dim):
     from oracle import hole_ccorr as oc
     n, B = 300, 257
@@ -40,7 +40,8 @@ def test_ccorr_score_matches_oracle(eng_mod, dim):
 
 
 @pytest.mark.parametrize("dim,side,margin", [(8, 0, 1.0), (8, 1, 0.2), (150, 0, 1.0), (150, 1, 1.0), (256, 0, 0.2),
-                                             (256, 1, 1.0), (384, 1, 1.0)])
+                                             (256, 1, 1.0), (384, 1, 1.0), (66, 0, 1.0), (290, 1, 1.0),
+                                             (450, 0, 0.2), (768, 1, 1.0)])
 def test_ccorr_train_steps_match_oracle(eng_mod, dim, side, margin):
     """Chained steps with duplicate rows (few entities, fewer relations), clipped and unclipped rows."""
     from oracle import hole_ccorr as oc
@@ -91,7 +92,7 @@ def test_ccorr_train_steps_device_loop_matches_single_steps(eng_mod):
     a.close(); b.close()
 
 
-@pytest.mark.parametrize("dim", [64, 150, 256])
+@pytest.mark.parametrize("dim", [64, 150, 256, 290, 320])
 @pytest.mark.parametrize("side", [0, 1])
 def test_ccorr_ranking_matches_fp64_oracle(eng_mod, dim, side):
     """All-candidate ranking in the archived mode (the score is linear in the candidate entity, so the same

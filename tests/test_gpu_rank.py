@@ -60,7 +60,7 @@ def _exact_from_operands(e, kg, queries, side, ent_begin, ent_end, raw, filt, ts
     return S, thr
 
 
-@pytest.mark.parametrize("dim", [64, 150, 256, 512])
+@pytest.mark.parametrize("dim", [64, 150, 256, 512, 2, 514, 640])     # 514, 640: 2-stage ring, 3 query-packer iterations
 @pytest.mark.parametrize("side", [0, 1])
 def test_rank_counts_exact_vs_own_operands(eng_mod, dim, side):
     kg, e = _setup(eng_mod, 11, 3000, 700, dim, seed=dim + side)
@@ -261,7 +261,7 @@ def test_full_size_config3_sample_against_fp64_contraction(eng_mod):
     assert torch.equal(raw2, raw)
 
 
-@pytest.mark.parametrize("dim", [64, 150, 256])
+@pytest.mark.parametrize("dim", [64, 150, 256, 258, 320])     # 258, 320: the 2-stage ring at bf16x3
 @pytest.mark.parametrize("side", [0, 1])
 def test_split_bf16_precision_matches_fp64_oracle(eng_mod, dim, side):
     """HOLE_RANK_BF16X3 (hi.hi + lo.hi + hi.lo on the tensor cores): ranks agree with the fp64

@@ -106,11 +106,15 @@ def test_selection_exact_vs_own_operands(eng_mod, side):
         assert np.isin(want_ids[q][want_s[q] < kth - 2e-6], g).all()
 
 
-@pytest.mark.parametrize("dim", [64, 150, 256])
+@pytest.mark.parametrize("dim,bf16", [pytest.param(d, False, id=str(d)) for d in (64, 150, 256, 2, 320)] +
+                         [pytest.param(640, True, id="640-bf16")])
 @pytest.mark.parametrize("side", [0, 1, 2])
-def test_topk_matches_fp64_oracle(eng_mod, dim, side):
+def test_topk_matches_fp64_oracle(eng_mod, dim, bf16, side):
     """Split-bf16: Q = 300 (not a multiple of 128) over [b + 7, en - 100) (not a multiple of 256), filtered,
-    k = 1, 10, 128; and Q = 1."""
+    k = 1, 10, 128; and Q = 1.  Dims 2 and 320 are the smallest and the largest bf16x3 builds; 640, the largest
+    plain bf16 build (3 query-packer iterations, 2-stage ring), runs in bf16: there the id set is exact outside
+    the bf16 score bound 4e-3 |q| |e| of the k-th score (|e| <= 1 after the clip), and the returned scores, which
+    the merge kernel recomputes in fp32, keep the fp32 tolerance."""
     kg, e = _setup(eng_mod, 9, 2600, 300, dim, seed=80 + dim + side)
     b, en = kg.n_relations + 7, kg.n_rows - 100
     assert (en - b) % 256 != 0
@@ -118,13 +122,19 @@ def test_topk_matches_fp64_oracle(eng_mod, dim, side):
     E64 = kg.E.astype(np.float64)
     S = _oracle_scores(E64, kg.triples, side, cand)
     foff, fids = _filters(kg, kg.triples, side, 94)
+    precision = eng_mod.HOLE_RANK_BF16 if bf16 else eng_mod.HOLE_RANK_BF16X3
+    band = BAND_X3
+    if bf16:
+        sides = ("tail", "head") if side == 2 else (("tail",) if side == 0 else ("head",))
+        qn = max(np.linalg.norm(O.query_vectors(E64, kg.triples, s, np.float64), axis=1).max() for s in sides)
+        band = 4e-3 * qn
     for k in (1, 10, 128):
-        ids, sc = e.topk(kg.triples, side, b, en, k, foff, fids)
+        ids, sc = e.topk(kg.triples, side, b, en, k, foff, fids, precision=precision)
         assert ids.shape == (S.shape[0], k)
-        _check_rows(ids.cpu().numpy(), sc.cpu().numpy(), S, cand, k, _filter_lists(foff, fids), BAND_X3)
-    ids, sc = e.topk(kg.triples[:1], side, b, en, 10)
+        _check_rows(ids.cpu().numpy(), sc.cpu().numpy(), S, cand, k, _filter_lists(foff, fids), band)
+    ids, sc = e.topk(kg.triples[:1], side, b, en, 10, precision=precision)
     S1 = _oracle_scores(E64, kg.triples[:1], side, cand)
-    _check_rows(ids.cpu().numpy(), sc.cpu().numpy(), S1, cand, 10, None, BAND_X3)
+    _check_rows(ids.cpu().numpy(), sc.cpu().numpy(), S1, cand, 10, None, band)
 
 
 def test_k_larger_than_the_candidates_pads(eng_mod):

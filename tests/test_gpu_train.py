@@ -37,7 +37,9 @@ def _engine(eng_mod, kg):
     return e, off, ids
 
 
-DIMS = [20, 64, 128, 150, 256, 512, 600]
+# 20 .. 600: round dims; 2, 66, 130, 258, 768: the first or last dim of a K1 lane-group regime
+# (tests/test_gpu_shapes.py lane_group)
+DIMS = [20, 64, 128, 150, 256, 512, 600, 2, 66, 130, 258, 768]
 
 
 @pytest.mark.parametrize("dim", DIMS)
@@ -293,7 +295,8 @@ def test_sharded_trainer_single_rank_matches_engine(eng_mod):
     assert np.abs(want - kg.E).max() > 1e-4
 
 
-@pytest.mark.parametrize("dim,k,l2", [(150, 1, 0.0), (256, 3, 0.0), (64, 2, 1e-5), (600, 2, 0.0)])
+@pytest.mark.parametrize("dim,k,l2", [(150, 1, 0.0), (256, 3, 0.0), (64, 2, 1e-5), (600, 2, 0.0), (720, 2, 0.0),
+                                      (66, 1, 1e-5)])
 def test_logloss_step_matches_oracle(eng_mod, dim, k, l2):
     """--log_loss branch (holE.py:194-196, 206-220): k corrupt batches drawn with virtual steps
     step*k + j (bit-exact vs the oracle's Philox), softplus rows, sparse gradients taken at the
@@ -356,14 +359,17 @@ def test_logloss_training_reduces_the_loss(eng_mod):
     assert abs(got - pos_loss(E)) < 1e-4
 
 
-@pytest.mark.parametrize("world", [1, 2, 3])
-def test_shard_route_and_post_virtual_ranks(eng_mod, world):
+@pytest.mark.parametrize("world,n_ent", [pytest.param(1, 1000, id="1"), pytest.param(2, 1000, id="2"),
+                                         pytest.param(3, 1000, id="3"), pytest.param(2, 3 << 24, id="2-4pass")])
+def test_shard_route_and_post_virtual_ranks(eng_mod, world, n_ent):
     """Request routing of the sharded step with `world` virtual ranks on one GPU (peer buffers are
-    local tensors): route == np.unique / searchsorted, post delivers every owner's slice."""
+    local tensors): route == np.unique / searchsorted, post delivers every owner's slice.  n_ent = 3 * 2^24:
+    ids above 2^24 (the largest one included), so the routing sort takes 4 byte passes; routing reads ids
+    only, so the engine's own table stays small."""
     from graphembeddings_b200.sharded import row_partition
     rng = np.random.default_rng(100 + world)
-    dim, R, n_ent, B = 150, 5, 1000, 257
-    e = eng_mod.HoleEngine(R + n_ent, dim)
+    dim, R, B = 150, 5, 257
+    e = eng_mod.HoleEngine(R + 1000, dim)
     cap = 3 * B
     rows_per = row_partition(n_ent, world)
     dev = e.device
@@ -374,6 +380,7 @@ def test_shard_route_and_post_virtual_ranks(eng_mod, world):
         pos = np.stack([R + rng.integers(0, n_ent, B), R + rng.integers(0, n_ent, B), rng.integers(0, R, B)], 1)
         pos[:5, 1] = pos[:5, 0]                                  # head == tail rows
         neg = R + rng.integers(0, n_ent, B)
+        neg[7] = R + n_ent - 1
         pos_t = torch.from_numpy(pos.astype(np.int32)).to(dev)
         neg_t = torch.from_numpy(neg.astype(np.int32)).to(dev)
         uniq = torch.full((cap,), -1, dtype=torch.int32, device=dev)
