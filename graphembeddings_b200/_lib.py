@@ -8,9 +8,9 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("HOLE_B200_LIB", os.path.join(_HERE, "libhole_b200.so"))   # override: A/B experiments
 
-HOLE_SIDE_TAIL, HOLE_SIDE_HEAD, HOLE_SIDE_BOTH = 0, 1, 2
+HOLE_SIDE_TAIL, HOLE_SIDE_HEAD, HOLE_SIDE_BOTH, HOLE_SIDE_RELATION = 0, 1, 2, 3
 HOLE_RANK_BF16, HOLE_RANK_BF16X3 = 0, 1
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 
 class HoleError(RuntimeError):

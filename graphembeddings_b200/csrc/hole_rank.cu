@@ -606,7 +606,9 @@ hole_rank_pack_cand_kernel(const float* __restrict__ table, int stride, int H, i
 }
 
 // Query operand (App. A.4): tail side q = h * r; head side q = r * conj(t) with the imaginary
-// half negated.  Also records the shard-local index of the true candidate.
+// half negated; relation side q = h * conj(t) with the imaginary half negated (the head side's product
+// with h as the first factor: s is linear in the relation row, App. A.3's ds/dy_r).  Also records the
+// shard-local index of the true candidate (t, h or r).
 // One warp per query; a lane holds groups of four complex components of both factor rows
 // (float4 loads of the [Re | pad | Im | pad] row layout) in registers between the norm pass and
 // the product pass.  PQ_ITERS = ceil(Hp / 128), at most 3 for the dimensions the ranking kernel's smem admits.
@@ -640,7 +642,7 @@ hole_rank_pack_query_kernel(const float* __restrict__ table, int stride, int H,
   }
   const int h = queries[3 * src], t = queries[3 * src + 1], r = queries[3 * src + 2];
   const int Hp = stride / 2, G4 = Hp / 4;
-  const float4* x1 = reinterpret_cast<const float4*>(table + (size_t)(side == HOLE_SIDE_TAIL ? h : r) * stride);
+  const float4* x1 = reinterpret_cast<const float4*>(table + (size_t)(side == HOLE_SIDE_HEAD ? r : h) * stride);
   const float4* x2 = reinterpret_cast<const float4*>(table + (size_t)(side == HOLE_SIDE_TAIL ? r : t) * stride);
   float4 A[PQ_ITERS], Bv[PQ_ITERS], C[PQ_ITERS], Dv[PQ_ITERS];   // (A,Bv) = first factor re/im, (C,Dv) = second
   float s1 = 0.f, s2 = 0.f;
@@ -675,7 +677,8 @@ hole_rank_pack_query_kernel(const float* __restrict__ table, int stride, int H,
       float re[4], im[4];
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
-        // tail: (a,b)=h (c,d)=r, q = h*r;  head: (a,b)=r (c,d)=t with b negated: q = (ac+bd, ad-bc)
+        // tail: (a,b)=h (c,d)=r, q = h*r;  head: (a,b)=r (c,d)=t with b negated: q = (ac+bd, ad-bc);
+        // relation: (a,b)=h (c,d)=t with b negated, the same product
         re[i] = a[i] * c[i] - b[i] * d[i];
         im[i] = a[i] * d[i] + b[i] * c[i];
       }
@@ -712,13 +715,15 @@ hole_rank_pack_query_kernel(const float* __restrict__ table, int stride, int H,
   __syncwarp();
 #pragma unroll 1
   for (int k = lane; k < row_vecs; k += 32) o4[k] = row4[k];
-  if (lane == 0) true_idx[qi] = (int32_t)((int64_t)(side == HOLE_SIDE_TAIL ? t : h) - ent_begin);
+  if (lane == 0)
+    true_idx[qi] = (int32_t)((int64_t)(side == HOLE_SIDE_TAIL ? t : (side == HOLE_SIDE_HEAD ? h : r)) - ent_begin);
 }
 
 // Query operand of the ARCHIVED score variant (hole_ccorr.cuh): s = Re sum_k rho_k c_k with rho = (1 - i) r is
 // linear in the candidate entity, so the all-candidate form is the same dense contraction with another
 // query vector:   tail side  s(h, r, .) = [Re t ; Im t] . [Re w ; -Im w],  w_m = sum_k rho_k conj(h_{m-k})
 //                 head side  s(., r, t) = [Re h ; Im h] . [Re u ;  Im u],  u_j = sum_k rho_k t_{j+k}
+//                 relation   s(h, ., t) = [Re r ; Im r] . [Re c + Im c ; Re c - Im c],  c_k = sum_j conj(h_j) t_{j+k}
 // One warp per query, one direct O(H^2) correlation out of shared memory.  tanh is monotone: ranking on s.
 template <int NV>
 __global__ void __launch_bounds__(256)
@@ -726,7 +731,7 @@ hole_rank_pack_query_ccorr_kernel(const float* __restrict__ table, int stride, i
                                   const int32_t* __restrict__ queries, int Q, int Qpad, int side,
                                   int64_t ent_begin, int K, int parts, __nv_bfloat16* __restrict__ out,
                                   int32_t* __restrict__ true_idx, float* __restrict__ qf) {
-  extern __shared__ float pqc_smem[];                   // per warp: entity row doubled (4H), rho (2H)
+  extern __shared__ float pqc_smem[];                   // per warp: entity row doubled (4H), rho or h (2H)
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   const int64_t qi = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
   if (qi >= Qpad) return;
@@ -746,13 +751,19 @@ hole_rank_pack_query_ccorr_kernel(const float* __restrict__ table, int stride, i
   const int Hp = stride / 2;
   float* sm = pqc_smem + (size_t)wib * (6 * H);
   float *e_re = sm, *e_im = sm + 2 * H, *rho_re = sm + 4 * H, *rho_im = sm + 5 * H;
+  const bool rel = side == HOLE_SIDE_RELATION;
   CVec<NV> yr;
-  // the relation row lands in the entity buffers first (overwritten below); rho = (1 - i) r
-  cc_load_row<NV>(table + (size_t)r * stride, H, Hp, lane, e_re, e_im, &yr);
+  // The fixed operand's row lands in the entity buffers first (overwritten below) and is kept in registers:
+  // cc_load_row writes a doubled row, which does not fit the 2H floats of the rho slot.
+  // rho = (1 - i) r, or for the relation side h itself.
+  cc_load_row<NV>(table + (size_t)(rel ? h : r) * stride, H, Hp, lane, e_re, e_im, &yr);
 #pragma unroll
   for (int v = 0; v < NV; ++v) {
     const int k = lane + 32 * v;
-    if (k < H) { rho_re[k] = yr.re[v] + yr.im[v]; rho_im[k] = yr.im[v] - yr.re[v]; }
+    if (k < H) {
+      rho_re[k] = rel ? yr.re[v] : yr.re[v] + yr.im[v];
+      rho_im[k] = rel ? yr.im[v] : yr.im[v] - yr.re[v];
+    }
   }
   __syncwarp();
   cc_load_row<NV>(table + (size_t)(side == HOLE_SIDE_TAIL ? h : t) * stride, H, Hp, lane, e_re, e_im, nullptr);
@@ -762,6 +773,14 @@ hole_rank_pack_query_ccorr_kernel(const float* __restrict__ table, int stride, i
     cc_corr<NV, false, true, false>(qv, rho_re, rho_im, e_re, e_im, H, lane);       // w; q = [Re w ; -Im w]
 #pragma unroll
     for (int v = 0; v < NV; ++v) qv.im[v] = -qv.im[v];
+  } else if (rel) {
+    cc_corr<NV, true, false, true>(qv, rho_re, rho_im, e_re, e_im, H, lane);        // c; q = [Re c + Im c ; Re c - Im c]
+#pragma unroll
+    for (int v = 0; v < NV; ++v) {
+      const float cr = qv.re[v], ci = qv.im[v];
+      qv.re[v] = cr + ci;
+      qv.im[v] = cr - ci;
+    }
   } else {
     cc_corr<NV, false, false, true>(qv, rho_re, rho_im, e_re, e_im, H, lane);       // u; q = [Re u ; Im u]
   }
@@ -783,7 +802,7 @@ hole_rank_pack_query_ccorr_kernel(const float* __restrict__ table, int stride, i
       }
     }
   }
-  if (lane == 0) true_idx[qi] = (int32_t)((int64_t)(side == HOLE_SIDE_TAIL ? t : h) - ent_begin);
+  if (lane == 0) true_idx[qi] = (int32_t)((int64_t)(side == HOLE_SIDE_TAIL ? t : (rel ? r : h)) - ent_begin);
 }
 
 // T[q] = packed candidate row of q's true candidate (zeros when it is not in this shard).
@@ -822,7 +841,9 @@ hole_rank_filter_kernel(const __nv_bfloat16* __restrict__ qp, const __nv_bfloat1
   int hits = 0;
   for (int64_t p = foff[qi]; p < foff[qi + 1]; ++p) {
     const int64_t j = (int64_t)fids[p] - ent_begin;
-    if (j < 0 || j >= Nc) continue;            // warp-uniform
+    // warp-uniform.  The true candidate never ranks before itself; its CUDA-core score may differ from the
+    // tensor-core threshold in the last bits, so it is skipped rather than compared.
+    if (j < 0 || j >= Nc || j == ti) continue;
     const __nv_bfloat16* crow = cand + (size_t)j * K * parts;
     float s = 0.f;
     for (int k = lane; k < K; k += 32) {
@@ -1032,7 +1053,8 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
                      int compute_true, int32_t* raw_before, int32_t* filt_before, void* stream,
                      bool prepare_only, const TopkArgs* tk = nullptr) {
   HOLE_CHECK_ARG(c && Q >= 0 && ent_begin >= 0 && ent_end >= ent_begin && ent_end <= c->n_rows);
-  HOLE_CHECK_ARG(side == HOLE_SIDE_TAIL || side == HOLE_SIDE_HEAD || side == HOLE_SIDE_BOTH);
+  HOLE_CHECK_ARG(side == HOLE_SIDE_TAIL || side == HOLE_SIDE_HEAD || side == HOLE_SIDE_BOTH ||
+                 side == HOLE_SIDE_RELATION);
   const bool topk = tk != nullptr;
   if (topk && Q > 0 && ent_end == ent_begin) {       // no candidates: every output row is padding
     HOLE_CHECK_ARG(queries != nullptr);

@@ -160,21 +160,20 @@ def build_filter_csr(queries, known_triples, side):
     """Per-query list of known-true candidates to filter (holE.py:413-422, 454-461).
 
     side "tail": for query (h, t, r) the known tails of (h, r); side "head": the known
-    heads of (t, r).  ``known_triples`` = train + valid triples [K, 3].  Returns
-    (off int64[Q+1], ids int32[.]) with ids ascending and de-duplicated per query."""
+    heads of (t, r); side "relation": the known relations of (h, t).  ``known_triples`` = train +
+    valid triples [K, 3].  Returns (off int64[Q+1], ids int32[.]) with ids ascending and
+    de-duplicated per query."""
     queries = np.asarray(queries, dtype=np.int64)
     known = np.asarray(known_triples, dtype=np.int64).reshape(-1, 3)
-    if side == "tail":
-        kq, kv = known[:, 0], known[:, 1]
-        qq = queries[:, 0]
-    elif side == "head":
-        kq, kv = known[:, 1], known[:, 0]
-        qq = queries[:, 1]
-    else:
+    # (first key column, second key column, value column)
+    cols = {"tail": (0, 2, 1), "head": (1, 2, 0), "relation": (0, 1, 2)}.get(side)
+    if cols is None:
         raise ValueError(side)
+    a, b, v = cols
+    kv = known[:, v]
     big = np.int64(1) << 32
-    kkey = kq * big + known[:, 2]
-    qkey = qq * big + queries[:, 2]
+    kkey = known[:, a] * big + known[:, b]
+    qkey = queries[:, a] * big + queries[:, b]
     order = np.lexsort((kv, kkey))
     kkey, kv = kkey[order], kv[order]
     if len(kkey):                                   # drop repeated (key, value) pairs once, globally

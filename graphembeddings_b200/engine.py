@@ -11,11 +11,11 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (HOLE_RANK_BF16, HOLE_RANK_BF16X3, HOLE_SIDE_BOTH, HOLE_SIDE_HEAD, HOLE_SIDE_TAIL,
-                   HoleError, check)
+from ._lib import (HOLE_RANK_BF16, HOLE_RANK_BF16X3, HOLE_SIDE_BOTH, HOLE_SIDE_HEAD, HOLE_SIDE_RELATION,
+                   HOLE_SIDE_TAIL, HoleError, check)
 
 __all__ = ["HoleEngine", "HoleError", "inverse_time_decay", "HOLE_SIDE_TAIL", "HOLE_SIDE_HEAD", "HOLE_SIDE_BOTH",
-           "HOLE_RANK_BF16", "HOLE_RANK_BF16X3"]
+           "HOLE_SIDE_RELATION", "HOLE_RANK_BF16", "HOLE_RANK_BF16X3"]
 
 
 def inverse_time_decay(lr0, step, decay_steps, decay_rate):
@@ -325,7 +325,9 @@ class HoleEngine:
         """All-candidate ranking of queries [Q,3] over candidate rows [ent_begin, ent_end)
         (eval_link_prediction holE.py:427-469 as a tensor-core contraction).  Returns
         (raw_before int32[Q], filt_before int32[Q], true_score float32[Q]); rank = 1 + count.
-        Counts are accumulated into raw_before / filt_before when given (candidate shards)."""
+        Counts are accumulated into raw_before / filt_before when given (candidate shards).
+        HOLE_SIDE_RELATION ranks each query's relation (column 2) over relation rows [ent_begin, ent_end),
+        normally [0, n_relations)."""
         q = self._triples(queries)
         Q = q.shape[0]
         nq = Q
@@ -338,7 +340,7 @@ class HoleEngine:
         if true_score is None:
             true_score = torch.zeros(Q, dtype=torch.float32, device=self.device)
         fo = fi = None
-        if filter_off is not None:
+        if filter_off is not None and len(filter_ids) > 0:      # no ids: nothing to filter (and no device pointer)
             fo = torch.as_tensor(filter_off).to(torch.int64).to(self.device).contiguous()
             fi = torch.as_tensor(filter_ids).to(torch.int32).to(self.device).contiguous()
         check(self.lib.hole_rank(self._ctx, _ptr(self.table), int(ent_begin), int(ent_end), _ptr(q),
@@ -352,7 +354,8 @@ class HoleEngine:
         """Top-k link prediction (the pop loop of eval_link_prediction, holE.py:427-472, over all candidates
         [ent_begin, ent_end)): for every query row the k candidates first in ascending (score, id) order,
         skipping its filter slice.  Returns (ids int32[Q', k], scores float32[Q', k]) on the device, Q' = Q or
-        2Q for HOLE_SIDE_BOTH; padding is id -1 / score +inf.  Each filter slice must be ascending."""
+        2Q for HOLE_SIDE_BOTH; padding is id -1 / score +inf.  Each filter slice must be ascending.
+        HOLE_SIDE_RELATION predicts the relations of (h, ?, t) over relation rows [ent_begin, ent_end)."""
         q = self._triples(queries)
         rows = q.shape[0] * (2 if int(side) == HOLE_SIDE_BOTH else 1)
         fo = fi = None
@@ -366,8 +369,9 @@ class HoleEngine:
             desc[starts[(starts > 0) & (starts < len(ids))] - 1] = False
             if desc.any():
                 raise HoleError("filter ids must be ascending within each query's slice")
-            fo = torch.as_tensor(off).to(self.device).contiguous()
-            fi = torch.as_tensor(ids.astype(np.int32)).to(self.device).contiguous()
+            if len(ids) > 0:                           # no ids: nothing to filter (and no device pointer)
+                fo = torch.as_tensor(off).to(self.device).contiguous()
+                fi = torch.as_tensor(ids.astype(np.int32)).to(self.device).contiguous()
         ids_out = torch.empty((rows, int(k)), dtype=torch.int32, device=self.device)
         scores = torch.empty((rows, int(k)), dtype=torch.float32, device=self.device)
         check(self.lib.hole_topk(self._ctx, _ptr(self.table), int(ent_begin), int(ent_end), _ptr(q), q.shape[0],

@@ -27,8 +27,15 @@ import torch
 from . import data as D
 from . import tf_bundle
 from . import tf_events
-from .engine import (HOLE_RANK_BF16, HOLE_RANK_BF16X3, HOLE_SIDE_HEAD, HOLE_SIDE_TAIL, HoleEngine,
-                     inverse_time_decay)
+from .engine import (HOLE_RANK_BF16, HOLE_RANK_BF16X3, HOLE_SIDE_HEAD, HOLE_SIDE_RELATION, HOLE_SIDE_TAIL,
+                     HoleEngine, inverse_time_decay)
+
+_SIDES = {"tail": HOLE_SIDE_TAIL, "head": HOLE_SIDE_HEAD, "relation": HOLE_SIDE_RELATION}
+
+
+def _candidate_range(side_name, relation_count, entity_count):
+    """Rows a side ranks: the entity rows for "tail" / "head", the relation rows for "relation"."""
+    return (0, relation_count) if side_name == "relation" else (relation_count, entity_count)
 
 FLAGS = None
 
@@ -370,6 +377,8 @@ def eval_link_prediction(eng, queries, known, relation_count, entity_count, side
     it (it cannot fire for the live model, SURVEY.md section 0).
     precision: split-bf16 by default (ranks match the fp32 reference except within ~3e-5 of a
     tie); HOLE_RANK_BF16 is 3x cheaper and what bench.py times.
+    Side "relation" ranks each triple's relation against all relation rows [0, relation_count),
+    filtered by the known relations of its (head, tail).
     Returns (raw_positions, filtered_positions) lists."""
     queries = np.unique(np.asarray(queries, dtype=np.int32).reshape(-1, 3), axis=0)   # test sets dedupe
     raw_positions, filtered_positions = [], []
@@ -377,14 +386,14 @@ def eval_link_prediction(eng, queries, known, relation_count, entity_count, side
     if len(queries) == 0:
         return raw_positions, filtered_positions
     for side_name in sides:
-        side = HOLE_SIDE_TAIL if side_name == "tail" else HOLE_SIDE_HEAD
+        side = _SIDES[side_name]
+        lo, hi = _candidate_range(side_name, relation_count, entity_count)
         foff, fids = D.build_filter_csr(queries, known, side_name)
-        raw, filt, ts = eng.rank(queries, side, relation_count, entity_count, foff, fids, precision=precision)
+        raw, filt, ts = eng.rank(queries, side, lo, hi, foff, fids, precision=precision)
         ok = np.ones(len(queries), bool)
         if threshold is not None:
             gate = torch.full((len(queries),), _logit(threshold), dtype=torch.float32, device=eng.device)
-            below, _, _ = eng.rank(queries, side, relation_count, entity_count, true_score=gate,
-                                   compute_true=False, precision=precision)
+            below, _, _ = eng.rank(queries, side, lo, hi, true_score=gate, compute_true=False, precision=precision)
             ok = below.cpu().numpy() > 0
         raw, filt, ts = raw.cpu().numpy(), filt.cpu().numpy(), ts.cpu().numpy()
         sig = 1.0 / (1.0 + np.exp(-ts.astype(np.float64)))
@@ -459,35 +468,44 @@ def eval_link_prediction_typed(eng, heads, candidate, true_triples, test_triples
 
 
 def predict_top_k(eng, test, known, relation_count, entity_count, k, path, precision=HOLE_RANK_BF16X3,
-                  value=None):
+                  value=None, sides=("tail", "head")):
     """The all-entity generalisation of the reference's `max_triples` cut of the pop loop (holE.py:427-472):
     the k best NEW tails of every distinct (head, relation) pair of the test file and the k best new heads of
-    every distinct (tail, relation) pair, filtered against the train + valid triples.  Writes one line per
+    every distinct (tail, relation) pair, filtered against the train + valid triples; with "relation" in
+    `sides`, also the k best new relations of every distinct (head, tail) pair.  Writes one line per
     prediction to `path`:  side  head  tail  relation  position  score  value  in_test
     (position 1-based, score = raw s, value = value(s) (sigma by default), in_test = the predicted triple is
     a test triple: the reference's MATCH vs GUESS).  Returns the number of lines written."""
     value = value or (lambda s: 1.0 / (1.0 + np.exp(-s)))
     test = np.asarray(test, dtype=np.int64).reshape(-1, 3)
     test_set = set(map(tuple, test.tolist()))
+    key_cols = {"tail": (0, 2), "head": (1, 2), "relation": (0, 1)}       # the query's known columns
     n = 0
     with open(path, 'w') as out:
-        for side_name, side, key_col in (("tail", HOLE_SIDE_TAIL, 0), ("head", HOLE_SIDE_HEAD, 1)):
-            pairs = np.unique(test[:, [key_col, 2]], axis=0)
+        for side_name in sides:
+            side, cols = _SIDES[side_name], list(key_cols[side_name])
+            pairs = np.unique(test[:, cols], axis=0)
             if len(pairs) == 0:
                 continue
             queries = np.zeros((len(pairs), 3), dtype=np.int32)     # the predicted column is ignored
-            queries[:, key_col] = pairs[:, 0]
-            queries[:, 2] = pairs[:, 1]
+            queries[:, cols] = pairs
             foff, fids = D.build_filter_csr(queries, known, side_name)
-            ids, scores = eng.topk(queries, side, relation_count, entity_count, k, foff, fids, precision=precision)
+            lo, hi = _candidate_range(side_name, relation_count, entity_count)
+            ids, scores = eng.topk(queries, side, lo, hi, k, foff, fids, precision=precision)
             ids, scores = ids.cpu().numpy(), scores.cpu().numpy().astype(np.float64)
             vals = value(scores)
-            for i, (a, r) in enumerate(pairs.tolist()):
+            for i, q in enumerate(queries.tolist()):
                 for pos in range(k):
                     c = int(ids[i, pos])
                     if c < 0:
                         break
-                    h, t = (a, c) if side == HOLE_SIDE_TAIL else (c, a)
+                    h, t, r = q
+                    if side == HOLE_SIDE_TAIL:
+                        t = c
+                    elif side == HOLE_SIDE_HEAD:
+                        h = c
+                    else:
+                        r = c
                     out.write('{}\t{}\t{}\t{}\t{}\t{:.9g}\t{:.6f}\t{}\n'.format(
                         side_name, h, t, r, pos + 1, scores[i, pos], vals[i, pos], (h, t, r) in test_set))
                     n += 1
@@ -512,17 +530,30 @@ def infer_triples(flags=None, log=print):
     raw, filt = eval_link_prediction(eng, data.test, data.known, data.relation_count, data.entity_count,
                                      threshold=threshold, results_path='inference_results.tsv',
                                      precision=precision)
+    relations = getattr(flags, 'relation_prediction', False)
     k = getattr(flags, 'predict_top_k', 0)
     if k:
         value = np.tanh if getattr(flags, 'score_variant', 'complex') != 'complex' else None
         path = os.path.join(flags.output_dir, 'predictions.tsv')
+        sides = ("tail", "head", "relation") if relations else ("tail", "head")
         n = predict_top_k(eng, data.test, data.known, data.relation_count, data.entity_count, k, path,
-                          precision=precision, value=value)
+                          precision=precision, value=value, sides=sides)
         log('Wrote {} predictions to {}'.format(n, path))
     if not raw:
         log('No test triple passed the confidence gate; no ranks recorded.')
-        return None
-    return score_mrr(raw, filt, log)
+        result = None
+    else:
+        result = score_mrr(raw, filt, log)
+    if relations:
+        # (h, ?, t) for every test triple: no confidence gate, nothing written to inference_results.tsv
+        rraw, rfilt = eval_link_prediction(eng, data.test, data.known, data.relation_count, data.entity_count,
+                                           sides=("relation",), precision=precision)
+        log('\nRelation prediction:')
+        if rraw:
+            result = dict(result or {}, relation=score_mrr(rraw, rfilt, log))
+        else:
+            log('No test triple to rank (every one is in-sample).')
+    return result
 
 
 # --------------------------------------------------------------------------------------
@@ -557,6 +588,12 @@ def build_parser():
     parser.add_argument('--predict_top_k', type=int, default=0,
                         help='With --infer: write the K best new tails of every (head, relation) and heads of every '
                              '(tail, relation) pair of the test file to <output_dir>/predictions.tsv (0 = off).')
+    parser.add_argument('--relation_prediction', action='store_true',
+                        help='With --infer: also rank every test triple\'s relation against all relations, (h, ?, t) '
+                             'filtered by the train + valid relations of (h, t), and log its MRR / Hits; with '
+                             '--predict_top_k, also write the K best new relations of every (head, tail) pair of the '
+                             'test file to predictions.tsv.  Writes nothing to inference_results.tsv; --infer_gate '
+                             'does not apply to it.')
     parser.add_argument('--valid_sample', action='store_true',
                         help='Validate on one sampled batch as holE.py does (default: the whole triples-valid.txt).')
     parser.add_argument('--score_variant', choices=['complex', 'ccorr_tanh'], default='complex',

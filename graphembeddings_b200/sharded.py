@@ -264,7 +264,11 @@ class RowShardedTrainer:
         The candidate operand is my block of the shard as it lies (packed once per call); the rows of the
         queries' other entities come from their owners into a small side table [relations | fetched rows].
         Phase 1 computes only the true candidates' scores (each by its owner), phase 2 counts."""
-        from .engine import HOLE_RANK_BF16, HOLE_SIDE_TAIL, HoleEngine
+        from .engine import HOLE_RANK_BF16, HOLE_SIDE_HEAD, HOLE_SIDE_TAIL, HoleEngine, HoleError
+        if side not in (HOLE_SIDE_TAIL, HOLE_SIDE_HEAD):
+            raise HoleError(f"sharded ranking supports the tail and head sides only, got side {side}; the relation "
+                            "rows are replicated, so rank relations on one GPU: HoleEngine.rank(..., "
+                            "HOLE_SIDE_RELATION, 0, n_relations) on a table from gather_embeddings()")
         precision = HOLE_RANK_BF16 if precision is None else precision
         dev = self.shard.device
         q = torch.as_tensor(queries).to(dev).long()

@@ -51,13 +51,14 @@ typedef struct hole_ctx hole_ctx;
 #define HOLE_SIDE_TAIL 0         /* corrupt / rank tails */
 #define HOLE_SIDE_HEAD 1         /* corrupt / rank heads */
 #define HOLE_SIDE_BOTH 2         /* hole_rank / hole_topk only: tails then heads in one pass */
+#define HOLE_SIDE_RELATION 3     /* hole_rank / hole_topk only: rank relations (h, ?, t); not part of BOTH */
 
 /* Operand precision of the tensor-core ranking contraction. */
 #define HOLE_RANK_BF16   0       /* bf16 operands, fp32 accumulate; dim <= 640           */
 #define HOLE_RANK_BF16X3 1       /* split-bf16 (hi*hi + lo*hi + hi*lo): ranks match fp32 except within ~3e-5 of a tie; dim <= 320 */
 
 /* ABI version of this header; hole_abi_version() returns the library's. */
-#define HOLE_ABI_VERSION 3
+#define HOLE_ABI_VERSION 4
 HOLE_API int hole_abi_version(void);
 
 /* Thread-local message of the last failing call on this thread ("" if none). */
@@ -273,6 +274,16 @@ HOLE_API int hole_train_steps_host(hole_ctx* ctx, float* table, const int32_t* t
  * cores.  For query q = (h, t, r) and side:
  *   TAIL: candidates j in [ent_begin, ent_end) scored s_j = clip(E_j) . (h * r)
  *   HEAD: candidates j scored s_j = clip(E_j) . (r * conj(t))~        (SURVEY App. A.4)
+ *   RELATION: candidates j scored s_j = clip(E_j) . (h * conj(t))~, i.e. [Re w ; -Im w] with
+ *         w = clip(h) o conj(clip(t)) (ds/dy_r of SURVEY App. A.3).  The caller passes the relation
+ *         rows, [ent_begin, ent_end) = [0, n_relations), as it passes the entity rows for TAIL / HEAD;
+ *         the true candidate is column 2 (r), a query's filter slice lists the known relations of
+ *         (h, t), ties go to the smaller relation id, and every per-query array has Q rows.
+ *         In HOLE_SCORE_CCORR_TANH mode the query vector is ds/dr = [Re c + Im c ; Re c - Im c] with
+ *         c_k = sum_j conj(h_j) t_{j+k} (rows clipped).  hole_rank_ex's query_table supplies h and t.
+ *         A relation call over another range than a hole_rank_prepare'd one re-packs the candidate
+ *         operand and drops the prepared one (the cache holds one range).
+ *   (~: imaginary half negated)
  * raw_before[q]  = #{j : (s_j, j) < (s_true, true_id)}  (ascending: lower is better,
  *                  holE.py:231, 446-453; ties by smaller candidate id, holE.py:434)
  * filt_before[q] = raw_before[q] - #{f in filter[q], f in range : (s_f, f) < (s_true, true_id)}
@@ -285,7 +296,8 @@ HOLE_API int hole_train_steps_host(hole_ctx* ctx, float* table, const int32_t* t
  * Counts are ADDED to raw_before / filt_before (caller zeroes them), so shards accumulate.
  * side == HOLE_SIDE_BOTH ranks both sides in one pass (candidates packed once): every
  * per-query array (true_score_io, raw_before, filt_before, and filter_off with 2Q+1 entries)
- * then has 2Q rows -- rows [0,Q) are the tail ranks, rows [Q,2Q) the head ranks. */
+ * then has 2Q rows -- rows [0,Q) are the tail ranks, rows [Q,2Q) the head ranks.  BOTH does not include
+ * relations; there is no three-side mode. */
 HOLE_API int hole_rank(hole_ctx* ctx, const float* table, int64_t ent_begin, int64_t ent_end,
               const int32_t* queries, int64_t Q, int side, int precision,
               const int64_t* filter_off, const int32_t* filter_ids,
@@ -299,8 +311,9 @@ HOLE_API int hole_rank(hole_ctx* ctx, const float* table, int64_t ent_begin, int
  *   raw_before == filt_before == NULL (with compute_true != 0): true scores only, no counting pass.
  * hole_rank_prepare packs the candidate operand of [ent_begin, ent_end) once; later hole_rank / hole_rank_ex
  * calls on the same (table, range, precision) reuse it instead of re-packing, until hole_rank_invalidate, a
- * training call on this context, or a call with another table / range.  The caller must invalidate after
- * changing the table by any other means. */
+ * training call on this context, or a call with another table / range -- a HOLE_SIDE_RELATION call over the
+ * relation rows included: the cache has a single slot, so the next entity call re-packs.  The caller must
+ * invalidate after changing the table by any other means. */
 HOLE_API int hole_rank_ex(hole_ctx* ctx, const float* table, int64_t ent_begin, int64_t ent_end,
                  const float* query_table, const int32_t* queries, int64_t Q, int side, int precision,
                  const int64_t* filter_off, const int32_t* filter_ids,
@@ -310,12 +323,13 @@ HOLE_API int hole_rank_prepare(hole_ctx* ctx, const float* table, int64_t ent_be
                       int precision, void* stream);
 HOLE_API int hole_rank_invalidate(hole_ctx* ctx);
 
-/* ---- top-k link prediction: the entities the model puts first for (h, r, ?) or (?, r, t).  Replaces the pop
+/* ---- top-k link prediction: the entities the model puts first for (h, r, ?) or (?, r, t), or with
+ * HOLE_SIDE_RELATION the relations it puts first for (h, ?, t) over [ent_begin, ent_end) = [0, n_relations).  Replaces the pop
  * loop of eval_link_prediction (holE.py:427-472: candidates popped in ascending order, at most
  * InferenceCandidates.max_triples of them) over ALL candidates [ent_begin, ent_end), on the same tensor-core
  * contraction as hole_rank (same operand packing, same hole_rank_prepare cache and invalidation rules).
  * For query q = (h, t, r) the candidate scores s_j are hole_rank's (TAIL / HEAD, or the HOLE_SCORE_CCORR_TANH
- * query vector in that mode); the id being predicted (t for TAIL, h for HEAD) is ignored.
+ * query vector in that mode); the id being predicted (t for TAIL, h for HEAD, r for RELATION) is ignored.
  * Row q of the output holds the k candidates first in ascending (s, id) order (lower is better, ties to the
  * smaller id: the heap's order, holE.py:231, 434, 446-453), skipping the ids of q's filter slice:
  *   ids_out    int32 [Q', k]  global row ids, sorted by (score, id)
