@@ -84,10 +84,8 @@ struct hole_ctx {
   int gs = 0, v = 0;   // lanes per row and float4s per lane per half (kernel variant)
   int sm_count = 0;
   int key_bits = 0;    // bits needed for a row id
-  int k1_smem = 0;     // dynamic shared memory of the first-generation K1 body (--log_loss passes)
   bool k1_ready = false;   // kernel attributes set (lazily, on the first training call)
-  int k1_block = 256;  // threads per K1 block
-  int k1v2_smem = 0;   // dynamic shared memory of hole_k1_kernel at k1_block threads
+  int k1v2_smem = 0;   // dynamic shared memory of hole_k1_kernel
   int k1_groups = 0;   // lane groups resident on the whole GPU (sizes T, the triples per group)
   int ramp_first = 0;  // hole_train_steps: steps in the first planned chunk, then x ramp_factor; 0 = no ramp
   int host_first = 0;  // hole_train_steps_host: steps in a short first chunk; 0 = off (measured slower: r02_e2e_ab.jsonl)
@@ -135,8 +133,9 @@ struct hole_ctx {
   size_t prof_used = 0;
 };
 
-// K1 / K3 `flags`: bits 0-1 = loss mode (0 hinge, 1 / 2 log-loss pass with / without the positive
-// term), bit 2 = add to the delta table instead of overwriting it
+// run_step / K3 `flags`: bits 0-1 = loss mode (0 hinge, 1 / 2 log-loss pass with / without the
+// positive term: K1 runs in DM 3, which always adds to the delta table), bit 2 = K3 adds to the
+// delta table instead of overwriting it
 constexpr int HOLE_K1_ACCUMULATE = 4;
 constexpr int HOLE_TREE_C = 32;      // fan-in of the deterministic gradient combine tree
 constexpr int HOLE_TREE_LEVELS = 6;  // 32^6 > any 4B

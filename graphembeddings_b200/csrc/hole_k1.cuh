@@ -1,11 +1,15 @@
-// K1, second generation: fused gather + norm clip + Hermitian score + sigmoid + hinge + backward
-// of one batch (holE.py:161-168, 191-192, 198, 231 and the backward TF derives for 296).
+// K1: fused gather + norm clip + Hermitian score + sigmoid + loss + backward of one batch
+// (holE.py:161-168, 191-192, 194-198, 231 and the backward TF derives for 296).
 // Included by hole_train.cu (uses its Row<> helpers).
 //
-// Differences from the first-generation body (kept as hole_train_fwd_bwd_ll_kernel for --log_loss):
+// A group of GS lanes walks T consecutive triples of the step's relation-grouped order (perm),
+// software-pipelined: the rows of the next two triples are in flight while the current one is
+// computed; the relation row is loaded once per run of equal relation and its gradient is summed
+// over the run in registers.  A row that occurs exactly once in the step (gslot == UNIQUE) is
+// read by nobody else during the step, so its change is written directly (see DM below);
+// otherwise its gradient is staged in G (for a relation run at the run's first triple) for K3.
 //   * rows are fetched with ONE 1-D bulk async copy per row (cp.async.bulk + mbarrier
-//     complete_tx, SASS UBLKCP) issued by one elected lane of the lane group, instead of
-//     2*V cp.async per lane;
+//     complete_tx, SASS UBLKCP) issued by one elected lane of the lane group;
 //   * rows stay UNSCALED in registers; the norm clip is carried as four scalars.  The score is
 //     trilinear, so s(y) = sc_h sc_r sc_t s(x): the three sums of squares and the two raw scores
 //     are reduced across the group in ONE round of shuffles;
@@ -17,8 +21,13 @@
 //   * DM selects where the step's row changes go: 0 in place on the table (single GPU),
 //     1 into a local delta table (hole_train_step_ex), 2 row-sharded: rows are gathered straight
 //     from their owners' shards over NVLink and every unique row's delta is stored into the
-//     owner's staging buffer (peer memory), fused into this kernel (hole_shard_step).
+//     owner's staging buffer (peer memory), fused into this kernel (hole_shard_step);
+//     3 is a --log_loss pass (hole_train_step_logloss): the table is read only and every unique
+//     row's delta is ADDED to the delta table, which sums the passes over one old table.  The
+//     loss is the only other difference; `loss` is null on the passes without the positive term.
 #pragma once
+
+constexpr int K1_THREADS = 256;  // threads per block; at dim 768 their landing rows take 221,376 B of 227 KB
 
 constexpr int K1V2_STAGES = 3;   // landing buffers per lane group: the triple being computed + 2 in flight
 
@@ -50,7 +59,7 @@ __device__ __forceinline__ void k1_bulk_g2s(void* smem_dst, const void* gsrc, ui
 }
 
 struct hole_k1_args {
-  float* E;                 // table (DM 0: updated in place; DM 1: read only; DM 2: unused)
+  float* E;                 // table (DM 0: updated in place; DM 1/3: read only; DM 2: unused)
   const int32_t* tri;       // [B,3] (head, tail, relation): rows to GATHER (DM 2: global row ids)
   const int32_t* neg;       // [B]   corrupt entity per triple
   const int32_t* perm;      // [B]   processing order (triples grouped by relation)
@@ -58,9 +67,9 @@ struct hole_k1_args {
   int side, B, T, nvec, stride;
   float margin, lr;
   float* G;                 // staged gradient rows (rows used more than once in the step)
-  float* loss;              // [B]
-  float* sigma;             // [2B] or null
-  float* Dtab;              // DM 1: delta table; DM 2: local delta rows of the replicated relation block
+  float* loss;              // [B]  (DM 3: log loss of the positives, null on the passes without them)
+  float* sigma;             // [2B] or null  (DM 3: [B] log loss of the pass's negatives)
+  float* Dtab;              // DM 1/3: delta table; DM 2: local delta rows of the replicated relation block
 };
 
 // DM 2 (row-sharded step): where rows live and where their deltas go
@@ -118,6 +127,7 @@ __device__ __forceinline__ void k1_row_from_smem(Row<V>& x, const float4* ssrc, 
 // carry the clip scales and the clip-backward projection), then
 //   unique row : DM 0  E[row] = x - lr dx   (skipped for an inactive hinge: dx == 0)
 //                DM 1/2  out[row] = -lr dx   (always written: the consumer adds every listed row)
+//                DM 3    out[row] += -lr dx
 //   otherwise  : G[gslot] = dx  for K3's ordered combine
 template <int GS, int V, bool FULL, int DM>
 __device__ __forceinline__ void k1_emit(const Row<V>& d, const Row<V>& x, float A, float Bc, bool uniq,
@@ -136,6 +146,11 @@ __device__ __forceinline__ void k1_emit(const Row<V>& d, const Row<V>& x, float 
       for (int k = 0; k < 4 * V; ++k) {
         o.re[k] = -lr * fmaf(A, d.re[k], -Bc * x.re[k]);
         o.im[k] = -lr * fmaf(A, d.im[k], -Bc * x.im[k]);
+      }
+      if (DM == 3) {
+        Row<V> p;
+        row_load<GS, V, false>(p, out_row, lane, nvec);
+        row_add(o, p);
       }
     }
     row_store<GS, V, FULL>(o, out_row, lane, nvec);
@@ -224,7 +239,7 @@ __device__ __forceinline__ void hole_k1_body(const hole_k1_args& a, const hole_k
       return static_cast<float*>(sh.stage.p[o]) +
              ((size_t)sh.me * (size_t)sh.cap + (size_t)(wrow - sh.R - s_cuts[o])) * stride;
     }
-    return (DM == 1 ? a.Dtab : a.E) + (size_t)id * stride;
+    return (DM == 0 ? a.E : a.Dtab) + (size_t)id * stride;
   };
   auto fetch = [&](const K1Ids& d, int stage) {
     if (lane == 0) {
@@ -338,13 +353,26 @@ __device__ __forceinline__ void hole_k1_body(const hole_k1_args& a, const hole_k
     const float sp = Sp * (sc_h * sc_r * sc_t);
     const float sn = Sn * (side == 0 ? (sc_h * sc_r * sc_n) : (sc_n * sc_r * sc_t));
     const float vp = sigmoidf_precise(sp), vn = sigmoidf_precise(sn);
-    const float pre = vp - vn + a.margin;
-    const bool act = pre >= 0.0f;                                  // TF Maximum grad: GreaterEqual
-    const float gp = act ? vp * (1.0f - vp) : 0.0f;
-    const float gn = act ? -(vn * (1.0f - vn)) : 0.0f;
-    if (lane == 0) {
-      a.loss[i] = fmaxf(pre, 0.0f);
-      if (a.sigma != nullptr) { a.sigma[i] = vp; a.sigma[B + i] = vn; }
+    bool act;
+    float gp, gn;
+    if constexpr (DM == 3) {  // (a plain `if` reorders DM 0-2's loop registers)
+      // --log_loss (holE.py:194-195): loss = log(1 + exp(-label * s)), d/ds = -label * sigmoid(-label * s)
+      act = true;
+      gp = (a.loss != nullptr) ? vp - 1.0f : 0.0f;
+      gn = vn;
+      if (lane == 0) {
+        if (a.loss != nullptr) a.loss[i] = logf(1.0f + expf(-sp));
+        a.sigma[i] = logf(1.0f + expf(sn));
+      }
+    } else {
+      const float pre = vp - vn + a.margin;
+      act = pre >= 0.0f;                                           // TF Maximum grad: GreaterEqual
+      gp = act ? vp * (1.0f - vp) : 0.0f;
+      gn = act ? -(vn * (1.0f - vn)) : 0.0f;
+      if (lane == 0) {
+        a.loss[i] = fmaxf(pre, 0.0f);
+        if (a.sigma != nullptr) { a.sigma[i] = vp; a.sigma[B + i] = vn; }
+      }
     }
     run_act = run_act || act;
     const float gs_p = gp * sp, gs_n = gn * sn, gs_b = gs_p + gs_n;   // y . dy of a row = g * s (Euler)
@@ -411,14 +439,10 @@ __device__ __forceinline__ void hole_k1_body(const hole_k1_args& a, const hole_k
   if (DM == 2) __threadfence_system();
 }
 
-#ifndef HOLE_K1_MAXTHREADS
-#define HOLE_K1_MAXTHREADS 256
-#endif
-#ifndef HOLE_K1_MINBLOCKS
-#define HOLE_K1_MINBLOCKS 1
-#endif
+// DM 3 at V 1 is held to two blocks per SM (128 registers, no spills), the occupancy DM 0 has there:
+// left free it takes 135 registers and one block per SM, and a log-loss step at d = 256 is 5-20 % slower
 template <int GS, int V, int DM>
-__global__ void __launch_bounds__(HOLE_K1_MAXTHREADS, HOLE_K1_MINBLOCKS)
+__global__ void __launch_bounds__(K1_THREADS, (DM == 3 && V == 1) ? 2 : 1)
 hole_k1_kernel(const hole_k1_args a, const hole_k1_shard sh) {
   // specialise on the corruption side and on "every lane owns valid float4s" (nvec == GS*V)
   const bool full = (a.nvec == GS * V);

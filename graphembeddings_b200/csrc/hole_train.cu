@@ -115,6 +115,17 @@ __device__ __forceinline__ void row_clip(Row<V>& x, float inv) {
   for (int k = 0; k < 4 * V; ++k) { x.re[k] *= sc; x.im[k] *= sc; }
 }
 
+template <int V>
+__device__ __forceinline__ void row_zero(Row<V>& x) {
+#pragma unroll
+  for (int k = 0; k < 4 * V; ++k) { x.re[k] = 0.f; x.im[k] = 0.f; }
+}
+template <int V>
+__device__ __forceinline__ void row_add(Row<V>& acc, const Row<V>& x) {
+#pragma unroll
+  for (int k = 0; k < 4 * V; ++k) { acc.re[k] += x.re[k]; acc.im[k] += x.im[k]; }
+}
+
 #ifdef HOLE_FAST_SIGMOID   // A/B only: ex2.approx + approximate division (|d sigma| ~ 1e-7)
 __device__ __forceinline__ float sigmoidf_precise(float s) { return __fdividef(1.0f, 1.0f + __expf(-s)); }
 #else
@@ -968,372 +979,6 @@ hole_score_kernel(const float* __restrict__ E, const int32_t* __restrict__ tripl
 }
 
 // ---------------------------------------------------------------------------------------
-// K1: fused forward + backward of one batch.
-// A group of GS lanes walks T consecutive triples of the step's relation-grouped order
-// (perm), software-pipelined: the next triple's three entity rows are in flight while the
-// current one is computed; the relation row is loaded once per run of equal relation and
-// its gradient is summed over the run in registers.
-// For each row a triple touches [relation, tail-slot, head-slot, corrupt entity] (rows
-// shared by the positive and the negative triple get the sum of both contributions; the
-// clip backward is linear in the incoming gradient, so merging before it is exact in real
-// arithmetic):
-//   * if the row occurs exactly once in this step (uniq flag from the plan) nobody else
-//     reads it during the step, so it is updated in place: E[row] = x - lr * dx;
-//   * otherwise the gradient row is staged in G (at slot*B + i; for a relation run at the
-//     position of the run's first triple) for K3.
-// ---------------------------------------------------------------------------------------
-enum { ROLE_T = 1, ROLE_H = 2, ROLE_N = 3 };
-
-template <int GS>
-__device__ __forceinline__ float group_sum_m(float v, unsigned gmask) {
-#pragma unroll
-  for (int o = GS / 2; o > 0; o >>= 1) v += __shfl_xor_sync(gmask, v, o);
-  return v;
-}
-
-template <int V>
-__device__ __forceinline__ void row_zero(Row<V>& x) {
-#pragma unroll
-  for (int k = 0; k < 4 * V; ++k) { x.re[k] = 0.f; x.im[k] = 0.f; }
-}
-template <int V>
-__device__ __forceinline__ void row_add(Row<V>& acc, const Row<V>& x) {
-#pragma unroll
-  for (int k = 0; k < 4 * V; ++k) { acc.re[k] += x.re[k]; acc.im[k] += x.im[k]; }
-}
-
-// Asynchronous row fetch into a per-lane landing buffer in shared memory: lane l copies
-// exactly the float4s it will later read itself, so no cross-lane synchronisation is
-// needed -- shared memory only holds the bytes in flight instead of registers.
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)),
-               "l"(gsrc)
-               : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-template <int GS, int V, bool FULL = false>
-__device__ __forceinline__ void row_fetch_async(float4* sdst, const float* grow, int lane, int nvec) {
-  const float4* p = reinterpret_cast<const float4*>(grow);
-#pragma unroll
-  for (int v = 0; v < V; ++v) {
-    const int idx = lane + v * GS;
-    if (FULL || idx < nvec) {
-      cp_async16(sdst + idx, p + idx);
-      cp_async16(sdst + nvec + idx, p + nvec + idx);
-    }
-  }
-}
-template <int GS, int V, bool FULL = false>
-__device__ __forceinline__ void row_from_smem(Row<V>& x, const float4* ssrc, int lane, int nvec) {
-#pragma unroll
-  for (int v = 0; v < V; ++v) {
-    const int idx = lane + v * GS;
-    float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a;
-    if (FULL || idx < nvec) { a = ssrc[idx]; b = ssrc[nvec + idx]; }
-    x.re[4 * v + 0] = a.x; x.re[4 * v + 1] = a.y; x.re[4 * v + 2] = a.z; x.re[4 * v + 3] = a.w;
-    x.im[4 * v + 0] = b.x; x.im[4 * v + 1] = b.y; x.im[4 * v + 2] = b.z; x.im[4 * v + 3] = b.w;
-  }
-}
-
-// through the norm clip (App. A.3): dx = clipped ? (dy - y (y.dy)) * inv : dy (y = clipped
-// row); then in place (unique row: E[row] = x - lr dx, x = y / s recovered as y * rs where
-// rs = 1/s is exact for the unclipped case s == 1) or staged.
-// xraw: the unscaled row as it was fetched (landing buffer), used for the in-place update.
-template <int GS, int V, bool FULL>
-__device__ __forceinline__ void finish_row(Row<V>& d, const Row<V>& y, const float4* xraw,
-                                           float inv_self, bool uniq, bool act, float lr,
-                                           float* erow, float* grow, int lane, int nvec,
-                                           unsigned gmask, int dmode) {
-  if (inv_self <= 1.0f) {          // group-uniform
-    float proj = 0.f;
-#pragma unroll
-    for (int k = 0; k < 4 * V; ++k) proj = fmaf(y.re[k], d.re[k], fmaf(y.im[k], d.im[k], proj));
-    proj = group_sum_m<GS>(proj, gmask);
-#pragma unroll
-    for (int k = 0; k < 4 * V; ++k) {
-      d.re[k] = (d.re[k] - y.re[k] * proj) * inv_self;
-      d.im[k] = (d.im[k] - y.im[k] * proj) * inv_self;
-    }
-  }
-  if (uniq) {
-    if (dmode != 0) {
-      // delta mode: erow points into the delta table.  Every row a step uses is written
-      // (zeros for an inactive hinge), so the caller only clears the relation block.
-      // dmode 2 adds to what the delta table holds (several passes over one old table).
-      const float sc = act ? -lr : 0.f;
-#pragma unroll
-      for (int k = 0; k < 4 * V; ++k) {
-        d.re[k] = act ? sc * d.re[k] : 0.f;
-        d.im[k] = act ? sc * d.im[k] : 0.f;
-      }
-      if (dmode == 2) {
-        Row<V> o;
-        row_load<GS, V, false>(o, erow, lane, nvec);
-        row_add(d, o);
-      }
-      row_store<GS, V, FULL>(d, erow, lane, nvec);
-    } else if (act) {              // inactive hinge: zero gradient, row unchanged
-      Row<V> x;
-      row_from_smem<GS, V, FULL>(x, xraw, lane, nvec);
-#pragma unroll
-      for (int k = 0; k < 4 * V; ++k) {
-        d.re[k] = x.re[k] - lr * d.re[k];
-        d.im[k] = x.im[k] - lr * d.im[k];
-      }
-      row_store<GS, V, FULL>(d, erow, lane, nvec);
-    }
-  } else {
-    row_store<GS, V, FULL>(d, grow, lane, nvec);
-  }
-}
-
-// yh, yt, yr, yn: the clipped rows (y = x * s)
-template <int GS, int V, int ROLE, int side, bool FULL>
-__device__ __forceinline__ void emit_row(const Row<V>& yh, const Row<V>& yt, const Row<V>& yr,
-                                         const Row<V>& yn, const float4* xraw, float inv_self,
-                                         float gp, float gn, bool uniq, bool act, float lr,
-                                         float* erow, float* grow, int lane, int nvec,
-                                         unsigned gmask, int dmode) {
-  Row<V> d;
-  const Row<V>& ys = (ROLE == ROLE_T) ? yt : (ROLE == ROLE_H) ? yh : yn;
-#pragma unroll
-  for (int k = 0; k < 4 * V; ++k) {
-    const float a = yh.re[k], b = yh.im[k], c = yr.re[k], dd = yr.im[k], e = yt.re[k], f = yt.im[k];
-    const float nr = yn.re[k], ni = yn.im[k];
-    float gre, gim;
-    if (ROLE == ROLE_T) {          // d/dt = g [a c - b d ; a d + b c]
-      gre = gp * (a * c - b * dd);
-      gim = gp * (a * dd + b * c);
-      if (side) {                  // negative (n, t, r) shares t
-        gre += gn * (nr * c - ni * dd);
-        gim += gn * (nr * dd + ni * c);
-      }
-    } else if (ROLE == ROLE_H) {   // d/dh = g [c e + d f ; c f - d e]
-      gre = gp * (c * e + dd * f);
-      gim = gp * (c * f - dd * e);
-      if (!side) {                 // negative (h, n, r) shares h
-        gre += gn * (c * nr + dd * ni);
-        gim += gn * (c * ni - dd * nr);
-      }
-    } else {                       // corrupt entity: head role if side else tail role
-      gre = side ? gn * (c * e + dd * f) : gn * (a * c - b * dd);
-      gim = side ? gn * (c * f - dd * e) : gn * (a * dd + b * c);
-    }
-    d.re[k] = gre;
-    d.im[k] = gim;
-  }
-  finish_row<GS, V, FULL>(d, ys, xraw, inv_self, uniq, act, lr, erow, grow, lane, nvec, gmask, dmode);
-}
-
-struct TripleIds { int i, h, t, r, n; };
-
-__device__ __forceinline__ TripleIds load_ids(const int32_t* __restrict__ tri,
-                                              const int32_t* __restrict__ neg,
-                                              const int32_t* __restrict__ perm, int g) {
-  TripleIds d;
-  d.i = perm[g];
-  d.h = tri[3 * d.i]; d.t = tri[3 * d.i + 1]; d.r = tri[3 * d.i + 2];
-  d.n = neg[d.i];
-  return d;
-}
-
-constexpr int K1_STAGES = 3;   // landing buffers per lane group: the triple being computed (its
-                               // unscaled rows are re-read for the in-place update) + 2 in flight
-
-template <int GS, int V, int side, bool FULL, bool LOGLOSS>
-__device__ __forceinline__ void
-hole_train_fwd_bwd_body(float* __restrict__ E, const int32_t* __restrict__ tri,
-                          const int32_t* __restrict__ neg, const int32_t* __restrict__ perm,
-                          const uint32_t* __restrict__ gslot, int B, int T, int nvec,
-                          int stride, float margin, float lr, float* __restrict__ G,
-                          float* __restrict__ loss, float* __restrict__ sigma, float* __restrict__ Dtab,
-                          int flags) {
-  extern __shared__ float4 k1_smem[];
-  // delta mode (multi-GPU step tables, log-loss passes): unique rows write -lr*dx into Dtab
-  // instead of updating E in place
-  const bool delta = Dtab != nullptr;
-  const int dmode = delta ? ((flags & HOLE_K1_ACCUMULATE) ? 2 : 1) : 0;
-  // 0 hinge; 1 / 2 = --log_loss pass with / without the positive term (own instantiation, so
-  // that the hinge kernel is compiled exactly as if the branch did not exist)
-  const int mode = LOGLOSS ? (flags & 3) : 0;
-  float* const Eout = delta ? Dtab : E;
-  const int lane = threadIdx.x % GS;
-  const int gbase = (threadIdx.x % 32) / GS * GS;
-  const unsigned gmask = (GS == 32) ? 0xffffffffu : (((1u << GS) - 1u) << gbase);
-  const int64_t w = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) / GS;
-  const int64_t g0l = w * T;
-  if (g0l >= B) return;
-  const int g0 = (int)g0l, g1 = min(B, g0 + T);
-  const int row4 = 2 * nvec;                                   // float4s per row
-  // per lane group: K1_STAGES x {h, t, n} landing rows, then one row for the relation
-  float4* my_smem = k1_smem + (size_t)(threadIdx.x / GS) * ((K1_STAGES * 3 + 1) * row4);
-  float4* rel_smem = my_smem + (size_t)K1_STAGES * 3 * row4;
-
-  auto fetch = [&](const TripleIds& d, int stage) {
-    float4* sb = my_smem + (size_t)stage * 3 * row4;
-    row_fetch_async<GS, V, FULL>(sb, E + (size_t)d.h * stride, lane, nvec);
-    row_fetch_async<GS, V, FULL>(sb + row4, E + (size_t)d.t * stride, lane, nvec);
-    row_fetch_async<GS, V, FULL>(sb + 2 * row4, E + (size_t)d.n * stride, lane, nvec);
-  };
-
-  TripleIds c = load_ids(tri, neg, perm, g0);
-  TripleIds n1 = (g0 + 1 < g1) ? load_ids(tri, neg, perm, g0 + 1) : c;
-  TripleIds n2 = (g0 + 2 < g1) ? load_ids(tri, neg, perm, g0 + 2) : c;
-  pdl_wait();                 // the previous step's K3 has finished updating the table
-  fetch(c, 0);
-  cp_async_commit();
-  if (g0 + 1 < g1) fetch(n1, 1);
-  cp_async_commit();
-
-  Row<V> yh, yt, yn, yr, acc;
-  row_zero(yr);
-  row_zero(acc);
-  int r_cur = -1, run_i = 0;
-  float ir = 0.f;
-  bool run_act = false;
-
-  // end of a run of equal relation: clip backward of the summed gradient, then apply / stage
-  auto flush_relation = [&]() {
-    const uint32_t sl = gslot[run_i];
-    finish_row<GS, V, FULL>(acc, yr, rel_smem, ir, sl == HOLE_SLOT_UNIQUE, run_act, lr,
-                      Eout + (size_t)r_cur * stride, G + (size_t)sl * stride, lane, nvec, gmask, dmode);
-  };
-
-  int stage = 0;
-  for (int g = g0; g < g1; ++g) {
-    TripleIds n3 = n2;
-    if (g + 3 < g1) n3 = load_ids(tri, neg, perm, g + 3);      // ids three ahead
-    if (g + 2 < g1) fetch(n2, (stage + 2) % K1_STAGES);         // rows two ahead
-    cp_async_commit();
-    cp_async_wait<2>();                                         // rows of triple g have landed
-    const float4* sb = my_smem + (size_t)stage * 3 * row4;
-    row_from_smem<GS, V, FULL>(yh, sb, lane, nvec);
-    row_from_smem<GS, V, FULL>(yt, sb + row4, lane, nvec);
-    row_from_smem<GS, V, FULL>(yn, sb + 2 * row4, lane, nvec);
-
-    if (c.r != r_cur) {                      // group-uniform
-      if (r_cur >= 0) flush_relation();
-      // the relation row: fetched synchronously once per run, unscaled copy kept in smem
-      row_load<GS, V, false>(yr, E + (size_t)c.r * stride, lane, nvec);
-      {
-        float4* rs = rel_smem;
-#pragma unroll
-        for (int v = 0; v < V; ++v) {
-          const int idx = lane + v * GS;
-          if (idx < nvec) {
-            rs[idx] = make_float4(yr.re[4 * v], yr.re[4 * v + 1], yr.re[4 * v + 2], yr.re[4 * v + 3]);
-            rs[nvec + idx] = make_float4(yr.im[4 * v], yr.im[4 * v + 1], yr.im[4 * v + 2], yr.im[4 * v + 3]);
-          }
-        }
-      }
-      ir = __frsqrt_rn(group_sum_m<GS>(row_sumsq(yr), gmask));
-      row_clip(yr, ir);
-      r_cur = c.r;
-      run_i = c.i;
-      run_act = false;
-      row_zero(acc);
-    }
-    const int i = c.i;
-    const uint32_t sl_t = gslot[B + i], sl_h = gslot[2 * B + i], sl_n = gslot[3 * B + i];
-
-    float ssh = row_sumsq(yh), sst = row_sumsq(yt), ssn = row_sumsq(yn);
-#pragma unroll
-    for (int o = GS / 2; o > 0; o >>= 1) {
-      ssh += __shfl_xor_sync(gmask, ssh, o);
-      sst += __shfl_xor_sync(gmask, sst, o);
-      ssn += __shfl_xor_sync(gmask, ssn, o);
-    }
-    // clip_by_norm(row, 1): y = x * min(rsqrt(sum x^2), 1)  (App. B)
-    const float ih = __frsqrt_rn(ssh), it = __frsqrt_rn(sst), in_ = __frsqrt_rn(ssn);
-    row_clip(yh, ih); row_clip(yt, it); row_clip(yn, in_);
-
-    // scores: s = sum (a c - b d) e + (a d + b c) f   with h=(a,b) r=(c,d) t=(e,f)
-    float sp = 0.f, sn = 0.f;
-#pragma unroll
-    for (int k = 0; k < 4 * V; ++k) {
-      const float a = yh.re[k], b = yh.im[k], cc = yr.re[k], d = yr.im[k], e = yt.re[k], f = yt.im[k];
-      const float nr = yn.re[k], ni = yn.im[k];
-      const float pr = a * cc - b * d, pi = a * d + b * cc;
-      sp += pr * e + pi * f;
-      if (side) sn += (nr * cc - ni * d) * e + (nr * d + ni * cc) * f;   // negative = (n, t, r)
-      else      sn += pr * nr + pi * ni;                                 // negative = (h, n, r)
-    }
-#pragma unroll
-    for (int o = GS / 2; o > 0; o >>= 1) {
-      sp += __shfl_xor_sync(gmask, sp, o);
-      sn += __shfl_xor_sync(gmask, sn, o);
-    }
-    const float vp = sigmoidf_precise(sp), vn = sigmoidf_precise(sn);
-    bool act;
-    float gp, gn;
-    if (mode == 0) {
-      const float pre = vp - vn + margin;
-      act = pre >= 0.0f;                                // TF Maximum grad: GreaterEqual
-      gp = act ? vp * (1.0f - vp) : 0.0f;
-      gn = act ? -(vn * (1.0f - vn)) : 0.0f;
-      if (lane == 0) {
-        loss[i] = fmaxf(pre, 0.0f);
-        if (sigma != nullptr) { sigma[i] = vp; sigma[B + i] = vn; }
-      }
-    } else {
-      // --log_loss (holE.py:194-195): loss = log(1 + exp(-label * s)), d/ds = -label * sigmoid(-label * s).
-      // `loss` takes the positives (pass 1 only), `sigma` this pass's negatives.
-      act = true;
-      gp = (mode == 1) ? vp - 1.0f : 0.0f;
-      gn = vn;
-      if (lane == 0) {
-        if (mode == 1) loss[i] = logf(1.0f + expf(-sp));
-        sigma[i] = logf(1.0f + expf(sn));
-      }
-    }
-    run_act = run_act || act;
-    // relation gradient, summed over the run before the clip backward:
-    // d/dr = g+ [a e + b f ; a f - b e] + g- [same with the negative's h, t]
-#pragma unroll
-    for (int k = 0; k < 4 * V; ++k) {
-      const float a = yh.re[k], b = yh.im[k], e = yt.re[k], f = yt.im[k];
-      const float nr = yn.re[k], ni = yn.im[k];
-      const float a2 = side ? nr : a, b2 = side ? ni : b, e2 = side ? e : nr, f2 = side ? f : ni;
-      acc.re[k] += gp * (a * e + b * f) + gn * (a2 * e2 + b2 * f2);
-      acc.im[k] += gp * (a * f - b * e) + gn * (a2 * f2 - b2 * e2);
-    }
-    emit_row<GS, V, ROLE_T, side, FULL>(yh, yt, yr, yn, sb + row4, it, gp, gn, sl_t == HOLE_SLOT_UNIQUE, act, lr,
-                            Eout + (size_t)c.t * stride, G + (size_t)sl_t * stride, lane, nvec, gmask, dmode);
-    emit_row<GS, V, ROLE_H, side, FULL>(yh, yt, yr, yn, sb, ih, gp, gn, sl_h == HOLE_SLOT_UNIQUE, act, lr,
-                            Eout + (size_t)c.h * stride, G + (size_t)sl_h * stride, lane, nvec, gmask, dmode);
-    emit_row<GS, V, ROLE_N, side, FULL>(yh, yt, yr, yn, sb + 2 * row4, in_, gp, gn, sl_n == HOLE_SLOT_UNIQUE, act, lr,
-                            Eout + (size_t)c.n * stride, G + (size_t)sl_n * stride, lane, nvec, gmask, dmode);
-    c = n1;
-    n1 = n2;
-    n2 = n3;
-    stage = (stage + 1) % K1_STAGES;
-  }
-  cp_async_wait<0>();
-  pdl_launch_dependents();    // K3 of this step may start its prologue
-  flush_relation();
-}
-
-#define HOLE_K1_BODY(SIDE, FULL_, LL) \
-  hole_train_fwd_bwd_body<GS, V, SIDE, FULL_, LL>(E, tri, neg, perm, gslot, B, T, nvec, stride, margin, lr, G, loss, sigma, Dtab, flags)
-
-// the --log_loss passes run the first-generation body (cp.async landing buffers, rows clipped in
-// registers); the hinge step runs hole_k1_kernel (hole_k1.cuh)
-template <int GS, int V>
-__global__ void __launch_bounds__(256)
-hole_train_fwd_bwd_ll_kernel(float* __restrict__ E, const int32_t* __restrict__ tri,
-                             const int32_t* __restrict__ neg, const int32_t* __restrict__ perm,
-                             const uint32_t* __restrict__ gslot, int side, int B, int T, int nvec,
-                             int stride, float margin, float lr, float* __restrict__ G,
-                             float* __restrict__ loss, float* __restrict__ sigma, float* __restrict__ Dtab,
-                             int flags) {
-  if (side) HOLE_K1_BODY(1, false, true); else HOLE_K1_BODY(0, false, true);
-}
-#undef HOLE_K1_BODY
-
-// ---------------------------------------------------------------------------------------
 // K3: deterministic sparse SGD update for rows that occur more than once in the step.
 // One group per sorted entry; only entries that head a chunk of C consecutive occurrences
 // of a row do work.  A row with n occurrences is reduced by a fixed C-ary tree over its
@@ -1722,19 +1367,17 @@ hole_loss_sum_kernel(const float* __restrict__ loss, int64_t B, float* __restric
 // ---------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------
-#define HOLE_DISPATCH_SMEM(ctx, KERNEL, grid, block, smem, stream, ...)                      \
+#define HOLE_DISPATCH(ctx, KERNEL, grid, block, stream, ...)                                 \
   do {                                                                                       \
-    if ((ctx)->gs == 8 && (ctx)->v == 1) KERNEL<8, 1><<<grid, block, smem, stream>>>(__VA_ARGS__);          \
-    else if ((ctx)->gs == 16 && (ctx)->v == 1) KERNEL<16, 1><<<grid, block, smem, stream>>>(__VA_ARGS__);   \
-    else if ((ctx)->gs == 32 && (ctx)->v == 1) KERNEL<32, 1><<<grid, block, smem, stream>>>(__VA_ARGS__);   \
-    else if ((ctx)->gs == 32 && (ctx)->v == 2) KERNEL<32, 2><<<grid, block, smem, stream>>>(__VA_ARGS__);   \
-    else if ((ctx)->gs == 32 && (ctx)->v == 3) KERNEL<32, 3><<<grid, block, smem, stream>>>(__VA_ARGS__);   \
+    if ((ctx)->gs == 8 && (ctx)->v == 1) KERNEL<8, 1><<<grid, block, 0, stream>>>(__VA_ARGS__);          \
+    else if ((ctx)->gs == 16 && (ctx)->v == 1) KERNEL<16, 1><<<grid, block, 0, stream>>>(__VA_ARGS__);   \
+    else if ((ctx)->gs == 32 && (ctx)->v == 1) KERNEL<32, 1><<<grid, block, 0, stream>>>(__VA_ARGS__);   \
+    else if ((ctx)->gs == 32 && (ctx)->v == 2) KERNEL<32, 2><<<grid, block, 0, stream>>>(__VA_ARGS__);   \
+    else if ((ctx)->gs == 32 && (ctx)->v == 3) KERNEL<32, 3><<<grid, block, 0, stream>>>(__VA_ARGS__);   \
     else return hole_set_error(HOLE_ERR_UNSUPPORTED, "no kernel variant for gs=%d v=%d",     \
                                (ctx)->gs, (ctx)->v);                                         \
     HOLE_LAUNCHED();                                                                         \
   } while (0)
-#define HOLE_DISPATCH(ctx, KERNEL, grid, block, stream, ...) \
-  HOLE_DISPATCH_SMEM(ctx, KERNEL, grid, block, 0, stream, __VA_ARGS__)
 
 // same, launched with programmatic stream serialization (see pdl_wait)
 #define HOLE_DISPATCH_PDL(ctx, KERNEL, grid_, block_, smem_, stream_, ...)                   \
@@ -1888,12 +1531,6 @@ extern "C" int hole_ctx_create(hole_ctx** out, int device, int64_t n_rows, int d
   c->row_passes = 1;
   while (((int64_t(1) << (8 * c->row_passes)) - 1) < n_rows) ++c->row_passes;
   c->rel_passes = c->row_passes;
-  // K1 landing buffers (first-generation body): K1_STAGES triples x 3 entity rows + 1 relation row per
-  // lane group.  Kernel attributes are set lazily by k1_prepare(): scoring / ranking contexts never
-  // need them.
-  c->k1_smem = (256 / c->gs) * (K1_STAGES * 3 + 1) * c->row_stride * (int)sizeof(float);
-  if (const char* e = getenv("HOLE_K1_BLOCK")) c->k1_block = atoi(e);
-  if (c->k1_block != 128 && c->k1_block != 192 && c->k1_block != 256) c->k1_block = 256;
   if (const char* e = getenv("HOLE_HOST_FIRST")) c->host_first = atoi(e);
   if (const char* e = getenv("HOLE_SORT_SMALL")) c->sort_small = atoi(e);   // 0 = always the radix chain, 2 = always one launch
   if (const char* e = getenv("HOLE_PLAN_RAMP")) {     // "first,factor"; "0" disables the ramp
@@ -2132,52 +1769,35 @@ static hole_k1_fn k1_fn(const hole_ctx* c) {
   return hole_k1_kernel<32, 3, DM>;
 }
 static hole_k1_fn k1_fn_dm(const hole_ctx* c, int dm) {
-  return dm == 0 ? k1_fn<0>(c) : dm == 1 ? k1_fn<1>(c) : k1_fn<2>(c);
+  return dm == 0 ? k1_fn<0>(c) : dm == 1 ? k1_fn<1>(c) : dm == 2 ? k1_fn<2>(c) : k1_fn<3>(c);
 }
 
 // Kernel attributes of the training kernels, set on the first training call of a context
 // (scoring / ranking contexts never pay for, or fail on, K1's shared-memory request).
 static int k1_prepare(hole_ctx* c) {
   if (c->k1_ready) return HOLE_OK;
-  const int limit = 227 * 1024;
-  // second generation: K1V2_STAGES x 3 landing rows + K1V2_STAGES mbarriers per lane group
-  int block = c->k1_block;
-  auto smem_of = [&](int blk) { return (blk / c->gs) * K1V2_STAGES * (3 * c->row_stride * (int)sizeof(float) + 8); };
-  while (block > 32 && smem_of(block) > limit) block -= 32;
-  if (smem_of(block) > limit || block < c->gs)
-    return hole_set_error(HOLE_ERR_UNSUPPORTED, "embedding_dim %d: a K1 lane group needs %d bytes of shared memory",
-                          c->dim, smem_of(c->gs));
-  c->k1_block = block;
-  c->k1v2_smem = smem_of(block);
+  // K1V2_STAGES x 3 landing rows + K1V2_STAGES mbarriers per lane group
+  c->k1v2_smem = (K1_THREADS / c->gs) * K1V2_STAGES * (3 * c->row_stride * (int)sizeof(float) + 8);
+  if (c->k1v2_smem > 227 * 1024)
+    return hole_set_error(HOLE_ERR_UNSUPPORTED, "embedding_dim %d: K1 needs %d bytes of shared memory",
+                          c->dim, c->k1v2_smem);
   int nb = 1;
-  for (int dm = 0; dm < 3; ++dm) {
+  for (int dm = 0; dm < 4; ++dm) {
     HOLE_CUDA_TRY(cudaFuncSetAttribute(k1_fn_dm(c, dm), cudaFuncAttributeMaxDynamicSharedMemorySize, c->k1v2_smem));
   }
-  HOLE_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k1_fn<0>(c), c->k1_block, c->k1v2_smem));
-  c->k1_groups = c->sm_count * std::max(nb, 1) * (c->k1_block / c->gs);
-  if (c->k1_smem <= limit) {       // first-generation body (--log_loss passes)
-    cudaError_t ea = cudaSuccess;
-#define HOLE_K1_ATTR(KERNEL)                                                                                   \
-    if (c->gs == 8) ea = cudaFuncSetAttribute(KERNEL<8, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, c->k1_smem);          \
-    else if (c->gs == 16) ea = cudaFuncSetAttribute(KERNEL<16, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, c->k1_smem);   \
-    else if (c->v == 1) ea = cudaFuncSetAttribute(KERNEL<32, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, c->k1_smem);     \
-    else if (c->v == 2) ea = cudaFuncSetAttribute(KERNEL<32, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, c->k1_smem);     \
-    else ea = cudaFuncSetAttribute(KERNEL<32, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, c->k1_smem);
-    HOLE_K1_ATTR(hole_train_fwd_bwd_ll_kernel)
-    HOLE_CUDA_TRY(ea);
-#undef HOLE_K1_ATTR
-  }
+  HOLE_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k1_fn<0>(c), K1_THREADS, c->k1v2_smem));
+  c->k1_groups = c->sm_count * std::max(nb, 1) * (K1_THREADS / c->gs);
   c->k1_ready = true;
   return HOLE_OK;
 }
 
 static int k1_launch(hole_ctx* c, int dm, const hole_k1_args& a, const hole_k1_shard& sh, cudaStream_t st,
                      bool pdl) {
-  const int per_block = c->k1_block / c->gs;
+  const int per_block = K1_THREADS / c->gs;
   const int64_t groups = ((int64_t)a.B + a.T - 1) / a.T;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)std::max<int64_t>(1, (groups + per_block - 1) / per_block));
-  cfg.blockDim = dim3((unsigned)c->k1_block);
+  cfg.blockDim = dim3((unsigned)K1_THREADS);
   cfg.dynamicSmemBytes = (size_t)c->k1v2_smem;
   cfg.stream = st;
   cudaLaunchAttribute at[1];
@@ -2319,23 +1939,17 @@ static int run_step(hole_ctx* c, hole_plan& pl, float* table, const int32_t* pos
                                    c->row_stride, margin, lr, c->G, loss_out, sigma_out)));
     HOLE_CUDA_TRY(cudaGetLastError());
     HOLE_LAUNCHED();
-  } else if ((flags & 3) == 0) {
+  } else {
     hole_k1_args ka = {};
     ka.E = table; ka.tri = shard ? shard_tri : pos; ka.neg = shard ? shard_neg : neg;
     ka.perm = pl.perm + (size_t)slot * B; ka.gslot = pl.gslot + off;
     ka.side = side; ka.B = (int)B; ka.T = pl.T; ka.nvec = c->nvec; ka.stride = c->row_stride;
-    ka.margin = margin; ka.lr = lr; ka.G = c->G; ka.loss = loss_out; ka.sigma = sigma_out; ka.Dtab = delta_out;
+    ka.margin = margin; ka.lr = lr; ka.G = c->G; ka.sigma = sigma_out; ka.Dtab = delta_out;
+    ka.loss = (flags & 3) == 2 ? nullptr : loss_out;       // a log-loss pass without the positive term
     static const hole_k1_shard no_shard = {};
-    const int dm = shard ? 2 : (delta_out ? 1 : 0);
+    const int dm = (flags & 3) ? 3 : shard ? 2 : (delta_out ? 1 : 0);
     int rc = k1_launch(c, dm, ka, shard ? *shard : no_shard, st, k1_follows_k3 && !c->profile);
     if (rc) return rc;
-  } else {
-    if (c->k1_smem > 227 * 1024)   // (hole_train_step_logloss refuses this at its entry; kept as a guard)
-      return hole_set_error(HOLE_ERR_UNSUPPORTED, "embedding_dim %d: the --log_loss kernel needs %d bytes of shared memory",
-                            c->dim, c->k1_smem);
-    HOLE_DISPATCH_SMEM(c, hole_train_fwd_bwd_ll_kernel, grid_for_groups((B + pl.T - 1) / pl.T, c->gs), 256,
-                       c->k1_smem, st, table, pos, neg, pl.perm + (size_t)slot * B, pl.gslot + off, side, (int)B, pl.T, c->nvec,
-                c->row_stride, margin, lr, c->G, loss_out, sigma_out, delta_out, flags);
   }
   if (pe) HOLE_CUDA_TRY(cudaEventRecord(pe[1], st));
   if (k1_done_mark) HOLE_CUDA_TRY(cudaEventRecord(k1_done_mark, st));
@@ -2453,10 +2067,6 @@ extern "C" int hole_train_step_logloss(hole_ctx* c, float* table, float* delta_w
   HOLE_CHECK_ARG(c && B >= 0 && negative_ratio >= 1 && negative_ratio <= 64);
   if (c->score_mode != HOLE_SCORE_COMPLEX)
     return hole_set_error(HOLE_ERR_UNSUPPORTED, "the archived ccorr/tanh score mode has no log-loss branch");
-  // Refuse before the workspace and the plan: a refused call launches nothing and leaves plan slot 0 as it was.
-  if (c->k1_smem > 227 * 1024)
-    return hole_set_error(HOLE_ERR_UNSUPPORTED, "embedding_dim %d: the --log_loss kernel needs %d bytes of shared memory",
-                          c->dim, c->k1_smem);
   if (B == 0) return HOLE_OK;
   HOLE_CHECK_ARG(table && delta_ws && triples && type_of && csr_off && csr_ids && loss_out);
   HOLE_CHECK_ARG(4 * B < (int64_t(1) << 31));

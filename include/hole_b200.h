@@ -70,8 +70,8 @@ HOLE_API int hole_row_stride(int dim);
 /* Create / destroy a context bound to CUDA device `device` for a table of n_rows x dim
  * (holE.py:263-264: one shared table for relations and entities).  Synchronous.
  * dim <= 768; a larger dim returns HOLE_ERR_UNSUPPORTED.  A call outside the limits of its own path
- * (ranking / top-k above, the --log_loss step: dim <= 720) returns HOLE_ERR_UNSUPPORTED before it
- * launches anything or writes any output, and the context stays usable. */
+ * (ranking / top-k above) returns HOLE_ERR_UNSUPPORTED before it launches anything or writes any
+ * output, and the context stays usable. */
 HOLE_API int hole_ctx_create(hole_ctx** out, int device, int64_t n_rows, int dim);
 HOLE_API int hole_ctx_destroy(hole_ctx* ctx);
 
@@ -161,8 +161,7 @@ HOLE_API int hole_train_step_plan(hole_ctx* ctx, const int32_t* pos, const int32
  *   loss_out     [(1 + negative_ratio) * B] device: positives, then each corrupt batch
  *   l2_loss_out  device scalar = sum(E_old^2) / 2 (tf.nn.l2_loss), or NULL
  *   neg_out      [negative_ratio * B] device int32 replacement entities, or NULL
- *   sides_out    [negative_ratio] HOST int32 (1 = heads replaced), or NULL
- * dim <= 720 (the kernel's landing buffers in shared memory); the hinge step builds up to 768. */
+ *   sides_out    [negative_ratio] HOST int32 (1 = heads replaced), or NULL */
 HOLE_API int hole_train_step_logloss(hole_ctx* ctx, float* table, float* delta_ws, const int32_t* triples,
                                      int64_t B, int negative_ratio, const int32_t* type_of,
                                      const int64_t* csr_off, const int32_t* csr_ids, uint64_t seed,

@@ -35,7 +35,7 @@ SUM_ATOL = 1e-3                                        # a step's loss sum again
 MARGIN = 0.2
 SS_CAP = 11264                   # duplicated row uses the one-launch row sort keeps in shared memory (hole_train.cu)
 SHARD_PREP_STEPS, SHARD_LOSS_CHUNK = 16, 64            # csrc/hole_shard.cuh
-ENV_KEYS = ("HOLE_PLAN_RAMP", "HOLE_HOST_FIRST", "HOLE_SORT_SMALL", "HOLE_K1_BLOCK")
+ENV_KEYS = ("HOLE_PLAN_RAMP", "HOLE_HOST_FIRST", "HOLE_SORT_SMALL")
 
 
 @pytest.fixture(scope="module")
@@ -383,43 +383,4 @@ def test_relation_ids_above_the_hint_are_trained_right(eng_mod, monkeypatch, hin
     b = _engine(eng_mod, monkeypatch, kg, env, n_rel_hint=hint)
     ref = _per_step(b, tri.to(b.device), B, seed, first_step, lrs, check_at=boundary_steps(layout))
     _assert_matches_per_step(f"hint {hint}", a.table, b.table, sums, ref, B, loss)
-    a.close(); b.close()
-
-
-# ---------------------------------------------------------------- 6. K1 block sizes
-@pytest.mark.parametrize("dim", [64, 150, 256, 600])
-@pytest.mark.parametrize("k1_block", [128, 192, 256])
-def test_k1_block_variants(eng_mod, monkeypatch, k1_block, dim):
-    """HOLE_K1_BLOCK = 128 | 192 | 256 threads per training-kernel block (d = 600 trims 256 to what shared
-    memory holds).  One step stays within the one-step tolerances of the fp64 oracle; a call of 8 steps in
-    chunks 1, 2, 4, 1 (HOLE_PLAN_RAMP=1,2) equals the per-step path bit for bit within the block size.  The
-    triples per lane group follow the number of lane groups and so the block size: results are not
-    compared across block sizes."""
-    B, n_steps = 4096, 8
-    layout = chunk_sizes(B, n_steps, (1, 2))
-    assert layout == [1, 2, 4, 1]
-    kg = D.synthetic_kg(11, 6000, (n_steps + 1) * B, 5, dim, seed=dim + k1_block, trained_scale=True,
-                        zipf_entities=True)
-    env = {"HOLE_K1_BLOCK": k1_block}
-    e = _engine(eng_mod, monkeypatch, kg, env)
-    off, ids = D.build_type_csr(kg.type_of)
-    pos = kg.triples[n_steps * B:]
-    side, neg = O.corrupt(pos, kg.type_of, off, ids, 8, 1)
-    loss, vp, vn = e.train_step(pos, neg, side, MARGIN, 0.1, return_sigma=True)
-    E64 = kg.E.astype(np.float64)
-    want, vp64, vn64 = O.sgd_step(E64, pos, neg, side, MARGIN, 0.1, np.float64, "tf")
-    assert np.abs(vp.cpu().numpy() - vp64).max() <= 1e-6 and np.abs(vn.cpu().numpy() - vn64).max() <= 1e-6
-    assert np.abs(loss.cpu().numpy() - want).max() <= LOSS_ATOL
-    got = e.embeddings().cpu().numpy()
-    err, tol = np.abs(got - E64), ROW_ATOL + ROW_RTOL * np.abs(E64)
-    assert (err <= tol).all(), float((err - tol).max())
-    e.close()
-    seed, first_step = 19, 90
-    lrs = _lrs(eng_mod, first_step, n_steps)
-    tri = torch.from_numpy(kg.triples[:n_steps * B].copy())
-    a = _engine(eng_mod, monkeypatch, kg, dict(env, HOLE_PLAN_RAMP="1,2"))
-    sums, loss = a.train_steps(tri, B, seed, first_step, MARGIN, lrs, want_loss=True)
-    b = _engine(eng_mod, monkeypatch, kg, env)
-    ref = _per_step(b, tri.to(b.device), B, seed, first_step, lrs, check_at=boundary_steps(layout))
-    _assert_matches_per_step(f"K1 block {k1_block}", a.table, b.table, sums, ref, B, loss)
     a.close(); b.close()

@@ -23,7 +23,6 @@ from graphembeddings_b200 import data as D
 from oracle import hole_oracle as O
 
 SMEM = 227 * 1024                 # opt-in shared memory per block
-K1_STAGES = 3                     # csrc/hole_train.cu
 EVEN_DIMS = range(2, 772, 2)      # 770 is the first dim the library refuses
 
 
@@ -76,13 +75,6 @@ def cc_nv(dim):
     return need, next(n for n in (1, 2, 3, 4, 6, 8, 12, need) if n >= need)
 
 
-def logloss_supported(dim):
-    """hole_train_step_logloss (csrc/hole_train.cu): the first-generation body's landing buffers,
-    k1_smem = (256 / gs) * (3 K1_STAGES + 1) * row_stride * 4 bytes, must fit 227 KB."""
-    lg = lane_group(dim)
-    return lg is not None and (256 // lg[0]) * (3 * K1_STAGES + 1) * row_stride(dim) * 4 <= SMEM
-
-
 def row_passes(n_rows):
     """hole_ctx_create (csrc/hole_train.cu): smallest p with 2^(8p) - 1 >= n_rows (the absent key sorts
     last).  Also the relation-sort passes without a hole_ctx_set_relations hint."""
@@ -132,13 +124,11 @@ def test_dispatch_mirror():
         (2, 64, (1, 1)), (66, 128, (2, 2)), (130, 192, (3, 3)), (194, 256, (4, 4)), (258, 320, (5, 6)),
         (322, 384, (6, 6)), (386, 448, (7, 8)), (450, 512, (8, 8)), (514, 576, (9, 12)), (578, 640, (10, 12)),
         (642, 704, (11, 12)), (706, 768, (12, 12)), (770, 770, (13, 13))]
-    assert regimes(logloss_supported) == [(2, 720, True), (722, 770, False)]
     assert last_kb_mmas(514) == 1 and last_kb_mmas(640) == 4 and last_kb_mmas(2) == 1
     # the edges the refusal tests below use, found from the mirror
     assert first_dim(lambda d: lane_group(d) is None) == 770
     assert first_dim(lambda d: rank_stages(d, 1) is None) == 642
     assert first_dim(lambda d: rank_stages(d, 2) is None) == 322
-    assert first_dim(lambda d: not logloss_supported(d)) == 722
     # table-size edges
     assert [row_passes(n) for n in (43, 255, 256, 65535, 65536, 2**24 - 1, 2**24)] == [1, 1, 2, 2, 3, 3, 4]
     assert [route_passes(n) for n in (1005, 256, 257, 2**24, 2**24 + 1, 3 * 2**24 + 5, 2**31)] == [2, 1, 2, 3, 4, 4, 4]
@@ -176,8 +166,7 @@ def test_parity_tests_reach_every_regime():
     assert {cc_nv(d)[0] for d in _dims_of(CC.test_ccorr_score_matches_oracle)} >= {5, 8, 9, 12}   # rounded up and exact
     assert {cc_nv(d)[1] for d in _dims_of(CC.test_ccorr_ranking_matches_fp64_oracle)} >= {6}
     assert {cc_nv(d)[1] for d in _dims_of(test_ccorr_rank_counts_exact_vs_own_operands)} == {8, 12}
-    ll = _dims_of(TR.test_logloss_step_matches_oracle)
-    assert max(ll) == max(d for d in EVEN_DIMS if logloss_supported(d)) and 66 in ll
+    assert {lane_group(d) for d in _dims_of(TR.test_logloss_step_matches_oracle)} == all_lane_groups
 
 
 # ---------------------------------------------------------------- GPU helpers
@@ -292,28 +281,6 @@ def test_bf16_refusal_then_scoring_and_training_on_the_same_context(eng_mod):
     want = O.evaluate_triples(kg.E.astype(np.float64), kg.triples, np.float64)
     assert np.abs(got - want).max() <= 1e-6
     _check_one_step(e, kg, 1024, side=1)
-    e.close()
-
-
-@pytest.mark.gpu
-def test_logloss_refusal_is_clean_and_the_hinge_step_still_works(eng_mod):
-    """First dim the --log_loss kernel does not build (722): HoleError before any kernel (no plan is built into
-    slot 0), table and delta workspace untouched; a hinge step on the same context then matches the oracle."""
-    dim = first_dim(lambda d: not logloss_supported(d))
-    assert lane_group(dim) is not None
-    kg = D.synthetic_kg(7, 500, 1024, 5, dim, seed=dim, trained_scale=True, zipf_entities=True)
-    e = _engine(eng_mod, kg)
-    table0 = e.table.clone()
-    e._delta_ws = torch.zeros_like(e.table)
-    ws = e._delta_ws
-    n0 = e.launch_count()
-    with pytest.raises(eng_mod.HoleError, match=f"embedding_dim {dim}"):
-        e.train_step_logloss(kg.triples[:300], 5, 0, 0.1, 1e-3, 2, want_l2_loss=True)
-    torch.cuda.synchronize()
-    assert e.launch_count() == n0
-    assert torch.equal(e.table, table0)
-    assert e._delta_ws is ws and not ws.any()
-    _check_one_step(e, kg, 1024, side=0)
     e.close()
 
 

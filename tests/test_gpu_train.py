@@ -296,7 +296,8 @@ def test_sharded_trainer_single_rank_matches_engine(eng_mod):
 
 
 @pytest.mark.parametrize("dim,k,l2", [(150, 1, 0.0), (256, 3, 0.0), (64, 2, 1e-5), (600, 2, 0.0), (720, 2, 0.0),
-                                      (66, 1, 1e-5)])
+                                      (66, 1, 1e-5), (56, 1, 0.0), (128, 2, 1e-5), (258, 2, 0.0), (512, 1, 1e-5),
+                                      (768, 2, 0.0)])
 def test_logloss_step_matches_oracle(eng_mod, dim, k, l2):
     """--log_loss branch (holE.py:194-196, 206-220): k corrupt batches drawn with virtual steps
     step*k + j (bit-exact vs the oracle's Philox), softplus rows, sparse gradients taken at the
