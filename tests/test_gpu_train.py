@@ -412,12 +412,13 @@ class _VirtualRanks:
     """`world` ranks of the row-sharded step on ONE GPU: one engine (library context) per rank, every
     "peer" buffer a local tensor.  A step runs its compute half on every rank, then its apply half on
     every rank, all on one stream -- so every flag a kernel waits for has been set by an earlier
-    kernel of the stream."""
+    kernel of the stream.  csr: the (offsets, ids) type table corruption draws from (default: built from
+    kg.type_of).  Trailing ranks may own no rows (e.g. 20 entities over 16 ranks)."""
 
-    def __init__(self, eng_mod, kg, world, B):
+    def __init__(self, eng_mod, kg, world, B, csr=None):
         from graphembeddings_b200.sharded import row_partition
-        self.world, self.B, self.R = world, B, kg.n_relations
-        off, ids = D.build_type_csr(kg.type_of)
+        self.world, self.B, self.R, self.n_rows = world, B, kg.n_relations, kg.n_rows
+        off, ids = D.build_type_csr(kg.type_of) if csr is None else csr
         self.rows_per = row_partition(kg.n_entities, world)
         self.engs, self.bufs = [], []
         for k in range(world):
@@ -425,8 +426,7 @@ class _VirtualRanks:
             e.set_relation_count(kg.n_relations)
             dev, w, cap = e.device, e.row_stride, 3 * B
             shard = torch.zeros((self.R + self.rows_per, w), dtype=torch.float32, device=dev)
-            b0 = self.R + k * self.rows_per
-            b1 = min(kg.n_rows, b0 + self.rows_per)
+            b0, b1 = self._block(k)
             full = eng_mod.HoleEngine(kg.n_rows, kg.dim).set_embeddings(kg.E)
             shard[: self.R] = full.table[: self.R]
             shard[self.R: self.R + (b1 - b0)] = full.table[b0:b1]
@@ -444,6 +444,11 @@ class _VirtualRanks:
             e.shard_init(world, k, self.R, kg.n_entities, self.rows_per, B, self.bufs[k][0],
                          *[pa([self.bufs[j][i] for j in range(world)]) for i in range(6)], self.bufs[k][6], 5.0)
         self.kg = kg
+
+    def _block(self, k):
+        """[b0, b1): the global rows rank k owns (empty for a trailing rank past the last entity)."""
+        b0 = self.R + k * self.rows_per
+        return b0, max(b0, min(self.n_rows, b0 + self.rows_per))
 
     def step(self, slices, seed, step, margin, lr, ahead=None):
         losses = []
@@ -463,8 +468,7 @@ class _VirtualRanks:
         for k in range(self.world):
             assert torch.equal(self.bufs[k][0][: self.R], rel)
             assert not self.engs[k].shard_poll()
-            b0 = self.R + k * self.rows_per
-            b1 = min(kg.n_rows, b0 + self.rows_per)
+            b0, b1 = self._block(k)
             ents.append(self.bufs[k][0][self.R: self.R + (b1 - b0)])
         tab = torch.cat([rel] + ents)
         tmp = self.engs[0].__class__(kg.n_rows, kg.dim)
