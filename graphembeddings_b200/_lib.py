@@ -10,7 +10,7 @@ LIB_PATH = os.environ.get("HOLE_B200_LIB", os.path.join(_HERE, "libhole_b200.so"
 
 HOLE_SIDE_TAIL, HOLE_SIDE_HEAD, HOLE_SIDE_BOTH, HOLE_SIDE_RELATION = 0, 1, 2, 3
 HOLE_RANK_BF16, HOLE_RANK_BF16X3 = 0, 1
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 
 class HoleError(RuntimeError):
@@ -59,6 +59,7 @@ SIGNATURES = {
     "hole_rank_prepare": (_int, [_p, _p, _i64, _i64, _int, _p]),
     "hole_rank_invalidate": (_int, [_p]),
     "hole_topk": (_int, [_p, _p, _i64, _i64, _p, _i64, _int, _int, _int, _p, _p, _p, _p, _p]),
+    "hole_neighbors": (_int, [_p, _p, _i64, _i64, _p, _i64, _int, _int, _p, _p, _p, _p, _p]),
     "hole_rank_debug_operands": (_int, [_p, _p, _p, C.POINTER(_i64), C.POINTER(_i64), C.POINTER(_int), _p]),
     "hole_profile_enable": (_int, [_p, _int]),
     "hole_profile_read": (_int, [_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(_i64)]),

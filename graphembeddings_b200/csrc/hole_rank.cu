@@ -67,6 +67,7 @@ struct RankParams {
   const int64_t* f_off;        // [Q+1] filter CSR, or null
   const int32_t* f_ids;        //       ids ascending within a query's slice
   int64_t ent_begin;
+  const int32_t* tk_self;      // [Qpad] hole_neighbors: shard-local index each query never returns (itself); else null
 };
 
 // ------------------------------------------------------------------------------------ PTX
@@ -259,6 +260,7 @@ struct TopkList {
   int n, k;
   float thr;
   int64_t f0, f1;            // the query's filter slice [f0, f1) of f_ids
+  int self;                  // local index never admitted (hole_neighbors: the query's own row), -1 for none
 };
 
 __device__ __forceinline__ bool in_filter(const int32_t* __restrict__ ids, int64_t lo, int64_t hi, int32_t id) {
@@ -323,7 +325,7 @@ __device__ __forceinline__ void epi_topk_admit(const uint32_t (&v)[32], int j0, 
 #pragma unroll
     for (int i = 0; i < 32; ++i) s = (i == c) ? __uint_as_float(v[i]) : s;     // no dynamic register index
     const int j = j0 + c;
-    if (!(s < L.thr) || j >= Nc) continue;                                     // thr may have dropped
+    if (!(s < L.thr) || j >= Nc || j == L.self) continue;                      // thr may have dropped
     if (L.f0 < L.f1 && in_filter(f_ids, L.f0, L.f1, (int32_t)(ent_begin + j))) continue;
     topk_insert(L, topk_key(s, (uint32_t)j));
   }
@@ -366,7 +368,7 @@ struct SmemLayout {
 // producer / issue loops carry none of the split mode's bookkeeping); EPI = EPI_RANK / EPI_TOPK (compile-time,
 // so that the counting epilogue carries none of the top-k code).
 // p is __grid_constant__ so that its fields are read in place from parameter space where they are used.  Passed
-// by value, the struct (128 bytes) is loaded into registers at entry, and each top-k instantiation compiles to
+// by value, the struct (136 bytes) is loaded into registers at entry, and each top-k instantiation compiles to
 // 112 more instructions.
 template <int PARTS, int EPI>
 __global__ void __launch_bounds__(RANK_THREADS, 1)
@@ -502,6 +504,7 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       L.thr = qok ? INFINITY : -INFINITY;            // rows past Q admit nothing
       L.f0 = L.f1 = 0;
       if (qok && p.f_off != nullptr) { L.f0 = p.f_off[q]; L.f1 = p.f_off[q + 1]; }
+      L.self = (qok && p.tk_self != nullptr) ? p.tk_self[q] : -1;
       const int t0 = chunk * p.chunk_tiles;
       const int t1 = min(p.n_tiles, t0 + p.chunk_tiles);
       for (int t = t0; t < t1; ++t) {
@@ -576,10 +579,11 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 }
 
 // ------------------------------------------------------------------------------------ operand packing
-// One warp per row.  Candidate operand: clip(E_j) rounded to bf16, [Re | Im | 0-pad] of K columns.
+// One warp per row.  Candidate operand: clip(E_j) rounded to bf16, [Re | Im | 0-pad] of K columns; with
+// `normalize` (hole_neighbors) E_j / |E_j| instead, and zero for a zero row.
 __global__ void __launch_bounds__(256)
 hole_rank_pack_cand_kernel(const float* __restrict__ table, int stride, int H, int64_t ent_begin,
-                           int Nc, int Npad, int K, int parts, __nv_bfloat16* __restrict__ out) {
+                           int Nc, int Npad, int K, int parts, int normalize, __nv_bfloat16* __restrict__ out) {
   const int lane = threadIdx.x & 31;
   const int64_t r = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
   if (r >= Npad) return;
@@ -594,7 +598,7 @@ hole_rank_pack_cand_kernel(const float* __restrict__ table, int stride, int H, i
   for (int k = lane; k < H; k += 32) { float a = x[k], b = x[Hp + k]; ss = fmaf(a, a, fmaf(b, b, ss)); }
 #pragma unroll
   for (int o2 = 16; o2 > 0; o2 >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o2);
-  const float sc = fminf(__frsqrt_rn(ss), 1.0f);
+  const float sc = normalize ? (ss > 0.f ? __frsqrt_rn(ss) : 0.f) : fminf(__frsqrt_rn(ss), 1.0f);
   for (int k = lane; k < K; k += 32) {
     float v = 0.f;
     if (k < H) v = x[k] * sc;
@@ -805,6 +809,46 @@ hole_rank_pack_query_ccorr_kernel(const float* __restrict__ table, int stride, i
   if (lane == 0) true_idx[qi] = (int32_t)((int64_t)(side == HOLE_SIDE_TAIL ? t : (rel ? r : h)) - ent_begin);
 }
 
+// Query operand of hole_neighbors: -E_q / |E_q| (zero for a zero row) of the row ids[q], negated so that the
+// ascending top-k epilogue selects the most similar candidates.  The norm is reduced in the candidate packer's
+// order, so a row and its own candidate row are exact negatives of each other.  Also writes the fp32 vector
+// before rounding (qf, [Re | Im] of K floats) and the shard-local index of the row itself, which the epilogue
+// never admits.  One warp per query.
+__global__ void __launch_bounds__(256)
+hole_neighbors_pack_query_kernel(const float* __restrict__ table, int stride, int H, const int32_t* __restrict__ ids,
+                                 int Q, int Qpad, int64_t ent_begin, int K, int parts,
+                                 __nv_bfloat16* __restrict__ out, int32_t* __restrict__ true_idx,
+                                 float* __restrict__ qf) {
+  const int lane = threadIdx.x & 31;
+  const int64_t qi = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+  if (qi >= Qpad) return;
+  __nv_bfloat16* o = out + (size_t)qi * K * parts;       // row = [hi part (K) | lo part (K)]
+  if (qi >= Q) {
+    for (int k = lane; k < K * parts; k += 32) o[k] = __float2bfloat16(0.f);
+    if (lane == 0) true_idx[qi] = -1;
+    return;
+  }
+  const int id = ids[qi];
+  const float* x = table + (size_t)id * stride;
+  const int Hp = stride / 2;
+  float ss = 0.f;
+  for (int k = lane; k < H; k += 32) { float a = x[k], b = x[Hp + k]; ss = fmaf(a, a, fmaf(b, b, ss)); }
+#pragma unroll
+  for (int o2 = 16; o2 > 0; o2 >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o2);
+  const float sc = ss > 0.f ? -__frsqrt_rn(ss) : 0.f;
+  float* qrow = qf + (size_t)qi * K;
+  for (int k = lane; k < K; k += 32) {
+    float v = 0.f;
+    if (k < H) v = x[k] * sc;
+    else if (k < 2 * H) v = x[Hp + (k - H)] * sc;
+    if (k < 2 * H) qrow[k] = v;
+    const __nv_bfloat16 hi = __float2bfloat16(v);
+    o[k] = hi;
+    if (parts == 2) o[K + k] = __float2bfloat16(v - __bfloat162float(hi));
+  }
+  if (lane == 0) true_idx[qi] = (int32_t)((int64_t)id - ent_begin);
+}
+
 // T[q] = packed candidate row of q's true candidate (zeros when it is not in this shard).
 // Eight lanes per row, four rows per warp: the kernel is two dependent loads deep, so rows in
 // flight per SM are what sets its speed.
@@ -867,11 +911,13 @@ hole_rank_filter_kernel(const __nv_bfloat16* __restrict__ qp, const __nv_bfloat1
 //     (real keys are unique -- each candidate lives in one list -- so only TOPK_EMPTY repeats);
 //  2. each selected candidate is rescored in fp32: the clipped fp32 table row times the fp32 query vector qf;
 //  3. the row is sorted by (fp32 score, id); slots without a candidate get id -1 and score +inf.
+// neighbors (hole_neighbors): the candidate row is unit-normalised instead of clipped, the score written is the
+// similarity -s, and empty slots get -inf.
 constexpr int TOPK_MAX = 128;
 constexpr int MERGE_THREADS = 256;
 __global__ void __launch_bounds__(MERGE_THREADS)
 hole_topk_merge_kernel(const uint64_t* __restrict__ keys, int n_lists, int k, const float* __restrict__ table,
-                       int stride, int H, int64_t ent_begin, const float* __restrict__ qf, int K,
+                       int stride, int H, int64_t ent_begin, const float* __restrict__ qf, int K, int neighbors,
                        int32_t* __restrict__ ids_out, float* __restrict__ scores_out) {
   __shared__ uint32_t hist[256];
   __shared__ uint64_t sel[TOPK_MAX];
@@ -882,8 +928,9 @@ hole_topk_merge_kernel(const uint64_t* __restrict__ keys, int n_lists, int k, co
   const int64_t q = blockIdx.x;
   int32_t* ido = ids_out + q * k;
   float* sco = scores_out + q * k;
+  const float pad = neighbors ? -INFINITY : INFINITY;
   if (n_lists == 0) {                                  // empty candidate range
-    for (int i = tid; i < k; i += MERGE_THREADS) { ido[i] = -1; sco[i] = INFINITY; }
+    for (int i = tid; i < k; i += MERGE_THREADS) { ido[i] = -1; sco[i] = pad; }
     return;
   }
   const int64_t L = (int64_t)n_lists * k;              // >= 2k: the k-th smallest key exists
@@ -944,7 +991,7 @@ hole_topk_merge_kernel(const uint64_t* __restrict__ keys, int n_lists, int k, co
     for (int c = lane; c < H; c += 32) { const float a = row[c], b = row[Hp + c]; ss = fmaf(a, a, fmaf(b, b, ss)); }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
-    const float scl = fminf(__frsqrt_rn(ss), 1.0f);
+    const float scl = neighbors ? (ss > 0.f ? __frsqrt_rn(ss) : 0.f) : fminf(__frsqrt_rn(ss), 1.0f);
     float d = 0.f;
     for (int c = lane; c < H; c += 32) d = fmaf(row[c] * scl, qrow[c], fmaf(row[Hp + c] * scl, qrow[H + c], d));
 #pragma unroll
@@ -960,8 +1007,12 @@ hole_topk_merge_kernel(const uint64_t* __restrict__ keys, int n_lists, int k, co
   if (tid < k) {
     int r = 0;
     for (int i = 0; i < k; ++i) { const uint64_t o = sel[i]; r += (o < mine || (o == mine && i < tid)) ? 1 : 0; }
-    if (mine == TOPK_EMPTY) { ido[r] = -1; sco[r] = INFINITY; }
-    else { ido[r] = (int32_t)(ent_begin + (uint32_t)mine); sco[r] = f32_from_order_bits((uint32_t)(mine >> 32)); }
+    if (mine == TOPK_EMPTY) { ido[r] = -1; sco[r] = pad; }
+    else {
+      const float s = f32_from_order_bits((uint32_t)(mine >> 32));
+      ido[r] = (int32_t)(ent_begin + (uint32_t)mine);
+      sco[r] = neighbors ? 0.f - s : s;                // 0 - s: a zero similarity is +0
+    }
   }
 }
 
@@ -1005,7 +1056,7 @@ struct hole_rank_ws {
   __nv_bfloat16* qp = nullptr;     // [Qpad, K]
   __nv_bfloat16* tq = nullptr;     // [Qpad + BN, K] gathered true rows
   int32_t* true_idx = nullptr;     // [Qpad]
-  size_t cand_cap = 0, q_cap = 0;  // elements
+  size_t cand_cap = 0, q_cap = 0, tq_cap = 0;  // elements
   float* qf = nullptr;             // hole_topk: [Qpad, K] fp32 query vectors
   uint64_t* tk_keys = nullptr;     // hole_topk: [Qpad][n_chunks][2][k] partial lists
   size_t qf_cap = 0, tk_cap = 0;   // elements
@@ -1043,10 +1094,14 @@ struct TopkArgs {
   int k;
   int32_t* ids_out;
   float* scores_out;
+  bool neighbors;      // hole_neighbors: `queries` is an id list [Q], cosine over unit-normalised operands
 };
 
 // prepare_only: pack (and keep) the candidate operand, nothing else
-// tk != null: hole_topk (the k best candidates per row instead of counts / true scores)
+// tk != null: hole_topk (the k best candidates per row instead of counts / true scores), or hole_neighbors.
+// hole_neighbors packs its own normalised candidate operand over the cache's buffer: it never reads the
+// cache and always drops it, so a clipped operand never meets a cosine query and a normalised one never
+// serves a ranking call.
 static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t ent_end,
                      const float* query_table, const int32_t* queries, int64_t Q, int side, int precision,
                      const int64_t* filter_off, const int32_t* filter_ids, float* true_score_io,
@@ -1056,13 +1111,14 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
   HOLE_CHECK_ARG(side == HOLE_SIDE_TAIL || side == HOLE_SIDE_HEAD || side == HOLE_SIDE_BOTH ||
                  side == HOLE_SIDE_RELATION);
   const bool topk = tk != nullptr;
+  const bool nb = topk && tk->neighbors;
   if (topk && Q > 0 && ent_end == ent_begin) {       // no candidates: every output row is padding
     HOLE_CHECK_ARG(queries != nullptr);
     HOLE_CUDA_TRY(cudaSetDevice(c->device));
     const int64_t rows = (side == HOLE_SIDE_BOTH) ? 2 * Q : Q;
     HOLE_CHECK_ARG(rows < (int64_t(1) << 30));
     hole_topk_merge_kernel<<<(unsigned)rows, MERGE_THREADS, 0, (cudaStream_t)stream>>>(
-        nullptr, 0, tk->k, nullptr, 0, 0, 0, nullptr, 0, tk->ids_out, tk->scores_out);
+        nullptr, 0, tk->k, nullptr, 0, 0, 0, nullptr, 0, nb ? 1 : 0, tk->ids_out, tk->scores_out);
     HOLE_LAUNCHED();
     return HOLE_OK;
   }
@@ -1107,15 +1163,24 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
   }
   if ((size_t)Qpad * Kall > w->q_cap) {
     HOLE_CUDA_TRY(cudaStreamSynchronize(st));
-    cudaFree(w->qp); cudaFree(w->tq); cudaFree(w->true_idx);
-    w->qp = w->tq = nullptr; w->true_idx = nullptr; w->q_cap = 0;
+    cudaFree(w->qp); cudaFree(w->true_idx);
+    w->qp = nullptr; w->true_idx = nullptr; w->q_cap = 0;
     if (cudaMalloc((void**)&w->qp, (size_t)Qpad * Kall * 2) != cudaSuccess ||
-        cudaMalloc((void**)&w->tq, (size_t)(Qpad + BN) * Kall * 2) != cudaSuccess ||
         cudaMalloc((void**)&w->true_idx, (size_t)Qpad * 4) != cudaSuccess) {
       cudaGetLastError();
       return hole_set_error(HOLE_ERR_ALLOC, "ranking query operand allocation failed");
     }
     w->q_cap = (size_t)Qpad * Kall;
+  }
+  // the gathered true rows serve only the diagonal pass: top-k and neighbour calls do not allocate them
+  if (compute_true && (size_t)(Qpad + BN) * Kall > w->tq_cap) {
+    HOLE_CUDA_TRY(cudaStreamSynchronize(st));
+    cudaFree(w->tq); w->tq = nullptr; w->tq_cap = 0;
+    if (cudaMalloc((void**)&w->tq, (size_t)(Qpad + BN) * Kall * 2) != cudaSuccess) {
+      cudaGetLastError();
+      return hole_set_error(HOLE_ERR_ALLOC, "ranking true-row allocation failed");
+    }
+    w->tq_cap = (size_t)(Qpad + BN) * Kall;
   }
   RankParams p{};
   p.m_tiles = Qpad / BM;
@@ -1147,11 +1212,12 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
 
   w->last_npad = Npad; w->last_K = Kall;
   // operands: the candidate operand is reused when hole_rank_prepare packed exactly this table / range
-  const bool cached = w->cache_valid && w->cache_table == table && w->cache_begin == ent_begin &&
+  const bool cached = !nb && w->cache_valid && w->cache_table == table && w->cache_begin == ent_begin &&
                       w->cache_end == ent_end && w->cache_parts == parts;
   if (!cached) {
     w->cache_valid = false;
-    hole_rank_pack_cand_kernel<<<(unsigned)((Npad + 7) / 8), 256, 0, st>>>(table, c->row_stride, c->H, ent_begin, Nc, Npad, K, parts, w->cand);
+    hole_rank_pack_cand_kernel<<<(unsigned)((Npad + 7) / 8), 256, 0, st>>>(table, c->row_stride, c->H, ent_begin, Nc, Npad, K, parts,
+                                                                           nb ? 1 : 0, w->cand);
     HOLE_LAUNCHED();
   }
   if (prepare_only) {
@@ -1160,7 +1226,13 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
     return HOLE_OK;
   }
   w->last_qpad = Qpad;
-  if (c->score_mode == HOLE_SCORE_CCORR_TANH) {
+  if (nb) {
+    // cosine does not depend on the score mode: one query packer for both
+    hole_neighbors_pack_query_kernel<<<(unsigned)((Qpad + 7) / 8), 256, 0, st>>>(table, c->row_stride, c->H, queries,
+                                                                                 (int)Q, Qpad, ent_begin, K, parts,
+                                                                                 w->qp, w->true_idx, w->qf);
+    HOLE_LAUNCHED();
+  } else if (c->score_mode == HOLE_SCORE_CCORR_TANH) {
     // archived score variant: another query vector, the same contraction (see the kernel's comment)
     const int nv = (c->row_stride / 2 + 31) / 32;
     const int warps = std::max(1, std::min(8, (200 * 1024) / (6 * c->H * (int)sizeof(float))));
@@ -1220,13 +1292,14 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
     p.f_off = filter_off;
     p.f_ids = filter_ids;
     p.ent_begin = ent_begin;
+    p.tk_self = nb ? w->true_idx : nullptr;
     const int grid = std::min(p.m_tiles * p.n_chunks, c->sm_count);
     if (parts == 2) hole_rank_kernel<2, EPI_TOPK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
     else hole_rank_kernel<1, EPI_TOPK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
     HOLE_LAUNCHED();
     hole_topk_merge_kernel<<<(unsigned)Q, MERGE_THREADS, 0, st>>>(w->tk_keys, p.n_chunks * 2, tk->k, table,
                                                                   c->row_stride, c->H, ent_begin, w->qf, K,
-                                                                  tk->ids_out, tk->scores_out);
+                                                                  nb ? 1 : 0, tk->ids_out, tk->scores_out);
     HOLE_LAUNCHED();
     return HOLE_OK;
   }
@@ -1288,8 +1361,18 @@ extern "C" int hole_topk(hole_ctx* c, const float* table, int64_t ent_begin, int
                          const int64_t* filter_off, const int32_t* filter_ids,
                          int32_t* ids_out, float* scores_out, void* stream) {
   HOLE_CHECK_ARG(c && k >= 1 && k <= TOPK_MAX && ids_out != nullptr && scores_out != nullptr);
-  const TopkArgs tk{k, ids_out, scores_out};
+  const TopkArgs tk{k, ids_out, scores_out, false};
   return rank_impl(c, table, ent_begin, ent_end, nullptr, queries, Q, side, precision, filter_off, filter_ids,
+                   nullptr, 0, nullptr, nullptr, stream, false, &tk);
+}
+
+extern "C" int hole_neighbors(hole_ctx* c, const float* table, int64_t ent_begin, int64_t ent_end,
+                              const int32_t* ids, int64_t Q, int precision, int k,
+                              const int64_t* filter_off, const int32_t* filter_ids,
+                              int32_t* ids_out, float* sim_out, void* stream) {
+  HOLE_CHECK_ARG(c && k >= 1 && k <= TOPK_MAX && ids_out != nullptr && sim_out != nullptr);
+  const TopkArgs tk{k, ids_out, sim_out, true};
+  return rank_impl(c, table, ent_begin, ent_end, nullptr, ids, Q, HOLE_SIDE_TAIL, precision, filter_off, filter_ids,
                    nullptr, 0, nullptr, nullptr, stream, false, &tk);
 }
 

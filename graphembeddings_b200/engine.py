@@ -358,26 +358,50 @@ class HoleEngine:
         HOLE_SIDE_RELATION predicts the relations of (h, ?, t) over relation rows [ent_begin, ent_end)."""
         q = self._triples(queries)
         rows = q.shape[0] * (2 if int(side) == HOLE_SIDE_BOTH else 1)
-        fo = fi = None
-        if filter_off is not None:
-            off = np.asarray(filter_off.cpu() if isinstance(filter_off, torch.Tensor) else filter_off, dtype=np.int64)
-            ids = np.asarray(filter_ids.cpu() if isinstance(filter_ids, torch.Tensor) else filter_ids, dtype=np.int64)
-            if off.shape != (rows + 1,) or off[0] != 0 or off[-1] != len(ids) or np.any(np.diff(off) < 0):
-                raise HoleError(f"filter_off must be a CSR offset array of {rows + 1} entries over {len(ids)} ids")
-            desc = np.diff(ids) < 0                    # descending step inside one slice
-            starts = off[1:-1]
-            desc[starts[(starts > 0) & (starts < len(ids))] - 1] = False
-            if desc.any():
-                raise HoleError("filter ids must be ascending within each query's slice")
-            if len(ids) > 0:                           # no ids: nothing to filter (and no device pointer)
-                fo = torch.as_tensor(off).to(self.device).contiguous()
-                fi = torch.as_tensor(ids.astype(np.int32)).to(self.device).contiguous()
+        fo, fi = self._filter_csr(filter_off, filter_ids, rows)
         ids_out = torch.empty((rows, int(k)), dtype=torch.int32, device=self.device)
         scores = torch.empty((rows, int(k)), dtype=torch.float32, device=self.device)
         check(self.lib.hole_topk(self._ctx, _ptr(self.table), int(ent_begin), int(ent_end), _ptr(q), q.shape[0],
                                  int(side), int(precision), int(k), _ptr(fo), _ptr(fi), _ptr(ids_out), _ptr(scores),
                                  _stream()))
         return ids_out, scores
+
+    def neighbors(self, ids, k, ent_begin, ent_end, filter_off=None, filter_ids=None, precision=HOLE_RANK_BF16X3):
+        """Nearest neighbours by cosine similarity of the whole stored rows: for every row ids[q], the k rows of
+        [ent_begin, ent_end) most similar to it, itself excluded, skipping its filter slice (ascending ids).
+        Returns (ids int32[Q, k], sims float32[Q, k]) on the device, by descending similarity with ties to the
+        smaller id; padding is id -1 / similarity -inf.  Independent of the score mode."""
+        q = torch.as_tensor(ids).reshape(-1)
+        if q.numel() and (int(q.min()) < 0 or int(q.max()) >= self.n_rows):
+            raise HoleError(f"neighbour query ids must lie in [0, {self.n_rows})")
+        q = q.to(torch.int32).to(self.device).contiguous()
+        rows = q.shape[0]
+        fo, fi = self._filter_csr(filter_off, filter_ids, rows)
+        ids_out = torch.empty((rows, int(k)), dtype=torch.int32, device=self.device)
+        sims = torch.empty((rows, int(k)), dtype=torch.float32, device=self.device)
+        check(self.lib.hole_neighbors(self._ctx, _ptr(self.table), int(ent_begin), int(ent_end), _ptr(q), rows,
+                                      int(precision), int(k), _ptr(fo), _ptr(fi), _ptr(ids_out), _ptr(sims),
+                                      _stream()))
+        return ids_out, sims
+
+    def _filter_csr(self, filter_off, filter_ids, rows):
+        """Checks a filter CSR of `rows` slices (ascending ids within each) and returns it as device tensors
+        (int64 offsets, int32 ids), or (None, None) for no filter or one without ids."""
+        if filter_off is None:
+            return None, None
+        off = np.asarray(filter_off.cpu() if isinstance(filter_off, torch.Tensor) else filter_off, dtype=np.int64)
+        ids = np.asarray(filter_ids.cpu() if isinstance(filter_ids, torch.Tensor) else filter_ids, dtype=np.int64)
+        if off.shape != (rows + 1,) or off[0] != 0 or off[-1] != len(ids) or np.any(np.diff(off) < 0):
+            raise HoleError(f"filter_off must be a CSR offset array of {rows + 1} entries over {len(ids)} ids")
+        desc = np.diff(ids) < 0                    # descending step inside one slice
+        starts = off[1:-1]
+        desc[starts[(starts > 0) & (starts < len(ids))] - 1] = False
+        if desc.any():
+            raise HoleError("filter ids must be ascending within each query's slice")
+        if len(ids) == 0:                          # no ids: nothing to filter (and no device pointer)
+            return None, None
+        return (torch.as_tensor(off).to(self.device).contiguous(),
+                torch.as_tensor(ids.astype(np.int32)).to(self.device).contiguous())
 
     def rank_prepare(self, ent_begin, ent_end, precision=HOLE_RANK_BF16):
         """Pack the candidate operand of [ent_begin, ent_end) once; later rank() calls on the same table /

@@ -512,6 +512,36 @@ def predict_top_k(eng, test, known, relation_count, entity_count, k, path, preci
     return n
 
 
+def write_nearest_neighbors(eng, test, relation_count, entity_count, k, path, id_to_metadata,
+                            precision=HOLE_RANK_BF16X3, chunk=65536):
+    """The k most similar rows (cosine of the whole embedding, HoleEngine.neighbors) of every distinct entity of
+    the test file among the entity rows [relation_count, entity_count), and of every distinct relation of the test
+    file among the relation rows [0, relation_count).  Writes one line per neighbour to `path`:
+    kind  row  neighbour  position  similarity  row_metadata  neighbour_metadata
+    (kind = entity / relation, position 1-based, metadata = entity_metadata.tsv's "id name").  Queries go to the
+    device `chunk` rows at a time, which bounds the workspace.  Returns the number of lines written."""
+    test = np.asarray(test, dtype=np.int64).reshape(-1, 3)
+    groups = (("entity", np.unique(test[:, :2]), relation_count, entity_count),
+              ("relation", np.unique(test[:, 2]), 0, relation_count))
+    n = 0
+    with open(path, 'w') as out:
+        for kind, rows, lo, hi in groups:
+            for c0 in range(0, len(rows), chunk):
+                part = rows[c0:c0 + chunk]
+                ids, sims = eng.neighbors(part, k, lo, hi, precision=precision)
+                ids, sims = ids.cpu().numpy(), sims.cpu().numpy()
+                for i, row in enumerate(part.tolist()):
+                    for pos in range(k):
+                        c = int(ids[i, pos])
+                        if c < 0:
+                            break
+                        out.write('{}\t{}\t{}\t{}\t{:.9g}\t{}\t{}\n'.format(
+                            kind, row, c, pos + 1, sims[i, pos], id_to_metadata.get(row, ''),
+                            id_to_metadata.get(c, '')))
+                        n += 1
+    return n
+
+
 def infer_triples(flags=None, log=print):
     """holE.py:530-582 with the all-entity filtered protocol."""
     flags = flags or FLAGS
@@ -539,6 +569,12 @@ def infer_triples(flags=None, log=print):
         n = predict_top_k(eng, data.test, data.known, data.relation_count, data.entity_count, k, path,
                           precision=precision, value=value, sides=sides)
         log('Wrote {} predictions to {}'.format(n, path))
+    nn_k = getattr(flags, 'nearest_neighbors', 0)
+    if nn_k:
+        path = os.path.join(flags.output_dir, 'neighbors.tsv')
+        n = write_nearest_neighbors(eng, data.test, data.relation_count, data.entity_count, nn_k, path,
+                                    data.id_to_metadata, precision=precision)
+        log('Wrote {} nearest-neighbour lines to {}'.format(n, path))
     if not raw:
         log('No test triple passed the confidence gate; no ranks recorded.')
         result = None
@@ -594,6 +630,10 @@ def build_parser():
                              '--predict_top_k, also write the K best new relations of every (head, tail) pair of the '
                              'test file to predictions.tsv.  Writes nothing to inference_results.tsv; --infer_gate '
                              'does not apply to it.')
+    parser.add_argument('--nearest_neighbors', type=int, default=0,
+                        help='With --infer: write the K entity rows most similar (cosine of the embeddings) to every '
+                             'entity of the test file, and the K relation rows most similar to every relation of it, '
+                             'to <output_dir>/neighbors.tsv (0 = off; K <= 128).')
     parser.add_argument('--valid_sample', action='store_true',
                         help='Validate on one sampled batch as holE.py does (default: the whole triples-valid.txt).')
     parser.add_argument('--score_variant', choices=['complex', 'ccorr_tanh'], default='complex',

@@ -58,7 +58,7 @@ typedef struct hole_ctx hole_ctx;
 #define HOLE_RANK_BF16X3 1       /* split-bf16 (hi*hi + lo*hi + hi*lo): ranks match fp32 except within ~3e-5 of a tie; dim <= 320 */
 
 /* ABI version of this header; hole_abi_version() returns the library's. */
-#define HOLE_ABI_VERSION 4
+#define HOLE_ABI_VERSION 5
 HOLE_API int hole_abi_version(void);
 
 /* Thread-local message of the last failing call on this thread ("" if none). */
@@ -347,6 +347,35 @@ HOLE_API int hole_topk(hole_ctx* ctx, const float* table, int64_t ent_begin, int
                        const int32_t* queries, int64_t Q, int side, int precision, int k,
                        const int64_t* filter_off, const int32_t* filter_ids,
                        int32_t* ids_out, float* scores_out, void* stream);
+
+/* ---- nearest neighbours: the rows of [ent_begin, ent_end) whose embeddings are most similar to row ids[q]
+ * (what holE.py leaves to the TensorBoard projector it configures, holE.py:334-337), on hole_topk's tensor-core
+ * contraction, top-k epilogue and merge.  Similarity is the cosine over the whole stored row as one real vector
+ * of dim components, cos(q, j) = E_q . E_j / (|E_q| |E_j|) = Re sum_k q_k conj(j_k); neither the norm clip nor
+ * the score mode enters it (HOLE_SCORE_COMPLEX and HOLE_SCORE_CCORR_TANH give the same result).  A row of zero
+ * norm has similarity exactly 0 with every row, as query and as candidate.
+ *   ids        int32 [Q]     query rows; the caller guarantees 0 <= ids[q] < n_rows (they may lie outside the range,
+ *                            e.g. an entity queried against the relation rows [0, n_relations))
+ *   ids_out    int32 [Q, k]  global row ids, by descending similarity, ties to the smaller id
+ *   sim_out    float32 [Q, k] their similarities, recomputed in fp32 from the fp32 table
+ * Row ids[q] itself is never returned; other rows with an identical embedding are.  The ids of q's filter slice
+ * (filter_off int64[Q+1] / filter_ids int32[.], may be NULL, ids ASCENDING within a slice) are skipped.  Fewer
+ * than k candidates left: the row is padded with id -1, similarity -inf.
+ * Precision, limits and errors as hole_topk: the id set is exact except within the precision's near-tie band of
+ * the k-th similarity (3e-5 for HOLE_RANK_BF16X3, 4e-3 for HOLE_RANK_BF16: both operands have unit norm);
+ * 1 <= k <= 128, else HOLE_ERR_ARG; dim <= 640 (bf16) / 320 (bf16x3), else HOLE_ERR_UNSUPPORTED before any launch
+ * or write -- except that an empty range (ent_begin == ent_end), which has no candidate to score, writes its
+ * all-padding rows and returns HOLE_OK at any dim, as hole_topk does; HOLE_ERR_ALLOC when the workspace does not
+ * fit: split Q.
+ * Operand cache: the call packs its own (unit-normalised) candidate operand into the single cache slot and drops a
+ * hole_rank_prepare'd one, which a later hole_rank / hole_topk call therefore re-packs.  A prepared (clipped)
+ * operand is never used for cosine, and a normalised one never for ranking.  hole_rank_debug_operands returns
+ * the operands of the last hole_neighbors call as it does for hole_rank / hole_topk.
+ * Row-sharded tables: gather the whole table onto one GPU first (gather_embeddings() of the sharded trainer). */
+HOLE_API int hole_neighbors(hole_ctx* ctx, const float* table, int64_t ent_begin, int64_t ent_end,
+                            const int32_t* ids, int64_t Q, int precision, int k,
+                            const int64_t* filter_off, const int32_t* filter_ids,
+                            int32_t* ids_out, float* sim_out, void* stream);
 
 /* Test hook: copy the bf16 operands the last hole_rank call packed (device to device).
  * cand_out [n_pad, K] / query_out [q_pad, K] may be NULL to query the shapes only. */
