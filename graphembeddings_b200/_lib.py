@@ -10,7 +10,8 @@ LIB_PATH = os.environ.get("HOLE_B200_LIB", os.path.join(_HERE, "libhole_b200.so"
 
 HOLE_SIDE_TAIL, HOLE_SIDE_HEAD, HOLE_SIDE_BOTH, HOLE_SIDE_RELATION = 0, 1, 2, 3
 HOLE_RANK_BF16, HOLE_RANK_BF16X3 = 0, 1
-ABI_VERSION = 5
+HOLE_OPT_SGD, HOLE_OPT_ADAGRAD = 0, 1
+ABI_VERSION = 6
 
 
 class HoleError(RuntimeError):
@@ -28,6 +29,7 @@ SIGNATURES = {
     "hole_ctx_destroy": (_int, [_p]),
     "hole_ctx_set_relations": (_int, [_p, _i64]),
     "hole_ctx_set_score_mode": (_int, [_p, _int]),
+    "hole_ctx_set_optimizer": (_int, [_p, _int, _p]),
     "hole_pack_rows": (_int, [_p, _p, _p, _i64, _p]),
     "hole_unpack_rows": (_int, [_p, _p, _p, _i64, _p]),
     "hole_corrupt": (_int, [_p, _p, _i64, _p, _p, _p, _u64, _u64, _p, _p, C.POINTER(_int), _p]),

@@ -93,6 +93,8 @@ struct hole_ctx {
                        //   a plan's latency is ~120 us of dependent launches whatever its size)
   int score_mode = 0;  // HOLE_SCORE_COMPLEX (live holE.py) or HOLE_SCORE_CCORR_TANH (archived variant, hole_ccorr.cuh)
   bool cc_ready = false;   // shared-memory attributes of the ccorr kernels set
+  int optimizer = 0;   // HOLE_OPT_SGD or HOLE_OPT_ADAGRAD (hole_ctx_set_optimizer)
+  float* accum = nullptr;  // AdaGrad accumulator [n_rows, row_stride] (caller-owned, kept by reference)
   int sort_small = 1;          // plan: one-launch sort + segments while the steps seen so far were small enough
                                //   (HOLE_SORT_SMALL: 0 never, 1 adaptive, 2 always -- tests of its large-step path)
   int64_t dup_seen_B = -1;     //   batch size the observation below belongs to

@@ -25,6 +25,8 @@
 //     3 is a --log_loss pass (hole_train_step_logloss): the table is read only and every unique
 //     row's delta is ADDED to the delta table, which sums the passes over one old table.  The
 //     loss is the only other difference; `loss` is null on the passes without the positive term.
+//     4 is DM 0 with AdaGrad (hole_ctx_set_optimizer): a unique row also reads and writes its row
+//     of the accumulator (carried in Dtab), with plain vector loads where the row is applied.
 #pragma once
 
 constexpr int K1_THREADS = 256;  // threads per block; at dim 768 their landing rows take 221,376 B of 227 KB
@@ -69,7 +71,8 @@ struct hole_k1_args {
   float* G;                 // staged gradient rows (rows used more than once in the step)
   float* loss;              // [B]  (DM 3: log loss of the positives, null on the passes without them)
   float* sigma;             // [2B] or null  (DM 3: [B] log loss of the pass's negatives)
-  float* Dtab;              // DM 1/3: delta table; DM 2: local delta rows of the replicated relation block
+  float* Dtab;              // DM 1/3: delta table; DM 2: local delta rows of the replicated relation block;
+                            // DM 4: the AdaGrad accumulator [n_rows, stride]
 };
 
 // DM 2 (row-sharded step): where rows live and where their deltas go
@@ -128,13 +131,29 @@ __device__ __forceinline__ void k1_row_from_smem(Row<V>& x, const float4* ssrc, 
 //   unique row : DM 0  E[row] = x - lr dx   (skipped for an inactive hinge: dx == 0)
 //                DM 1/2  out[row] = -lr dx   (always written: the consumer adds every listed row)
 //                DM 3    out[row] += -lr dx
+//                DM 4    S[row] += dx^2,  E[row] = x - lr dx rsqrt(S[row])  (S: the accumulator row
+//                        s_row; skipped for an inactive hinge)
 //   otherwise  : G[gslot] = dx  for K3's ordered combine
 template <int GS, int V, bool FULL, int DM>
 __device__ __forceinline__ void k1_emit(const Row<V>& d, const Row<V>& x, float A, float Bc, bool uniq,
-                                        bool act, float lr, float* out_row, float* g_row, int lane, int nvec) {
+                                        bool act, float lr, float* out_row, float* g_row, int lane, int nvec,
+                                        float* s_row = nullptr) {
   Row<V> o;
   if (uniq) {
-    if (DM == 0) {
+    if constexpr (DM == 4) {
+      if (!act) return;
+      Row<V> acc;
+      row_load<GS, V, false>(acc, s_row, lane, nvec);
+#pragma unroll
+      for (int k = 0; k < 4 * V; ++k) {
+        const float gr = fmaf(A, d.re[k], -Bc * x.re[k]), gi = fmaf(A, d.im[k], -Bc * x.im[k]);
+        acc.re[k] = fmaf(gr, gr, acc.re[k]);
+        acc.im[k] = fmaf(gi, gi, acc.im[k]);
+        o.re[k] = fmaf(-lr * gr, __frsqrt_rn(acc.re[k]), x.re[k]);
+        o.im[k] = fmaf(-lr * gi, __frsqrt_rn(acc.im[k]), x.im[k]);
+      }
+      row_store<GS, V, FULL>(acc, s_row, lane, nvec);
+    } else if (DM == 0) {
       if (!act) return;
 #pragma unroll
       for (int k = 0; k < 4 * V; ++k) {
@@ -239,7 +258,7 @@ __device__ __forceinline__ void hole_k1_body(const hole_k1_args& a, const hole_k
       return static_cast<float*>(sh.stage.p[o]) +
              ((size_t)sh.me * (size_t)sh.cap + (size_t)(wrow - sh.R - s_cuts[o])) * stride;
     }
-    return (DM == 0 ? a.E : a.Dtab) + (size_t)id * stride;
+    return (DM == 0 || DM == 4 ? a.E : a.Dtab) + (size_t)id * stride;
   };
   auto fetch = [&](const K1Ids& d, int stage) {
     if (lane == 0) {
@@ -272,7 +291,7 @@ __device__ __forceinline__ void hole_k1_body(const hole_k1_args& a, const hole_k
   int r_cur = -1, run_i = 0;
   float inv_r = 0.f, sc_r = 1.f, proj_r = 0.f;
   bool run_act = false;
-  float* const rel_out = (DM == 0) ? a.E : a.Dtab;
+  float* const rel_out = (DM == 0 || DM == 4) ? a.E : a.Dtab;
 
   // end of a run of equal relation: clip backward of the summed gradient, then apply / stage
   auto flush_relation = [&]() {
@@ -280,7 +299,7 @@ __device__ __forceinline__ void hole_k1_body(const hole_k1_args& a, const hole_k
     const bool cl = inv_r <= 1.0f;
     k1_emit<GS, V, FULL, DM>(acc, xr, cl ? inv_r : 1.0f, cl ? sc_r * proj_r * inv_r : 0.0f,
                              sl == HOLE_SLOT_UNIQUE, run_act, a.lr, rel_out + (size_t)r_cur * stride,
-                             a.G + (size_t)sl * stride, lane, nvec);
+                             a.G + (size_t)sl * stride, lane, nvec, a.Dtab + (size_t)r_cur * stride);
   };
 
   int stage = 0;
@@ -292,6 +311,9 @@ __device__ __forceinline__ void hole_k1_body(const hole_k1_args& a, const hole_k
     if (g + 2 < g1) fetch(n2, (stage + 2) % K1V2_STAGES);         // rows two ahead
     const int i = c.i;
     const uint32_t sl_t = a.gslot[B + i], sl_h = a.gslot[2 * B + i], sl_n = a.gslot[3 * B + i];
+    float* const sr_h = DM == 4 ? a.Dtab + (size_t)c.h * stride : nullptr;     // DM 4: accumulator rows
+    float* const sr_t = DM == 4 ? a.Dtab + (size_t)c.t * stride : nullptr;
+    float* const sr_n = DM == 4 ? a.Dtab + (size_t)c.n * stride : nullptr;
     if (c.r != r_cur) {                      // group-uniform
       if (r_cur >= 0) flush_relation();
       // the relation row: once per run, straight from L2 (DM 2: my replica)
@@ -388,9 +410,11 @@ __device__ __forceinline__ void hole_k1_body(const hole_k1_args& a, const hole_k
     if (side == 0) {
       const float hr = sc_h * sc_r;
       k1_emit<GS, V, FULL, DM>(P, xt, gp * hr * (cl_t ? inv_t : 1.0f), cl_t ? sc_t * gs_p * inv_t : 0.0f,
-                               sl_t == HOLE_SLOT_UNIQUE, act, lr, dst_t, a.G + (size_t)sl_t * stride, lane, nvec);
+                               sl_t == HOLE_SLOT_UNIQUE, act, lr, dst_t, a.G + (size_t)sl_t * stride, lane, nvec,
+                               sr_t);
       k1_emit<GS, V, FULL, DM>(P, xn, gn * hr * (cl_n ? inv_n : 1.0f), cl_n ? sc_n * gs_n * inv_n : 0.0f,
-                               sl_n == HOLE_SLOT_UNIQUE, act, lr, dst_n, a.G + (size_t)sl_n * stride, lane, nvec);
+                               sl_n == HOLE_SLOT_UNIQUE, act, lr, dst_n, a.G + (size_t)sl_n * stride, lane, nvec,
+                               sr_n);
       const float bt = gp * sc_t, bn = gn * sc_n;
       Row<V> d;
 #pragma unroll
@@ -404,13 +428,16 @@ __device__ __forceinline__ void hole_k1_body(const hole_k1_args& a, const hole_k
         acc.im[k] += fmaf(ha, ws, -hb * us);
       }
       k1_emit<GS, V, FULL, DM>(d, xh, sc_r * (cl_h ? inv_h : 1.0f), cl_h ? sc_h * gs_b * inv_h : 0.0f,
-                               sl_h == HOLE_SLOT_UNIQUE, act, lr, dst_h, a.G + (size_t)sl_h * stride, lane, nvec);
+                               sl_h == HOLE_SLOT_UNIQUE, act, lr, dst_h, a.G + (size_t)sl_h * stride, lane, nvec,
+                               sr_h);
     } else {
       const float rt = sc_r * sc_t;
       k1_emit<GS, V, FULL, DM>(P, xh, gp * rt * (cl_h ? inv_h : 1.0f), cl_h ? sc_h * gs_p * inv_h : 0.0f,
-                               sl_h == HOLE_SLOT_UNIQUE, act, lr, dst_h, a.G + (size_t)sl_h * stride, lane, nvec);
+                               sl_h == HOLE_SLOT_UNIQUE, act, lr, dst_h, a.G + (size_t)sl_h * stride, lane, nvec,
+                               sr_h);
       k1_emit<GS, V, FULL, DM>(P, xn, gn * rt * (cl_n ? inv_n : 1.0f), cl_n ? sc_n * gs_n * inv_n : 0.0f,
-                               sl_n == HOLE_SLOT_UNIQUE, act, lr, dst_n, a.G + (size_t)sl_n * stride, lane, nvec);
+                               sl_n == HOLE_SLOT_UNIQUE, act, lr, dst_n, a.G + (size_t)sl_n * stride, lane, nvec,
+                               sr_n);
       const float bh = gp * sc_h, bn = gn * sc_n;
       Row<V> d;
 #pragma unroll
@@ -424,7 +451,8 @@ __device__ __forceinline__ void hole_k1_body(const hole_k1_args& a, const hole_k
         acc.im[k] += fmaf(us, tf, -ws * te);
       }
       k1_emit<GS, V, FULL, DM>(d, xt, sc_r * (cl_t ? inv_t : 1.0f), cl_t ? sc_t * gs_b * inv_t : 0.0f,
-                               sl_t == HOLE_SLOT_UNIQUE, act, lr, dst_t, a.G + (size_t)sl_t * stride, lane, nvec);
+                               sl_t == HOLE_SLOT_UNIQUE, act, lr, dst_t, a.G + (size_t)sl_t * stride, lane, nvec,
+                               sr_t);
     }
     c = n1;
     n1 = n2;
@@ -440,9 +468,10 @@ __device__ __forceinline__ void hole_k1_body(const hole_k1_args& a, const hole_k
 }
 
 // DM 3 at V 1 is held to two blocks per SM (128 registers, no spills), the occupancy DM 0 has there:
-// left free it takes 135 registers and one block per SM, and a log-loss step at d = 256 is 5-20 % slower
+// left free it takes 135 registers and one block per SM, and a log-loss step at d = 256 is 5-20 % slower.
+// DM 4 at V 1 likewise (128 registers, no spills; DESIGN §7c)
 template <int GS, int V, int DM>
-__global__ void __launch_bounds__(K1_THREADS, (DM == 3 && V == 1) ? 2 : 1)
+__global__ void __launch_bounds__(K1_THREADS, ((DM == 3 || DM == 4) && V == 1) ? 2 : 1)
 hole_k1_kernel(const hole_k1_args a, const hole_k1_shard sh) {
   // specialise on the corruption side and on "every lane owns valid float4s" (nvec == GS*V)
   const bool full = (a.nvec == GS * V);

@@ -232,6 +232,8 @@ extern "C" int hole_shard_init(hole_ctx* c, int world, int me, int64_t n_relatio
   HOLE_CHECK_ARG(err_flag && type_of && csr_off && csr_ids);
   if (c->score_mode != HOLE_SCORE_COMPLEX)
     return hole_set_error(HOLE_ERR_UNSUPPORTED, "the archived ccorr/tanh score mode has no row-sharded step");
+  int rc = optimizer_refusal(c, HOLE_STEP_SHARD);
+  if (rc) return rc;
   HOLE_CHECK_ARG(world >= 1 && world <= HOLE_MAX_RANKS && me >= 0 && me < world);
   HOLE_CHECK_ARG(n_relations >= 0 && n_entities > 0 && rows_per_rank > 0 && rows_per_rank * world >= n_entities);
   HOLE_CHECK_ARG(n_relations + rows_per_rank * world < (int64_t(1) << 31));
@@ -242,7 +244,7 @@ extern "C" int hole_shard_init(hole_ctx* c, int world, int me, int64_t n_relatio
   // that the side stream's routing / plan kernels of the next chunk run beside it, not after it
   int reserve = 12;
   if (const char* e = getenv("HOLE_SHARD_RESERVE_SMS")) reserve = atoi(e);
-  int rc = hole_ws_reserve(c, max_batch, SHARD_PREP_STEPS);
+  rc = hole_ws_reserve(c, max_batch, SHARD_PREP_STEPS);
   if (rc) return rc;
   if (world > 1 && reserve > 0 && reserve < c->sm_count / 2)
     c->k1_groups = c->k1_groups / c->sm_count * (c->sm_count - reserve);
@@ -331,6 +333,8 @@ static int shard_prepare(hole_ctx* c, const int32_t* pos, int64_t B, int64_t n_s
 
 static int shard_check_args(hole_ctx* c, const int32_t* pos, int64_t B) {
   HOLE_CHECK_ARG(c != nullptr);
+  int rc = optimizer_refusal(c, HOLE_STEP_SHARD);
+  if (rc) return rc;
   if (c->shard_state == nullptr) return hole_set_error(HOLE_ERR_ARG, "hole_shard_init has not been called");
   HOLE_CHECK_ARG(pos != nullptr && B > 0 && B <= c->shard_state->max_batch);
   return HOLE_OK;
@@ -431,6 +435,8 @@ extern "C" int hole_shard_step_compute(hole_ctx* c, const int32_t* pos, int64_t 
 // apply of the step: every peer's deltas -> my shard
 extern "C" int hole_shard_step_apply(hole_ctx* c, void* stream) {
   HOLE_CHECK_ARG(c != nullptr);
+  int rc = optimizer_refusal(c, HOLE_STEP_SHARD);
+  if (rc) return rc;
   if (c->shard_state == nullptr) return hole_set_error(HOLE_ERR_ARG, "hole_shard_init has not been called");
   HOLE_CUDA_TRY(cudaSetDevice(c->device));
   hole_shard_state* s = c->shard_state;

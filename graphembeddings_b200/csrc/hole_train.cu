@@ -979,7 +979,7 @@ hole_score_kernel(const float* __restrict__ E, const int32_t* __restrict__ tripl
 }
 
 // ---------------------------------------------------------------------------------------
-// K3: deterministic sparse SGD update for rows that occur more than once in the step.
+// K3: deterministic sparse SGD (or AdaGrad) update for rows that occur more than once in the step.
 // One group per sorted entry; only entries that head a chunk of C consecutive occurrences
 // of a row do work.  A row with n occurrences is reduced by a fixed C-ary tree over its
 // sorted occurrences (order: slot, then batch index); the last group to finish a node's
@@ -1018,11 +1018,13 @@ struct hole_k3_shard {
   hole_peer_ptrs stage;     // PEER: rank o's delta staging [world][cap][stride]
 };
 
-template <int GS, int V>
-__global__ void __launch_bounds__(256)
-hole_apply_kernel(float* __restrict__ E, float* __restrict__ G, const uint4* __restrict__ heads,
-                  const int* __restrict__ nheads, int* __restrict__ counters, int M, int nvec,
-                  int stride, float lr, float* __restrict__ Dtab, int flags, const hole_k3_shard sh) {
+// ADA: the root applies the AdaGrad update with the accumulator S (hole_ctx_set_optimizer) instead of SGD
+template <int GS, int V, bool ADA>
+__device__ __forceinline__ void hole_apply_body(float* __restrict__ E, float* __restrict__ G,
+                                                const uint4* __restrict__ heads, const int* __restrict__ nheads,
+                                                int* __restrict__ counters, int M, int nvec, int stride, float lr,
+                                                float* __restrict__ Dtab, int flags, const hole_k3_shard& sh,
+                                                float* __restrict__ S) {
   constexpr int C = HOLE_TREE_C;
   const int lane = threadIdx.x % GS;
   const int gbase = (threadIdx.x % 32) / GS * GS;
@@ -1039,10 +1041,11 @@ hole_apply_kernel(float* __restrict__ E, float* __restrict__ G, const uint4* __r
     const int rel = j - s;
     const int cnt = min(C, n - rel);
     float* erow = E + (size_t)row * stride;
-    Row<V> acc, x;
+    Row<V> acc, x, s2;
     const bool delta = Dtab != nullptr;   // delta mode: write -lr * sum into Dtab, leave E alone
     const bool single = n <= C && !delta; // this leaf is also the root: fetch the table row alongside
     if (single) row_load<GS, V, false>(x, erow, lane, nvec);
+    if constexpr (ADA) { if (single) row_load<GS, V, false>(s2, S + (size_t)row * stride, lane, nvec); }
     sum_rows<GS, V>(acc, G, j, 1, cnt, stride, lane, nvec);
     int level = 0, idx = rel / C, nl = (n + C - 1) / C;
     int64_t span = C;   // sorted entries covered by one node of this level
@@ -1068,10 +1071,22 @@ hole_apply_kernel(float* __restrict__ E, float* __restrict__ G, const uint4* __r
           break;
         }
         if (!single) row_load<GS, V, false>(x, erow, lane, nvec);
+        if constexpr (ADA) {    // S[row] += acc^2;  E[row] -= lr * acc * rsqrt(S[row])  (SparseApplyAdagrad)
+          if (!single) row_load<GS, V, false>(s2, S + (size_t)row * stride, lane, nvec);
 #pragma unroll
-        for (int k = 0; k < 4 * V; ++k) {
-          x.re[k] -= lr * acc.re[k];
-          x.im[k] -= lr * acc.im[k];
+          for (int k = 0; k < 4 * V; ++k) {
+            s2.re[k] = fmaf(acc.re[k], acc.re[k], s2.re[k]);
+            s2.im[k] = fmaf(acc.im[k], acc.im[k], s2.im[k]);
+            x.re[k] = fmaf(-lr * acc.re[k], __frsqrt_rn(s2.re[k]), x.re[k]);
+            x.im[k] = fmaf(-lr * acc.im[k], __frsqrt_rn(s2.im[k]), x.im[k]);
+          }
+          row_store<GS, V>(s2, S + (size_t)row * stride, lane, nvec);
+        } else {
+#pragma unroll
+          for (int k = 0; k < 4 * V; ++k) {
+            x.re[k] -= lr * acc.re[k];
+            x.im[k] -= lr * acc.im[k];
+          }
         }
         row_store<GS, V>(x, erow, lane, nvec);
         break;
@@ -1097,6 +1112,24 @@ hole_apply_kernel(float* __restrict__ E, float* __restrict__ G, const uint4* __r
     }
   }
   if (sh.world > 0) __threadfence_system();   // delta rows stored to peer memory: see hole_k1_body
+}
+
+template <int GS, int V>
+__global__ void __launch_bounds__(256)
+hole_apply_kernel(float* __restrict__ E, float* __restrict__ G, const uint4* __restrict__ heads,
+                  const int* __restrict__ nheads, int* __restrict__ counters, int M, int nvec,
+                  int stride, float lr, float* __restrict__ Dtab, int flags, const hole_k3_shard sh) {
+  hole_apply_body<GS, V, false>(E, G, heads, nheads, counters, M, nvec, stride, lr, Dtab, flags, sh, nullptr);
+}
+
+// K3 of an AdaGrad step: in place on the table E and the accumulator S
+template <int GS, int V>
+__global__ void __launch_bounds__(256)
+hole_adagrad_apply_kernel(float* __restrict__ E, float* __restrict__ G, const uint4* __restrict__ heads,
+                          const int* __restrict__ nheads, int* __restrict__ counters, int M, int nvec,
+                          int stride, float lr, float* __restrict__ S) {
+  const hole_k3_shard sh = {};
+  hole_apply_body<GS, V, true>(E, G, heads, nheads, counters, M, nvec, stride, lr, nullptr, 0, sh, S);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1461,6 +1494,16 @@ extern "C" int hole_ctx_set_score_mode(hole_ctx* c, int mode) {
   return HOLE_OK;
 }
 
+extern "C" int hole_ctx_set_optimizer(hole_ctx* c, int optimizer, float* accum) {
+  HOLE_CHECK_ARG(c != nullptr);
+  HOLE_CHECK_ARG((optimizer == HOLE_OPT_SGD && accum == nullptr) || (optimizer == HOLE_OPT_ADAGRAD && accum != nullptr));
+  if (optimizer == HOLE_OPT_ADAGRAD && c->shard_state != nullptr)
+    return hole_set_error(HOLE_ERR_UNSUPPORTED, "AdaGrad has no row-sharded step");
+  c->optimizer = optimizer;
+  c->accum = accum;
+  return HOLE_OK;
+}
+
 static int ctx_create_streams(hole_ctx* c) {
   HOLE_CUDA_TRY(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
   {   // the plan is small integer work that the next step waits for: highest priority
@@ -1769,7 +1812,7 @@ static hole_k1_fn k1_fn(const hole_ctx* c) {
   return hole_k1_kernel<32, 3, DM>;
 }
 static hole_k1_fn k1_fn_dm(const hole_ctx* c, int dm) {
-  return dm == 0 ? k1_fn<0>(c) : dm == 1 ? k1_fn<1>(c) : dm == 2 ? k1_fn<2>(c) : k1_fn<3>(c);
+  return dm == 0 ? k1_fn<0>(c) : dm == 1 ? k1_fn<1>(c) : dm == 2 ? k1_fn<2>(c) : dm == 3 ? k1_fn<3>(c) : k1_fn<4>(c);
 }
 
 // Kernel attributes of the training kernels, set on the first training call of a context
@@ -1782,7 +1825,7 @@ static int k1_prepare(hole_ctx* c) {
     return hole_set_error(HOLE_ERR_UNSUPPORTED, "embedding_dim %d: K1 needs %d bytes of shared memory",
                           c->dim, c->k1v2_smem);
   int nb = 1;
-  for (int dm = 0; dm < 4; ++dm) {
+  for (int dm = 0; dm < 5; ++dm) {
     HOLE_CUDA_TRY(cudaFuncSetAttribute(k1_fn_dm(c, dm), cudaFuncAttributeMaxDynamicSharedMemorySize, c->k1v2_smem));
   }
   HOLE_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k1_fn<0>(c), K1_THREADS, c->k1v2_smem));
@@ -1896,6 +1939,22 @@ static int plan_steps(hole_ctx* c, hole_plan& pl, const int32_t* triples_dev, in
   return HOLE_OK;
 }
 
+// The training calls without an AdaGrad form refuse it here, before they enqueue anything (a refused call
+// leaves the context as it was): the delta-table and log-loss steps, the row-sharded steps, and every
+// training call in the archived ccorr/tanh score mode.
+enum { HOLE_STEP_TABLE, HOLE_STEP_DELTA, HOLE_STEP_LOGLOSS, HOLE_STEP_SHARD };
+static int optimizer_refusal(const hole_ctx* c, int kind) {
+  if (c->optimizer == HOLE_OPT_SGD) return HOLE_OK;
+  if (kind == HOLE_STEP_DELTA)
+    return hole_set_error(HOLE_ERR_UNSUPPORTED, "AdaGrad updates the table in place: no delta-table step");
+  if (kind == HOLE_STEP_LOGLOSS)
+    return hole_set_error(HOLE_ERR_UNSUPPORTED, "AdaGrad has no log-loss step (its L2 gradient is dense)");
+  if (kind == HOLE_STEP_SHARD) return hole_set_error(HOLE_ERR_UNSUPPORTED, "AdaGrad has no row-sharded step");
+  if (c->score_mode != HOLE_SCORE_COMPLEX)
+    return hole_set_error(HOLE_ERR_UNSUPPORTED, "the archived ccorr/tanh score mode has no AdaGrad step");
+  return HOLE_OK;
+}
+
 // K1 + K3 of one step whose plan is slot `slot` of pl.
 // shard != nullptr (hole_shard_step): pos / neg are the step's triples as request-list rows (what the
 // plan was built on), shard_tri / shard_neg the same triples as global row ids (what K1 gathers).
@@ -1947,16 +2006,25 @@ static int run_step(hole_ctx* c, hole_plan& pl, float* table, const int32_t* pos
     ka.margin = margin; ka.lr = lr; ka.G = c->G; ka.sigma = sigma_out; ka.Dtab = delta_out;
     ka.loss = (flags & 3) == 2 ? nullptr : loss_out;       // a log-loss pass without the positive term
     static const hole_k1_shard no_shard = {};
-    const int dm = (flags & 3) ? 3 : shard ? 2 : (delta_out ? 1 : 0);
+    int dm = (flags & 3) ? 3 : shard ? 2 : (delta_out ? 1 : 0);
+    if (c->optimizer == HOLE_OPT_ADAGRAD) {     // (optimizer_refusal: only the in-place step gets here)
+      dm = 4;
+      ka.Dtab = c->accum;
+    }
     int rc = k1_launch(c, dm, ka, shard ? *shard : no_shard, st, k1_follows_k3 && !c->profile);
     if (rc) return rc;
   }
   if (pe) HOLE_CUDA_TRY(cudaEventRecord(pe[1], st));
   if (k1_done_mark) HOLE_CUDA_TRY(cudaEventRecord(k1_done_mark, st));
   const unsigned k3_grid = std::min<unsigned>(grid_for_groups(pl.heads_cap, c->gs), (unsigned)c->sm_count * 4);
-  HOLE_DISPATCH_PDL(c, hole_apply_kernel, k3_grid, 256, 0, st, table, c->G,
-                pl.heads + (size_t)slot * pl.heads_cap, pl.nheads + slot, c->counters, M, c->nvec,
-                c->row_stride, lr, delta_out, flags, k3s);
+  if (c->optimizer == HOLE_OPT_ADAGRAD)
+    HOLE_DISPATCH_PDL(c, hole_adagrad_apply_kernel, k3_grid, 256, 0, st, table, c->G,
+                      pl.heads + (size_t)slot * pl.heads_cap, pl.nheads + slot, c->counters, M, c->nvec,
+                      c->row_stride, lr, c->accum);
+  else
+    HOLE_DISPATCH_PDL(c, hole_apply_kernel, k3_grid, 256, 0, st, table, c->G,
+                  pl.heads + (size_t)slot * pl.heads_cap, pl.nheads + slot, c->counters, M, c->nvec,
+                  c->row_stride, lr, delta_out, flags, k3s);
   if (pe) HOLE_CUDA_TRY(cudaEventRecord(pe[2], st));
   return HOLE_OK;
 }
@@ -2014,11 +2082,13 @@ extern "C" int hole_train_step_ex(hole_ctx* c, float* table, float* delta_out, c
                                   const int32_t* neg_ent, int side, int64_t B, float margin, float lr,
                                   float* loss_out, float* sigma_out, void* stream) {
   HOLE_CHECK_ARG(c && B >= 0 && (side == 0 || side == 1));
+  int rc = optimizer_refusal(c, delta_out ? HOLE_STEP_DELTA : HOLE_STEP_TABLE);
+  if (rc) return rc;
   if (B == 0) return HOLE_OK;   // an empty batch is a no-op
   HOLE_CHECK_ARG(table && pos && neg_ent && loss_out);
   HOLE_CHECK_ARG(4 * B < (int64_t(1) << 31));
   HOLE_CUDA_TRY(cudaSetDevice(c->device));
-  int rc = hole_ws_reserve(c, B, 1);
+  rc = hole_ws_reserve(c, B, 1);
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   int slot_ix = -1;
@@ -2067,12 +2137,14 @@ extern "C" int hole_train_step_logloss(hole_ctx* c, float* table, float* delta_w
   HOLE_CHECK_ARG(c && B >= 0 && negative_ratio >= 1 && negative_ratio <= 64);
   if (c->score_mode != HOLE_SCORE_COMPLEX)
     return hole_set_error(HOLE_ERR_UNSUPPORTED, "the archived ccorr/tanh score mode has no log-loss branch");
+  int rc = optimizer_refusal(c, HOLE_STEP_LOGLOSS);
+  if (rc) return rc;
   if (B == 0) return HOLE_OK;
   HOLE_CHECK_ARG(table && delta_ws && triples && type_of && csr_off && csr_ids && loss_out);
   HOLE_CHECK_ARG(4 * B < (int64_t(1) << 31));
   HOLE_CUDA_TRY(cudaSetDevice(c->device));
   const int k = negative_ratio;
-  int rc = hole_ws_reserve(c, B, k);
+  rc = hole_ws_reserve(c, B, k);
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   hole_plan& pl = c->plan[0];
@@ -2305,12 +2377,14 @@ extern "C" int hole_train_steps(hole_ctx* c, float* table, const int32_t* triple
                                 float margin, const float* lr, float* loss_out, float* loss_sum_out,
                                 void* stream) {
   HOLE_CHECK_ARG(c && B >= 0 && n_steps >= 0);
+  int rc = optimizer_refusal(c, HOLE_STEP_TABLE);
+  if (rc) return rc;
   if (B == 0 || n_steps == 0) return HOLE_OK;
   HOLE_CHECK_ARG(table && triples && type_of && csr_off && csr_ids && lr);
   HOLE_CHECK_ARG(4 * B < (int64_t(1) << 31));
   HOLE_CUDA_TRY(cudaSetDevice(c->device));
   const int64_t S = plan_chunk(B);
-  int rc = hole_ws_reserve(c, B, S);
+  rc = hole_ws_reserve(c, B, S);
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   // the plan stream may only read the caller's triples once the caller's stream got here
@@ -2345,12 +2419,14 @@ extern "C" int hole_train_steps_host(hole_ctx* c, float* table, const int32_t* t
                                      float margin, const float* lr, float* loss_sum_host,
                                      void* stream) {
   HOLE_CHECK_ARG(c && B >= 0 && n_steps >= 0);
+  int rc = optimizer_refusal(c, HOLE_STEP_TABLE);
+  if (rc) return rc;
   if (B == 0 || n_steps == 0) return HOLE_OK;
   HOLE_CHECK_ARG(table && triples_host && type_of && csr_off && csr_ids && lr && loss_sum_host);
   HOLE_CHECK_ARG(4 * B < (int64_t(1) << 31));
   HOLE_CUDA_TRY(cudaSetDevice(c->device));
   const int64_t S = plan_chunk(B);
-  int rc = hole_ws_reserve(c, B, S);
+  rc = hole_ws_reserve(c, B, S);
   if (rc) return rc;
   const int64_t stage_elems = S * B * 3;
   if (stage_elems > c->cap_stage) {

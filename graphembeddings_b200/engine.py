@@ -51,6 +51,7 @@ class HoleEngine:
         check(self.lib.hole_ctx_create(C.byref(h), device, self.n_rows, self.dim))
         self._ctx = h
         self.table = None
+        self.accum = None          # AdaGrad accumulator (set_optimizer)
         self.type_of = self.csr_off = self.csr_ids = None
 
     def set_relation_count(self, n_relations):
@@ -63,6 +64,52 @@ class HoleEngine:
         variant of holE-20170724/graph.pbtxt:6221-6521: tanh of r-weighted circular correlation)."""
         code = {"complex": 0, "ccorr_tanh": 1}.get(mode, mode)      # HOLE_SCORE_COMPLEX / HOLE_SCORE_CCORR_TANH
         check(self.lib.hole_ctx_set_score_mode(self._ctx, int(code)))
+        return self
+
+    def set_optimizer(self, optimizer, initial_accumulator=0.1):
+        """"sgd" (holE.py:296's GradientDescentOptimizer, the default) or "adagrad" (TF's
+        AdagradOptimizer(lr, initial_accumulator_value) in its place).  "adagrad" allocates the accumulator
+        [n_rows, row_stride] and fills all of it, pad columns included, with initial_accumulator (> 0);
+        "sgd" drops it.  AdaGrad trains through train_step / train_steps / train_steps_host only."""
+        if optimizer == "sgd":
+            check(self.lib.hole_ctx_set_optimizer(self._ctx, _lib.HOLE_OPT_SGD, None))
+            self.accum = None
+            return self
+        if optimizer != "adagrad":
+            raise HoleError(f"unknown optimizer {optimizer!r}: 'sgd' or 'adagrad'")
+        if not float(initial_accumulator) > 0.0:
+            raise HoleError(f"initial_accumulator must be > 0, got {initial_accumulator}")
+        accum = torch.full((self.n_rows, self.row_stride), float(initial_accumulator), dtype=torch.float32,
+                           device=self.device)
+        check(self.lib.hole_ctx_set_optimizer(self._ctx, _lib.HOLE_OPT_ADAGRAD, _ptr(accum)))
+        self.accum, self.initial_accumulator = accum, float(initial_accumulator)
+        return self
+
+    def accumulator(self):
+        """The AdaGrad accumulator as a [N, dim] float32 CUDA tensor (checkpoint layout, the slot
+        `embeddings/Adagrad`)."""
+        if getattr(self, "accum", None) is None:
+            raise HoleError("the optimizer is not adagrad: there is no accumulator")
+        out = torch.empty((self.n_rows, self.dim), dtype=torch.float32, device=self.device)
+        check(self.lib.hole_unpack_rows(self._ctx, _ptr(self.accum), _ptr(out), self.n_rows, _stream()))
+        return out
+
+    def set_accumulator(self, A):
+        """A: [N, dim] float32 (checkpoint layout), every element > 0.  The pad columns of the device layout
+        are refilled with the initial value (packing writes zeros there)."""
+        if getattr(self, "accum", None) is None:
+            raise HoleError("the optimizer is not adagrad: there is no accumulator")
+        A = torch.as_tensor(A, dtype=torch.float32)
+        assert A.shape == (self.n_rows, self.dim), A.shape
+        src = A.to(self.device).contiguous()
+        if not bool((src > 0).all()):
+            raise HoleError("every accumulator element must be > 0")
+        check(self.lib.hole_pack_rows(self._ctx, _ptr(src), _ptr(self.accum), self.n_rows, _stream()))
+        half, H = self.row_stride // 2, self.dim // 2
+        if H < half:
+            self.accum[:, H:half] = self.initial_accumulator
+            self.accum[:, half + H:] = self.initial_accumulator
+        torch.cuda.current_stream().synchronize()   # src may be freed by the caller
         return self
 
     def close(self):

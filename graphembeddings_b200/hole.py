@@ -194,11 +194,28 @@ def summarize(var):
             "max": float(var.max()), "min": float(var.min())}
 
 
+ADAGRAD_SLOT = "embeddings/Adagrad"
+
+
+def check_optimizer_flags(flags):
+    """The training branches that have no AdaGrad form exit before anything is trained."""
+    if getattr(flags, 'optimizer', 'sgd') != 'adagrad':
+        return
+    if flags.log_loss:
+        raise SystemExit("--optimizer adagrad has no --log_loss branch (its L2 gradient would make the update dense)")
+    if getattr(flags, 'score_variant', 'complex') != 'complex':
+        raise SystemExit("--optimizer adagrad is not available with --score_variant ccorr_tanh")
+    if not flags.adagrad_initial_accumulator > 0:
+        raise SystemExit("--adagrad_initial_accumulator must be > 0")
+
+
 def save_checkpoint(eng, output_dir, global_step, metadata_names=None):
     """saver.save(sess, output_dir + '/model.ckpt') (holE.py:359) + checkpoint state file."""
     E = eng.embeddings().cpu().numpy()
-    tf_bundle.save_bundle(os.path.join(output_dir, 'model.ckpt'),
-                          {"embeddings": E, "batch/Variable": np.array(global_step, dtype=np.int32)})
+    tensors = {"embeddings": E, "batch/Variable": np.array(global_step, dtype=np.int32)}
+    if eng.accum is not None:       # AdagradOptimizer's slot, under the name TF's Saver gives it
+        tensors[ADAGRAD_SLOT] = eng.accumulator().cpu().numpy()
+    tf_bundle.save_bundle(os.path.join(output_dir, 'model.ckpt'), tensors)
     tf_bundle.write_checkpoint_state(output_dir)
 
 
@@ -206,6 +223,16 @@ def load_checkpoint(output_dir):
     """saver.restore(sess, output_dir + '/model.ckpt') (holE.py:313-314)."""
     b = tf_bundle.load_bundle(os.path.join(output_dir, 'model.ckpt'), names={"embeddings", "batch/Variable"})
     return b["embeddings"], int(np.asarray(b.get("batch/Variable", 0)).reshape(-1)[0])
+
+
+def load_accumulator(output_dir):
+    """The AdaGrad slot of the checkpoint; a checkpoint without one is refused, as TF's Saver refuses to
+    restore a variable the checkpoint does not hold."""
+    b = tf_bundle.load_bundle(os.path.join(output_dir, 'model.ckpt'), names={ADAGRAD_SLOT})
+    if ADAGRAD_SLOT not in b:
+        raise SystemExit(f"--optimizer adagrad: the checkpoint in {output_dir} has no {ADAGRAD_SLOT} slot "
+                         "(it was not trained with AdaGrad); resume it with --optimizer sgd")
+    return b[ADAGRAD_SLOT]
 
 
 # --------------------------------------------------------------------------------------
@@ -218,6 +245,7 @@ def run_training(data, flags=None, seed=0, max_steps=None, log=print):
         'Batch count: ', batch_count)
     if flags.embedding_dim % 2:
         raise ValueError("embedding_dim must be even (holE.py:164-165 splits the row in halves)")
+    check_optimizer_flags(flags)
     # Warning: this will clobber existing summaries (holE.py:253-260)
     if not flags.resume_checkpoint and os.path.isdir(flags.output_dir):
         raise Exception("WARNING: " + flags.output_dir + " already exists!")
@@ -228,12 +256,20 @@ def run_training(data, flags=None, seed=0, max_steps=None, log=print):
             raise
 
     global_step = 0
+    adagrad = getattr(flags, 'optimizer', 'sgd') == 'adagrad'
+    A = None
     if flags.resume_checkpoint:
         E, global_step = load_checkpoint(flags.output_dir)
+        if adagrad:
+            A = load_accumulator(flags.output_dir)      # (--optimizer sgd ignores a saved accumulator)
         # TODO (reference, holE.py:315): the epoch counter restarts
     else:
         E = D.init_embeddings(data.entity_count, flags.embedding_dim, np.random.default_rng(seed))
     eng = make_engine(data.entity_count, data.relation_count, flags.embedding_dim, E, data.id_to_type)
+    if adagrad:      # tf.train.AdagradOptimizer(lr, initial_accumulator_value) in place of holE.py:296's SGD
+        eng.set_optimizer("adagrad", flags.adagrad_initial_accumulator)
+        if A is not None:
+            eng.set_accumulator(A)
     if getattr(flags, 'score_variant', 'complex') != 'complex':
         if flags.log_loss:
             raise SystemExit("--score_variant ccorr_tanh has no --log_loss branch")
@@ -640,6 +676,11 @@ def build_parser():
                         help="Score function: 'complex' = holE.py:191-198 (default); 'ccorr_tanh' = the archived "
                              "variant of the holE-20170724 run (tanh of the r-weighted circular correlation, "
                              "trained there with --margin 1.0); no --log_loss branch.")
+    parser.add_argument('--optimizer', choices=['sgd', 'adagrad'], default='sgd',
+                        help="sgd: holE.py's GradientDescentOptimizer; adagrad: tf.train.AdagradOptimizer in its "
+                             "place (checkpoints then hold its slot embeddings/Adagrad); hinge loss, complex score only.")
+    parser.add_argument('--adagrad_initial_accumulator', type=float, default=0.1,
+                        help='AdagradOptimizer initial_accumulator_value (> 0).')
     parser.add_argument('--seed', type=int, default=0)
     parser.add_argument('--max_steps', type=int, default=None, help='Stop after this many steps (testing).')
     return parser
@@ -653,6 +694,7 @@ def main(argv=None):
     if FLAGS.infer:
         infer_triples(FLAGS)
     else:
+        check_optimizer_flags(FLAGS)
         training_data = init_data(FLAGS)
         run_training(training_data, FLAGS, seed=FLAGS.seed, max_steps=FLAGS.max_steps)
 

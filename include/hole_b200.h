@@ -58,7 +58,7 @@ typedef struct hole_ctx hole_ctx;
 #define HOLE_RANK_BF16X3 1       /* split-bf16 (hi*hi + lo*hi + hi*lo): ranks match fp32 except within ~3e-5 of a tie; dim <= 320 */
 
 /* ABI version of this header; hole_abi_version() returns the library's. */
-#define HOLE_ABI_VERSION 5
+#define HOLE_ABI_VERSION 6
 HOLE_API int hole_abi_version(void);
 
 /* Thread-local message of the last failing call on this thread ("" if none). */
@@ -94,6 +94,25 @@ HOLE_API int hole_ctx_set_relations(hole_ctx* ctx, int64_t n_relations);
 #define HOLE_SCORE_CCORR_TANH 1
 HOLE_API int hole_ctx_set_score_mode(hole_ctx* ctx, int mode);
 
+/* Optimizer of the training step.  HOLE_OPT_SGD (default; accum must be NULL) is holE.py:296's
+ * GradientDescentOptimizer: table[i] -= lr * g_i.  HOLE_OPT_ADAGRAD is TF 1.2's AdagradOptimizer in its place
+ * (SparseApplyAdagrad after the duplicate indices are summed), per touched row i and element, in fp32:
+ *     accum[i] += g_i^2;   table[i] -= lr * g_i * rsqrt(accum[i])
+ * with the NEW accumulator and no epsilon; g_i is the gradient the SGD step applies (duplicates summed in the
+ * same fixed order), and a row whose hinge is inactive (g_i = 0) keeps its table and accumulator rows.
+ *   accum  float32 [n_rows, row_stride], the table's row layout, caller-owned and kept by reference (like the
+ *          type tables of hole_corrupt) until the next hole_ctx_set_optimizer call.  EVERY element must be
+ *          > 0, the pad columns included (TF starts it at initial_accumulator_value, 0.1 by default): a zero
+ *          pad element would make the pad column 0 * rsqrt(0) = NaN instead of keeping it zero.
+ * In AdaGrad mode hole_train_step, hole_train_steps and hole_train_steps_host update the table and the
+ * accumulator.  hole_train_step_ex with a delta_out, hole_train_step_logloss, every hole_shard_* call, and
+ * every training call in HOLE_SCORE_CCORR_TANH mode return HOLE_ERR_UNSUPPORTED before they launch anything
+ * or write anything, and the context stays usable.  AdaGrad on a context bound by hole_shard_init is
+ * HOLE_ERR_UNSUPPORTED too.  Switching back to HOLE_OPT_SGD restores the SGD step exactly. */
+#define HOLE_OPT_SGD 0
+#define HOLE_OPT_ADAGRAD 1
+HOLE_API int hole_ctx_set_optimizer(hole_ctx* ctx, int optimizer, float* accum);
+
 /* Checkpoint layout [n, dim] <-> device layout [n, row_stride]. */
 HOLE_API int hole_pack_rows(hole_ctx* ctx, const float* src_nd, float* dst_padded, int64_t n, void* stream);
 HOLE_API int hole_unpack_rows(hole_ctx* ctx, const float* src_padded, float* dst_nd, int64_t n, void* stream);
@@ -126,7 +145,8 @@ HOLE_API int hole_score(hole_ctx* ctx, const float* table, const int32_t* triple
 
 /* ---- one training step: replaces evaluate_batch's hinge branch (holE.py:222-234) plus
  * GradientDescentOptimizer.minimize (holE.py:296) -- forward, backward and the sparse
- * update table[idx] -= lr * g with duplicates accumulated in a fixed order.
+ * update table[idx] -= lr * g with duplicates accumulated in a fixed order (or the AdaGrad
+ * update, see hole_ctx_set_optimizer).
  *   neg_ent int32[B]: replacement entity per triple; side: HOLE_SIDE_*.
  *   loss_out float32[B] (hinge per triple); sigma_out float32[2B] or NULL
  *   (sigma+ then sigma-, the tensors holE.py:200 summarises). */
@@ -384,7 +404,7 @@ HOLE_API int hole_rank_debug_operands(hole_ctx* ctx, void* cand_out, void* query
 
 /* ---- measurement hooks (bench.py's roofline figure).  With profiling enabled every
  * training step records CUDA events on `stream` around its two hot kernels (K1 =
- * hole_train_fwd_bwd_kernel, K3 = hole_apply_kernel).  hole_profile_read synchronises and
+ * hole_k1_kernel, K3 = hole_apply_kernel or, with AdaGrad, hole_adagrad_apply_kernel).  hole_profile_read synchronises and
  * returns the summed kernel times in milliseconds and the number of steps measured since
  * the last hole_profile_enable call. */
 HOLE_API int hole_profile_enable(hole_ctx* ctx, int on);
