@@ -11,7 +11,7 @@ LIB_PATH = os.environ.get("HOLE_B200_LIB", os.path.join(_HERE, "libhole_b200.so"
 HOLE_SIDE_TAIL, HOLE_SIDE_HEAD, HOLE_SIDE_BOTH, HOLE_SIDE_RELATION = 0, 1, 2, 3
 HOLE_RANK_BF16, HOLE_RANK_BF16X3 = 0, 1
 HOLE_OPT_SGD, HOLE_OPT_ADAGRAD = 0, 1
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 
 class HoleError(RuntimeError):
@@ -50,6 +50,7 @@ SIGNATURES = {
     "hole_shard_steps": (_int, [_p, _p, _i64, _i64, _u64, _u64, _f32, _p, _p, _p]),
     "hole_shard_steps_host": (_int, [_p, _p, _i64, _i64, _u64, _u64, _f32, _p, _p, _p]),
     "hole_shard_poll": (_int, [_p, C.POINTER(_int), _p]),
+    "hole_shard_set_optimizer": (_int, [_p, _int, _p]),
     "hole_shard_profile_read": (_int, [_p, C.POINTER(C.c_double), C.POINTER(_i64)]),
     "hole_enable_peer_access": (_int, [_p, _int]),
     "hole_gather_rows": (_int, [_p, _p, _p, _i64, _p, _i64, _p]),

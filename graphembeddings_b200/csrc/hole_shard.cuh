@@ -26,6 +26,10 @@
 //             relation block takes every rank's deltas in rank order, so the result is
 //             deterministic and the replicas stay bit-identical -- then signals flag A
 //
+// AdaGrad (hole_shard_set_optimizer): compute runs unchanged with lr = -1, so the staged rows are gradients;
+// the owner's apply (hole_shard_adagrad_apply_kernel) sums a row's gradients in rank order, then updates the
+// row and its accumulator row once.  The exchange is byte for byte that of an SGD step.
+//
 // No NCCL call and no host synchronisation inside a step; two flag waits per step, both at the
 // head of a kernel that has work to do anyway.  Flags only grow (epoch = steps completed).
 #pragma once
@@ -72,6 +76,11 @@ struct hole_shard_state {
   hole_shard_prep prep[2];
   int prep_toggle = 0;
   int epoch = 0;                         // steps completed
+  int optimizer = HOLE_OPT_SGD;          // hole_shard_set_optimizer: the optimizer of the following steps
+  float* accum = nullptr;                // AdaGrad: accumulator shard [R + rows_per, stride] (caller-owned)
+  int step_optimizer = HOLE_OPT_SGD;     // latched by hole_shard_step_compute for the step's apply
+  float step_lr = 0.f;
+  float* step_accum = nullptr;
   std::vector<cudaEvent_t> prof_ev;      // hole_profile_enable: 6 events per step (phase boundaries)
   size_t prof_used = 0;
 };
@@ -204,6 +213,90 @@ hole_shard_apply_kernel(float* __restrict__ shard, const int32_t* __restrict__ i
   }
 }
 
+// Owner side, pass 2 of an AdaGrad step (hole_shard_set_optimizer).  The compute half ran with lr = -1, so the
+// staged rows are the ranks' summed gradients (-(-1) * g and 1 * g are exact).  Same items, claim / slot protocol
+// and flag A as hole_shard_apply_kernel, but a row's gradients are summed first, then applied once, as
+// SparseApplyAdagrad after TF's duplicate-index sum:
+//   g = sum_k staged_k[row] (rank order);  A[row] += g^2;  E[row] -= lr * g * rsqrt(A[row])
+// with the expressions of the single-GPU step (k1_emit DM 4, the root of hole_apply_body<.., true>).  Relation
+// rows (items [0, R)) take g = sum_k relstage[k][r] on every rank, so the table and accumulator replicas stay
+// bit-identical.  A row whose gradient is zero everywhere keeps both rows (A + 0 = A, x + (-lr * 0) * s = x).
+template <int GS, int V>
+__global__ void __launch_bounds__(256)
+hole_shard_adagrad_apply_kernel(float* __restrict__ shard, float* __restrict__ accum,
+                                const int32_t* __restrict__ inbox, const int32_t* __restrict__ meta,
+                                const float* __restrict__ stage, const float* __restrict__ relstage, int R, int world,
+                                int me, int64_t cap, int64_t row0, int64_t rows_per, unsigned* __restrict__ claim,
+                                const int32_t* __restrict__ slot, hole_peer_ptrs flags, int signal_epoch,
+                                unsigned* __restrict__ done, int nvec, int stride, float lr) {
+  __shared__ int s_pre[HOLE_MAX_RANKS + 1];
+  __shared__ bool s_last;
+  if (threadIdx.x == 0) {
+    int pre = 0;
+    for (int k = 0; k < world; ++k) { s_pre[k] = pre; pre += meta[2 * k]; }
+    s_pre[world] = pre;
+  }
+  __syncthreads();
+  const int lane = threadIdx.x % GS;
+  const int total = R + s_pre[world];
+  const int gstride = (gridDim.x * blockDim.x) / GS;
+  for (int item = (blockIdx.x * blockDim.x + threadIdx.x) / GS; item < total; item += gstride) {
+    Row<V> g, d;
+    size_t r;                                            // shard / accumulator row
+    if (item < R) {
+      r = (size_t)item;
+      row_zero(g);
+      for (int k = 0; k < world; ++k) {
+        row_load<GS, V, false>(d, relstage + ((size_t)k * R + item) * stride, lane, nvec);
+        row_add(g, d);
+      }
+    } else {
+      const int e = item - R;
+      int k = 0;
+      while (e >= s_pre[k + 1]) ++k;
+      const int64_t row = (int64_t)inbox[(size_t)k * cap + (e - s_pre[k])] - row0;
+      unsigned m = __ldcg(claim + row);
+      if ((m & (0u - m)) != (1u << k)) continue;         // a lower rank's group owns this row (or it is done)
+      r = (size_t)(R + row);
+      row_zero(g);
+      while (m != 0) {
+        const int l = __ffs(m) - 1;
+        m &= m - 1;
+        const int gi = __ldcg(slot + (size_t)l * rows_per + row);
+        row_load<GS, V, false>(d, stage + ((size_t)l * cap + gi) * stride, lane, nvec);
+        row_add(g, d);
+      }
+      if (lane == 0) claim[row] = 0;                     // ready for the next step
+    }
+    float* erow = shard + r * stride;
+    float* arow = accum + r * stride;
+    Row<V> x, a;
+    row_load<GS, V, false>(x, erow, lane, nvec);
+    row_load<GS, V, false>(a, arow, lane, nvec);
+#pragma unroll
+    for (int k = 0; k < 4 * V; ++k) {
+      a.re[k] = fmaf(g.re[k], g.re[k], a.re[k]);
+      a.im[k] = fmaf(g.im[k], g.im[k], a.im[k]);
+      x.re[k] = fmaf(-lr * g.re[k], __frsqrt_rn(a.re[k]), x.re[k]);
+      x.im[k] = fmaf(-lr * g.im[k], __frsqrt_rn(a.im[k]), x.im[k]);
+    }
+    row_store<GS, V>(a, arow, lane, nvec);
+    row_store<GS, V>(x, erow, lane, nvec);
+  }
+  __threadfence_system();
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = atomicAdd(done, 1u) == gridDim.x - 1;
+  __syncthreads();
+  if (s_last) {
+    if (threadIdx.x == 0) *done = 0;
+    __threadfence_system();
+    if (threadIdx.x < world) {
+      int* theirs = static_cast<int*>(flags.p[threadIdx.x]) + me;             // flags[0][me] on that rank
+      asm volatile("st.release.sys.global.s32 [%0], %1;" ::"l"(theirs), "r"(signal_epoch) : "memory");
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------ host side
 static void shard_free(hole_ctx* c) {
   hole_shard_state* s = c->shard_state;
@@ -296,6 +389,18 @@ extern "C" int hole_shard_init(hole_ctx* c, int world, int me, int64_t n_relatio
   rc = route_reserve(c, 3 * max_batch, SHARD_PREP_STEPS);
   if (rc) { shard_free(c); return rc; }
   HOLE_CUDA_TRY(cudaDeviceSynchronize());
+  return HOLE_OK;
+}
+
+// The optimizer of the row-sharded steps; it lives in the shard state (hole_shard_init resets it to SGD) and
+// leaves the context's own optimizer (hole_ctx_set_optimizer) alone.
+extern "C" int hole_shard_set_optimizer(hole_ctx* c, int optimizer, float* accum_shard) {
+  HOLE_CHECK_ARG(c != nullptr);
+  if (c->shard_state == nullptr) return hole_set_error(HOLE_ERR_ARG, "hole_shard_init has not been called");
+  HOLE_CHECK_ARG((optimizer == HOLE_OPT_SGD && accum_shard == nullptr) ||
+                 (optimizer == HOLE_OPT_ADAGRAD && accum_shard != nullptr));
+  c->shard_state->optimizer = optimizer;
+  c->shard_state->accum = accum_shard;
   return HOLE_OK;
 }
 
@@ -414,8 +519,12 @@ extern "C" int hole_shard_step_compute(hole_ctx* c, const int32_t* pos, int64_t 
   sh.me = me; sh.world = world; sh.cap = s->cap; sh.timeout_ns = s->timeout_ns;
   sh.shard = s->p_shard; sh.stage = s->p_stage;
   sh.uniq = p_uniq; sh.inbox = ib; sh.meta = mt;          // the request lists are posted by K1 itself
-  rc = run_step(c, pl, s->shard, p_pos_w, p_neg_w, side, B, margin, lr, loss_out, nullptr, k, st, s->Drel, false, 0,
-                &sh, pos, p_neg, c->profile ? s->prof_ev[s->prof_used - 6 + 2] : nullptr);
+  // AdaGrad: K1 / K3 stage -(-1) * g = g, the ranks' summed gradients, and the owners apply lr (latched here
+  // for hole_shard_step_apply)
+  const bool ada = s->optimizer == HOLE_OPT_ADAGRAD;
+  s->step_optimizer = s->optimizer; s->step_lr = lr; s->step_accum = s->accum;
+  rc = run_step(c, pl, s->shard, p_pos_w, p_neg_w, side, B, margin, ada ? -1.0f : lr, loss_out, nullptr, k, st,
+                s->Drel, false, 0, &sh, pos, p_neg, c->profile ? s->prof_ev[s->prof_used - 6 + 2] : nullptr);
   if (rc) return rc;
   if ((rc = shard_mark(c, 3, st))) return rc;
   p.consumed += 1;
@@ -449,10 +558,16 @@ extern "C" int hole_shard_step_apply(hole_ctx* c, void* stream) {
       inbox, meta, world, s->cap, row0, s->rows_per, s->claim, s->slot, static_cast<const int*>(s->p_flags.p[me]),
       s->epoch + 1, s->err, s->timeout_ns);
   HOLE_LAUNCHED();
-  HOLE_DISPATCH(c, hole_shard_apply_kernel, (unsigned)c->sm_count * 16, 256, st, s->shard, inbox, meta,
-                static_cast<const float*>(s->p_stage.p[me]), static_cast<const float*>(s->p_relstage.p[me]),
-                (int)s->R, world, me, s->cap, row0, s->rows_per, s->claim, s->slot, s->p_flags, s->epoch + 1,
-                s->done + 1, c->nvec, c->row_stride);
+  if (s->step_optimizer == HOLE_OPT_ADAGRAD)                 // the optimizer and lr of the step's compute half
+    HOLE_DISPATCH(c, hole_shard_adagrad_apply_kernel, (unsigned)c->sm_count * 16, 256, st, s->shard, s->step_accum,
+                  inbox, meta, static_cast<const float*>(s->p_stage.p[me]),
+                  static_cast<const float*>(s->p_relstage.p[me]), (int)s->R, world, me, s->cap, row0, s->rows_per,
+                  s->claim, s->slot, s->p_flags, s->epoch + 1, s->done + 1, c->nvec, c->row_stride, s->step_lr);
+  else
+    HOLE_DISPATCH(c, hole_shard_apply_kernel, (unsigned)c->sm_count * 16, 256, st, s->shard, inbox, meta,
+                  static_cast<const float*>(s->p_stage.p[me]), static_cast<const float*>(s->p_relstage.p[me]),
+                  (int)s->R, world, me, s->cap, row0, s->rows_per, s->claim, s->slot, s->p_flags, s->epoch + 1,
+                  s->done + 1, c->nvec, c->row_stride);
   s->epoch += 1;
   return shard_mark(c, 5, (cudaStream_t)stream);
 }

@@ -258,6 +258,15 @@ class HoleEngine:
                                        peer_relstage, peer_inbox, peer_meta, peer_flags, _ptr(err_flag),
                                        float(timeout_s), _ptr(self.type_of), _ptr(self.csr_off), _ptr(self.csr_ids)))
 
+    def shard_set_optimizer(self, optimizer, accum_shard=None):
+        """hole_shard_set_optimizer: the optimizer of the following sharded steps ("sgd" with no accumulator,
+        "adagrad" with accum_shard = float32 CUDA [n_relations + rows_per_rank, row_stride], every element > 0,
+        kept alive here while bound).  Call after shard_init, on every rank before the same step."""
+        code = {"sgd": _lib.HOLE_OPT_SGD, "adagrad": _lib.HOLE_OPT_ADAGRAD}.get(optimizer, optimizer)
+        check(self.lib.hole_shard_set_optimizer(self._ctx, int(code), _ptr(accum_shard)))
+        self._shard_accum = accum_shard
+        return self
+
     def shard_prepare(self, pos_i32, seed, step):
         check(self.lib.hole_shard_prepare(self._ctx, _ptr(pos_i32), pos_i32.shape[0], int(seed), int(step), _stream()))
 

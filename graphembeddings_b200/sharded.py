@@ -148,9 +148,21 @@ class RowShardedTrainer:
         self.shard = self.be.pad_rows(mine)
         return self
 
+    def set_optimizer(self, optimizer, initial_accumulator=0.1):
+        """This all-to-all trainer trains with SGD only; AdaGrad runs on P2PRowShardedTrainer."""
+        if optimizer == "sgd":
+            return self
+        from ._lib import HoleError
+        raise HoleError(f"{type(self).__name__} (the all-to-all row-sharded trainer) trains with 'sgd' only; "
+                        f"optimizer {optimizer!r} on several GPUs needs P2PRowShardedTrainer (NVLink peer memory)")
+
     def gather_embeddings(self):
         """Full [N, dim] table on every rank (tests / checkpointing)."""
-        mine = self.be.unpad_rows(self.shard[self.R:]).contiguous()
+        return self._gather(self.shard)
+
+    def _gather(self, P):
+        """Full [N, dim] array on every rank from every rank's [relations | block] rows P (device layout)."""
+        mine = self.be.unpad_rows(P[self.R:]).contiguous()
         if self.world == 1:
             ents = mine
         else:
@@ -159,7 +171,7 @@ class RowShardedTrainer:
             out = [torch.empty_like(buf) for _ in range(self.world)]
             self.dist.all_gather(out, buf)
             ents = torch.cat(out, dim=0)[: self.n_ent]
-        return torch.cat([self.be.unpad_rows(self.shard[: self.R]), ents], dim=0)
+        return torch.cat([self.be.unpad_rows(P[: self.R]), ents], dim=0)
 
     # ------------------------------------------------------------------ exchange helpers
     def _a2a(self, send, send_counts, recv_counts, out=None):
@@ -364,6 +376,7 @@ class P2PRowShardedTrainer(RowShardedTrainer):
         self.meta = torch.zeros((2, G, 2), dtype=torch.int32, device=dev)
         self.flags = torch.zeros((2, G), dtype=torch.int32, device=dev)
         self.barrier_err = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.accum = None          # AdaGrad accumulator shard (set_optimizer), the layout of self.shard
         mine = [self.shard, self.stage, self.relstage, self.inbox, self.meta, self.flags]
         if G == 1:
             peers = [mine]
@@ -418,6 +431,56 @@ class P2PRowShardedTrainer(RowShardedTrainer):
         if self.world > 1:
             self.dist.barrier()
         self.shard = self.stage = self.relstage = self.inbox = self.meta = self.flags = None
+        self.accum = None
+
+    def set_optimizer(self, optimizer, initial_accumulator=0.1):
+        """"sgd" (the default) or "adagrad" (TF's AdagradOptimizer(lr, initial_accumulator_value), applied by each
+        row's owner to the gradient summed over every rank that uses the row; hole_shard_set_optimizer).
+        "adagrad" allocates this rank's accumulator shard [relations | my block] and fills all of it, pad columns
+        and the unused trailing rows included, with initial_accumulator (> 0); "sgd" drops it.  Every rank must
+        make the same call before the same step."""
+        from ._lib import HoleError
+        eng = self.be.eng
+        if optimizer == "sgd":
+            eng.shard_set_optimizer("sgd", None)
+            self.accum = None
+            return self
+        if optimizer != "adagrad":
+            raise HoleError(f"unknown optimizer {optimizer!r}: 'sgd' or 'adagrad'")
+        if not float(initial_accumulator) > 0.0:
+            raise HoleError(f"initial_accumulator must be > 0, got {initial_accumulator}")
+        accum = torch.full_like(self.shard, float(initial_accumulator))
+        eng.shard_set_optimizer("adagrad", accum)
+        self.accum, self.initial_accumulator = accum, float(initial_accumulator)
+        return self
+
+    def load_accumulator(self, A):
+        """A: the full [N, dim] AdaGrad accumulator (checkpoint layout, the slot `embeddings/Adagrad`), every element
+        > 0, available on every rank; keeps this rank's part.  The pad columns and unused rows keep the initial
+        value."""
+        from ._lib import HoleError
+        if getattr(self, "accum", None) is None:
+            raise HoleError("the optimizer is not adagrad: there is no accumulator")
+        A = torch.as_tensor(A, dtype=torch.float32)
+        assert A.shape == (self.R + self.n_ent, self.dim), A.shape
+        mine = torch.cat([A[: self.R], A[self.begin:self.end]], dim=0).to(self.accum.device)
+        if not bool((mine > 0).all()):
+            raise HoleError("every accumulator element must be > 0")
+        H, Hp = self.dim // 2, self.be.width // 2
+        self.accum.fill_(self.initial_accumulator)
+        self.accum[: mine.shape[0], :H] = mine[:, :H]
+        self.accum[: mine.shape[0], Hp:Hp + H] = mine[:, H:]
+        torch.cuda.current_stream().synchronize()   # A may be freed by the caller
+        return self
+
+    def gather_accumulator(self):
+        """Full [N, dim] AdaGrad accumulator on every rank (checkpoint layout: the `embeddings/Adagrad` slot of
+        tf_bundle).  Collective, like gather_embeddings()."""
+        from ._lib import HoleError
+        if getattr(self, "accum", None) is None:
+            raise HoleError("the optimizer is not adagrad: there is no accumulator")
+        self.check_barriers()
+        return self._gather(self.accum)
 
     def load_embeddings(self, E):
         E = torch.as_tensor(E)

@@ -58,7 +58,7 @@ typedef struct hole_ctx hole_ctx;
 #define HOLE_RANK_BF16X3 1       /* split-bf16 (hi*hi + lo*hi + hi*lo): ranks match fp32 except within ~3e-5 of a tie; dim <= 320 */
 
 /* ABI version of this header; hole_abi_version() returns the library's. */
-#define HOLE_ABI_VERSION 6
+#define HOLE_ABI_VERSION 7
 HOLE_API int hole_abi_version(void);
 
 /* Thread-local message of the last failing call on this thread ("" if none). */
@@ -108,7 +108,9 @@ HOLE_API int hole_ctx_set_score_mode(hole_ctx* ctx, int mode);
  * accumulator.  hole_train_step_ex with a delta_out, hole_train_step_logloss, every hole_shard_* call, and
  * every training call in HOLE_SCORE_CCORR_TANH mode return HOLE_ERR_UNSUPPORTED before they launch anything
  * or write anything, and the context stays usable.  AdaGrad on a context bound by hole_shard_init is
- * HOLE_ERR_UNSUPPORTED too.  Switching back to HOLE_OPT_SGD restores the SGD step exactly. */
+ * HOLE_ERR_UNSUPPORTED too.  Switching back to HOLE_OPT_SGD restores the SGD step exactly.
+ * This call sets the optimizer of the single-table steps only.  The row-sharded steps have their own,
+ * hole_shard_set_optimizer below, which this call neither reads nor changes. */
 #define HOLE_OPT_SGD 0
 #define HOLE_OPT_ADAGRAD 1
 HOLE_API int hole_ctx_set_optimizer(hole_ctx* ctx, int optimizer, float* accum);
@@ -219,7 +221,24 @@ HOLE_API int hole_train_step_logloss(hole_ctx* ctx, float* table, float* delta_w
  *   [n_steps*B, 3] (this rank's slices), one step prepared ahead; lr [host] float32[n_steps];
  *   loss sums of my slices to loss_sum_out (device) / loss_sum_host (blocks until they are there).
  * hole_shard_poll: synchronises `stream` and reports whether a flag wait has timed out; the tables
- *   are then inconsistent and the caller must stop. */
+ *   are then inconsistent and the caller must stop.
+ * hole_shard_set_optimizer: the optimizer of the following sharded steps (after hole_shard_init, which resets
+ *   it to HOLE_OPT_SGD; before it, HOLE_ERR_ARG).  HOLE_OPT_SGD needs accum_shard == NULL, HOLE_OPT_ADAGRAD a
+ *   non-NULL one; any other id is HOLE_ERR_ARG.  A refused call changes nothing.
+ *     accum_shard  float32 [n_relations + rows_per_rank, row_stride], the shard's layout (replicated relation
+ *                  rows, then my block), caller-owned and kept by reference.  EVERY element must be > 0, the pad
+ *                  columns and the unused trailing rows of the last rank's block included (see
+ *                  hole_ctx_set_optimizer).
+ *   AdaGrad step, per row i listed by ranks k1 < k2 < ... and per element, in fp32:
+ *     g_i = sum_k staged_k[i] (rank order);  A[i] += g_i^2;  E[i] -= lr * g_i * rsqrt(A[i])
+ *   with staged_k[i] rank k's summed gradient of row i; a relation row r takes g_r = sum over every rank's
+ *   relation gradient in rank order, applied by every rank to its replicas of the table and the accumulator,
+ *   which stay bit-identical.  A row whose gradient is zero on every rank keeps both rows.  The NVLink exchange
+ *   is that of an SGD step.  hole_shard_step_compute latches the optimizer and lr of a step and
+ *   hole_shard_step_apply applies with them; hole_shard_step(s)(_host) do both per step.  Every rank must set
+ *   the same optimizer before the same step (like the (B, seed, step) sequence).  The context's own optimizer
+ *   (hole_ctx_set_optimizer) is separate: it must stay HOLE_OPT_SGD on a sharded context, and the single-table
+ *   calls on such a context keep their behaviour. */
 #define HOLE_MAX_RANKS 16
 HOLE_API int hole_shard_init(hole_ctx* ctx, int world, int me, int64_t n_relations, int64_t n_entities,
                              int64_t rows_per_rank, int64_t max_batch, float* shard,
@@ -241,6 +260,7 @@ HOLE_API int hole_shard_steps_host(hole_ctx* ctx, const int32_t* triples_host, i
                                    uint64_t seed, uint64_t first_step, float margin, const float* lr,
                                    float* loss_sum_host, void* stream);
 HOLE_API int hole_shard_poll(hole_ctx* ctx, int* timed_out, void* stream);
+HOLE_API int hole_shard_set_optimizer(hole_ctx* ctx, int optimizer, float* accum_shard);
 /* Measurement hook: with hole_profile_enable on, summed milliseconds of the step's phases
  * [post, K1 (incl. its wait for the peers' shards), K3, finish, apply (incl. its wait for the peers'
  * deltas)] -> phase_ms5 [host, double[5]], and the number of steps measured since the last read. */
