@@ -11,11 +11,13 @@
 //   warp 1      MMA issuer (one elected lane): tcgen05.mma cta_group::1, M=128 N=256 K=16,
 //               accumulators double-buffered in TMEM (2 x 256 columns)
 //   warps 2..9  epilogue: tcgen05.ld 32 columns at a time, compare against the row's
-//               threshold, count; two warps per TMEM lane quarter split the columns
+//               threshold, count, and merge-join the row's filter slice with the counted columns;
+//               two warps per TMEM lane quarter split the columns
 #include <cuda.h>
 #include <cuda_bf16.h>
 
 #include <algorithm>
+#include <climits>
 
 #include "hole_common.cuh"
 #include "hole_ccorr_core.cuh"
@@ -59,11 +61,12 @@ struct RankParams {
   const float* true_score;     // [Q]   COUNT: thresholds
   const int32_t* true_idx;     // [Qpad] shard-local index of the true candidate (may be out of range)
   int32_t* raw_cnt;            // [Q]   COUNT: += count
-  int32_t* filt_cnt;           // [Q]   COUNT: += count (filter hits are subtracted afterwards)
+  int32_t* filt_cnt;           // [Q]   COUNT: += count minus the filtered candidates among it
   float* true_out;             // [Q]   DIAG: score of the true candidate if it lives in this shard
   // top-k epilogue (EPI_TOPK)
   int topk;                    // k
   uint64_t* tk_keys;           // [Qpad][n_chunks][2][k] per-thread candidate lists (binary max-heaps)
+  // COUNT and EPI_TOPK
   const int64_t* f_off;        // [Q+1] filter CSR, or null
   const int32_t* f_ids;        //       ids ascending within a query's slice
   int64_t ent_begin;
@@ -196,12 +199,47 @@ __host__ __device__ constexpr uint32_t umma_idesc_bf16(int M, int N) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
+// A thread's place in its query row's filter slice (known-true candidates, holE.py:454-461), whose ids are
+// ascending: the thread meets its columns in ascending order, so the slice is merge-joined with them.
+struct FilterCursor {
+  int64_t fp, f1;            // f_ids[fp .. f1): ids not yet passed
+  int next, after;           // shard-local indices of f_ids[fp] and f_ids[fp + 1], INT_MAX past the end; `after`
+                             // is loaded one step ahead, so that a step of the cursor does not wait for memory
+};
+
+__device__ __forceinline__ int filter_id_at(const int32_t* __restrict__ ids, int64_t i, int64_t f1, int64_t ent_begin) {
+  return i < f1 ? (int)((int64_t)ids[i] - ent_begin) : INT_MAX;
+}
+
+// First id of f_ids[lo, hi) that is >= id (hi if none).
+__device__ __forceinline__ int64_t lower_bound_id(const int32_t* __restrict__ ids, int64_t lo, int64_t hi, int64_t id) {
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) >> 1;
+    if ((int64_t)ids[mid] < id) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+
+// Moves the cursor past every copy of the id it stands on (a repeated id is one candidate).
+__device__ __forceinline__ void filter_advance(FilterCursor& f, const int32_t* __restrict__ ids, int64_t ent_begin) {
+  const int cur = f.next;
+  do {
+    ++f.fp;
+    f.next = f.after;
+    f.after = filter_id_at(ids, f.fp + 1, f.f1, ent_begin);
+  } while (f.next <= cur);
+}
+
 // Rank-count epilogue of 32 accumulator columns held by one thread (one query row): how many of the
-// candidates j0 .. j0+31 rank before the true one.  thr_hi = nextafter(thr): s <= thr <=> s < thr_hi;
-// candidates with index < tie win ties (holE.py:427-469 walks the heap in index order).
+// candidates j0 .. j0+31 rank before the true one (c0), and how many of those are filtered (fc).
+// thr_hi = nextafter(thr): s <= thr <=> s < thr_hi; candidates with index < tie win ties (holE.py:427-469
+// walks the heap in index order).  A filtered column is subtracted exactly when this very compare counted
+// it, so filt_before is exact with respect to raw_before; the true column itself never counts (s == thr,
+// j == tie), whether or not it is filtered.
 __device__ __forceinline__ void epi_count32(const uint32_t (&v)[32], int j0, float thr, float thr_hi, int tie,
-                                            int Nc, int& c0) {
-  const bool slow = (j0 < tie && tie < j0 + 32) || (j0 + 32 > Nc);
+                                            int Nc, int& c0, FilterCursor& f, const int32_t* __restrict__ f_ids,
+                                            int64_t ent_begin, int& fc) {
+  const bool slow = (j0 < tie && tie < j0 + 32) || (j0 + 32 > Nc) || (f.next < j0 + 32);
   if (!__any_sync(0xffffffffu, slow)) {
     const float tt = (j0 + 32 <= tie) ? thr_hi : thr;
     // (A two-instruction FSETP + predicated-add form on four independent counters measured 2-5 %
@@ -215,26 +253,40 @@ __device__ __forceinline__ void epi_count32(const uint32_t (&v)[32], int j0, flo
       const float tt = (j < tie) ? thr_hi : thr;
       c0 += (j < Nc && __uint_as_float(v[k]) < tt) ? 1 : 0;
     }
+    // ids below j0 (the other column group's half of a tile, or before this thread's first column) are passed
+    // without a compare
+    while (f.next < j0 + 32) {
+      const int j = f.next, c = j - j0;
+      if (c >= 0) {
+        float s = 0.f;
+#pragma unroll
+        for (int i = 0; i < 32; ++i) s = (i == c) ? __uint_as_float(v[i]) : s;     // no dynamic register index
+        const float tt = (j < tie) ? thr_hi : thr;
+        fc += (j < Nc && s < tt) ? 1 : 0;
+      }
+      filter_advance(f, f_ids, ent_begin);
+    }
+    __syncwarp();          // reconverge before the next .sync.aligned tcgen05 instruction
   }
 }
 // 128 columns (four chunks) of one accumulator row; the TMEM load of a chunk is in flight while
 // the previous one is counted.
-__device__ __forceinline__ int epi_count128(uint32_t taddr0, int j0, float thr, float thr_hi, int tie, int Nc) {
+__device__ __forceinline__ void epi_count128(uint32_t taddr0, int j0, float thr, float thr_hi, int tie, int Nc,
+                                             int& c0, FilterCursor& f, const int32_t* __restrict__ f_ids,
+                                             int64_t ent_begin, int& fc) {
   uint32_t va[32], vb[32];
-  int c0 = 0;
   tmem_ld32_async(taddr0, va);
   tmem_ld_wait(va);
   tmem_ld32_async(taddr0 + 32, vb);
-  epi_count32(va, j0, thr, thr_hi, tie, Nc, c0);
+  epi_count32(va, j0, thr, thr_hi, tie, Nc, c0, f, f_ids, ent_begin, fc);
   tmem_ld_wait(vb);
   tmem_ld32_async(taddr0 + 64, va);
-  epi_count32(vb, j0 + 32, thr, thr_hi, tie, Nc, c0);
+  epi_count32(vb, j0 + 32, thr, thr_hi, tie, Nc, c0, f, f_ids, ent_begin, fc);
   tmem_ld_wait(va);
   tmem_ld32_async(taddr0 + 96, vb);
-  epi_count32(va, j0 + 64, thr, thr_hi, tie, Nc, c0);
+  epi_count32(va, j0 + 64, thr, thr_hi, tie, Nc, c0, f, f_ids, ent_begin, fc);
   tmem_ld_wait(vb);
-  epi_count32(vb, j0 + 96, thr, thr_hi, tie, Nc, c0);
-  return c0;
+  epi_count32(vb, j0 + 96, thr, thr_hi, tie, Nc, c0, f, f_ids, ent_begin, fc);
 }
 
 // ---- top-k epilogue.  A candidate is the 64-bit key (order-preserving bits of s, local index j): ascending
@@ -531,24 +583,37 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       const int m_tile = item / p.n_chunks, chunk = item % p.n_chunks;
       const int q = m_tile * BM + row_in_tile;
       const bool qok = q < p.Q;
-      float thr = -INFINITY, thr_hi = -INFINITY;
-      int tie = 0;
-      if (p.mode == MODE_COUNT && qok) {
-        thr = p.true_score[q];
-        thr_hi = nextafterf(thr, INFINITY);          // s <= thr  <=>  s < thr_hi
-        const int ti = p.true_idx[q];
-        tie = ti < 0 ? 0 : (ti > p.Nc ? p.Nc : ti);  // candidates with local index < tie win ties
-      }
-      int cnt = 0;
       const int t0 = chunk * p.chunk_tiles;
       const int t1 = (p.mode == MODE_DIAG) ? t0 + 1 : min(p.n_tiles, t0 + p.chunk_tiles);
+      float thr = -INFINITY, thr_hi = -INFINITY;
+      int tie = 0;
+      FilterCursor fcur{0, 0, INT_MAX, INT_MAX};
+      if (p.mode == MODE_COUNT && qok) {
+        int64_t f0 = 0;
+        if (p.f_off != nullptr) { f0 = p.f_off[q]; fcur.f1 = p.f_off[q + 1]; }
+        thr = p.true_score[q];
+        const int ti = p.true_idx[q];
+        if (p.f_off != nullptr) {
+          // A long slice is entered by binary search at this thread's first column; a short one from its start
+          // (the merge-join passes ids below the thread's columns).
+          if (fcur.f1 - f0 > 16)
+            f0 = lower_bound_id(p.f_ids, f0, fcur.f1, p.ent_begin + (int64_t)t0 * BN + cgrp * EPI_COLS);
+          fcur.fp = f0;
+          fcur.next = filter_id_at(p.f_ids, f0, fcur.f1, p.ent_begin);
+          fcur.after = filter_id_at(p.f_ids, f0 + 1, fcur.f1, p.ent_begin);
+        }
+        thr_hi = nextafterf(thr, INFINITY);          // s <= thr  <=>  s < thr_hi
+        tie = ti < 0 ? 0 : (ti > p.Nc ? p.Nc : ti);  // candidates with local index < tie win ties
+      }
+      int cnt = 0, fcnt = 0;
       for (int t = t0; t < t1; ++t) {
         mbar_wait(&sl->tmem_full[acc], acc_phase);
         tc_fence_after();
         const uint32_t taddr0 = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * BN + cgrp * EPI_COLS);
         if (p.mode == MODE_COUNT) {
           static_assert(EPI_COLS == 128, "epi_count128 covers 128 columns per warp");
-          cnt += epi_count128(taddr0, t * BN + cgrp * EPI_COLS, thr, thr_hi, tie, p.Nc);
+          epi_count128(taddr0, t * BN + cgrp * EPI_COLS, thr, thr_hi, tie, p.Nc, cnt, fcur, p.f_ids, p.ent_begin,
+                       fcnt);
         } else if (cgrp == (quarter * 32) / EPI_COLS) {
           // DIAG: row i of the tile wants column i, which lives in chunk `quarter`, register `lane`
           uint32_t v[32];
@@ -568,7 +633,7 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       }
       if (p.mode == MODE_COUNT && qok && cnt != 0) {
         atomicAdd(&p.raw_cnt[q], cnt);
-        atomicAdd(&p.filt_cnt[q], cnt);
+        atomicAdd(&p.filt_cnt[q], cnt - fcnt);
       }
     }
   }
@@ -865,44 +930,6 @@ hole_rank_gather_true_kernel(const __nv_bfloat16* __restrict__ cand, const int32
   const int nv = K / 8;                                  // a multiple of 8 (K is a multiple of 64)
 #pragma unroll 4
   for (int k = sub; k < nv; k += 8) dst[k] = ok ? src[k] : make_uint4(0, 0, 0, 0);
-}
-
-// Filtered counts: one warp per query walks its filter list (known-true candidates,
-// holE.py:454-461) and removes those that rank before the true one.  Scores are fp32 dot
-// products of the same bf16 operands (CUDA cores): identical to the tensor-core value except
-// for accumulation order, i.e. only exact near-ties can differ.
-__global__ void __launch_bounds__(256)
-hole_rank_filter_kernel(const __nv_bfloat16* __restrict__ qp, const __nv_bfloat16* __restrict__ cand,
-                        int K, int parts, const int64_t* __restrict__ foff, const int32_t* __restrict__ fids,
-                        int64_t ent_begin, int Nc, const float* __restrict__ true_score,
-                        const int32_t* __restrict__ true_idx, int Q, int32_t* __restrict__ filt_cnt) {
-  const int lane = threadIdx.x & 31;
-  const int64_t qi = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
-  if (qi >= Q) return;
-  const float thr = true_score[qi];
-  const int ti = true_idx[qi];
-  const __nv_bfloat16* qrow = qp + (size_t)qi * K * parts;
-  int hits = 0;
-  for (int64_t p = foff[qi]; p < foff[qi + 1]; ++p) {
-    const int64_t j = (int64_t)fids[p] - ent_begin;
-    // warp-uniform.  The true candidate never ranks before itself; its CUDA-core score may differ from the
-    // tensor-core threshold in the last bits, so it is skipped rather than compared.
-    if (j < 0 || j >= Nc || j == ti) continue;
-    const __nv_bfloat16* crow = cand + (size_t)j * K * parts;
-    float s = 0.f;
-    for (int k = lane; k < K; k += 32) {
-      const float qh = __bfloat162float(qrow[k]), ch = __bfloat162float(crow[k]);
-      s = fmaf(qh, ch, s);
-      if (parts == 2) {
-        s = fmaf(__bfloat162float(qrow[K + k]), ch, s);
-        s = fmaf(qh, __bfloat162float(crow[K + k]), s);
-      }
-    }
-#pragma unroll
-    for (int o2 = 16; o2 > 0; o2 >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o2);
-    hits += (s < thr || (s == thr && j < ti)) ? 1 : 0;
-  }
-  if (lane == 0 && hits != 0) atomicSub(&filt_cnt[qi], hits);
 }
 
 // hole_topk, after the contraction: one block per output row.
@@ -1329,14 +1356,13 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
   p.true_score = true_score_io;
   p.raw_cnt = raw_before;
   p.filt_cnt = filt_before;
+  p.f_off = filter_off;
+  p.f_ids = filter_ids;
+  p.ent_begin = ent_begin;
   const int grid = std::min(p.m_tiles * p.n_chunks, c->sm_count);
   if (parts == 2) hole_rank_kernel<2, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
   else hole_rank_kernel<1, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
   HOLE_LAUNCHED();
-  if (filter_off != nullptr) {
-    hole_rank_filter_kernel<<<(unsigned)((Q + 7) / 8), 256, 0, st>>>(w->qp, w->cand, K, parts, filter_off, filter_ids, ent_begin, Nc, true_score_io, w->true_idx, (int)Q, filt_before);
-    HOLE_LAUNCHED();
-  }
   return HOLE_OK;
 }
 

@@ -327,8 +327,13 @@ HOLE_API int hole_train_steps_host(hole_ctx* ctx, float* table, const int32_t* t
  *                  holE.py:231, 446-453; ties by smaller candidate id, holE.py:434)
  * filt_before[q] = raw_before[q] - #{f in filter[q], f in range : (s_f, f) < (s_true, true_id)}
  *                  (train/valid-true candidates do not advance the filtered rank,
- *                  holE.py:454-463).  rank = 1 + count.
- * filter_off int64[Q+1] / filter_ids int32[.] may be NULL (no filtering).
+ *                  holE.py:454-463), with s_f the very score raw_before was counted with: a filtered
+ *                  candidate is subtracted exactly when it was counted.  With compute_true != 0 the true
+ *                  candidate never counts (it is not before itself); with compute_true == 0 its column is an
+ *                  ordinary candidate against the given threshold.  rank = 1 + count.
+ * filter_off int64[Q+1] / filter_ids int32[.] may be NULL (no filtering); the ids of each slice must be
+ * ASCENDING (the count epilogue merge-joins them with its columns; data.build_filter_csr produces them so).
+ * A slice is a set: an id listed twice is subtracted once.  Ids outside [ent_begin, ent_end) are ignored.
  * true_score_io float32[Q]: if compute_true != 0 it is written for queries whose true
  * candidate lies in [ent_begin, ent_end) and left untouched otherwise (so candidate shards
  * on several GPUs can be combined by the caller); if compute_true == 0 it is read.

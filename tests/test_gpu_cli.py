@@ -178,7 +178,7 @@ def test_typed_candidate_protocol_matches_heap_restatement():
     # bf16 operands move a score by at most 4e-3 |q||e| <= 4e-3, so a rank may differ from the exact one only
     # by candidates within 8e-3 of the item's own fp64 score
     E64 = kg.E.astype(np.float64)
-    k = 0
+    k = n_exact = 0
     for h in heads:
         triples = np.array([(h, t, r) for t in tails for r in rels])
         s64 = O.score(E64, triples, np.float64)
@@ -194,8 +194,11 @@ def test_typed_candidate_protocol_matches_heap_restatement():
                 f_sure = int(((s64 < me - 8e-3) & insample).sum())
                 f_maybe = int(((s64 <= me + 8e-3) & insample).sum())
                 assert lo - f_maybe + 1 <= filt[k] <= hi - f_sure + 1
+                if hi == lo:                   # no other candidate inside the band: both ranks are exact
+                    assert raw[k] == lo + 1 and filt[k] == lo - f_sure + 1
+                    n_exact += 1
                 k += 1
-    assert k == len(raw)
+    assert k == len(raw) and n_exact > 0
     m = hole.score_mrr(raw, filt, log=lambda *a: None)
     mw = O.score_mrr(want_r, want_f)
     assert abs(m["filtered_mrr"] - mw["filtered_mrr"]) < 5e-3
