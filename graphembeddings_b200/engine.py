@@ -170,11 +170,13 @@ class HoleEngine:
                                        C.byref(side), _stream()))
         return int(side.value), neg
 
-    def evaluate_triples(self, triples):
-        """holE.py:179 evaluate_triples -> sigma(score) float32[B] on device."""
+    def evaluate_triples(self, triples, table=None):
+        """holE.py:179 evaluate_triples -> sigma(score) float32[B] on device.  table: a device-layout table to
+        score on instead of self.table (a side table of fetched rows, sharded.score_on_shards)."""
         t = self._triples(triples)
         out = torch.empty(t.shape[0], dtype=torch.float32, device=self.device)
-        check(self.lib.hole_score(self._ctx, _ptr(self.table), _ptr(t), t.shape[0], _ptr(out), _stream()))
+        check(self.lib.hole_score(self._ctx, _ptr(self.table if table is None else table), _ptr(t), t.shape[0],
+                                  _ptr(out), _stream()))
         return out
 
     def train_step(self, pos, neg_ent, side, margin, lr, return_sigma=False):

@@ -3,6 +3,7 @@ outputs in --output_dir, no TensorFlow.
 
     python -m graphembeddings_b200.hole --data_dir D --output_dir O [flags of holE.py:598-619]
     python -m graphembeddings_b200.hole --data_dir D --output_dir O --infer
+    python -m torch.distributed.run --nproc-per-node N -m graphembeddings_b200.hole --data_dir D --output_dir O --gpus N
 
 Function names follow the reference: init_data (holE.py:44-94), evaluate_batch (205-234),
 run_training (249-370), init_inference_data (381-424), eval_link_prediction (427-472),
@@ -144,19 +145,24 @@ def init_inference_data(flags=None):
 # --------------------------------------------------------------------------------------
 # model pieces on the engine
 # --------------------------------------------------------------------------------------
+def type_tables(entity_count, id_to_type):
+    """(type_of, csr_off, csr_ids) of the corruption sampler from the metadata's row -> type map."""
+    names = {}
+    type_of = np.full(entity_count, -1, dtype=np.int32)
+    for idx, t in id_to_type.items():
+        type_of[idx] = names.setdefault(t, len(names))
+    if (type_of < 0).any():
+        raise ValueError(f"{int((type_of < 0).sum())} table rows have no type in the metadata "
+                         f"(first: {int(np.flatnonzero(type_of < 0)[0])})")
+    off, ids = D.build_type_csr(type_of, len(names))
+    return type_of, off, ids
+
+
 def make_engine(entity_count, relation_count, dim, embeddings, id_to_type=None, device=0):
     eng = HoleEngine(entity_count, dim, device).set_embeddings(embeddings)
     eng.set_relation_count(max(1, relation_count))
     if id_to_type is not None:
-        names = {}
-        type_of = np.full(entity_count, -1, dtype=np.int32)
-        for idx, t in id_to_type.items():
-            type_of[idx] = names.setdefault(t, len(names))
-        if (type_of < 0).any():
-            raise ValueError(f"{int((type_of < 0).sum())} table rows have no type in the metadata "
-                             f"(first: {int(np.flatnonzero(type_of < 0)[0])})")
-        off, ids = D.build_type_csr(type_of, len(names))
-        eng.set_types(type_of, off, ids)
+        eng.set_types(*type_tables(entity_count, id_to_type))
     return eng
 
 
@@ -211,12 +217,42 @@ def check_optimizer_flags(flags):
 
 def save_checkpoint(eng, output_dir, global_step, metadata_names=None):
     """saver.save(sess, output_dir + '/model.ckpt') (holE.py:359) + checkpoint state file."""
-    E = eng.embeddings().cpu().numpy()
-    tensors = {"embeddings": E, "batch/Variable": np.array(global_step, dtype=np.int32)}
-    if eng.accum is not None:       # AdagradOptimizer's slot, under the name TF's Saver gives it
-        tensors[ADAGRAD_SLOT] = eng.accumulator().cpu().numpy()
+    write_checkpoint(output_dir, eng.embeddings(), global_step,
+                     eng.accumulator() if eng.accum is not None else None)
+
+
+def write_checkpoint(output_dir, E, global_step, A=None):
+    """The bundle of save_checkpoint from the [N, dim] table E and AdaGrad accumulator A (None: no slot)."""
+    tensors = {"embeddings": E.cpu().numpy(), "batch/Variable": np.array(global_step, dtype=np.int32)}
+    if A is not None:       # AdagradOptimizer's slot, under the name TF's Saver gives it
+        tensors[ADAGRAD_SLOT] = A.cpu().numpy()
     tf_bundle.save_bundle(os.path.join(output_dir, 'model.ckpt'), tensors)
     tf_bundle.write_checkpoint_state(output_dir)
+
+
+def write_summaries(slog, events, global_step, lr_now, parts, batch_parts=None):
+    """One validation point's summaries.tsv row and TensorBoard event; returns valid_loss_mean.  parts: the
+    validation twin's (name, tensor) pairs, "loss" among them; batch_parts: (loss, sigma+, sigma-) of the next
+    training batch (scored, not trained on) or None.  The merged summaries of holE.py:352-353, under the
+    reference's name scopes."""
+    vlm = float(dict(parts)["loss"].mean())
+    row = {"step": global_step, "valid_loss_mean": vlm, "learning_rate": lr_now}
+    for nm, var in parts:
+        row.update({f"{nm}_{k}": v for k, v in summarize(var).items()})
+    slog.write("\t".join(f"{k}={v}" for k, v in row.items()) + "\n")
+    slog.flush()
+    scal, hist = {"batch/learn/learning_rate": lr_now}, {}
+    scopes = {"pos": "validation/positive/eval", "neg": "validation/corrupt/eval", "loss": "validation"}
+    for nm, var in parts:
+        sc_, hi_ = tf_events.summarize_tags(scopes[nm], var.float().cpu().numpy())
+        scal.update(sc_); hist.update(hi_)
+    if batch_parts is not None:
+        tl, tp, tn = batch_parts
+        for scope, var in (("batch/eval/positive/eval", tp), ("batch/eval/corrupt/eval", tn), ("batch/eval", tl)):
+            sc_, hi_ = tf_events.summarize_tags(scope, var.float().cpu().numpy())
+            scal.update(sc_); hist.update(hi_)
+    events.add_summary(global_step, scal, hist)
+    return vlm
 
 
 def load_checkpoint(output_dir):
@@ -313,31 +349,13 @@ def run_training(data, flags=None, seed=0, max_steps=None, log=print):
                         else:
                             vloss, vp, vn = evaluate_batch(eng, vb, seed, global_step, flags.margin)
                             parts = (("pos", vp), ("neg", vn), ("loss", vloss))
-                        vlm = float(vloss.mean())
                         lr_now = float(inverse_time_decay(flags.learning_rate, global_step, decay_steps,
                                                           flags.learning_decay_rate))
-                        row = {"step": global_step, "valid_loss_mean": vlm, "learning_rate": lr_now}
-                        for nm, var in parts:
-                            row.update({f"{nm}_{k}": v for k, v in summarize(var).items()})
-                        slog.write("\t".join(f"{k}={v}" for k, v in row.items()) + "\n")
-                        slog.flush()
-                        # the merged summaries of holE.py:352-353: the validation twin's scalars and
-                        # histograms, the training graph's on the next training batch (scored, not
-                        # trained on), and the learning rate -- under the reference's name scopes
-                        scal, hist = {"batch/learn/learning_rate": lr_now}, {}
-                        scopes = {"pos": "validation/positive/eval", "neg": "validation/corrupt/eval",
-                                  "loss": "validation"}
-                        for nm, var in parts:
-                            sc_, hi_ = tf_events.summarize_tags(scopes[nm], var.float().cpu().numpy())
-                            scal.update(sc_); hist.update(hi_)
+                        batch_parts = None
                         if not flags.log_loss:
                             tb = shuffled[(batch - 1) * B:batch * B]
-                            tl, tp, tn = evaluate_batch(eng, tb, seed, global_step, flags.margin)
-                            for scope, var in (("batch/eval/positive/eval", tp), ("batch/eval/corrupt/eval", tn),
-                                               ("batch/eval", tl)):
-                                sc_, hi_ = tf_events.summarize_tags(scope, var.float().cpu().numpy())
-                                scal.update(sc_); hist.update(hi_)
-                        events.add_summary(global_step, scal, hist)
+                            batch_parts = evaluate_batch(eng, tb, seed, global_step, flags.margin)
+                        vlm = write_summaries(slog, events, global_step, lr_now, parts, batch_parts)
                         log('\tStep {} Validation Loss: {}...'.format(global_step, vlm))
                         if vlm < pocket_loss:       # pocket checkpoint (holE.py:357-360)
                             pocket_loss = vlm
@@ -374,6 +392,234 @@ def run_training(data, flags=None, seed=0, max_steps=None, log=print):
         save_checkpoint(eng, flags.output_dir, global_step)    # never validated: still leave a model
     log('Trained {} steps in {:.1f}s'.format(steps_done, time.time() - t_start))
     return eng, global_step
+
+
+# --------------------------------------------------------------------------------------
+# training driver on several GPUs (--gpus N): the row-sharded trainer of sharded.py
+# --------------------------------------------------------------------------------------
+def check_gpus_flags(flags, world):
+    """The refusals of a --gpus run, all made before any CUDA work.  world: WORLD_SIZE of the launch."""
+    n = flags.gpus
+    launch = (f"python -m torch.distributed.run --nproc-per-node {n} -m graphembeddings_b200.hole ... --gpus {n}"
+              if n > 1 else "python -m graphembeddings_b200.hole ... (no torch.distributed.run)")
+    if n < 1:
+        raise SystemExit(f"--gpus must be >= 1, got {n}")
+    if world != n:
+        raise SystemExit(f"--gpus {n} but WORLD_SIZE={world}: launch with {launch}")
+    if flags.infer:
+        if n > 1:
+            raise SystemExit("--infer runs on one GPU (the checkpoint holds the whole table): run it with --gpus 1 "
+                             "and without torch.distributed.run")
+        return
+    if flags.batch_size % n:
+        lo = flags.batch_size - flags.batch_size % n
+        raise SystemExit(f"--batch_size {flags.batch_size} is the global batch and must be a multiple of --gpus {n}: "
+                         f"use --batch_size {lo or n} or {lo + n}")
+    if flags.log_loss:
+        raise SystemExit("--log_loss has no row-sharded step: train it on one GPU (--gpus 1)")
+    if getattr(flags, 'score_variant', 'complex') != 'complex':
+        raise SystemExit("--score_variant ccorr_tanh has no row-sharded step: train it on one GPU (--gpus 1)")
+    if getattr(flags, 'optimizer', 'sgd') == 'adagrad' and os.environ.get("HOLE_SHARDED_NCCL") == "1":
+        raise SystemExit("--optimizer adagrad on several GPUs needs the NVLink peer-memory trainer, which "
+                         "HOLE_SHARDED_NCCL=1 turns off: unset it, or train with --optimizer sgd")
+
+
+def rank_rows(order, batch_size, world, rank):
+    """This rank's share of every whole global batch of `order` (1-D), step-major: rows [s*b, (s+1)*b) of the
+    result, b = batch_size / world, are rows [s*batch_size + rank*b, s*batch_size + (rank+1)*b) of `order`."""
+    b = batch_size // world
+    n = order.shape[0] // batch_size
+    return order[:n * batch_size].view(n, world, b)[:, rank].reshape(-1)
+
+
+def valid_split(n, world):
+    """Offsets o_0 = 0 <= o_1 <= ... <= o_world = n: rank k scores rows [o_k, o_{k+1}) of a validation batch."""
+    return [k * n // world for k in range(world + 1)]
+
+
+def _from_rank0(dist, value):
+    """Rank 0's value on every rank: a decision that leads into a collective is made once."""
+    if dist is None:
+        return value
+    box = [value]
+    dist.broadcast_object_list(box, src=0)
+    return box[0]
+
+
+def _gather_in_rank_order(dist, world, x, sizes):
+    """Every rank's 1-D x (rank k's has sizes[k] entries), concatenated in rank order, on every rank."""
+    if world == 1:
+        return x
+    buf = torch.zeros(max(sizes), dtype=x.dtype, device=x.device)
+    buf[:x.shape[0]] = x
+    out = [torch.empty_like(buf) for _ in range(world)]
+    dist.all_gather(out, buf)
+    return torch.cat([o[:s] for o, s in zip(out, sizes)])
+
+
+def evaluate_batch_sharded(tr, offsets, part, seed, step, margin, dist):
+    """evaluate_batch on the row-sharded table.  The batch is split at offsets o_0 = 0 <= ... <= o_world; `part` is
+    this rank's rows [o_rank, o_rank+1) (device [n,3]), corrupted with the draws hole_corrupt makes for them over the
+    whole batch (index_base = o_rank) and scored on the shards.  Every rank gets the whole (loss, sigma+, sigma-) in
+    batch order.  Collective."""
+    world = len(offsets) - 1
+    base = offsets[tr.my_rank]
+    assert part.shape[0] == offsets[tr.my_rank + 1] - base
+    side, neg = tr.be.eng.corrupt_batch(part, seed, step, base)
+    corrupt = part.clone()
+    corrupt[:, 0 if side else 1] = neg
+    s = tr.score(torch.cat([part, corrupt]))
+    sizes = [offsets[k + 1] - offsets[k] for k in range(world)]
+    vp, vn = (_gather_in_rank_order(dist, world, x, sizes) for x in (s[:part.shape[0]], s[part.shape[0]:]))
+    return torch.clamp(vp - vn + margin, min=0.0), vp, vn
+
+
+def run_training_sharded(data, flags, dist, rank, world, local_rank, seed=0, max_steps=None, log=print):
+    """run_training on `world` GPUs, one process per GPU (dist = torch.distributed, or None at world 1): the table is
+    row-sharded (sharded.make_trainer) and each rank trains rows [rank*B/world, (rank+1)*B/world) of every global
+    batch of B = --batch_size triples, taken from the one-GPU driver's shuffled order.  The steps, learning rates,
+    seeds, validation points, summaries, pocket checkpoints and outputs are the one-GPU driver's; rank 0 logs and
+    writes the files.  Returns the final global step."""
+    from . import sharded
+    say = log if rank == 0 else (lambda *a: None)
+    batch_count = data.triple_count // flags.batch_size
+    say('Embedding dimension: ', flags.embedding_dim, 'Batch size: ', flags.batch_size,
+        'Batch count: ', batch_count, 'GPUs: ', world)
+    if flags.embedding_dim % 2:
+        raise ValueError("embedding_dim must be even (holE.py:164-165 splits the row in halves)")
+    check_optimizer_flags(flags)
+    check_gpus_flags(flags, world)
+    # Warning: this will clobber existing summaries (holE.py:253-260).  Rank 0 decides, or rank 1 would find the
+    # directory rank 0 has just made.
+    refuse = False
+    if rank == 0:
+        refuse = not flags.resume_checkpoint and os.path.isdir(flags.output_dir)
+        if not refuse:
+            os.makedirs(flags.output_dir, exist_ok=True)
+    if _from_rank0(dist, refuse):
+        raise Exception("WARNING: " + flags.output_dir + " already exists!")
+
+    global_step = 0
+    adagrad = getattr(flags, 'optimizer', 'sgd') == 'adagrad'
+    A = None
+    if flags.resume_checkpoint:
+        E, global_step = load_checkpoint(flags.output_dir)
+        if adagrad:
+            A = load_accumulator(flags.output_dir)
+    else:
+        E = D.init_embeddings(data.entity_count, flags.embedding_dim, np.random.default_rng(seed))
+    B, R = flags.batch_size, data.relation_count
+    Bl = B // world
+    be = sharded.CudaBackend(R, flags.embedding_dim, Bl, local_rank, *type_tables(data.entity_count, data.id_to_type))
+    tr = sharded.make_trainer(R, data.entity_count - R, flags.embedding_dim, be, dist, log=say)
+    p2p = isinstance(tr, sharded.P2PRowShardedTrainer)
+    if adagrad:
+        if not p2p:
+            raise SystemExit("--optimizer adagrad on several GPUs needs the NVLink peer-memory trainer, and the GPUs "
+                             "of this job cannot map each other's memory: train with --optimizer sgd")
+        tr.set_optimizer("adagrad", flags.adagrad_initial_accumulator)
+    tr.load_embeddings(E)
+    if A is not None:
+        tr.load_accumulator(A)
+    del E, A
+    dev = be.device
+
+    def save(step):
+        """All ranks gather (collective), rank 0 writes the one-GPU checkpoint layout."""
+        E_, A_ = tr.gather_embeddings(), tr.gather_accumulator() if adagrad else None
+        if rank == 0:
+            write_checkpoint(flags.output_dir, E_, step, A_)
+
+    triples_dev = torch.from_numpy(data.triples).to(dev)
+    valid = data.validation_triples
+    decay_steps = flags.learning_decay_steps * batch_count
+    valid_every = max(1, batch_count // 16)      # holE.py:351 (divides by zero if batch_count < 16)
+    gen = torch.Generator(device=dev)
+    gen.manual_seed(seed)
+    vrng = np.random.default_rng(seed + 1)
+    valid_dev = torch.from_numpy(np.ascontiguousarray(valid)).to(dev) if len(valid) else None
+    events = tf_events.EventFileWriter(flags.output_dir) if rank == 0 else None
+    slog = open(os.path.join(flags.output_dir, 'summaries.tsv'), 'a') if rank == 0 else None
+    pocket_loss = 2.
+    steps_done = 0
+    t_start = time.time()
+    try:
+        for epoch in range(1, flags.num_epochs + 1):
+            say('Initializing projector...')
+            if rank == 0:
+                tf_bundle.write_projector_config(flags.output_dir)
+            say('Training epoch {}...'.format(epoch))
+            perm = torch.randperm(data.triple_count, device=dev, generator=gen)
+            if epoch == 1 and world > 1:      # a different shuffle on one rank would silently train another model
+                ck = (perm.long() * torch.arange(1, data.triple_count + 1, device=dev)).sum().view(1)
+                cks = [torch.empty_like(ck) for _ in range(world)]
+                dist.all_gather(cks, ck)
+                if any(int(c) != int(cks[0]) for c in cks):
+                    raise RuntimeError(f"the ranks drew different epoch permutations (checksums "
+                                       f"{[int(c) for c in cks]}): every rank must run the same torch build and GPU model")
+            mine = triples_dev[rank_rows(perm, B, world, rank)]          # [batch_count * Bl, 3], step-major
+            batch = 1                       # for batch in range(1, batch_count)  (holE.py:340)
+            while batch < batch_count:
+                if batch % valid_every == 0 and len(valid) > 0:
+                    vb = (torch.from_numpy(valid[vrng.integers(0, len(valid), size=B)]).to(dev)
+                          if getattr(flags, "valid_sample", False) else valid_dev)
+                    vo = valid_split(len(vb), world)
+                    vloss, vp, vn = evaluate_batch_sharded(tr, vo, vb[vo[rank]:vo[rank + 1]], seed, global_step,
+                                                           flags.margin, dist)
+                    # the next training batch: my share of it is rows [rank*Bl, (rank+1)*Bl)
+                    tl, tp, tn = evaluate_batch_sharded(tr, [k * Bl for k in range(world + 1)],
+                                                        mine[(batch - 1) * Bl:batch * Bl], seed, global_step,
+                                                        flags.margin, dist)
+                    vlm = None
+                    if rank == 0:
+                        lr_now = float(inverse_time_decay(flags.learning_rate, global_step, decay_steps,
+                                                          flags.learning_decay_rate))
+                        vlm = write_summaries(slog, events, global_step, lr_now,
+                                              (("pos", vp), ("neg", vn), ("loss", vloss)), (tl, tp, tn))
+                        say('\tStep {} Validation Loss: {}...'.format(global_step, vlm))
+                    vlm = _from_rank0(dist, vlm)
+                    if vlm < pocket_loss:       # pocket checkpoint (holE.py:357-360), one decision on every rank
+                        pocket_loss = vlm
+                        save(global_step)
+                        say('Epoch {}, (Model saved with loss {})'.format(epoch, vlm))
+                nxt = min(batch_count, (batch // valid_every + 1) * valid_every)
+                n = nxt - batch
+                if max_steps is not None:
+                    n = min(n, max_steps - steps_done)
+                lrs = [inverse_time_decay(flags.learning_rate, global_step + k, decay_steps,
+                                          flags.learning_decay_rate) for k in range(n)]
+                chunk = mine[(batch - 1) * Bl:(batch - 1 + n) * Bl]
+                if p2p:
+                    tr.train_steps(chunk, Bl, seed, global_step, flags.margin, lrs)
+                else:                           # the all-to-all trainer has no multi-step call
+                    for k in range(n):
+                        tr.train_step(chunk[k * Bl:(k + 1) * Bl], seed, global_step + k, flags.margin, lrs[k])
+                batch += n
+                global_step += n
+                steps_done += n
+                if max_steps is not None and steps_done >= max_steps:
+                    raise StopIteration
+        say('Done training -- epoch limit reached')
+    except StopIteration:
+        say('Done training -- step limit reached')
+    finally:
+        say('Stopping training...')
+        if rank == 0:
+            events.close()
+            slog.close()
+    torch.cuda.synchronize()
+    if p2p:
+        tr.check_barriers()
+    elapsed = time.time() - t_start
+    # never validated: still leave a model (rank 0 looks, every rank enters the gather)
+    if _from_rank0(dist, rank == 0 and not os.path.exists(os.path.join(flags.output_dir, 'model.ckpt.index'))):
+        save(global_step)
+    say('Trained {} steps in {:.1f}s on {} GPUs: {:.4g} triples/s'.format(
+        steps_done, elapsed, world, steps_done * B / max(elapsed, 1e-9)))
+    if p2p:
+        tr.close()
+    be.eng.close()
+    return global_step
 
 
 # --------------------------------------------------------------------------------------
@@ -681,6 +927,11 @@ def build_parser():
                              "place (checkpoints then hold its slot embeddings/Adagrad); hinge loss, complex score only.")
     parser.add_argument('--adagrad_initial_accumulator', type=float, default=0.1,
                         help='AdagradOptimizer initial_accumulator_value (> 0).')
+    parser.add_argument('--gpus', type=int, default=1,
+                        help='Train on N GPUs of this node, the table row-sharded over them and --batch_size the '
+                             'global batch (a multiple of N); N > 1 is launched as python -m torch.distributed.run '
+                             '--nproc-per-node N -m graphembeddings_b200.hole ... --gpus N.  Hinge loss, complex '
+                             'score; --infer runs on one GPU.')
     parser.add_argument('--seed', type=int, default=0)
     parser.add_argument('--max_steps', type=int, default=None, help='Stop after this many steps (testing).')
     return parser
@@ -691,12 +942,35 @@ def main(argv=None):
     FLAGS, _ = build_parser().parse_known_args(argv)
     if FLAGS.save_embeddings:
         raise SystemExit("--save_embeddings (holE.py:501-527, a py2-only debug dump) is out of scope")
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if FLAGS.gpus != 1 or world != 1:
+        check_gpus_flags(FLAGS, world)
     if FLAGS.infer:
         infer_triples(FLAGS)
     else:
         check_optimizer_flags(FLAGS)
-        training_data = init_data(FLAGS)
-        run_training(training_data, FLAGS, seed=FLAGS.seed, max_steps=FLAGS.max_steps)
+        if world > 1:
+            train_distributed(FLAGS, world)
+        else:
+            training_data = init_data(FLAGS)
+            run_training(training_data, FLAGS, seed=FLAGS.seed, max_steps=FLAGS.max_steps)
+
+
+def train_distributed(flags, world):
+    """One rank of a torch.distributed.run launch: device LOCAL_RANK; the NCCL process group serves the rendezvous,
+    the IPC handle exchange and the driver's few host-side collectives."""
+    import contextlib
+    import io
+    import torch.distributed as dist
+    rank, local_rank = int(os.environ["RANK"]), int(os.environ["LOCAL_RANK"])
+    torch.cuda.set_device(local_rank)
+    dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
+    with contextlib.redirect_stdout(sys.stdout if rank == 0 else io.StringIO()):
+        data = init_data(flags)
+    run_training_sharded(data, flags, dist, rank, world, local_rank, seed=flags.seed, max_steps=flags.max_steps)
+    # Only after a clean run: a rank that raised (rank 0 alone writes the files, so an I/O error is rank 0's) must
+    # exit at once rather than wait in a teardown the others never reach; torch.distributed.run then stops them.
+    dist.destroy_process_group()
 
 
 if __name__ == '__main__':

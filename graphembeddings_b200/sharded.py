@@ -268,6 +268,21 @@ class RowShardedTrainer:
                 off += n_k
         return loss
 
+    # ------------------------------------------------------------------ scoring
+    def score(self, triples):
+        """sigma (hole_score) of this rank's triples [n,3] (global row ids) on the sharded table.  Collective: every
+        rank calls it with its own triples (possibly none).  The rows of the heads and tails come from their owners
+        by all-to-all into a side table [relations | fetched rows], as in rank()."""
+        dev = self.shard.device
+        t = torch.as_tensor(triples).to(dev).long()
+        n, R = t.shape[0], self.R
+        uniq, inv = torch.unique(t[:, :2].reshape(-1), return_inverse=True)
+        send_counts, recv_counts = self._route(uniq)
+        ids_in = self._a2a(uniq, send_counts, recv_counts)
+        rows_in = self._a2a(self.shard.index_select(0, ids_in - self.begin + R), recv_counts, send_counts)
+        side = torch.cat([self.shard[:R], rows_in], dim=0)
+        return self.be.eng.evaluate_triples(_side_triples(t, inv, R), table=side)
+
     # ------------------------------------------------------------------ ranking
     def rank(self, queries, side, filter_off=None, filter_ids=None, precision=None):
         """All-entity ranking of (replicated) queries [Q,3] with candidates sharded by row block.
@@ -329,6 +344,41 @@ class RowShardedTrainer:
         finally:
             eng.table = None
         return cnt[0], cnt[1]
+
+
+def _side_triples(t, inv, n_relations):
+    """triples t [n,3] re-indexed to a side table [relations | fetched rows] (inv: torch.unique's inverse of
+    t[:, :2].reshape(-1))."""
+    q = torch.empty((t.shape[0], 3), dtype=torch.int32, device=t.device)
+    q[:, :2] = (n_relations + inv.view(-1, 2)).to(torch.int32)
+    q[:, 2] = t[:, 2].to(torch.int32)
+    return q
+
+
+def score_on_shards(eng, peer_shards, me, n_relations, rows_per, triples):
+    """sigma (hole_score) of triples [n,3] (global row ids) on a row-sharded table read in place.  peer_shards[k] is
+    rank k's shard [relations | entity rows n_relations + k*rows_per, ...], possibly another GPU's memory mapped into
+    eng's device; me: the caller's rank, whose replica of the relation rows is read.  The relation rows and the rows of
+    the heads and tails are copied (hole_gather_rows) into a side table [relations | fetched rows], the triples
+    re-indexed to it and scored there, so sigma is bit for bit that of hole_score on the whole table.  eng: any context
+    of the table's dim on this device.  The caller orders the reads after the owners' last update and before their
+    next one (P2PRowShardedTrainer.score)."""
+    dev = eng.device
+    t = torch.as_tensor(triples).to(dev).long()
+    n, R, world = t.shape[0], int(n_relations), len(peer_shards)
+    if n == 0:
+        return torch.empty(0, dtype=torch.float32, device=dev)
+    uniq, inv = torch.unique(t[:, :2].reshape(-1), return_inverse=True)       # ascending: one run per owner
+    bounds = R + rows_per * torch.arange(1, world + 1, device=dev)
+    cuts = [0] + torch.searchsorted(uniq, bounds).tolist()
+    side = torch.zeros((R + uniq.shape[0], eng.row_stride), dtype=torch.float32, device=dev)
+    if R:          # the relation replicas are bit-identical on every rank: read the local one
+        eng.gather_rows(peer_shards[me], torch.arange(R, device=dev), 0, side[:R])
+    for k in range(world):
+        a, b = cuts[k], cuts[k + 1]
+        if b > a:      # global row g lies at row g - k*rows_per of rank k's shard
+            eng.gather_rows(peer_shards[k], uniq[a:b].contiguous(), -k * rows_per, side[R + a:R + b])
+    return eng.evaluate_triples(_side_triples(t, inv, R), table=side)
 
 
 class PeerMemoryUnavailable(RuntimeError):
@@ -510,6 +560,20 @@ class P2PRowShardedTrainer(RowShardedTrainer):
     def rank(self, *a, **kw):
         self.check_barriers()
         return super().rank(*a, **kw)
+
+    def score(self, triples):
+        """sigma of this rank's triples [n,3] on the sharded table, read in place from the owners' shards over peer
+        memory (score_on_shards).  Collective.  Two conditions keep the reads consistent:
+          1. before the first read, torch.cuda.synchronize(), dist.barrier() and check_barriers(): every owner's
+             apply of the last step has completed, on every rank, and no barrier timed out;
+          2. the gathers are enqueued on this rank's current stream, ahead of its next hole_shard_steps call.  An
+             owner's next apply waits for every rank's "delivered" flag of that step, which a rank raises only after
+             its K1 / K3 of the step, so after these gathers: no row is overwritten under a reader."""
+        torch.cuda.synchronize()
+        if self.world > 1:
+            self.dist.barrier()
+        self.check_barriers()
+        return score_on_shards(self.be.eng, [p[0] for p in self._peers], self.my_rank, self.R, self.rows_per, triples)
 
     def _as_slice(self, pos):
         pos = torch.as_tensor(pos)
