@@ -16,7 +16,6 @@ all-entity filtered head+tail protocol with the unreachable `infer_threshold` ga
 --negative_ratio and --l2_regularization select the logistic branch (holE.py:194-196, 206-220).
 """
 import argparse
-import errno
 import os
 import sys
 import time
@@ -166,14 +165,20 @@ def make_engine(entity_count, relation_count, dim, embeddings, id_to_type=None, 
     return eng
 
 
+def _corrupt_triples(eng, t, seed, step, index_base=0):
+    """t [n,3] (device int32) with the column corrupt_batch draws replaced by its negatives: the head if the side
+    it returns is nonzero, else the tail."""
+    side, neg = eng.corrupt_batch(t, seed, step, index_base)
+    corrupt = t.clone()
+    corrupt[:, 0 if side else 1] = neg
+    return corrupt
+
+
 def evaluate_batch(eng, triple_batch, seed, step, margin):
     """holE.py:222-234 without the update: corrupt, score both, hinge.  Returns
     (loss[B], sigma_pos[B], sigma_neg[B]) device tensors."""
     t = torch.as_tensor(triple_batch, dtype=torch.int32).to(eng.device)
-    side, neg = eng.corrupt_batch(t, seed, step)
-    corrupt = t.clone()
-    corrupt[:, 0 if side else 1] = neg
-    vp, vn = eng.evaluate_triples(t), eng.evaluate_triples(corrupt)
+    vp, vn = eng.evaluate_triples(t), eng.evaluate_triples(_corrupt_triples(eng, t, seed, step))
     return torch.clamp(vp - vn + margin, min=0.0), vp, vn
 
 
@@ -184,11 +189,8 @@ def evaluate_batch_logloss(eng, triple_batch, seed, step, l2, negative_ratio):
     t = torch.as_tensor(triple_batch, dtype=torch.int32).to(eng.device)
     k = int(negative_ratio)
     rows = [-torch.log(eng.evaluate_triples(t))]                 # log(1+exp(-s)) = -log(sigmoid(s))
-    for j in range(k):
-        side, neg = eng.corrupt_batch(t, seed, step * k + j)
-        corrupt = t.clone()
-        corrupt[:, 0 if side else 1] = neg
-        rows.append(-torch.log1p(-eng.evaluate_triples(corrupt)))  # log(1+exp(s)) = -log(1 - sigmoid(s))
+    for j in range(k):                                           # log(1+exp(s)) = -log(1 - sigmoid(s))
+        rows.append(-torch.log1p(-eng.evaluate_triples(_corrupt_triples(eng, t, seed, step * k + j))))
     l2_loss = 0.5 * (eng.table.double() ** 2).sum()
     return torch.stack(rows) + float(l2) * l2_loss.float()
 
@@ -274,123 +276,158 @@ def load_accumulator(output_dir):
 # --------------------------------------------------------------------------------------
 # training driver
 # --------------------------------------------------------------------------------------
-def run_training(data, flags=None, seed=0, max_steps=None, log=print):
-    flags = flags or FLAGS
-    batch_count = data.triple_count // flags.batch_size
-    log('Embedding dimension: ', flags.embedding_dim, 'Batch size: ', flags.batch_size,
-        'Batch count: ', batch_count)
+def _train_loop(data, flags, dist, rank, world, seed, max_steps, log, open_table):
+    """holE.py's training loop (249-370) on `world` ranks (dist None, rank 0, world 1: one GPU).  open_table(E, A)
+    makes the table from the initial [N, dim] embeddings and AdaGrad accumulator (None: none to restore) and returns
+    (device, train, score, save):
+      train(rows, first_step, lrs)  trains len(lrs) consecutive steps on this rank's rows [len(lrs)*B/world, 3];
+      score(vb, tb, step)           scores the validation triples vb and this rank's rows tb of the next training
+                                    batch: (parts, batch_parts) of write_summaries on rank 0 (collective);
+      save(step)                    writes the checkpoint (collective).
+    Rank 0 logs and writes the files.  Returns the final global step."""
+    say = log if rank == 0 else (lambda *a: None)
     if flags.embedding_dim % 2:
         raise ValueError("embedding_dim must be even (holE.py:164-165 splits the row in halves)")
     check_optimizer_flags(flags)
-    # Warning: this will clobber existing summaries (holE.py:253-260)
-    if not flags.resume_checkpoint and os.path.isdir(flags.output_dir):
+    if getattr(flags, 'score_variant', 'complex') != 'complex' and flags.log_loss:
+        raise SystemExit("--score_variant ccorr_tanh has no --log_loss branch")
+    # Warning: this will clobber existing summaries (holE.py:253-260).  Rank 0 decides, or rank 1 would find the
+    # directory rank 0 has just made.
+    refuse = False
+    if rank == 0:
+        refuse = not flags.resume_checkpoint and os.path.isdir(flags.output_dir)
+        if not refuse:
+            os.makedirs(flags.output_dir, exist_ok=True)
+    if _from_rank0(dist, refuse):
         raise Exception("WARNING: " + flags.output_dir + " already exists!")
-    try:
-        os.makedirs(flags.output_dir)
-    except OSError as e:
-        if e.errno != errno.EEXIST:
-            raise
 
-    global_step = 0
-    adagrad = getattr(flags, 'optimizer', 'sgd') == 'adagrad'
-    A = None
+    global_step, A = 0, None
     if flags.resume_checkpoint:
         E, global_step = load_checkpoint(flags.output_dir)
-        if adagrad:
+        if getattr(flags, 'optimizer', 'sgd') == 'adagrad':
             A = load_accumulator(flags.output_dir)      # (--optimizer sgd ignores a saved accumulator)
         # TODO (reference, holE.py:315): the epoch counter restarts
     else:
         E = D.init_embeddings(data.entity_count, flags.embedding_dim, np.random.default_rng(seed))
-    eng = make_engine(data.entity_count, data.relation_count, flags.embedding_dim, E, data.id_to_type)
-    if adagrad:      # tf.train.AdagradOptimizer(lr, initial_accumulator_value) in place of holE.py:296's SGD
-        eng.set_optimizer("adagrad", flags.adagrad_initial_accumulator)
-        if A is not None:
-            eng.set_accumulator(A)
-    if getattr(flags, 'score_variant', 'complex') != 'complex':
-        if flags.log_loss:
-            raise SystemExit("--score_variant ccorr_tanh has no --log_loss branch")
-        eng.set_score_mode(flags.score_variant)      # archived FFT / tanh score (holE-20170724/graph.pbtxt:6221-6521)
-    B = flags.batch_size
-    triples_dev = torch.from_numpy(data.triples).to(eng.device)
+    dev, train, score, save = open_table(E, A)
+    del E, A
+    B, Bl = flags.batch_size, flags.batch_size // world
+    batch_count = data.triple_count // B
+    triples_dev = torch.from_numpy(data.triples).to(dev)
     valid = data.validation_triples
     decay_steps = flags.learning_decay_steps * batch_count
     valid_every = max(1, batch_count // 16)      # holE.py:351 (divides by zero if batch_count < 16)
-    gen = torch.Generator(device=eng.device)
+    gen = torch.Generator(device=dev)
     gen.manual_seed(seed)
     vrng = np.random.default_rng(seed + 1)
-    valid_dev = torch.from_numpy(np.ascontiguousarray(valid)).to(eng.device) if len(valid) else None
-    log_path = os.path.join(flags.output_dir, 'summaries.tsv')
-    events = tf_events.EventFileWriter(flags.output_dir)      # summary_writer (holE.py:317)
+    valid_dev = torch.from_numpy(np.ascontiguousarray(valid)).to(dev) if len(valid) else None
+    events = tf_events.EventFileWriter(flags.output_dir) if rank == 0 else None     # summary_writer (holE.py:317)
+    slog = open(os.path.join(flags.output_dir, 'summaries.tsv'), 'a') if rank == 0 else None
     pocket_loss = 2.
     steps_done = 0
     t_start = time.time()
     try:
-        with open(log_path, 'a') as slog:
-            for epoch in range(1, flags.num_epochs + 1):
-                log('Initializing projector...')
+        for epoch in range(1, flags.num_epochs + 1):
+            say('Initializing projector...')
+            if rank == 0:
                 tf_bundle.write_projector_config(flags.output_dir)
-                log('Training epoch {}...'.format(epoch))
-                perm = torch.randperm(data.triple_count, device=eng.device, generator=gen)
-                shuffled = triples_dev[perm]
-                batch = 1                       # for batch in range(1, batch_count)  (holE.py:340)
-                while batch < batch_count:
-                    if batch % valid_every == 0 and len(valid) > 0:
-                        # The reference scores ONE shuffled batch of the validation file and notes
-                        # "TODO: this should run the entire validation set" (holE.py:350): the whole file
-                        # is scored on the device here (--valid_sample restores the sampled batch).
-                        if getattr(flags, "valid_sample", False):
-                            vb = valid[vrng.integers(0, len(valid), size=B)]
-                        else:
-                            vb = valid_dev
-                        if flags.log_loss:
-                            vloss = evaluate_batch_logloss(eng, vb, seed, global_step, flags.l2_regularization,
-                                                           flags.negative_ratio)
-                            parts = (("loss", vloss),)
-                        else:
-                            vloss, vp, vn = evaluate_batch(eng, vb, seed, global_step, flags.margin)
-                            parts = (("pos", vp), ("neg", vn), ("loss", vloss))
+            say('Training epoch {}...'.format(epoch))
+            perm = torch.randperm(data.triple_count, device=dev, generator=gen)
+            if epoch == 1 and world > 1:      # a different shuffle on one rank would silently train another model
+                ck = (perm.long() * torch.arange(1, data.triple_count + 1, device=dev)).sum().view(1)
+                cks = [torch.empty_like(ck) for _ in range(world)]
+                dist.all_gather(cks, ck)
+                if any(int(c) != int(cks[0]) for c in cks):
+                    raise RuntimeError(f"the ranks drew different epoch permutations (checksums "
+                                       f"{[int(c) for c in cks]}): every rank must run the same torch build and GPU model")
+            mine = triples_dev[rank_rows(perm, B, world, rank)]          # [batch_count * Bl, 3], step-major
+            batch = 1                       # for batch in range(1, batch_count)  (holE.py:340)
+            while batch < batch_count:
+                if batch % valid_every == 0 and len(valid) > 0:
+                    # The reference scores ONE shuffled batch of the validation file and notes
+                    # "TODO: this should run the entire validation set" (holE.py:350): the whole file
+                    # is scored on the device here (--valid_sample restores the sampled batch).
+                    vb = (torch.from_numpy(valid[vrng.integers(0, len(valid), size=B)]).to(dev)
+                          if getattr(flags, "valid_sample", False) else valid_dev)
+                    parts, batch_parts = score(vb, mine[(batch - 1) * Bl:batch * Bl], global_step)
+                    vlm = None
+                    if rank == 0:
                         lr_now = float(inverse_time_decay(flags.learning_rate, global_step, decay_steps,
                                                           flags.learning_decay_rate))
-                        batch_parts = None
-                        if not flags.log_loss:
-                            tb = shuffled[(batch - 1) * B:batch * B]
-                            batch_parts = evaluate_batch(eng, tb, seed, global_step, flags.margin)
                         vlm = write_summaries(slog, events, global_step, lr_now, parts, batch_parts)
-                        log('\tStep {} Validation Loss: {}...'.format(global_step, vlm))
-                        if vlm < pocket_loss:       # pocket checkpoint (holE.py:357-360)
-                            pocket_loss = vlm
-                            save_checkpoint(eng, flags.output_dir, global_step)
-                            log('Epoch {}, (Model saved with loss {})'.format(epoch, vlm))
-                    # run up to the next validation point without returning to the host per step
-                    nxt = min(batch_count, (batch // valid_every + 1) * valid_every)
-                    n = nxt - batch
-                    if max_steps is not None:
-                        n = min(n, max_steps - steps_done)
-                    lrs = [inverse_time_decay(flags.learning_rate, global_step + k, decay_steps,
-                                              flags.learning_decay_rate) for k in range(n)]
-                    if flags.log_loss:
-                        for k in range(n):       # one library call per step (k corrupt batches inside)
-                            eng.train_step_logloss(shuffled[(batch - 1 + k) * B:(batch + k) * B], seed,
-                                                   global_step + k, lrs[k], flags.l2_regularization,
-                                                   flags.negative_ratio)
-                    else:
-                        eng.train_steps(shuffled[(batch - 1) * B:(batch - 1 + n) * B], B, seed, global_step,
-                                        flags.margin, lrs)
-                    batch += n
-                    global_step += n
-                    steps_done += n
-                    if max_steps is not None and steps_done >= max_steps:
-                        raise StopIteration
-            log('Done training -- epoch limit reached')
+                        say('\tStep {} Validation Loss: {}...'.format(global_step, vlm))
+                    vlm = _from_rank0(dist, vlm)
+                    if vlm < pocket_loss:       # pocket checkpoint (holE.py:357-360), one decision on every rank
+                        pocket_loss = vlm
+                        save(global_step)
+                        say('Epoch {}, (Model saved with loss {})'.format(epoch, vlm))
+                # run up to the next validation point without returning to the host per step
+                nxt = min(batch_count, (batch // valid_every + 1) * valid_every)
+                n = nxt - batch
+                if max_steps is not None:
+                    n = min(n, max_steps - steps_done)
+                lrs = [inverse_time_decay(flags.learning_rate, global_step + k, decay_steps,
+                                          flags.learning_decay_rate) for k in range(n)]
+                train(mine[(batch - 1) * Bl:(batch - 1 + n) * Bl], global_step, lrs)
+                batch += n
+                global_step += n
+                steps_done += n
+                if max_steps is not None and steps_done >= max_steps:
+                    raise StopIteration
+        say('Done training -- epoch limit reached')
     except StopIteration:
-        log('Done training -- step limit reached')
+        say('Done training -- step limit reached')
     finally:
-        log('Stopping training...')
-        events.close()
+        say('Stopping training...')
+        if rank == 0:
+            events.close()
+            slog.close()
     torch.cuda.synchronize()
-    if not os.path.exists(os.path.join(flags.output_dir, 'model.ckpt.index')):
-        save_checkpoint(eng, flags.output_dir, global_step)    # never validated: still leave a model
-    log('Trained {} steps in {:.1f}s'.format(steps_done, time.time() - t_start))
+    elapsed = time.time() - t_start
+    # never validated: still leave a model (rank 0 looks, every rank enters the gather)
+    if _from_rank0(dist, rank == 0 and not os.path.exists(os.path.join(flags.output_dir, 'model.ckpt.index'))):
+        save(global_step)
+    say('Trained {} steps in {:.1f}s on {} GPUs: {:.4g} triples/s'.format(
+        steps_done, elapsed, world, steps_done * B / max(elapsed, 1e-9)))
+    return global_step
+
+
+def run_training(data, flags=None, seed=0, max_steps=None, log=print):
+    """holE.py's run_training on one GPU (HoleEngine).  Returns (engine, final global step)."""
+    flags = flags or FLAGS
+    B = flags.batch_size
+    log('Embedding dimension: ', flags.embedding_dim, 'Batch size: ', B, 'Batch count: ', data.triple_count // B)
+    eng = None
+
+    def open_table(E, A):
+        nonlocal eng
+        eng = make_engine(data.entity_count, data.relation_count, flags.embedding_dim, E, data.id_to_type)
+        if getattr(flags, 'optimizer', 'sgd') == 'adagrad':
+            # tf.train.AdagradOptimizer(lr, initial_accumulator_value) in place of holE.py:296's SGD
+            eng.set_optimizer("adagrad", flags.adagrad_initial_accumulator)
+            if A is not None:
+                eng.set_accumulator(A)
+        if getattr(flags, 'score_variant', 'complex') != 'complex':
+            eng.set_score_mode(flags.score_variant)      # archived FFT / tanh score (holE-20170724/graph.pbtxt:6221-6521)
+
+        def train(rows, first_step, lrs):
+            if flags.log_loss:
+                for k, lr in enumerate(lrs):       # one library call per step (k corrupt batches inside)
+                    eng.train_step_logloss(rows[k * B:(k + 1) * B], seed, first_step + k, lr, flags.l2_regularization,
+                                           flags.negative_ratio)
+            else:
+                eng.train_steps(rows, B, seed, first_step, flags.margin, lrs)
+
+        def score(vb, tb, step):
+            if flags.log_loss:
+                return (("loss", evaluate_batch_logloss(eng, vb, seed, step, flags.l2_regularization,
+                                                        flags.negative_ratio)),), None
+            vloss, vp, vn = evaluate_batch(eng, vb, seed, step, flags.margin)
+            return (("pos", vp), ("neg", vn), ("loss", vloss)), evaluate_batch(eng, tb, seed, step, flags.margin)
+
+        return eng.device, train, score, lambda step: save_checkpoint(eng, flags.output_dir, step)
+
+    global_step = _train_loop(data, flags, None, 0, 1, seed, max_steps, log, open_table)
     return eng, global_step
 
 
@@ -465,10 +502,7 @@ def evaluate_batch_sharded(tr, offsets, part, seed, step, margin, dist):
     world = len(offsets) - 1
     base = offsets[tr.my_rank]
     assert part.shape[0] == offsets[tr.my_rank + 1] - base
-    side, neg = tr.be.eng.corrupt_batch(part, seed, step, base)
-    corrupt = part.clone()
-    corrupt[:, 0 if side else 1] = neg
-    s = tr.score(torch.cat([part, corrupt]))
+    s = tr.score(torch.cat([part, _corrupt_triples(tr.be.eng, part, seed, step, base)]))
     sizes = [offsets[k + 1] - offsets[k] for k in range(world)]
     vp, vn = (_gather_in_rank_order(dist, world, x, sizes) for x in (s[:part.shape[0]], s[part.shape[0]:]))
     return torch.clamp(vp - vn + margin, min=0.0), vp, vn
@@ -481,143 +515,49 @@ def run_training_sharded(data, flags, dist, rank, world, local_rank, seed=0, max
     seeds, validation points, summaries, pocket checkpoints and outputs are the one-GPU driver's; rank 0 logs and
     writes the files.  Returns the final global step."""
     from . import sharded
-    say = log if rank == 0 else (lambda *a: None)
-    batch_count = data.triple_count // flags.batch_size
-    say('Embedding dimension: ', flags.embedding_dim, 'Batch size: ', flags.batch_size,
-        'Batch count: ', batch_count, 'GPUs: ', world)
-    if flags.embedding_dim % 2:
-        raise ValueError("embedding_dim must be even (holE.py:164-165 splits the row in halves)")
-    check_optimizer_flags(flags)
-    check_gpus_flags(flags, world)
-    # Warning: this will clobber existing summaries (holE.py:253-260).  Rank 0 decides, or rank 1 would find the
-    # directory rank 0 has just made.
-    refuse = False
+    B = flags.batch_size
     if rank == 0:
-        refuse = not flags.resume_checkpoint and os.path.isdir(flags.output_dir)
-        if not refuse:
-            os.makedirs(flags.output_dir, exist_ok=True)
-    if _from_rank0(dist, refuse):
-        raise Exception("WARNING: " + flags.output_dir + " already exists!")
-
-    global_step = 0
+        log('Embedding dimension: ', flags.embedding_dim, 'Batch size: ', B, 'Batch count: ', data.triple_count // B,
+            'GPUs: ', world)
+    check_gpus_flags(flags, world)
     adagrad = getattr(flags, 'optimizer', 'sgd') == 'adagrad'
-    A = None
-    if flags.resume_checkpoint:
-        E, global_step = load_checkpoint(flags.output_dir)
+    be = tr = None
+
+    def open_table(E, A):
+        nonlocal be, tr
+        R, Bl = data.relation_count, B // world
+        be = sharded.CudaBackend(R, flags.embedding_dim, Bl, local_rank, *type_tables(data.entity_count,
+                                                                                      data.id_to_type))
+        tr = sharded.make_trainer(R, data.entity_count - R, flags.embedding_dim, be, dist,
+                                  log=log if rank == 0 else None)
         if adagrad:
-            A = load_accumulator(flags.output_dir)
-    else:
-        E = D.init_embeddings(data.entity_count, flags.embedding_dim, np.random.default_rng(seed))
-    B, R = flags.batch_size, data.relation_count
-    Bl = B // world
-    be = sharded.CudaBackend(R, flags.embedding_dim, Bl, local_rank, *type_tables(data.entity_count, data.id_to_type))
-    tr = sharded.make_trainer(R, data.entity_count - R, flags.embedding_dim, be, dist, log=say)
-    p2p = isinstance(tr, sharded.P2PRowShardedTrainer)
-    if adagrad:
-        if not p2p:
-            raise SystemExit("--optimizer adagrad on several GPUs needs the NVLink peer-memory trainer, and the GPUs "
-                             "of this job cannot map each other's memory: train with --optimizer sgd")
-        tr.set_optimizer("adagrad", flags.adagrad_initial_accumulator)
-    tr.load_embeddings(E)
-    if A is not None:
-        tr.load_accumulator(A)
-    del E, A
-    dev = be.device
+            if not isinstance(tr, sharded.P2PRowShardedTrainer):
+                raise SystemExit("--optimizer adagrad on several GPUs needs the NVLink peer-memory trainer, and the "
+                                 "GPUs of this job cannot map each other's memory: train with --optimizer sgd")
+            tr.set_optimizer("adagrad", flags.adagrad_initial_accumulator)
+        tr.load_embeddings(E)
+        if A is not None:
+            tr.load_accumulator(A)
 
-    def save(step):
-        """All ranks gather (collective), rank 0 writes the one-GPU checkpoint layout."""
-        E_, A_ = tr.gather_embeddings(), tr.gather_accumulator() if adagrad else None
-        if rank == 0:
-            write_checkpoint(flags.output_dir, E_, step, A_)
+        def score(vb, tb, step):
+            vo = valid_split(len(vb), world)
+            vloss, vp, vn = evaluate_batch_sharded(tr, vo, vb[vo[rank]:vo[rank + 1]], seed, step, flags.margin, dist)
+            # the next training batch: my share of it is rows [rank*Bl, (rank+1)*Bl)
+            return (("pos", vp), ("neg", vn), ("loss", vloss)), evaluate_batch_sharded(
+                tr, [k * Bl for k in range(world + 1)], tb, seed, step, flags.margin, dist)
 
-    triples_dev = torch.from_numpy(data.triples).to(dev)
-    valid = data.validation_triples
-    decay_steps = flags.learning_decay_steps * batch_count
-    valid_every = max(1, batch_count // 16)      # holE.py:351 (divides by zero if batch_count < 16)
-    gen = torch.Generator(device=dev)
-    gen.manual_seed(seed)
-    vrng = np.random.default_rng(seed + 1)
-    valid_dev = torch.from_numpy(np.ascontiguousarray(valid)).to(dev) if len(valid) else None
-    events = tf_events.EventFileWriter(flags.output_dir) if rank == 0 else None
-    slog = open(os.path.join(flags.output_dir, 'summaries.tsv'), 'a') if rank == 0 else None
-    pocket_loss = 2.
-    steps_done = 0
-    t_start = time.time()
-    try:
-        for epoch in range(1, flags.num_epochs + 1):
-            say('Initializing projector...')
+        def save(step):
+            """All ranks gather (collective), rank 0 writes the one-GPU checkpoint layout."""
+            E_, A_ = tr.gather_embeddings(), tr.gather_accumulator() if adagrad else None
             if rank == 0:
-                tf_bundle.write_projector_config(flags.output_dir)
-            say('Training epoch {}...'.format(epoch))
-            perm = torch.randperm(data.triple_count, device=dev, generator=gen)
-            if epoch == 1 and world > 1:      # a different shuffle on one rank would silently train another model
-                ck = (perm.long() * torch.arange(1, data.triple_count + 1, device=dev)).sum().view(1)
-                cks = [torch.empty_like(ck) for _ in range(world)]
-                dist.all_gather(cks, ck)
-                if any(int(c) != int(cks[0]) for c in cks):
-                    raise RuntimeError(f"the ranks drew different epoch permutations (checksums "
-                                       f"{[int(c) for c in cks]}): every rank must run the same torch build and GPU model")
-            mine = triples_dev[rank_rows(perm, B, world, rank)]          # [batch_count * Bl, 3], step-major
-            batch = 1                       # for batch in range(1, batch_count)  (holE.py:340)
-            while batch < batch_count:
-                if batch % valid_every == 0 and len(valid) > 0:
-                    vb = (torch.from_numpy(valid[vrng.integers(0, len(valid), size=B)]).to(dev)
-                          if getattr(flags, "valid_sample", False) else valid_dev)
-                    vo = valid_split(len(vb), world)
-                    vloss, vp, vn = evaluate_batch_sharded(tr, vo, vb[vo[rank]:vo[rank + 1]], seed, global_step,
-                                                           flags.margin, dist)
-                    # the next training batch: my share of it is rows [rank*Bl, (rank+1)*Bl)
-                    tl, tp, tn = evaluate_batch_sharded(tr, [k * Bl for k in range(world + 1)],
-                                                        mine[(batch - 1) * Bl:batch * Bl], seed, global_step,
-                                                        flags.margin, dist)
-                    vlm = None
-                    if rank == 0:
-                        lr_now = float(inverse_time_decay(flags.learning_rate, global_step, decay_steps,
-                                                          flags.learning_decay_rate))
-                        vlm = write_summaries(slog, events, global_step, lr_now,
-                                              (("pos", vp), ("neg", vn), ("loss", vloss)), (tl, tp, tn))
-                        say('\tStep {} Validation Loss: {}...'.format(global_step, vlm))
-                    vlm = _from_rank0(dist, vlm)
-                    if vlm < pocket_loss:       # pocket checkpoint (holE.py:357-360), one decision on every rank
-                        pocket_loss = vlm
-                        save(global_step)
-                        say('Epoch {}, (Model saved with loss {})'.format(epoch, vlm))
-                nxt = min(batch_count, (batch // valid_every + 1) * valid_every)
-                n = nxt - batch
-                if max_steps is not None:
-                    n = min(n, max_steps - steps_done)
-                lrs = [inverse_time_decay(flags.learning_rate, global_step + k, decay_steps,
-                                          flags.learning_decay_rate) for k in range(n)]
-                chunk = mine[(batch - 1) * Bl:(batch - 1 + n) * Bl]
-                if p2p:
-                    tr.train_steps(chunk, Bl, seed, global_step, flags.margin, lrs)
-                else:                           # the all-to-all trainer has no multi-step call
-                    for k in range(n):
-                        tr.train_step(chunk[k * Bl:(k + 1) * Bl], seed, global_step + k, flags.margin, lrs[k])
-                batch += n
-                global_step += n
-                steps_done += n
-                if max_steps is not None and steps_done >= max_steps:
-                    raise StopIteration
-        say('Done training -- epoch limit reached')
-    except StopIteration:
-        say('Done training -- step limit reached')
-    finally:
-        say('Stopping training...')
-        if rank == 0:
-            events.close()
-            slog.close()
-    torch.cuda.synchronize()
-    if p2p:
-        tr.check_barriers()
-    elapsed = time.time() - t_start
-    # never validated: still leave a model (rank 0 looks, every rank enters the gather)
-    if _from_rank0(dist, rank == 0 and not os.path.exists(os.path.join(flags.output_dir, 'model.ckpt.index'))):
-        save(global_step)
-    say('Trained {} steps in {:.1f}s on {} GPUs: {:.4g} triples/s'.format(
-        steps_done, elapsed, world, steps_done * B / max(elapsed, 1e-9)))
-    if p2p:
-        tr.close()
+                write_checkpoint(flags.output_dir, E_, step, A_)
+
+        return (be.device, lambda rows, first_step, lrs: tr.train_steps(rows, Bl, seed, first_step, flags.margin, lrs),
+                score, save)
+
+    global_step = _train_loop(data, flags, dist, rank, world, seed, max_steps, log, open_table)
+    tr.check_barriers()
+    tr.close()
     be.eng.close()
     return global_step
 

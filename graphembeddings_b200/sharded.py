@@ -268,6 +268,25 @@ class RowShardedTrainer:
                 off += n_k
         return loss
 
+    def train_steps(self, triples_i32, batch_size, seed, first_step, margin, lrs):
+        """n_steps consecutive train_step calls on device-resident slices [n_steps*B, 3] (lrs: at least n_steps
+        rates).  Returns this rank's per-step loss sums (device)."""
+        n_steps = triples_i32.shape[0] // batch_size
+        sums = torch.empty(n_steps, dtype=torch.float32, device=triples_i32.device)
+        for k in range(n_steps):
+            sums[k] = self.train_step(triples_i32[k * batch_size:(k + 1) * batch_size], seed, first_step + k, margin,
+                                      lrs[k]).sum()
+        return sums
+
+    def check_barriers(self):
+        """Nothing to check: the all-to-all trainer has no step barriers of its own."""
+
+    def close(self):
+        """Releases the ranking context of rank()."""
+        if getattr(self, "_rank_eng", None) is not None:
+            self._rank_eng.close()
+            self._rank_eng = None
+
     # ------------------------------------------------------------------ scoring
     def score(self, triples):
         """sigma (hole_score) of this rank's triples [n,3] (global row ids) on the sharded table.  Collective: every
@@ -475,9 +494,7 @@ class P2PRowShardedTrainer(RowShardedTrainer):
             return
         torch.cuda.synchronize()
         self._peers = None
-        if getattr(self, "_rank_eng", None) is not None:
-            self._rank_eng.close()
-            self._rank_eng = None
+        super().close()
         if self.world > 1:
             self.dist.barrier()
         self.shard = self.stage = self.relstage = self.inbox = self.meta = self.flags = None
@@ -672,8 +689,7 @@ def parity_case(dist, rank, world, local, dim, Bl, steps, n_ent, seed, chunked, 
         e2.close()
     flag = torch.tensor([1 if ok else 0], device="cuda")
     dist.broadcast(flag, 0)
-    if hasattr(tr, "close"):
-        tr.close()
+    tr.close()
     be.eng.close()
     return bool(flag.item()), res
 
