@@ -51,6 +51,8 @@ SIGNATURES = {
     "hole_shard_steps_host": (_int, [_p, _p, _i64, _i64, _u64, _u64, _f32, _p, _p, _p]),
     "hole_shard_poll": (_int, [_p, C.POINTER(_int), _p]),
     "hole_shard_set_optimizer": (_int, [_p, _int, _p]),
+    "hole_shard_step_logloss": (_int, [_p, _p, _i64, _int, _u64, _u64, _f32, _f32, _p, _p, _p, _p, _p]),
+    "hole_shard_step_logloss_compute": (_int, [_p, _p, _i64, _int, _u64, _u64, _f32, _f32, _p, _p, _p, _p, _p]),
     "hole_shard_profile_read": (_int, [_p, C.POINTER(C.c_double), C.POINTER(_i64)]),
     "hole_enable_peer_access": (_int, [_p, _int]),
     "hole_gather_rows": (_int, [_p, _p, _p, _i64, _p, _i64, _p]),

@@ -30,6 +30,12 @@
 // the owner's apply (hole_shard_adagrad_apply_kernel) sums a row's gradients in rank order, then updates the
 // row and its accumulator row once.  The exchange is byte for byte that of an SGD step.
 //
+// Log loss (hole_shard_step_logloss, DESIGN 7d): the k passes of a --log_loss step all read the OLD table, so the
+// rows are gathered once into a local step table W = [my relation replica | request-list rows] (gather kernel,
+// after flag A), the one-GPU step's K1 (DM 3) / K3 passes run on W into a local delta table D, and the push
+// kernel stores D's request-list rows into the owners' staging buffers; finish, claim and apply are the SGD
+// step's.  Between claim and apply the owner decays its shard by the L2 factor the compute half latched.
+//
 // No NCCL call and no host synchronisation inside a step; two flag waits per step, both at the
 // head of a kernel that has work to do anyway.  Flags only grow (epoch = steps completed).
 #pragma once
@@ -81,6 +87,19 @@ struct hole_shard_state {
   int step_optimizer = HOLE_OPT_SGD;     // latched by hole_shard_step_compute for the step's apply
   float step_lr = 0.f;
   float* step_accum = nullptr;
+  bool step_decay = false;               // latched by hole_shard_step_logloss_compute: decay my shard before the
+  float step_scale = 1.f;                //   apply, by step_scale, and write half its sum of squares to step_l2_out
+  float* step_l2_out = nullptr;
+  // log-loss step, allocated by its first call (hole_shard_step_logloss_compute)
+  hole_plan ll_plan;                     // the k passes' plan (c->plan[] may hold a hinge chunk prepared ahead)
+  int64_t ll_S = 0;                      // passes ll_plan is sized for
+  int32_t* ll_uniq = nullptr;            // [cap] request list
+  int32_t* ll_cuts = nullptr;            // [HOLE_MAX_RANKS+1]
+  int32_t* ll_pos_w = nullptr;           // [max_batch,3] my triples as step-table rows
+  int32_t* ll_neg_w = nullptr;           // [ll_S][max_batch] the corrupt entities as step-table rows
+  float* ll_W = nullptr;                 // [R + cap, stride] step table
+  float* ll_D = nullptr;                 // [R + cap, stride] its deltas (zero between steps)
+  float* ll_partial = nullptr;           // [2 * 8 * sm_count] block partials of the decay's sum of squares
   std::vector<cudaEvent_t> prof_ev;      // hole_profile_enable: 6 events per step (phase boundaries)
   size_t prof_used = 0;
 };
@@ -297,10 +316,70 @@ hole_shard_adagrad_apply_kernel(float* __restrict__ shard, float* __restrict__ a
   }
 }
 
+// Log-loss step: the step table W = [my relation replica | request-list rows], once every peer's shard is current
+// (flag A).  One warp per row, float4 by float4; a request-list row comes from its owner's shard (over NVLink).
+__global__ void __launch_bounds__(256)
+hole_shard_gather_kernel(float4* __restrict__ W, const int32_t* __restrict__ uniq, const int32_t* __restrict__ cuts,
+                         hole_peer_ptrs shard, int R, int rows_per, int me, int world, int row4,
+                         const int* __restrict__ my_flags, int wait_epoch, int* __restrict__ err,
+                         unsigned long long timeout_ns) {
+  hole_flags_wait(my_flags, world, wait_epoch, err, timeout_ns);
+  const int lane = threadIdx.x & 31;
+  const int n = R + cuts[world];
+  for (int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; row < n; row += (gridDim.x * blockDim.x) >> 5) {
+    const float4* src;
+    if (row < R) {
+      src = static_cast<const float4*>(shard.p[me]) + (size_t)row * row4;
+    } else {
+      const int id = uniq[row - R], o = (id - R) / rows_per;
+      src = static_cast<const float4*>(shard.p[o]) + (size_t)(id - o * rows_per) * row4;
+    }
+    float4* dst = W + (size_t)row * row4;
+    for (int q = lane; q < row4; q += 32) dst[q] = src[q];
+  }
+}
+
+// Log-loss step: request-list row R + j of the delta table D -> slot j - cuts[o] of my slice of owner o's staging
+// buffer (the layout hole_shard_apply_kernel reads), and the row back to zero.  Each thread fences its own peer
+// stores: the finish kernel raises flag B after this kernel.
+__global__ void __launch_bounds__(256)
+hole_shard_push_kernel(float4* __restrict__ D, const int32_t* __restrict__ cuts, hole_peer_ptrs stage, int R,
+                       int me, int world, int64_t cap, int row4) {
+  __shared__ int s_cuts[HOLE_MAX_RANKS + 1];
+  if (threadIdx.x <= world) s_cuts[threadIdx.x] = cuts[threadIdx.x];
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const int U = s_cuts[world];
+  const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < U; j += (gridDim.x * blockDim.x) >> 5) {
+    int o = 0;
+    while (j >= s_cuts[o + 1]) ++o;
+    float4* src = D + (size_t)(R + j) * row4;
+    float4* dst = static_cast<float4*>(stage.p[o]) + ((size_t)me * cap + (size_t)(j - s_cuts[o])) * row4;
+    for (int q = lane; q < row4; q += 32) {
+      dst[q] = src[q];
+      src[q] = z;
+    }
+  }
+  __threadfence_system();
+}
+
 // ------------------------------------------------------------------------------------ host side
+static void shard_ll_free(hole_shard_state* s) {
+  plan_free(s->ll_plan);
+  cudaFree(s->ll_uniq); cudaFree(s->ll_cuts); cudaFree(s->ll_pos_w); cudaFree(s->ll_neg_w);
+  cudaFree(s->ll_W); cudaFree(s->ll_D); cudaFree(s->ll_partial);
+  s->ll_uniq = s->ll_cuts = s->ll_pos_w = s->ll_neg_w = nullptr;
+  s->ll_W = s->ll_D = s->ll_partial = nullptr;
+  s->ll_S = 0;
+}
+
 static void shard_free(hole_ctx* c) {
   hole_shard_state* s = c->shard_state;
   if (s == nullptr) return;
+  shard_ll_free(s);
+  if (s->ll_plan.ready) cudaEventDestroy(s->ll_plan.ready);
+  if (s->ll_plan.released) cudaEventDestroy(s->ll_plan.released);
   for (int b = 0; b < 2; ++b) {
     cudaFree(s->prep[b].uniq); cudaFree(s->prep[b].cuts); cudaFree(s->prep[b].pos_w);
     cudaFree(s->prep[b].neg_w); cudaFree(s->prep[b].neg);
@@ -523,6 +602,7 @@ extern "C" int hole_shard_step_compute(hole_ctx* c, const int32_t* pos, int64_t 
   // for hole_shard_step_apply)
   const bool ada = s->optimizer == HOLE_OPT_ADAGRAD;
   s->step_optimizer = s->optimizer; s->step_lr = lr; s->step_accum = s->accum;
+  s->step_decay = false;
   rc = run_step(c, pl, s->shard, p_pos_w, p_neg_w, side, B, margin, ada ? -1.0f : lr, loss_out, nullptr, k, st,
                 s->Drel, false, 0, &sh, pos, p_neg, c->profile ? s->prof_ev[s->prof_used - 6 + 2] : nullptr);
   if (rc) return rc;
@@ -558,6 +638,29 @@ extern "C" int hole_shard_step_apply(hole_ctx* c, void* stream) {
       inbox, meta, world, s->cap, row0, s->rows_per, s->claim, s->slot, static_cast<const int*>(s->p_flags.p[me]),
       s->epoch + 1, s->err, s->timeout_ns);
   HOLE_LAUNCHED();
+  if (s->step_decay) {
+    // log-loss step: no peer reads my shard any more (claim has seen every flag B), so decay it in place
+    // (E <- E * scale, as the one-GPU step's dense pass) and sum the squares of its old rows -- the relation
+    // replica on rank 0 only, so that the ranks' parts add up to the whole table's
+    const size_t rel4 = (size_t)s->R * c->row_stride / 4, ent4 = (size_t)s->rows_per * c->row_stride / 4;
+    const int blocks = c->sm_count * 8;
+    float4* sh4 = reinterpret_cast<float4*>(s->shard);
+    if (me == 0) {
+      hole_l2_scale_kernel<<<blocks, 256, 0, st>>>(sh4, rel4 + ent4, s->step_scale, s->ll_partial);
+      HOLE_LAUNCHED();
+    } else {
+      if (s->step_scale != 1.0f && rel4 > 0) {
+        hole_l2_scale_kernel<<<blocks, 256, 0, st>>>(sh4, rel4, s->step_scale, s->ll_partial + blocks);
+        HOLE_LAUNCHED();
+      }
+      hole_l2_scale_kernel<<<blocks, 256, 0, st>>>(sh4 + rel4, ent4, s->step_scale, s->ll_partial);
+      HOLE_LAUNCHED();
+    }
+    if (s->step_l2_out != nullptr) {
+      hole_l2_finish_kernel<<<1, 256, 0, st>>>(s->ll_partial, blocks, s->step_l2_out);
+      HOLE_LAUNCHED();
+    }
+  }
   if (s->step_optimizer == HOLE_OPT_ADAGRAD)                 // the optimizer and lr of the step's compute half
     HOLE_DISPATCH(c, hole_shard_adagrad_apply_kernel, (unsigned)c->sm_count * 16, 256, st, s->shard, s->step_accum,
                   inbox, meta, static_cast<const float*>(s->p_stage.p[me]),
@@ -596,6 +699,147 @@ extern "C" int hole_shard_profile_read(hole_ctx* c, double* phase_ms5, int64_t* 
 extern "C" int hole_shard_step(hole_ctx* c, const int32_t* pos, int64_t B, uint64_t seed, uint64_t step,
                                float margin, float lr, float* loss_out, void* stream) {
   int rc = hole_shard_step_compute(c, pos, B, seed, step, margin, lr, loss_out, stream);
+  if (rc) return rc;
+  return hole_shard_step_apply(c, stream);
+}
+
+// Buffers of the log-loss step for up to S passes (grown on demand; growing synchronises the device).
+static int shard_ll_reserve(hole_ctx* c, int64_t S) {
+  hole_shard_state* s = c->shard_state;
+  if (s->ll_W != nullptr && S <= s->ll_S) return HOLE_OK;
+  S = std::max(S, s->ll_S);
+  HOLE_CUDA_TRY(cudaDeviceSynchronize());                    // an earlier step may still read the old buffers
+  shard_ll_free(s);
+  if (s->ll_plan.ready == nullptr) {
+    HOLE_CUDA_TRY(cudaEventCreateWithFlags(&s->ll_plan.ready, cudaEventDisableTiming));
+    HOLE_CUDA_TRY(cudaEventCreateWithFlags(&s->ll_plan.released, cudaEventDisableTiming));
+  }
+  int rc = plan_alloc(c, s->ll_plan, s->max_batch, S);
+  if (rc) return rc;
+  const size_t rows = (size_t)(s->R + s->cap), bytes = rows * c->row_stride * sizeof(float);
+#define LL_ALLOC(ptr, n)                                                                 \
+  do {                                                                                   \
+    if (cudaMalloc((void**)&(ptr), (n)) != cudaSuccess) {                                \
+      cudaGetLastError();                                                                \
+      shard_ll_free(s);                                                                  \
+      return hole_set_error(HOLE_ERR_ALLOC, "log-loss step allocation of %zu bytes failed", (size_t)(n)); \
+    }                                                                                    \
+  } while (0)
+  LL_ALLOC(s->ll_uniq, (size_t)s->cap * 4);
+  LL_ALLOC(s->ll_cuts, (size_t)(HOLE_MAX_RANKS + 1) * 4);
+  LL_ALLOC(s->ll_pos_w, (size_t)s->max_batch * 12);
+  LL_ALLOC(s->ll_neg_w, (size_t)S * s->max_batch * 4);
+  LL_ALLOC(s->ll_W, bytes);
+  LL_ALLOC(s->ll_D, bytes);
+  LL_ALLOC(s->ll_partial, (size_t)2 * 8 * c->sm_count * sizeof(float));
+#undef LL_ALLOC
+  if (cudaMemset(s->ll_D, 0, bytes) != cudaSuccess) {
+    cudaGetLastError();
+    shard_ll_free(s);
+    return hole_set_error(HOLE_ERR_CUDA, "log-loss step: clearing the delta table failed");
+  }
+  s->ll_S = S;
+  return HOLE_OK;
+}
+
+// Log-loss step, compute half: corruption + route on the call's stream, then the k passes' plan on the side stream
+// beside post + gather, the k passes (K1 DM 3 + K3 accumulating into D), push + finish.  Latches the decay for
+// hole_shard_step_apply.
+extern "C" int hole_shard_step_logloss_compute(hole_ctx* c, const int32_t* pos, int64_t B, int negative_ratio,
+                                               uint64_t seed, uint64_t step, float lr, float l2, float* loss_out,
+                                               float* l2_part_out, int32_t* neg_out, int32_t* sides_out,
+                                               void* stream) {
+  HOLE_CHECK_ARG(c != nullptr);
+  if (c->score_mode != HOLE_SCORE_COMPLEX)
+    return hole_set_error(HOLE_ERR_UNSUPPORTED, "the archived ccorr/tanh score mode has no log-loss branch");
+  int rc = optimizer_refusal(c, HOLE_STEP_SHARD);
+  if (rc) return rc;
+  hole_shard_state* s = c->shard_state;
+  if (s == nullptr) return hole_set_error(HOLE_ERR_ARG, "hole_shard_init has not been called");
+  if (s->optimizer != HOLE_OPT_SGD)
+    return hole_set_error(HOLE_ERR_UNSUPPORTED, "AdaGrad has no log-loss step (its L2 gradient is dense)");
+  const int k = negative_ratio;
+  HOLE_CHECK_ARG(pos != nullptr && loss_out != nullptr && B > 0 && k >= 1 && k <= 64);
+  // the (2 + k)B entity uses fit the staging / inbox slices, and their step-table rows the plan's row bitmaps
+  HOLE_CHECK_ARG((2 + k) * B <= s->cap && s->R + (2 + k) * B <= c->n_rows);
+  HOLE_CUDA_TRY(cudaSetDevice(c->device));
+  if ((rc = shard_ll_reserve(c, k))) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int world = s->world, me = s->me;
+  if ((rc = shard_mark(c, 0, st))) return rc;
+  // 1. corruption + route.  The route scratch is shared with the hinge chunks prepared on the side stream: after them
+  HOLE_CUDA_TRY(cudaEventRecord(c->ev_entry, c->plan_stream));
+  HOLE_CUDA_TRY(cudaStreamWaitEvent(st, c->ev_entry, 0));
+  hole_plan& pl = s->ll_plan;
+  const uint64_t v0 = step * (uint64_t)k;                    // pass j is virtual step v0 + j
+  const uint64_t index_base = (uint64_t)me * (uint64_t)B;    // my slice of the global batch
+  for (int j = 0; j < k; ++j) {
+    hole_corrupt_kernel<<<(unsigned)std::min<int64_t>((B + 255) / 256, 65535), 256, 0, st>>>(
+        pos, B, 1, s->type_of, s->csr_off, s->csr_ids, seed, v0 + (uint64_t)j, index_base, pl.neg + (size_t)j * B,
+        nullptr);
+    HOLE_LAUNCHED();
+  }
+  rc = shard_route(c, pos, pl.neg, B, s->R, s->R + s->rows_per * world, s->rows_per, world, s->ll_uniq, s->ll_cuts,
+                   s->ll_pos_w, s->ll_neg_w, st, 1, s->cap, k);
+  if (rc) return rc;
+  // the passes' plan on the side stream, while this stream posts and gathers (the plan waits for the previous
+  // call's passes: pl.released)
+  HOLE_CUDA_TRY(cudaEventRecord(c->ev_entry, st));
+  HOLE_CUDA_TRY(cudaStreamWaitEvent(c->plan_stream, c->ev_entry, 0));
+  rc = plan_steps(c, pl, s->ll_pos_w, B, k, nullptr, nullptr, nullptr, seed, v0, s->ll_neg_w, c->plan_stream,
+                  /*tstride=*/0);
+  if (rc) return rc;
+  // 2. my request lists -> the owners' inboxes of this step's parity; the step table, once every shard is current
+  const int par = s->epoch & 1;
+  hole_peer_ptrs ib, mt;
+  for (int o = 0; o < HOLE_MAX_RANKS; ++o) {
+    ib.p[o] = o < world ? static_cast<int32_t*>(s->p_inbox.p[o]) + (size_t)par * world * s->cap : nullptr;
+    mt.p[o] = o < world ? static_cast<int32_t*>(s->p_meta.p[o]) + (size_t)par * world * 2 : nullptr;
+  }
+  hole_shard_post_kernel<<<(unsigned)std::min<int64_t>((s->cap + 255) / 256, c->sm_count * 4), 256, 0, st>>>(
+      s->ll_uniq, s->ll_cuts, world, me, s->cap, ib, mt);
+  HOLE_LAUNCHED();
+  if ((rc = shard_mark(c, 1, st))) return rc;
+  const int row4 = c->row_stride / 4;
+  hole_shard_gather_kernel<<<(unsigned)c->sm_count * 8, 256, 0, st>>>(
+      reinterpret_cast<float4*>(s->ll_W), s->ll_uniq, s->ll_cuts, s->p_shard, (int)s->R, (int)s->rows_per, me, world,
+      row4, static_cast<const int*>(s->p_flags.p[me]), s->epoch, s->err, s->timeout_ns);
+  HOLE_LAUNCHED();
+  if ((rc = shard_mark(c, 2, st))) return rc;
+  // 3. the k passes of the one-GPU step on W (pass 0 carries the positive term), every delta added into D
+  HOLE_CUDA_TRY(cudaStreamWaitEvent(st, pl.ready, 0));
+  for (int j = 0; j < k; ++j) {
+    const int side = hole_side_coin(seed, v0 + (uint64_t)j);
+    if (sides_out) sides_out[j] = side;
+    rc = run_step(c, pl, s->ll_W, s->ll_pos_w, s->ll_neg_w + (size_t)j * B, side, B, 0.0f, lr, loss_out,
+                  loss_out + (size_t)(1 + j) * B, j, st, s->ll_D, false, (j == 0 ? 1 : 2) | HOLE_K1_ACCUMULATE);
+    if (rc) return rc;
+  }
+  if (neg_out)
+    HOLE_CUDA_TRY(cudaMemcpyAsync(neg_out, pl.neg, (size_t)k * B * 4, cudaMemcpyDeviceToDevice, st));
+  pl.used = true;
+  HOLE_CUDA_TRY(cudaEventRecord(pl.released, st));
+  if ((rc = shard_mark(c, 3, st))) return rc;
+  // 4. entity deltas -> the owners' staging buffers, relation deltas -> every peer, then flag B
+  hole_shard_push_kernel<<<(unsigned)c->sm_count * 8, 256, 0, st>>>(
+      reinterpret_cast<float4*>(s->ll_D), s->ll_cuts, s->p_stage, (int)s->R, me, world, s->cap, row4);
+  HOLE_LAUNCHED();
+  const unsigned fgrid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((s->R + (256 / c->gs) - 1) / (256 / c->gs), c->sm_count));
+  HOLE_DISPATCH(c, hole_shard_finish_kernel, fgrid, 256, st, s->ll_D, (int)s->R, me, world, s->p_relstage, s->p_flags,
+                s->epoch + 1, s->done, c->nvec, c->row_stride);
+  // the owner's half: SGD apply of the staged deltas, after the decay (one-GPU expression, global batch size)
+  s->step_optimizer = HOLE_OPT_SGD;
+  s->step_decay = l2 != 0.0f || l2_part_out != nullptr;
+  s->step_scale = 1.0f - lr * (float)(1 + k) * (float)((int64_t)world * B) * l2;
+  s->step_l2_out = l2_part_out;
+  return shard_mark(c, 4, st);
+}
+
+extern "C" int hole_shard_step_logloss(hole_ctx* c, const int32_t* pos, int64_t B, int negative_ratio, uint64_t seed,
+                                       uint64_t step, float lr, float l2, float* loss_out, float* l2_part_out,
+                                       int32_t* neg_out, int32_t* sides_out, void* stream) {
+  int rc = hole_shard_step_logloss_compute(c, pos, B, negative_ratio, seed, step, lr, l2, loss_out, l2_part_out,
+                                           neg_out, sides_out, stream);
   if (rc) return rc;
   return hole_shard_step_apply(c, stream);
 }

@@ -1647,6 +1647,42 @@ extern "C" int hole_ctx_destroy(hole_ctx* c) {
 
 static int k1_prepare(hole_ctx* c);
 
+// Buffers of one plan for chunks of S steps of batch B (freed again on failure).
+static int plan_alloc(hole_ctx* c, hole_plan& p, int64_t B, int64_t S) {
+  const size_t M = (size_t)4 * B;
+  const size_t tiles = (M + ST_TILE - 1) / ST_TILE;
+#define PL_ALLOC(ptr, bytes)                                                             \
+  do {                                                                                   \
+    if (cudaMalloc((void**)&(ptr), (bytes)) != cudaSuccess) {                            \
+      cudaGetLastError();                                                                \
+      plan_free(p);                                                                      \
+      return hole_set_error(HOLE_ERR_ALLOC, "workspace allocation of %zu bytes failed", (size_t)(bytes)); \
+    }                                                                                    \
+  } while (0)
+  PL_ALLOC(p.keysA, S * M * 4); PL_ALLOC(p.keysB, S * M * 4); PL_ALLOC(p.keysC, S * M * 4);
+  PL_ALLOC(p.valsA, S * M * 4); PL_ALLOC(p.valsB, S * M * 4);
+  {
+    const size_t W = (size_t)(c->n_rows + 31) / 32;
+    p.bitmap_words = (size_t)S * W;
+    PL_ALLOC(p.seen, 2 * p.bitmap_words * 4);
+    HOLE_CUDA_TRY(cudaMemset(p.seen, 0, 2 * p.bitmap_words * 4));
+    p.dup = p.seen + p.bitmap_words;
+    PL_ALLOC(p.done, (size_t)S * sizeof(unsigned));
+    HOLE_CUDA_TRY(cudaMemset(p.done, 0, (size_t)S * sizeof(unsigned)));
+    PL_ALLOC(p.blkcnt, (size_t)S * ((M + DP_TILE - 1) / DP_TILE + 1) * 4);
+    PL_ALLOC(p.mdup, (size_t)S * 4);
+  }
+  PL_ALLOC(p.gslot, S * M * 4);
+  PL_ALLOC(p.heads, (size_t)S * (M / 2 + 1) * sizeof(uint4));
+  PL_ALLOC(p.nheads, (size_t)S * 4);
+  PL_ALLOC(p.neg, (size_t)S * B * 4);
+  PL_ALLOC(p.perm, (size_t)S * B * 4);
+  PL_ALLOC(p.ghist, (size_t)S * 256 * tiles * 4);
+  p.used = false;
+#undef PL_ALLOC
+  return HOLE_OK;
+}
+
 // Workspace for chunks of S steps of batch B.  Reallocation synchronises the device.
 int hole_ws_reserve(hole_ctx* c, int64_t B, int64_t S) {
   hole_rank_cache_invalidate(c);     // every training entry point comes through here
@@ -1661,7 +1697,6 @@ int hole_ws_reserve(hole_ctx* c, int64_t B, int64_t S) {
   S = std::max(S, c->cap_S);
   ws_free(c);
   const size_t M = (size_t)4 * B;
-  const size_t tiles = (M + ST_TILE - 1) / ST_TILE;
 #define WS_ALLOC(ptr, bytes)                                                             \
   do {                                                                                   \
     if (cudaMalloc((void**)&(ptr), (bytes)) != cudaSuccess) {                            \
@@ -1675,27 +1710,8 @@ int hole_ws_reserve(hole_ctx* c, int64_t B, int64_t S) {
   WS_ALLOC(c->loss, (size_t)S * B * 4);
   WS_ALLOC(c->loss_sum, (size_t)S * 4);
   for (int k = 0; k < 2; ++k) {
-    hole_plan& p = c->plan[k];
-    WS_ALLOC(p.keysA, S * M * 4); WS_ALLOC(p.keysB, S * M * 4); WS_ALLOC(p.keysC, S * M * 4);
-    WS_ALLOC(p.valsA, S * M * 4); WS_ALLOC(p.valsB, S * M * 4);
-    {
-      const size_t W = (size_t)(c->n_rows + 31) / 32;
-      p.bitmap_words = (size_t)S * W;
-      WS_ALLOC(p.seen, 2 * p.bitmap_words * 4);
-      HOLE_CUDA_TRY(cudaMemset(p.seen, 0, 2 * p.bitmap_words * 4));
-      p.dup = p.seen + p.bitmap_words;
-      WS_ALLOC(p.done, (size_t)S * sizeof(unsigned));
-      HOLE_CUDA_TRY(cudaMemset(p.done, 0, (size_t)S * sizeof(unsigned)));
-      WS_ALLOC(p.blkcnt, (size_t)S * ((M + DP_TILE - 1) / DP_TILE + 1) * 4);
-      WS_ALLOC(p.mdup, (size_t)S * 4);
-    }
-    WS_ALLOC(p.gslot, S * M * 4);
-    WS_ALLOC(p.heads, (size_t)S * (M / 2 + 1) * sizeof(uint4));
-    WS_ALLOC(p.nheads, (size_t)S * 4);
-    WS_ALLOC(p.neg, (size_t)S * B * 4);
-    WS_ALLOC(p.perm, (size_t)S * B * 4);
-    WS_ALLOC(p.ghist, (size_t)S * 256 * tiles * 4);
-    p.used = false;
+    const int rc = plan_alloc(c, c->plan[k], B, S);
+    if (rc) { ws_free(c); return rc; }
   }
 #undef WS_ALLOC
   HOLE_CUDA_TRY(cudaMemset(c->counters, 0, (size_t)HOLE_TREE_LEVELS * M * 4));
@@ -1933,9 +1949,12 @@ static int plan_steps(hole_ctx* c, hole_plan& pl, const int32_t* triples_dev, in
   }
   HOLE_CUDA_TRY(cudaEventRecord(pl.ready, ps));
   // (off the consumer's path) clean bitmaps for the next plan in this slot; report the largest step to the host
+  // (the plans of the context's two slots report; the row-sharded log-loss step's own plan does not)
   HOLE_CUDA_TRY(cudaMemsetAsync(pl.seen, 0, (size_t)2 * pl.bitmap_words * 4, ps));   // seen | dup (one allocation)
-  hole_plan_dupmax_kernel<<<1, 256, 0, ps>>>(pl.mdup, (int)S, c->dup_max_host_dev + (&pl - c->plan));
-  HOLE_LAUNCHED();
+  if (&pl == &c->plan[0] || &pl == &c->plan[1]) {
+    hole_plan_dupmax_kernel<<<1, 256, 0, ps>>>(pl.mdup, (int)S, c->dup_max_host_dev + (&pl - c->plan));
+    HOLE_LAUNCHED();
+  }
   return HOLE_OK;
 }
 
@@ -2250,17 +2269,20 @@ static int route_reserve(hole_ctx* c, int64_t M, int64_t S = 1) {
 }
 
 // S steps at once: pos [S][B][3], neg_ent [S][B] -> uniq_out [S][uniq_stride], cuts_out [S][HOLE_MAX_RANKS+1]
-// (S == 1: exactly world+1 entries are written), pos_w [S][B][3], neg_w [S][B]
+// (S == 1: exactly world+1 entries are written), pos_w [S][B][3], neg_w [S][B].
+// n_neg > 1 (one step, a log-loss step's k corrupt batches): neg_ent and neg_w are [n_neg][B], and the request
+// list is the union of the (2 + n_neg)B entity uses.
 static int shard_route(hole_ctx* c, const int32_t* pos, const int32_t* neg_ent, int64_t B,
                        int64_t n_relations, int64_t n_rows_global, int64_t rows_per_rank,
                        int world, int32_t* uniq_out, int32_t* cuts_out, int32_t* pos_w,
-                       int32_t* neg_w, void* stream, int64_t S = 1, int64_t uniq_stride = 0) {
+                       int32_t* neg_w, void* stream, int64_t S = 1, int64_t uniq_stride = 0, int n_neg = 1) {
   HOLE_CHECK_ARG(c && pos && neg_ent && uniq_out && cuts_out && pos_w && neg_w);
-  HOLE_CHECK_ARG(B > 0 && 3 * B < (int64_t(1) << 31) && world >= 1 && world <= HOLE_MAX_RANKS && S >= 1);
+  HOLE_CHECK_ARG(n_neg >= 1 && (n_neg == 1 || S == 1));
+  HOLE_CHECK_ARG(B > 0 && (2 + n_neg) * B < (int64_t(1) << 31) && world >= 1 && world <= HOLE_MAX_RANKS && S >= 1);
   HOLE_CHECK_ARG(n_relations >= 0 && rows_per_rank > 0 && n_rows_global > n_relations &&
                  n_rows_global <= (int64_t(1) << 31));
   HOLE_CUDA_TRY(cudaSetDevice(c->device));
-  const int M = (int)(3 * B);
+  const int M = (int)((2 + n_neg) * B);
   if (uniq_stride <= 0) uniq_stride = M;
   int rc = route_reserve(c, M, S);
   if (rc) return rc;
@@ -2272,6 +2294,10 @@ static int shard_route(hole_ctx* c, const int32_t* pos, const int32_t* neg_ent, 
   dim3 kgrid((unsigned)std::min<int64_t>((B + 255) / 256, 1024), (unsigned)S);
   hole_shard_keys_kernel<<<kgrid, 256, 0, st>>>(pos, neg_ent, (int)B, kA);
   HOLE_LAUNCHED();
+  // the further corrupt columns are keys as they are (a row id is its own key): keys [3B, (2 + n_neg)B).  The
+  // assign kernel sends a sorted entry p >= 2B to neg_w[p - 2B], i.e. column (p - 2B) / B
+  if (n_neg > 1)
+    HOLE_CUDA_TRY(cudaMemcpyAsync(kA + 3 * B, neg_ent + B, (size_t)(n_neg - 1) * B * 4, cudaMemcpyDeviceToDevice, st));
   uint32_t *sk, *sp;
   rc = radix_sort(ghist, kA, kB, vA, vB, nullptr, S, M, passes, st, &sk, &sp, c->route_done);
   if (rc) return rc;

@@ -285,6 +285,30 @@ class HoleEngine:
         check(fn(self._ctx, _ptr(pos_i32), B, int(seed), int(step), float(margin), float(lr), _ptr(loss_out), _stream()))
         return loss_out
 
+    def shard_step_logloss(self, pos_i32, seed, step, lr, l2=0.0, negative_ratio=1, phase=None, want_corruption=False,
+                           want_l2_loss=None):
+        """One row-sharded --log_loss step (hole_shard_step_logloss) on this rank's slice (int32 CUDA [B,3], global
+        row ids) of the global batch.  Returns (loss [(1+k), B] device: my slice's rows without the L2 term,
+        l2_part device scalar: half the sum of squares of the old rows I own, relation rows on rank 0 only -- the
+        sum over ranks is train_step_logloss's l2_loss) and, with want_corruption, also (sides list,
+        neg [k, B] device).  The scalar is computed, like train_step_logloss's, only when l2 != 0 unless
+        want_l2_loss=True.  phase: None = whole step, "compute" = its first half (the l2 part is then written by
+        the apply half, shard_step(None, ..., phase="apply"))."""
+        if phase not in (None, "compute"):
+            raise HoleError(f"phase must be None or 'compute', got {phase!r} (the apply half is shard_step's)")
+        B, k = pos_i32.shape[0], int(negative_ratio)
+        loss = torch.empty((1 + max(k, 0), B), dtype=torch.float32, device=self.device)
+        l2_part = torch.zeros((), dtype=torch.float32, device=self.device)
+        neg = torch.empty((max(k, 0), B), dtype=torch.int32, device=self.device) if want_corruption else None
+        sides = (C.c_int32 * max(k, 1))()
+        fn = self.lib.hole_shard_step_logloss if phase is None else self.lib.hole_shard_step_logloss_compute
+        check(fn(self._ctx, _ptr(pos_i32), B, k, int(seed), int(step), float(lr), float(l2), _ptr(loss),
+                 _ptr(l2_part) if (want_l2_loss or (want_l2_loss is None and l2 != 0.0)) else None,
+                 None if neg is None else _ptr(neg), sides, _stream()))
+        if want_corruption:
+            return loss, l2_part, list(sides)[:k], neg
+        return loss, l2_part
+
     def shard_steps(self, triples_i32, batch_size, seed, first_step, margin, lrs):
         """n_steps consecutive sharded steps on device-resident slices [n_steps*B, 3]; returns the
         per-step loss sums of this rank's slices (device float32)."""

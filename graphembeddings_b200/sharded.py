@@ -127,6 +127,21 @@ class CudaBackend:
     def add_rows(self, table, ids, id_offset, rows):
         self.eng.add_rows(table, ids.contiguous(), id_offset, rows.contiguous())
 
+    def reserve_step_rows(self, max_batch):
+        """Room for R + 3 * max_batch step-table rows in the engine's context (a row-sharded log-loss step with k
+        negatives lists up to (2 + k) B rows): replaces the engine by a larger one if it is smaller.  Call before
+        anything is bound to the engine."""
+        if self.R + 3 * int(max_batch) <= self.eng.n_rows:
+            return self
+        from .engine import HoleEngine
+        old = self.eng
+        eng = HoleEngine(self.R + 3 * int(max_batch), self.dim, self.device.index or 0)
+        eng.set_relation_count(self.R)
+        eng.type_of, eng.csr_off, eng.csr_ids = old.type_of, old.csr_off, old.csr_ids
+        old.close()
+        self.eng = eng
+        return self
+
 
 class RowShardedTrainer:
     def __init__(self, n_relations, n_entities, dim, backend, dist=None, max_batch=None):
@@ -155,6 +170,12 @@ class RowShardedTrainer:
         from ._lib import HoleError
         raise HoleError(f"{type(self).__name__} (the all-to-all row-sharded trainer) trains with 'sgd' only; "
                         f"optimizer {optimizer!r} on several GPUs needs P2PRowShardedTrainer (NVLink peer memory)")
+
+    def train_step_logloss(self, pos_local, seed, step, lr, l2, negative_ratio):
+        """This all-to-all trainer has no --log_loss step; it runs on P2PRowShardedTrainer."""
+        from ._lib import HoleError
+        raise HoleError(f"{type(self).__name__} (the all-to-all row-sharded trainer) has no log-loss step; "
+                        f"--log_loss on several GPUs needs P2PRowShardedTrainer (NVLink peer memory)")
 
     def gather_embeddings(self):
         """Full [N, dim] table on every rank (tests / checkpointing)."""
@@ -428,14 +449,19 @@ class P2PRowShardedTrainer(RowShardedTrainer):
 
     No NCCL call and no host synchronisation inside a step."""
 
-    def __init__(self, n_relations, n_entities, dim, backend, dist, timeout_s=0.0, check_every=256):
+    def __init__(self, n_relations, n_entities, dim, backend, dist, timeout_s=0.0, check_every=256,
+                 negative_ratio=1):
+        """negative_ratio: the largest k of the train_step_logloss calls to come.  A log-loss step lists up to
+        (2 + k) B rows of B = backend.max_batch triples, so the staging buffers and inboxes hold
+        3 * max(B, ceil((2 + k) B / 3)) rows."""
         super().__init__(n_relations, n_entities, dim, backend, dist)
         from torch.multiprocessing.reductions import reduce_tensor
         dev, G, R = backend.device, self.world, self.R
-        eng = backend.eng
-        if eng.type_of is None:
+        if backend.eng.type_of is None:
             raise ValueError("the backend needs the type tables (type_of, csr_off, csr_ids) for the corruption")
-        self.max_batch = backend.max_batch
+        B = backend.max_batch
+        self.max_batch = max(B, -(-(2 + int(negative_ratio)) * B // 3))
+        eng = backend.reserve_step_rows(self.max_batch).eng
         self.cap = 3 * self.max_batch
         width = backend.width
         self.shard = torch.zeros((R + self.rows_per, width), dtype=torch.float32, device=dev)
@@ -619,6 +645,21 @@ class P2PRowShardedTrainer(RowShardedTrainer):
         if self.check_every and self._since_check >= self.check_every:
             self.check_barriers()
         return loss
+
+    def train_step_logloss(self, pos_local, seed, step, lr, l2, negative_ratio):
+        """One --log_loss step (holE.py:194-196, 206-220, 296; hole_shard_step_logloss) of the global batch: the
+        result of HoleEngine.train_step_logloss on the concatenated slices.  pos_local: this rank's [B,3] slice;
+        negative_ratio <= the trainer's.  Returns (loss rows of my slice [(1+k), B] device, without the L2 term;
+        my l2 part, a device scalar: half the sum of squares of the old rows I own, the relation rows counted on
+        rank 0 -- summed over the ranks, the global l2_loss; zero when l2 == 0).  A hinge step prepared ahead with
+        next_pos stays prepared."""
+        pos = self._as_slice(pos_local)
+        loss, l2_part = self.be.eng.shard_step_logloss(pos, seed, step, lr, l2, negative_ratio)
+        self._keep_logloss = pos                            # read by the step's kernels
+        self._since_check += 1
+        if self.check_every and self._since_check >= self.check_every:
+            self.check_barriers()
+        return loss, l2_part
 
     def train_steps(self, triples_i32, batch_size, seed, first_step, margin, lrs):
         """n_steps consecutive steps on device-resident slices [n_steps*B, 3] without returning to the

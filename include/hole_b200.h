@@ -261,9 +261,44 @@ HOLE_API int hole_shard_steps_host(hole_ctx* ctx, const int32_t* triples_host, i
                                    float* loss_sum_host, void* stream);
 HOLE_API int hole_shard_poll(hole_ctx* ctx, int* timed_out, void* stream);
 HOLE_API int hole_shard_set_optimizer(hole_ctx* ctx, int optimizer, float* accum_shard);
+/* hole_shard_step_logloss: one batch-synchronous --log_loss step (hole_train_step_logloss) of the GLOBAL
+ *   batch, the ranks' `pos` slices of B triples concatenated in rank order (world*B triples).  The result is
+ *   hole_train_step_logloss's on that global batch with the same (seed, step, lr, l2, k = negative_ratio):
+ *     negatives  pass j is virtual step step*k + j: side hole_side_coin(seed, step*k + j), Philox draws keyed
+ *                on the global triple index me*B + i, so the negatives and sides do not depend on `world`;
+ *     gradients  every pass of every rank reads rows no rank has changed in this step (the old table);
+ *     loss_out   device float32 [(1+k)*B]: my positives, then each corrupt batch, without the L2 term;
+ *     update     E <- E * (1 - lr*(1+k)*(world*B)*l2) + sum of the deltas (the one-GPU fp32 expression with
+ *                the global B).  The owner of an entity row adds the staged deltas of every listing rank in
+ *                rank order; every rank decays its relation replica and adds every rank's relation deltas in
+ *                rank order, so the replicas stay bit-identical.  Rows no triple touches are only scaled.
+ *                With l2 == 0 and no l2_part_out there is no dense pass;
+ *     l2_part_out  optional device float32 scalar: half the sum of squares of the OLD rows I own (my entity
+ *                block, and the relation rows on rank 0 only); the sum over ranks is the one-GPU l2_loss.
+ *                Written by the apply half;
+ *     neg_out    optional device int32 [k][B] (global row ids), sides_out optional HOST int32 [k].
+ *   Every rank must call it with the same (B, k, seed, step, lr, l2) sequence; log-loss steps may sit between
+ *   hinge hole_shard_step(s) calls on one context (they advance the same epochs and leave a hinge step prepared
+ *   ahead by hole_shard_prepare in place).  Rows are gathered once per step into a local step table, whatever k
+ *   is.  Needs (2+k)*B <= 3*max_batch and n_relations + (2+k)*B <= the context's n_rows; k in [1, 64]; the
+ *   shard optimizer HOLE_OPT_SGD.  Otherwise, or before hole_shard_init, HOLE_ERR_ARG / HOLE_ERR_UNSUPPORTED,
+ *   and nothing is launched or written.  The step's buffers are allocated by its first call (and grown with k).
+ * hole_shard_step_logloss_compute: its first half (corruption and routing, the passes' plan on a side
+ *   stream beside the post and the gather, the k passes, push, finish); it latches the decay and l2_part_out for the next hole_shard_step_apply, which is the
+ *   second half.  After a hinge compute half nothing is latched. */
+HOLE_API int hole_shard_step_logloss(hole_ctx* ctx, const int32_t* pos, int64_t B, int negative_ratio, uint64_t seed,
+                                     uint64_t step, float lr, float l2, float* loss_out, float* l2_part_out,
+                                     int32_t* neg_out, int32_t* sides_out, void* stream);
+HOLE_API int hole_shard_step_logloss_compute(hole_ctx* ctx, const int32_t* pos, int64_t B, int negative_ratio,
+                                             uint64_t seed, uint64_t step, float lr, float l2, float* loss_out,
+                                             float* l2_part_out, int32_t* neg_out, int32_t* sides_out,
+                                             void* stream);
 /* Measurement hook: with hole_profile_enable on, summed milliseconds of the step's phases
  * [post, K1 (incl. its wait for the peers' shards), K3, finish, apply (incl. its wait for the peers'
- * deltas)] -> phase_ms5 [host, double[5]], and the number of steps measured since the last read. */
+ * deltas)] -> phase_ms5 [host, double[5]], and the number of steps measured since the last read.
+ * A log-loss step's five phases are [corruption + route + post, gather (incl. its wait for the peers'
+ * shards), the k passes (incl. the wait for their plan, built on the side stream beside the post and the
+ * gather), push + finish, apply (incl. its wait and the decay)]. */
 HOLE_API int hole_shard_profile_read(hole_ctx* ctx, double* phase_ms5, int64_t* n_steps);
 
 /* Building blocks of the step, exported for tests.
