@@ -65,6 +65,8 @@ SIGNATURES = {
     "hole_rank_invalidate": (_int, [_p]),
     "hole_topk": (_int, [_p, _p, _i64, _i64, _p, _i64, _int, _int, _int, _p, _p, _p, _p, _p]),
     "hole_neighbors": (_int, [_p, _p, _i64, _i64, _p, _i64, _int, _int, _p, _p, _p, _p, _p]),
+    "hole_rank_typed": (_int, [_p, _p, _p, _i64, _int, _int, _p, _p, _p, _i64, _p, _p, _p, _p, _p, _p]),
+    "hole_topk_typed": (_int, [_p, _p, _p, _p, _i64, _int, _int, _int, _p, _p, _i64, _p, _p, _p, _p, _p]),
     "hole_rank_debug_operands": (_int, [_p, _p, _p, C.POINTER(_i64), C.POINTER(_i64), C.POINTER(_int), _p]),
     "hole_profile_enable": (_int, [_p, _int]),
     "hole_profile_read": (_int, [_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(_i64)]),

@@ -45,6 +45,14 @@ enum { MODE_COUNT = 0, MODE_DIAG = 1 };
 // each thread's k best candidates (hole_topk)
 enum { EPI_RANK = 0, EPI_TOPK = 1 };
 
+// One work item of a typed call: query slots [q0, min(q0 + BM, q_end)) of type tau against candidate tiles
+// [t0, t1) of the type's operand segment, rows [seg, seg + n).  Top-k: the list of slot q0 + i, column group g
+// is list l0 + i * lstride + g.
+struct TypedItem {
+  int32_t q0, q_end, seg, n, t0, t1, tau, lstride;
+  int64_t l0;
+};
+
 struct RankParams {
   int mode;
   int num_kb;        // k-blocks of ONE operand part: round_up(D, 64) / 64
@@ -71,6 +79,13 @@ struct RankParams {
   const int32_t* f_ids;        //       ids ascending within a query's slice
   int64_t ent_begin;
   const int32_t* tk_self;      // [Qpad] hole_neighbors: shard-local index each query never returns (itself); else null
+  // typed calls (TYPED instantiations): work items from the device plan, rows in slot order (queries grouped by type)
+  const TypedItem* t_items;
+  const int32_t* t_n_items;    // item count, written by the plan
+  const int32_t* t_perm;       // [Q] slot -> caller row (the filter CSR is in caller rows)
+  const int32_t* type_of;      // [n_rows]
+  const int32_t* t_pos;        // [n_rows] position of an id within its type's slice of csr_ids, -1 if none
+  const int32_t* csr_ids;
 };
 
 // ------------------------------------------------------------------------------------ PTX
@@ -207,8 +222,30 @@ struct FilterCursor {
                              // is loaded one step ahead, so that a step of the cursor does not wait for memory
 };
 
-__device__ __forceinline__ int filter_id_at(const int32_t* __restrict__ ids, int64_t i, int64_t f1, int64_t ent_begin) {
-  return i < f1 ? (int)((int64_t)ids[i] - ent_begin) : INT_MAX;
+// Candidate columns of a call, as seen by the epilogue: column j is global id gid_of(cm, j); a filter id is column
+// col_of(cm, id).  cm = ent_begin: the contiguous range [ent_begin, ...).  cm = TypeCols: the segment of one type,
+// ids ascending with the column; a filter id of another type maps to -1, which the merge-join passes like an id
+// below its columns.
+struct TypeCols {
+  const int32_t* __restrict__ type_of;
+  const int32_t* __restrict__ pos;
+  const int32_t* __restrict__ seg_ids;     // csr_ids + the segment's start
+  int tau, n;
+  __device__ __forceinline__ int col(int32_t id) const { return type_of[id] == tau ? pos[id] : -1; }
+  __device__ __forceinline__ int64_t gid(int j) const { return seg_ids[j]; }
+  __device__ __forceinline__ int64_t lb_key(int j) const { return j < n ? (int64_t)seg_ids[j] : (int64_t)INT_MAX + 1; }
+};
+__device__ __forceinline__ int col_of(int64_t ent_begin, int32_t id) { return (int)((int64_t)id - ent_begin); }
+__device__ __forceinline__ int col_of(const TypeCols& cm, int32_t id) { return cm.col(id); }
+__device__ __forceinline__ int64_t gid_of(int64_t ent_begin, int j) { return ent_begin + j; }
+__device__ __forceinline__ int64_t gid_of(const TypeCols& cm, int j) { return cm.gid(j); }
+// the low half of a top-k key: the local index, or in a typed call the global id (ascending with the column)
+__device__ __forceinline__ int key_of(int64_t, int j) { return j; }
+__device__ __forceinline__ int key_of(const TypeCols& cm, int j) { return (int)cm.gid(j); }
+
+template <class Cols>
+__device__ __forceinline__ int filter_id_at(const int32_t* __restrict__ ids, int64_t i, int64_t f1, Cols cm) {
+  return i < f1 ? col_of(cm, ids[i]) : INT_MAX;
 }
 
 // First id of f_ids[lo, hi) that is >= id (hi if none).
@@ -221,12 +258,13 @@ __device__ __forceinline__ int64_t lower_bound_id(const int32_t* __restrict__ id
 }
 
 // Moves the cursor past every copy of the id it stands on (a repeated id is one candidate).
-__device__ __forceinline__ void filter_advance(FilterCursor& f, const int32_t* __restrict__ ids, int64_t ent_begin) {
+template <class Cols>
+__device__ __forceinline__ void filter_advance(FilterCursor& f, const int32_t* __restrict__ ids, Cols cm) {
   const int cur = f.next;
   do {
     ++f.fp;
     f.next = f.after;
-    f.after = filter_id_at(ids, f.fp + 1, f.f1, ent_begin);
+    f.after = filter_id_at(ids, f.fp + 1, f.f1, cm);
   } while (f.next <= cur);
 }
 
@@ -236,9 +274,10 @@ __device__ __forceinline__ void filter_advance(FilterCursor& f, const int32_t* _
 // walks the heap in index order).  A filtered column is subtracted exactly when this very compare counted
 // it, so filt_before is exact with respect to raw_before; the true column itself never counts (s == thr,
 // j == tie), whether or not it is filtered.
+template <class Cols>
 __device__ __forceinline__ void epi_count32(const uint32_t (&v)[32], int j0, float thr, float thr_hi, int tie,
                                             int Nc, int& c0, FilterCursor& f, const int32_t* __restrict__ f_ids,
-                                            int64_t ent_begin, int& fc) {
+                                            Cols cm, int& fc) {
   const bool slow = (j0 < tie && tie < j0 + 32) || (j0 + 32 > Nc) || (f.next < j0 + 32);
   if (!__any_sync(0xffffffffu, slow)) {
     const float tt = (j0 + 32 <= tie) ? thr_hi : thr;
@@ -264,29 +303,30 @@ __device__ __forceinline__ void epi_count32(const uint32_t (&v)[32], int j0, flo
         const float tt = (j < tie) ? thr_hi : thr;
         fc += (j < Nc && s < tt) ? 1 : 0;
       }
-      filter_advance(f, f_ids, ent_begin);
+      filter_advance(f, f_ids, cm);
     }
     __syncwarp();          // reconverge before the next .sync.aligned tcgen05 instruction
   }
 }
 // 128 columns (four chunks) of one accumulator row; the TMEM load of a chunk is in flight while
 // the previous one is counted.
+template <class Cols>
 __device__ __forceinline__ void epi_count128(uint32_t taddr0, int j0, float thr, float thr_hi, int tie, int Nc,
                                              int& c0, FilterCursor& f, const int32_t* __restrict__ f_ids,
-                                             int64_t ent_begin, int& fc) {
+                                             Cols cm, int& fc) {
   uint32_t va[32], vb[32];
   tmem_ld32_async(taddr0, va);
   tmem_ld_wait(va);
   tmem_ld32_async(taddr0 + 32, vb);
-  epi_count32(va, j0, thr, thr_hi, tie, Nc, c0, f, f_ids, ent_begin, fc);
+  epi_count32(va, j0, thr, thr_hi, tie, Nc, c0, f, f_ids, cm, fc);
   tmem_ld_wait(vb);
   tmem_ld32_async(taddr0 + 64, va);
-  epi_count32(vb, j0 + 32, thr, thr_hi, tie, Nc, c0, f, f_ids, ent_begin, fc);
+  epi_count32(vb, j0 + 32, thr, thr_hi, tie, Nc, c0, f, f_ids, cm, fc);
   tmem_ld_wait(va);
   tmem_ld32_async(taddr0 + 96, vb);
-  epi_count32(va, j0 + 64, thr, thr_hi, tie, Nc, c0, f, f_ids, ent_begin, fc);
+  epi_count32(va, j0 + 64, thr, thr_hi, tie, Nc, c0, f, f_ids, cm, fc);
   tmem_ld_wait(vb);
-  epi_count32(vb, j0 + 96, thr, thr_hi, tie, Nc, c0, f, f_ids, ent_begin, fc);
+  epi_count32(vb, j0 + 96, thr, thr_hi, tie, Nc, c0, f, f_ids, cm, fc);
 }
 
 // ---- top-k epilogue.  A candidate is the 64-bit key (order-preserving bits of s, local index j): ascending
@@ -365,8 +405,9 @@ __device__ __forceinline__ bool epi_topk_vote(const uint32_t (&v)[32], float thr
 }
 // Slow path, only for a warp in which some lane admits a candidate of columns j0 .. j0+31: bounds, filter,
 // heap insert.  Runs while no tcgen05.ld is in flight (the loaded registers are final).
+template <class Cols>
 __device__ __forceinline__ void epi_topk_admit(const uint32_t (&v)[32], int j0, TopkList& L, int Nc,
-                                               const int32_t* __restrict__ f_ids, int64_t ent_begin) {
+                                               const int32_t* __restrict__ f_ids, Cols cm) {
   uint32_t m = 0;
 #pragma unroll
   for (int c = 0; c < 32; ++c) m |= (__uint_as_float(v[c]) < L.thr ? 1u : 0u) << c;
@@ -378,31 +419,32 @@ __device__ __forceinline__ void epi_topk_admit(const uint32_t (&v)[32], int j0, 
     for (int i = 0; i < 32; ++i) s = (i == c) ? __uint_as_float(v[i]) : s;     // no dynamic register index
     const int j = j0 + c;
     if (!(s < L.thr) || j >= Nc || j == L.self) continue;                      // thr may have dropped
-    if (L.f0 < L.f1 && in_filter(f_ids, L.f0, L.f1, (int32_t)(ent_begin + j))) continue;
-    topk_insert(L, topk_key(s, (uint32_t)j));
+    if (L.f0 < L.f1 && in_filter(f_ids, L.f0, L.f1, (int32_t)gid_of(cm, j))) continue;
+    topk_insert(L, topk_key(s, (uint32_t)key_of(cm, j)));
   }
   __syncwarp();          // reconverge before the next .sync.aligned tcgen05 instruction
 }
 // 128 columns of one accumulator row.  The next chunk's TMEM load is in flight during the vote on the current
 // one; the slow path of a chunk runs after that load has landed.
+template <class Cols>
 __device__ __forceinline__ void epi_topk128(uint32_t taddr0, int j0, TopkList& L, int Nc,
-                                            const int32_t* __restrict__ f_ids, int64_t ent_begin) {
+                                            const int32_t* __restrict__ f_ids, Cols cm) {
   uint32_t va[32], vb[32];
   tmem_ld32_async(taddr0, va);
   tmem_ld_wait(va);
   tmem_ld32_async(taddr0 + 32, vb);
   bool h = epi_topk_vote(va, L.thr);
   tmem_ld_wait(vb);
-  if (h) epi_topk_admit(va, j0, L, Nc, f_ids, ent_begin);
+  if (h) epi_topk_admit(va, j0, L, Nc, f_ids, cm);
   tmem_ld32_async(taddr0 + 64, va);
   h = epi_topk_vote(vb, L.thr);
   tmem_ld_wait(va);
-  if (h) epi_topk_admit(vb, j0 + 32, L, Nc, f_ids, ent_begin);
+  if (h) epi_topk_admit(vb, j0 + 32, L, Nc, f_ids, cm);
   tmem_ld32_async(taddr0 + 96, vb);
   h = epi_topk_vote(va, L.thr);
   tmem_ld_wait(vb);
-  if (h) epi_topk_admit(va, j0 + 64, L, Nc, f_ids, ent_begin);
-  if (epi_topk_vote(vb, L.thr)) epi_topk_admit(vb, j0 + 96, L, Nc, f_ids, ent_begin);
+  if (h) epi_topk_admit(va, j0 + 64, L, Nc, f_ids, cm);
+  if (epi_topk_vote(vb, L.thr)) epi_topk_admit(vb, j0 + 96, L, Nc, f_ids, cm);
 }
 
 struct SmemLayout {
@@ -418,11 +460,12 @@ struct SmemLayout {
 // ------------------------------------------------------------------------------------ kernel
 // PARTS = 1 plain bf16, 2 split-bf16 (compile-time, so that the bf16 instantiation's single-thread
 // producer / issue loops carry none of the split mode's bookkeeping); EPI = EPI_RANK / EPI_TOPK (compile-time,
-// so that the counting epilogue carries none of the top-k code).
+// so that the counting epilogue carries none of the top-k code); TYPED (compile-time, so that the all-candidate
+// instantiations are unchanged): items are TypedItems of the device plan, each against one type's segment.
 // p is __grid_constant__ so that its fields are read in place from parameter space where they are used.  Passed
 // by value, the struct (136 bytes) is loaded into registers at entry, and each top-k instantiation compiles to
 // 112 more instructions.
-template <int PARTS, int EPI>
+template <int PARTS, int EPI, bool TYPED = false>
 __global__ void __launch_bounds__(RANK_THREADS, 1)
 hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const __grid_constant__ RankParams p) {
@@ -435,7 +478,7 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   SmemLayout* sl = reinterpret_cast<SmemLayout*>(sB + (size_t)p.stages * B_KB_BYTES);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int n_items = p.m_tiles * p.n_chunks;
+  const int n_items = TYPED ? *p.t_n_items : p.m_tiles * p.n_chunks;
 
   if (warp == WARP_TMA && lane == 0) {
     tma_prefetch_desc(&tmA);
@@ -460,15 +503,19 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       const uint32_t b_bytes = (p.mode == MODE_DIAG) ? B_KB_BYTES / 2 : B_KB_BYTES;
       for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
         const int m_tile = item / p.n_chunks, chunk = item % p.n_chunks;
+        // typed: the query tile starts at any row (rows past the operand are zero-filled, rows of the next type
+        // are inactive in the epilogue), the candidate tiles at the type's segment
+        TypedItem it{};
+        if constexpr (TYPED) it = p.t_items[item];
         mbar_wait(&sl->a_empty, a_phase ^ 1);
         mbar_expect_tx(&sl->a_full, (uint32_t)nkb_all * A_KB_BYTES);
         for (int kb = 0; kb < nkb_all; ++kb)
-          tma_load_2d(sA + (size_t)kb * A_KB_BYTES, &tmA, &sl->a_full, kb * BK, m_tile * BM);
+          tma_load_2d(sA + (size_t)kb * A_KB_BYTES, &tmA, &sl->a_full, kb * BK, TYPED ? it.q0 : m_tile * BM);
         a_phase ^= 1;
-        const int t0 = chunk * p.chunk_tiles;
-        const int t1 = (p.mode == MODE_DIAG) ? t0 + 1 : min(p.n_tiles, t0 + p.chunk_tiles);
+        const int t0 = TYPED ? it.t0 : chunk * p.chunk_tiles;
+        const int t1 = TYPED ? it.t1 : (p.mode == MODE_DIAG) ? t0 + 1 : min(p.n_tiles, t0 + p.chunk_tiles);
         for (int t = t0; t < t1; ++t) {
-          const int row0 = (p.mode == MODE_DIAG) ? m_tile * BM : t * BN;
+          const int row0 = (p.mode == MODE_DIAG) ? m_tile * BM : (TYPED ? it.seg : 0) + t * BN;
           for (int kb = 0; kb < nkb_all; ++kb) {
             mbar_wait(&sl->empty[stage], phase ^ 1);
             mbar_expect_tx(&sl->full[stage], b_bytes);
@@ -490,8 +537,8 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         mbar_wait(&sl->a_full, a_phase);
         a_phase ^= 1;
         tc_fence_after();
-        const int t0 = chunk * p.chunk_tiles;
-        const int t1 = (p.mode == MODE_DIAG) ? t0 + 1 : min(p.n_tiles, t0 + p.chunk_tiles);
+        const int t0 = TYPED ? p.t_items[item].t0 : chunk * p.chunk_tiles;
+        const int t1 = TYPED ? p.t_items[item].t1 : (p.mode == MODE_DIAG) ? t0 + 1 : min(p.n_tiles, t0 + p.chunk_tiles);
         for (int t = t0; t < t1; ++t) {
           mbar_wait(&sl->tmem_empty[acc], acc_phase ^ 1);
           tc_fence_after();
@@ -548,6 +595,32 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     int acc = 0; uint32_t acc_phase = 0;
     for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
       const int m_tile = item / p.n_chunks, chunk = item % p.n_chunks;
+      if constexpr (TYPED) {
+        const TypedItem it = p.t_items[item];
+        const int q = it.q0 + row_in_tile;
+        const bool qok = q < it.q_end;
+        TopkList L;
+        L.heap = p.tk_keys + (size_t)(it.l0 + (int64_t)row_in_tile * it.lstride + cgrp) * p.topk;
+        L.n = 0; L.k = p.topk;
+        L.thr = qok ? INFINITY : -INFINITY;          // rows of another type admit nothing
+        L.f0 = L.f1 = 0;
+        if (qok && p.f_off != nullptr) { const int cq = p.t_perm[q]; L.f0 = p.f_off[cq]; L.f1 = p.f_off[cq + 1]; }
+        L.self = -1;
+        const TypeCols cm{p.type_of, p.t_pos, p.csr_ids + it.seg, it.tau, it.n};
+        for (int t = it.t0; t < it.t1; ++t) {
+          mbar_wait(&sl->tmem_full[acc], acc_phase);
+          tc_fence_after();
+          const uint32_t taddr0 = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * BN + cgrp * EPI_COLS);
+          epi_topk128(taddr0, t * BN + cgrp * EPI_COLS, L, it.n, p.f_ids, cm);
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) mbar_arrive(&sl->tmem_empty[acc]);
+          if (++acc == 2) { acc = 0; acc_phase ^= 1; }
+        }
+        if (qok)
+          for (int i = L.n; i < L.k; ++i) L.heap[i] = TOPK_EMPTY;
+        continue;
+      }
       const int q = m_tile * BM + row_in_tile;
       const bool qok = q < p.Q;
       TopkList L;
@@ -581,6 +654,47 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     int acc = 0; uint32_t acc_phase = 0;
     for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
       const int m_tile = item / p.n_chunks, chunk = item % p.n_chunks;
+      if constexpr (TYPED) {
+        // counts only (the diagonal pass runs untyped on the slot-ordered operands); rows in slot order
+        const TypedItem it = p.t_items[item];
+        const int q = it.q0 + row_in_tile;
+        const bool qok = q < it.q_end;
+        const TypeCols cm{p.type_of, p.t_pos, p.csr_ids + it.seg, it.tau, it.n};
+        float thr = -INFINITY, thr_hi = -INFINITY;
+        int tie = 0;
+        FilterCursor fcur{0, 0, INT_MAX, INT_MAX};
+        if (qok) {
+          thr = p.true_score[q];
+          if (p.f_off != nullptr) {
+            const int cq = p.t_perm[q];
+            int64_t f0 = p.f_off[cq];
+            fcur.f1 = p.f_off[cq + 1];
+            if (fcur.f1 - f0 > 16) f0 = lower_bound_id(p.f_ids, f0, fcur.f1, cm.lb_key(it.t0 * BN + cgrp * EPI_COLS));
+            fcur.fp = f0;
+            fcur.next = filter_id_at(p.f_ids, f0, fcur.f1, cm);
+            fcur.after = filter_id_at(p.f_ids, f0 + 1, fcur.f1, cm);
+          }
+          thr_hi = nextafterf(thr, INFINITY);
+          const int ti = p.true_idx[q] - it.seg;     // the true candidate's column in the segment
+          tie = ti < 0 ? 0 : (ti > it.n ? it.n : ti);
+        }
+        int cnt = 0, fcnt = 0;
+        for (int t = it.t0; t < it.t1; ++t) {
+          mbar_wait(&sl->tmem_full[acc], acc_phase);
+          tc_fence_after();
+          const uint32_t taddr0 = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * BN + cgrp * EPI_COLS);
+          epi_count128(taddr0, t * BN + cgrp * EPI_COLS, thr, thr_hi, tie, it.n, cnt, fcur, p.f_ids, cm, fcnt);
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) mbar_arrive(&sl->tmem_empty[acc]);
+          if (++acc == 2) { acc = 0; acc_phase ^= 1; }
+        }
+        if (qok && cnt != 0) {
+          atomicAdd(&p.raw_cnt[q], cnt);
+          atomicAdd(&p.filt_cnt[q], cnt - fcnt);
+        }
+        continue;
+      }
       const int q = m_tile * BM + row_in_tile;
       const bool qok = q < p.Q;
       const int t0 = chunk * p.chunk_tiles;
@@ -612,8 +726,8 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         const uint32_t taddr0 = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * BN + cgrp * EPI_COLS);
         if (p.mode == MODE_COUNT) {
           static_assert(EPI_COLS == 128, "epi_count128 covers 128 columns per warp");
-          epi_count128(taddr0, t * BN + cgrp * EPI_COLS, thr, thr_hi, tie, p.Nc, cnt, fcur, p.f_ids, p.ent_begin,
-                       fcnt);
+          epi_count128(taddr0, t * BN + cgrp * EPI_COLS, thr, thr_hi, tie, p.Nc, cnt, fcur, p.f_ids,
+                       p.ent_begin, fcnt);
         } else if (cgrp == (quarter * 32) / EPI_COLS) {
           // DIAG: row i of the tile wants column i, which lives in chunk `quarter`, register `lane`
           uint32_t v[32];
@@ -646,18 +760,22 @@ hole_rank_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 // ------------------------------------------------------------------------------------ operand packing
 // One warp per row.  Candidate operand: clip(E_j) rounded to bf16, [Re | Im | 0-pad] of K columns; with
 // `normalize` (hole_neighbors) E_j / |E_j| instead, and zero for a zero row.
+// GATHER (typed calls): row r is table row gather[r], for r < *gather_n (the type tables' csr_ids and
+// csr_off[n_types]), so that each type's candidates are contiguous operand rows; Nc is then unused.
+template <bool GATHER = false>
 __global__ void __launch_bounds__(256)
 hole_rank_pack_cand_kernel(const float* __restrict__ table, int stride, int H, int64_t ent_begin,
-                           int Nc, int Npad, int K, int parts, int normalize, __nv_bfloat16* __restrict__ out) {
+                           int Nc, int Npad, int K, int parts, int normalize, __nv_bfloat16* __restrict__ out,
+                           const int32_t* __restrict__ gather = nullptr, const int64_t* __restrict__ gather_n = nullptr) {
   const int lane = threadIdx.x & 31;
   const int64_t r = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
   if (r >= Npad) return;
   __nv_bfloat16* o = out + (size_t)r * K * parts;       // row = [hi part (K) | lo part (K)]
-  if (r >= Nc) {
+  if (GATHER ? r >= *gather_n : r >= Nc) {
     for (int k = lane; k < K * parts; k += 32) o[k] = __float2bfloat16(0.f);
     return;
   }
-  const float* x = table + (size_t)(ent_begin + r) * stride;
+  const float* x = table + (size_t)(GATHER ? (int64_t)gather[r] : ent_begin + r) * stride;
   const int Hp = stride / 2;
   float ss = 0.f;
   for (int k = lane; k < H; k += 32) { float a = x[k], b = x[Hp + k]; ss = fmaf(a, a, fmaf(b, b, ss)); }
@@ -1043,6 +1161,185 @@ hole_topk_merge_kernel(const uint64_t* __restrict__ keys, int n_lists, int k, co
   }
 }
 
+// ------------------------------------------------------------------------------------ typed-call plan
+// hole_rank_typed / hole_topk_typed rank each query against the candidates of one type.  The candidate operand is
+// packed in csr_ids order, so type tau is the operand rows [csr_off[tau], csr_off[tau+1]) (its segment); the plan
+// below groups the queries by type (slots), and writes the work items, on the device:
+//   typed_pos    t_pos[id] = id's position in its type's segment
+//   typed_count  each query's type, and its place among the queries of that type (arrival order: a query's
+//                results do not depend on its slot)
+//   typed_scan   per type: first slot, items per query window, first item; the item count
+//   typed_place  slot-ordered triples, slot -> caller row, slot types, the true candidate's operand row
+//   typed_items  one TypedItem per (query window of <= BM slots, chunk of the type's candidate tiles)
+constexpr int PLAN_THREADS = 1024;
+
+__global__ void __launch_bounds__(256)
+hole_typed_pos_kernel(const int32_t* __restrict__ type_of, const int64_t* __restrict__ csr_off,
+                      const int32_t* __restrict__ csr_ids, int64_t n_types, int32_t* __restrict__ t_pos) {
+  const int64_t n = csr_off[n_types];
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int32_t id = csr_ids[i];
+    t_pos[id] = (int32_t)(i - csr_off[type_of[id]]);
+  }
+}
+
+// query_type != null: hole_topk_typed's caller-given types; else the type of the true candidate (t / h)
+__global__ void __launch_bounds__(256)
+hole_typed_count_kernel(const int32_t* __restrict__ queries, const int32_t* __restrict__ query_type, int Q, int side,
+                        const int32_t* __restrict__ type_of, int32_t* __restrict__ qtype, int32_t* __restrict__ qrank,
+                        int32_t* __restrict__ tcount) {
+  const int q = blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= Q) return;
+  const int tau = query_type != nullptr ? query_type[q] : type_of[queries[3 * q + (side == HOLE_SIDE_TAIL ? 1 : 0)]];
+  qtype[q] = tau;
+  qrank[q] = atomicAdd(&tcount[tau], 1);
+}
+
+// Exclusive block-wide scan of one value per thread (PLAN_THREADS threads); returns the thread's prefix.
+__device__ int64_t block_excl_scan(int64_t v, int64_t* warp_sums, int64_t* total) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int64_t inc = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int64_t y = __shfl_up_sync(0xffffffffu, inc, o);
+    if (lane >= o) inc += y;
+  }
+  if (lane == 31) warp_sums[warp] = inc;
+  __syncthreads();
+  if (warp == 0) {
+    int64_t w = warp_sums[lane], wi = w;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int64_t y = __shfl_up_sync(0xffffffffu, wi, o);
+      if (lane >= o) wi += y;
+    }
+    warp_sums[lane] = wi - w;
+    if (lane == 31) *total = wi;
+  }
+  __syncthreads();
+  const int64_t r = warp_sums[warp] + inc - v;
+  __syncthreads();
+  return r;
+}
+
+// One block.  chunk_tiles: the target candidate tiles per item (split_chunks of the all-candidate shape, so that
+// no type has more chunks than that shape, and the item count stays within the workspace sized for it); a type's
+// tiles are cut into nch[tau] equal chunks of tper[tau] tiles.  A type without candidates gets no items (its top-k rows are padding).
+__global__ void __launch_bounds__(PLAN_THREADS)
+hole_typed_scan_kernel(const int32_t* __restrict__ tcount, const int64_t* __restrict__ csr_off, int n_types,
+                       int chunk_tiles, int32_t* __restrict__ qoff, int32_t* __restrict__ nch,
+                       int32_t* __restrict__ tper, int32_t* __restrict__ ioff, int32_t* __restrict__ n_items) {
+  __shared__ int64_t ws[32], tot;
+  const int per = (n_types + PLAN_THREADS - 1) / PLAN_THREADS;
+  const int b = min(n_types, (int)threadIdx.x * per), e = min(n_types, b + per);
+  auto chunks = [&](int tau, int& ch, int& tp) {
+    const int64_t n = csr_off[tau + 1] - csr_off[tau];
+    const int tiles = (int)((n + BN - 1) / BN);
+    ch = 0; tp = 0;
+    if (tcount[tau] > 0 && tiles > 0) {
+      tp = (tiles + (tiles + chunk_tiles - 1) / chunk_tiles - 1) / ((tiles + chunk_tiles - 1) / chunk_tiles);
+      ch = (tiles + tp - 1) / tp;
+    }
+  };
+  int64_t sq = 0, si = 0;
+  for (int tau = b; tau < e; ++tau) {
+    int ch, tp;
+    chunks(tau, ch, tp);
+    const int c = tcount[tau];
+    sq += c;
+    si += (int64_t)ch * ((c + BM - 1) / BM);
+  }
+  int64_t pq = block_excl_scan(sq, ws, &tot);
+  int64_t pi = block_excl_scan(si, ws, &tot);
+  if (threadIdx.x == 0) *n_items = (int32_t)tot;
+  for (int tau = b; tau < e; ++tau) {
+    int ch, tp;
+    chunks(tau, ch, tp);
+    const int c = tcount[tau];
+    qoff[tau] = (int32_t)pq; nch[tau] = ch; tper[tau] = tp; ioff[tau] = (int32_t)pi;
+    pq += c;
+    pi += (int64_t)ch * ((c + BM - 1) / BM);
+  }
+}
+
+// Slots [Q, Qpad) get true_row -1 (padding rows of the query operand).
+__global__ void __launch_bounds__(256)
+hole_typed_place_kernel(const int32_t* __restrict__ queries, int Q, int Qpad, int side,
+                        const int32_t* __restrict__ qtype, const int32_t* __restrict__ qrank,
+                        const int32_t* __restrict__ qoff, const int64_t* __restrict__ csr_off,
+                        const int32_t* __restrict__ t_pos, int32_t* __restrict__ sorted, int32_t* __restrict__ perm,
+                        int32_t* __restrict__ slot_type, int32_t* __restrict__ true_row) {
+  const int q = blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= Qpad) return;
+  if (q >= Q) { true_row[q] = -1; return; }
+  const int tau = qtype[q];
+  const int s = qoff[tau] + qrank[q];
+  const int h = queries[3 * q], t = queries[3 * q + 1], r = queries[3 * q + 2];
+  sorted[3 * s] = h; sorted[3 * s + 1] = t; sorted[3 * s + 2] = r;
+  perm[s] = q;
+  slot_type[s] = tau;
+  const int tp = t_pos != nullptr ? t_pos[side == HOLE_SIDE_TAIL ? t : h] : -1;      // top-k: no true candidate
+  true_row[s] = tp < 0 ? -1 : (int32_t)(csr_off[tau] + tp);
+}
+
+// One warp per type.  Top-k lists are laid out as hole_topk's, [slot][n_chunks][2][k]: a type with fewer chunks
+// leaves the rest of its slots' lists empty.
+__global__ void __launch_bounds__(256)
+hole_typed_items_kernel(const int32_t* __restrict__ tcount, const int64_t* __restrict__ csr_off, int n_types,
+                        const int32_t* __restrict__ qoff, const int32_t* __restrict__ nch,
+                        const int32_t* __restrict__ tper, const int32_t* __restrict__ ioff, int n_chunks,
+                        TypedItem* __restrict__ items) {
+  const int64_t tau = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (tau >= n_types) return;
+  const int c = tcount[tau], ch = nch[tau];
+  if (c == 0 || ch == 0) return;
+  const int64_t seg = csr_off[tau];
+  const int n = (int)(csr_off[tau + 1] - seg);
+  const int tiles = (n + BN - 1) / BN, tp = tper[tau];
+  const int windows = (c + BM - 1) / BM;
+  for (int i = lane; i < windows * ch; i += 32) {
+    const int w = i / ch, ci = i % ch;
+    TypedItem it;
+    it.q0 = qoff[tau] + w * BM;
+    it.q_end = qoff[tau] + c;
+    it.seg = (int32_t)seg;
+    it.n = n;
+    it.t0 = ci * tp;
+    it.t1 = min(tiles, it.t0 + tp);
+    it.tau = (int32_t)tau;
+    it.lstride = 2 * n_chunks;
+    it.l0 = ((int64_t)it.q0 * n_chunks + ci) * 2;
+    items[ioff[tau] + i] = it;
+  }
+}
+
+// hole_rank_typed's outputs, from slot order to the caller's rows.
+__global__ void __launch_bounds__(256)
+hole_typed_unpermute_kernel(const int32_t* __restrict__ perm, int Q, const int32_t* __restrict__ raw_s,
+                            const int32_t* __restrict__ filt_s, const float* __restrict__ true_s,
+                            int32_t* __restrict__ raw, int32_t* __restrict__ filt, float* __restrict__ true_out) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= Q) return;
+  const int q = perm[s];
+  raw[q] = raw_s[s];
+  filt[q] = filt_s[s];
+  true_out[q] = true_s[s];
+}
+
+// hole_topk_typed's rows, from slot order to the caller's rows.
+__global__ void __launch_bounds__(256)
+hole_typed_unpermute_rows_kernel(const int32_t* __restrict__ perm, int Q, int k, const int32_t* __restrict__ ids_s,
+                                 const float* __restrict__ scores_s, int32_t* __restrict__ ids,
+                                 float* __restrict__ scores) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i >= (int64_t)Q * k) return;
+  const int64_t s = i / k, c = i % k;
+  const int64_t o = (int64_t)perm[s] * k + c;
+  ids[o] = ids_s[i];
+  scores[o] = scores_s[i];
+}
+
 // ------------------------------------------------------------------------------------ host
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
@@ -1095,6 +1392,14 @@ struct hole_rank_ws {
   int64_t cache_begin = -1, cache_end = -1;
   int cache_parts = 0;
   bool cache_valid = false;
+  // typed calls (the plan above)
+  int32_t* t_pos = nullptr;        // [n_rows]
+  int32_t* t_q = nullptr;          // [TQ_ARRAYS][Qpad] per-query / per-slot arrays (see rank_impl)
+  int32_t* t_type = nullptr;       // [TT_ARRAYS][n_types + 1] per-type arrays, then the item count
+  TypedItem* t_items = nullptr;
+  int32_t* t_ids = nullptr;        // top-k: [Qpad, k] ids and scores in slot order
+  float* t_scores = nullptr;
+  size_t t_pos_cap = 0, t_q_cap = 0, t_type_cap = 0, t_items_cap = 0, t_ids_cap = 0, t_scores_cap = 0;   // elements
 };
 
 void hole_rank_cache_invalidate(hole_ctx* c) {
@@ -1105,6 +1410,8 @@ void hole_rank_ws_free(hole_ctx* c) {
   if (c->rank == nullptr) return;
   cudaFree(c->rank->cand); cudaFree(c->rank->qp); cudaFree(c->rank->tq); cudaFree(c->rank->true_idx);
   cudaFree(c->rank->qf); cudaFree(c->rank->tk_keys);
+  cudaFree(c->rank->t_pos); cudaFree(c->rank->t_q); cudaFree(c->rank->t_type);
+  cudaFree(c->rank->t_items); cudaFree(c->rank->t_ids); cudaFree(c->rank->t_scores);
   delete c->rank;
   c->rank = nullptr;
 }
@@ -1116,6 +1423,33 @@ static void split_chunks(RankParams& p, int sm_count) {
   p.chunk_tiles = (p.n_tiles + chunks - 1) / chunks;
   p.n_chunks = (p.n_tiles + p.chunk_tiles - 1) / p.chunk_tiles;
 }
+
+// Grows a workspace buffer to n elements (contents are not kept).  False when the allocation fails.
+template <class T>
+static bool ws_grow(T*& ptr, size_t& cap, size_t n, cudaStream_t st) {
+  if (n <= cap) return true;
+  cudaStreamSynchronize(st);
+  cudaFree(ptr); ptr = nullptr; cap = 0;
+  if (cudaMalloc((void**)&ptr, n * sizeof(T)) != cudaSuccess) {
+    cudaGetLastError();
+    return false;
+  }
+  cap = n;
+  return true;
+}
+
+// hole_rank_typed / hole_topk_typed: candidates are the rows of one type per query (the type tables of
+// hole_corrupt); query_type != null gives the types (top-k), else each query's true candidate's type.
+struct TypedArgs {
+  const int32_t* type_of;
+  const int64_t* csr_off;
+  const int32_t* csr_ids;
+  int64_t n_types;
+  const int32_t* query_type;
+};
+enum { TQ_TYPE, TQ_RANK, TQ_TRIPLES, TQ_PERM = TQ_TRIPLES + 3, TQ_SLOT_TYPE, TQ_TRUE_ROW, TQ_RAW, TQ_FILT, TQ_TRUE,
+       TQ_ARRAYS };
+enum { TT_COUNT, TT_QOFF, TT_NCH, TT_TPER, TT_IOFF, TT_ARRAYS };
 
 struct TopkArgs {
   int k;
@@ -1133,7 +1467,7 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
                      const float* query_table, const int32_t* queries, int64_t Q, int side, int precision,
                      const int64_t* filter_off, const int32_t* filter_ids, float* true_score_io,
                      int compute_true, int32_t* raw_before, int32_t* filt_before, void* stream,
-                     bool prepare_only, const TopkArgs* tk = nullptr) {
+                     bool prepare_only, const TopkArgs* tk = nullptr, const TypedArgs* ty = nullptr) {
   HOLE_CHECK_ARG(c && Q >= 0 && ent_begin >= 0 && ent_end >= ent_begin && ent_end <= c->n_rows);
   HOLE_CHECK_ARG(side == HOLE_SIDE_TAIL || side == HOLE_SIDE_HEAD || side == HOLE_SIDE_BOTH ||
                  side == HOLE_SIDE_RELATION);
@@ -1229,23 +1563,83 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
       w->qf_cap = qf_n; w->tk_cap = tk_n;
     }
   }
+  // typed calls: the chunk target and the workspace bounds come from the all-candidate shape (Q x n_rows):
+  // no type has more tiles, so no type has more items per query window than that shape has chunks
+  RankParams tshape{};
+  size_t t_items_max = 0;
+  if (ty) {
+    tshape.m_tiles = Qpad / BM;
+    tshape.n_tiles = Npad / BN;
+    split_chunks(tshape, c->sm_count);
+    t_items_max = (size_t)tshape.n_chunks * ((size_t)Qpad / BM + (size_t)std::min<int64_t>(Q, ty->n_types));
+    if ((ty->type_of && !ws_grow(w->t_pos, w->t_pos_cap, (size_t)c->n_rows, st)) ||
+        !ws_grow(w->t_q, w->t_q_cap, (size_t)TQ_ARRAYS * Qpad, st) ||
+        !ws_grow(w->t_type, w->t_type_cap, (size_t)TT_ARRAYS * (ty->n_types + 1) + 1, st) ||
+        !ws_grow(w->t_items, w->t_items_cap, t_items_max, st) ||
+        (topk && !ws_grow(w->t_ids, w->t_ids_cap, (size_t)Qpad * tk->k, st)) ||
+        (topk && !ws_grow(w->t_scores, w->t_scores_cap, (size_t)Qpad * tk->k, st)))
+      return hole_set_error(HOLE_ERR_ALLOC, "typed ranking workspace allocation failed");
+  }
   if (!w->attr_set) {
     HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<1, EPI_RANK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<2, EPI_RANK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<1, EPI_TOPK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<2, EPI_TOPK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<1, EPI_RANK, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<2, EPI_RANK, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<1, EPI_TOPK, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    HOLE_CUDA_TRY(cudaFuncSetAttribute(hole_rank_kernel<2, EPI_TOPK, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     w->attr_set = true;
   }
 
   w->last_npad = Npad; w->last_K = Kall;
   // operands: the candidate operand is reused when hole_rank_prepare packed exactly this table / range
-  const bool cached = !nb && w->cache_valid && w->cache_table == table && w->cache_begin == ent_begin &&
+  // (a typed call packs its own operand in type order, over the cache's buffer, and drops the cache)
+  const bool cached = !nb && !ty && w->cache_valid && w->cache_table == table && w->cache_begin == ent_begin &&
                       w->cache_end == ent_end && w->cache_parts == parts;
-  if (!cached) {
+  if (ty) {
+    w->cache_valid = false;
+    hole_rank_pack_cand_kernel<true><<<(unsigned)((Npad + 7) / 8), 256, 0, st>>>(table, c->row_stride, c->H, 0, Nc, Npad, K,
+                                                                                 parts, 0, w->cand, ty->csr_ids,
+                                                                                 ty->csr_off + ty->n_types);
+    HOLE_LAUNCHED();
+  } else if (!cached) {
     w->cache_valid = false;
     hole_rank_pack_cand_kernel<<<(unsigned)((Npad + 7) / 8), 256, 0, st>>>(table, c->row_stride, c->H, ent_begin, Nc, Npad, K, parts,
                                                                            nb ? 1 : 0, w->cand);
     HOLE_LAUNCHED();
+  }
+  // typed calls: the plan, then the query packers below run on the slot-ordered triples
+  int32_t* const tq_arr = ty ? w->t_q : nullptr;
+  auto tq = [&](int a) { return tq_arr + (size_t)a * Qpad; };
+  int32_t* const tt_arr = ty ? w->t_type : nullptr;
+  const int64_t n_types = ty ? ty->n_types : 0;
+  auto tt = [&](int a) { return tt_arr + (size_t)a * (n_types + 1); };
+  int32_t* const t_n_items = ty ? tt(TT_ARRAYS) : nullptr;
+  const int32_t* const t_pos = (ty && ty->type_of) ? w->t_pos : nullptr;   // ranking only
+  if (ty) {
+    if (t_pos) {
+      HOLE_CUDA_TRY(cudaMemsetAsync(w->t_pos, 0xff, (size_t)c->n_rows * 4, st));
+      hole_typed_pos_kernel<<<(unsigned)std::min<int64_t>(4 * c->sm_count, (c->n_rows + 255) / 256), 256, 0, st>>>(
+          ty->type_of, ty->csr_off, ty->csr_ids, n_types, w->t_pos);
+      HOLE_LAUNCHED();
+    }
+    HOLE_CUDA_TRY(cudaMemsetAsync(tt(TT_COUNT), 0, (size_t)n_types * 4, st));
+    hole_typed_count_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, st>>>(queries, ty->query_type, (int)Q, side, ty->type_of,
+                                                                         tq(TQ_TYPE), tq(TQ_RANK), tt(TT_COUNT));
+    HOLE_LAUNCHED();
+    hole_typed_scan_kernel<<<1, PLAN_THREADS, 0, st>>>(tt(TT_COUNT), ty->csr_off, (int)n_types, tshape.chunk_tiles,
+                                                       tt(TT_QOFF), tt(TT_NCH), tt(TT_TPER), tt(TT_IOFF), t_n_items);
+    HOLE_LAUNCHED();
+    hole_typed_place_kernel<<<(unsigned)((Qpad + 255) / 256), 256, 0, st>>>(
+        queries, (int)Q, Qpad, side, tq(TQ_TYPE), tq(TQ_RANK), tt(TT_QOFF), ty->csr_off, t_pos, tq(TQ_TRIPLES),
+        tq(TQ_PERM), tq(TQ_SLOT_TYPE), tq(TQ_TRUE_ROW));
+    HOLE_LAUNCHED();
+    hole_typed_items_kernel<<<(unsigned)((n_types * 32 + 255) / 256), 256, 0, st>>>(
+        tt(TT_COUNT), ty->csr_off, (int)n_types, tt(TT_QOFF), tt(TT_NCH), tt(TT_TPER), tt(TT_IOFF), tshape.n_chunks,
+        w->t_items);
+    HOLE_LAUNCHED();
+    queries = tq(TQ_TRIPLES);
   }
   if (prepare_only) {
     w->cache_table = table; w->cache_begin = ent_begin; w->cache_end = ent_end; w->cache_parts = parts;
@@ -1308,7 +1702,6 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
   p.stages = stages;
   p.Q = (int)Q;
   p.Nc = Nc;
-  p.true_idx = w->true_idx;
 
   if (topk) {
     rc = make_map(&mapB, w->cand, Npad, Kall, BN);
@@ -1320,6 +1713,24 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
     p.f_ids = filter_ids;
     p.ent_begin = ent_begin;
     p.tk_self = nb ? w->true_idx : nullptr;
+    if (ty) {
+      p.t_items = w->t_items; p.t_n_items = t_n_items; p.t_perm = tq(TQ_PERM);
+      p.type_of = ty->type_of; p.t_pos = w->t_pos; p.csr_ids = ty->csr_ids;
+      // the lists of a type with fewer chunks than the shape stay empty; keys hold global ids, so the merge
+      // runs unchanged (ent_begin 0) into slot-ordered rows
+      HOLE_CUDA_TRY(cudaMemsetAsync(w->tk_keys, 0xff, (size_t)Qpad * p.n_chunks * 2 * tk->k * sizeof(uint64_t), st));
+      const int grid = (int)std::min<size_t>(t_items_max, (size_t)c->sm_count);
+      if (parts == 2) hole_rank_kernel<2, EPI_TOPK, true><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+      else hole_rank_kernel<1, EPI_TOPK, true><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+      HOLE_LAUNCHED();
+      hole_topk_merge_kernel<<<(unsigned)Q, MERGE_THREADS, 0, st>>>(w->tk_keys, p.n_chunks * 2, tk->k, table, c->row_stride,
+                                                                    c->H, 0, w->qf, K, 0, w->t_ids, w->t_scores);
+      HOLE_LAUNCHED();
+      hole_typed_unpermute_rows_kernel<<<(unsigned)((Q * tk->k + 255) / 256), 256, 0, st>>>(
+          tq(TQ_PERM), (int)Q, tk->k, w->t_ids, w->t_scores, tk->ids_out, tk->scores_out);
+      HOLE_LAUNCHED();
+      return HOLE_OK;
+    }
     const int grid = std::min(p.m_tiles * p.n_chunks, c->sm_count);
     if (parts == 2) hole_rank_kernel<2, EPI_TOPK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
     else hole_rank_kernel<1, EPI_TOPK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
@@ -1331,16 +1742,20 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
     return HOLE_OK;
   }
 
+  // typed: the diagonal pass runs untyped on the slot-ordered operands, against the true candidates' operand rows
+  int32_t* const true_idx = ty ? tq(TQ_TRUE_ROW) : w->true_idx;
+  float* const true_s = ty ? reinterpret_cast<float*>(tq(TQ_TRUE)) : true_score_io;
+  p.true_idx = true_idx;
   if (compute_true) {
     const int rows = Qpad + BN;
-    hole_rank_gather_true_kernel<<<(unsigned)((Qpad + 31) / 32), 256, 0, st>>>(w->cand, w->true_idx, Nc, Qpad, Kall, w->tq);
+    hole_rank_gather_true_kernel<<<(unsigned)((Qpad + 31) / 32), 256, 0, st>>>(w->cand, true_idx, Nc, Qpad, Kall, w->tq);
     HOLE_LAUNCHED();
     HOLE_CUDA_TRY(cudaMemsetAsync(w->tq + (size_t)Qpad * Kall, 0, (size_t)BN * Kall * 2, st));
     rc = make_map(&mapB, w->tq, rows, Kall, BN / 2);      // DIAG tiles: the query tile's own 128 true rows
     if (rc) return rc;
     p.mode = MODE_DIAG;
     p.n_tiles = 1; p.chunk_tiles = 1; p.n_chunks = 1;
-    p.true_out = true_score_io;
+    p.true_out = true_s;
     const int grid = std::min(p.m_tiles, c->sm_count);
     if (parts == 2) hole_rank_kernel<2, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
     else hole_rank_kernel<1, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
@@ -1359,6 +1774,21 @@ static int rank_impl(hole_ctx* c, const float* table, int64_t ent_begin, int64_t
   p.f_off = filter_off;
   p.f_ids = filter_ids;
   p.ent_begin = ent_begin;
+  if (ty) {
+    // counts into zeroed slot-ordered buffers, then every output row is written in the caller's order
+    HOLE_CUDA_TRY(cudaMemsetAsync(tq(TQ_RAW), 0, (size_t)2 * Qpad * 4, st));      // TQ_RAW and TQ_FILT
+    p.true_score = true_s; p.raw_cnt = tq(TQ_RAW); p.filt_cnt = tq(TQ_FILT);
+    p.t_items = w->t_items; p.t_n_items = t_n_items; p.t_perm = tq(TQ_PERM);
+    p.type_of = ty->type_of; p.t_pos = w->t_pos; p.csr_ids = ty->csr_ids;
+    const int grid = (int)std::min<size_t>(t_items_max, (size_t)c->sm_count);
+    if (parts == 2) hole_rank_kernel<2, EPI_RANK, true><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+    else hole_rank_kernel<1, EPI_RANK, true><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
+    HOLE_LAUNCHED();
+    hole_typed_unpermute_kernel<<<(unsigned)((Q + 255) / 256), 256, 0, st>>>(tq(TQ_PERM), (int)Q, tq(TQ_RAW), tq(TQ_FILT),
+                                                                             true_s, raw_before, filt_before, true_score_io);
+    HOLE_LAUNCHED();
+    return HOLE_OK;
+  }
   const int grid = std::min(p.m_tiles * p.n_chunks, c->sm_count);
   if (parts == 2) hole_rank_kernel<2, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
   else hole_rank_kernel<1, EPI_RANK><<<grid, RANK_THREADS, smem_bytes, st>>>(mapA, mapB, p);
@@ -1400,6 +1830,32 @@ extern "C" int hole_neighbors(hole_ctx* c, const float* table, int64_t ent_begin
   const TopkArgs tk{k, ids_out, sim_out, true};
   return rank_impl(c, table, ent_begin, ent_end, nullptr, ids, Q, HOLE_SIDE_TAIL, precision, filter_off, filter_ids,
                    nullptr, 0, nullptr, nullptr, stream, false, &tk);
+}
+
+extern "C" int hole_rank_typed(hole_ctx* c, const float* table, const int32_t* queries, int64_t Q, int side,
+                               int precision, const int32_t* type_of, const int64_t* csr_off, const int32_t* csr_ids,
+                               int64_t n_types, const int64_t* filter_off, const int32_t* filter_ids,
+                               float* true_score_out, int32_t* raw_before, int32_t* filt_before, void* stream) {
+  HOLE_CHECK_ARG(c && (side == HOLE_SIDE_TAIL || side == HOLE_SIDE_HEAD));
+  HOLE_CHECK_ARG(type_of && csr_off && csr_ids && n_types >= 1 && n_types < (int64_t(1) << 30));
+  HOLE_CHECK_ARG(Q == 0 || (true_score_out && raw_before && filt_before));
+  const TypedArgs ty{type_of, csr_off, csr_ids, n_types, nullptr};
+  return rank_impl(c, table, 0, c->n_rows, nullptr, queries, Q, side, precision, filter_off, filter_ids,
+                   true_score_out, 1, raw_before, filt_before, stream, false, nullptr, &ty);
+}
+
+extern "C" int hole_topk_typed(hole_ctx* c, const float* table, const int32_t* queries, const int32_t* query_type,
+                               int64_t Q, int side, int precision, int k, const int64_t* csr_off,
+                               const int32_t* csr_ids, int64_t n_types, const int64_t* filter_off,
+                               const int32_t* filter_ids, int32_t* ids_out, float* scores_out, void* stream) {
+  HOLE_CHECK_ARG(c && k >= 1 && k <= TOPK_MAX && (Q == 0 || (query_type && ids_out && scores_out)));
+  HOLE_CHECK_ARG(side == HOLE_SIDE_TAIL || side == HOLE_SIDE_HEAD);
+  HOLE_CHECK_ARG(csr_off && csr_ids && n_types >= 1 && n_types < (int64_t(1) << 30));
+  // (no type_of: the top-k epilogue tests filter ids by their global id, and there is no true candidate)
+  const TypedArgs ty{nullptr, csr_off, csr_ids, n_types, query_type};
+  const TopkArgs tk{k, ids_out, scores_out, false};
+  return rank_impl(c, table, 0, c->n_rows, nullptr, queries, Q, side, precision, filter_off, filter_ids,
+                   nullptr, 0, nullptr, nullptr, stream, false, &tk, &ty);
 }
 
 extern "C" int hole_rank_prepare(hole_ctx* c, const float* table, int64_t ent_begin, int64_t ent_end,

@@ -466,6 +466,59 @@ class HoleEngine:
                                       _stream()))
         return ids_out, sims
 
+    def _typed_tables(self):
+        if self.type_of is None:
+            raise HoleError("type-constrained ranking needs the type tables: call set_types() first")
+        return self.type_of, self.csr_off, self.csr_ids, self.csr_off.shape[0] - 1
+
+    def _typed_queries(self, queries):
+        q = self._triples(queries)
+        if q.shape[0] and (int(q.min()) < 0 or int(q.max()) >= self.n_rows):
+            raise HoleError(f"query ids must lie in [0, {self.n_rows})")
+        return q
+
+    def rank_typed(self, queries, side, filter_off=None, filter_ids=None, precision=HOLE_RANK_BF16):
+        """Type-constrained ranking (hole_rank_typed): each query's true tail (HOLE_SIDE_TAIL) or head
+        (HOLE_SIDE_HEAD) ranked among the entities of its own type in the set_types() tables.  Returns
+        (raw_before int32[Q], filt_before int32[Q], true_score float32[Q]) on the device; rank = 1 + count.
+        Filter slices hold global ids, ascending; ids of other types are ignored."""
+        type_of, csr_off, csr_ids, n_types = self._typed_tables()
+        q = self._typed_queries(queries)
+        Q = q.shape[0]
+        if Q and int(side) in (HOLE_SIDE_TAIL, HOLE_SIDE_HEAD):
+            tau = type_of[q[:, 1 if int(side) == HOLE_SIDE_TAIL else 0].long()]
+            if int(tau.min()) < 0 or int(tau.max()) >= n_types:
+                raise HoleError("every query's true entity must have a type in [0, n_types)")
+        fo, fi = self._filter_csr(filter_off, filter_ids, Q)
+        raw = torch.zeros(Q, dtype=torch.int32, device=self.device)
+        filt = torch.zeros(Q, dtype=torch.int32, device=self.device)
+        true_score = torch.zeros(Q, dtype=torch.float32, device=self.device)
+        check(self.lib.hole_rank_typed(self._ctx, _ptr(self.table), _ptr(q), Q, int(side), int(precision),
+                                       _ptr(type_of), _ptr(csr_off), _ptr(csr_ids), n_types, _ptr(fo), _ptr(fi),
+                                       _ptr(true_score), _ptr(raw), _ptr(filt), _stream()))
+        return raw, filt, true_score
+
+    def topk_typed(self, queries, side, query_types, k, filter_off=None, filter_ids=None,
+                   precision=HOLE_RANK_BF16X3):
+        """Type-constrained top-k (hole_topk_typed): for query q, the k entities of type query_types[q] first in
+        ascending (score, id), skipping its filter slice (global ids, ascending).  Returns (ids int32[Q, k],
+        scores float32[Q, k]) on the device; padding is id -1 / score +inf."""
+        _, csr_off, csr_ids, n_types = self._typed_tables()
+        q = self._typed_queries(queries)
+        Q = q.shape[0]
+        qt = np.asarray(query_types.cpu() if isinstance(query_types, torch.Tensor) else query_types,
+                        dtype=np.int64).reshape(-1)
+        if qt.shape != (Q,) or (Q and (qt.min() < 0 or qt.max() >= n_types)):
+            raise HoleError(f"query_types must hold one type in [0, {n_types}) per query")
+        qt = torch.as_tensor(qt.astype(np.int32)).to(self.device).contiguous()
+        fo, fi = self._filter_csr(filter_off, filter_ids, Q)
+        ids_out = torch.empty((Q, int(k)), dtype=torch.int32, device=self.device)
+        scores = torch.empty((Q, int(k)), dtype=torch.float32, device=self.device)
+        check(self.lib.hole_topk_typed(self._ctx, _ptr(self.table), _ptr(q), _ptr(qt), Q, int(side), int(precision),
+                                       int(k), _ptr(csr_off), _ptr(csr_ids), n_types, _ptr(fo), _ptr(fi),
+                                       _ptr(ids_out), _ptr(scores), _stream()))
+        return ids_out, scores
+
     def _filter_csr(self, filter_off, filter_ids, rows):
         """Checks a filter CSR of `rows` slices (ascending ids within each) and returns it as device tensors
         (int64 offsets, int32 ids), or (None, None) for no filter or one without ids."""

@@ -628,6 +628,26 @@ def eval_link_prediction(eng, queries, known, relation_count, entity_count, side
     return raw_positions, filtered_positions
 
 
+def eval_link_prediction_type_constrained(eng, queries, known, sides=("tail", "head"), precision=HOLE_RANK_BF16X3):
+    """Type-constrained counterpart of eval_link_prediction: every test triple's tail (head) is ranked among the
+    entities of its own type in the engine's set_types() tables -- the candidates the corruption sampler draws
+    from and the reference's per-type pools (holE.py:381-424, 427-469) -- ascending by (score, id), on
+    HoleEngine.rank_typed.  Test triples are deduplicated, in-sample ones skipped, and train/valid-true
+    candidates do not advance the filtered rank.  No confidence gate, nothing written to inference_results.tsv.
+    Returns (raw_positions, filtered_positions) lists."""
+    queries = np.unique(np.asarray(queries, dtype=np.int32).reshape(-1, 3), axis=0)
+    queries = queries[~D.rows_in(queries, known)]
+    raw_positions, filtered_positions = [], []
+    if len(queries) == 0:
+        return raw_positions, filtered_positions
+    for side_name in sides:
+        foff, fids = D.build_filter_csr(queries, known, side_name)
+        raw, filt, _ = eng.rank_typed(queries, _SIDES[side_name], foff, fids, precision=precision)
+        raw_positions += (raw.cpu().numpy() + 1).tolist()
+        filtered_positions += (filt.cpu().numpy() + 1).tolist()
+    return raw_positions, filtered_positions
+
+
 def eval_link_prediction_typed(eng, heads, candidate, true_triples, test_triples, threshold=None):
     """The reference's own protocol (holE.py:564-573 + 427-469): for every head, the triples
     product([head], candidate.tail_candidates, candidate.relations) are ranked JOINTLY,
@@ -690,30 +710,40 @@ def eval_link_prediction_typed(eng, heads, candidate, true_triples, test_triples
 
 
 def predict_top_k(eng, test, known, relation_count, entity_count, k, path, precision=HOLE_RANK_BF16X3,
-                  value=None, sides=("tail", "head")):
+                  value=None, sides=("tail", "head"), type_of=None):
     """The all-entity generalisation of the reference's `max_triples` cut of the pop loop (holE.py:427-472):
     the k best NEW tails of every distinct (head, relation) pair of the test file and the k best new heads of
     every distinct (tail, relation) pair, filtered against the train + valid triples; with "relation" in
     `sides`, also the k best new relations of every distinct (head, tail) pair.  Writes one line per
     prediction to `path`:  side  head  tail  relation  position  score  value  in_test
     (position 1-based, score = raw s, value = value(s) (sigma by default), in_test = the predicted triple is
-    a test triple: the reference's MATCH vs GUESS).  Returns the number of lines written."""
+    a test triple: the reference's MATCH vs GUESS).  Returns the number of lines written.
+    type_of (entity sides only): type-constrained prediction on HoleEngine.topk_typed with the engine's
+    set_types() tables; the queries are then the distinct (known pair, type of its test answer), and each gets
+    the k best new entities of that type."""
     value = value or (lambda s: 1.0 / (1.0 + np.exp(-s)))
     test = np.asarray(test, dtype=np.int64).reshape(-1, 3)
     test_set = set(map(tuple, test.tolist()))
     key_cols = {"tail": (0, 2), "head": (1, 2), "relation": (0, 1)}       # the query's known columns
+    answer_col = {"tail": 1, "head": 0}
     n = 0
     with open(path, 'w') as out:
         for side_name in sides:
             side, cols = _SIDES[side_name], list(key_cols[side_name])
-            pairs = np.unique(test[:, cols], axis=0)
+            keys = test[:, cols]
+            if type_of is not None:                                    # (pair, type of its answer)
+                keys = np.concatenate([keys, np.asarray(type_of, np.int64)[test[:, answer_col[side_name]], None]], 1)
+            pairs = np.unique(keys, axis=0)
             if len(pairs) == 0:
                 continue
             queries = np.zeros((len(pairs), 3), dtype=np.int32)     # the predicted column is ignored
-            queries[:, cols] = pairs
+            queries[:, cols] = pairs[:, :2]
             foff, fids = D.build_filter_csr(queries, known, side_name)
-            lo, hi = _candidate_range(side_name, relation_count, entity_count)
-            ids, scores = eng.topk(queries, side, lo, hi, k, foff, fids, precision=precision)
+            if type_of is not None:
+                ids, scores = eng.topk_typed(queries, side, pairs[:, 2], k, foff, fids, precision=precision)
+            else:
+                lo, hi = _candidate_range(side_name, relation_count, entity_count)
+                ids, scores = eng.topk(queries, side, lo, hi, k, foff, fids, precision=precision)
             ids, scores = ids.cpu().numpy(), scores.cpu().numpy().astype(np.float64)
             vals = value(scores)
             for i, q in enumerate(queries.tolist()):
@@ -811,6 +841,23 @@ def infer_triples(flags=None, log=print):
             result = dict(result or {}, relation=score_mrr(rraw, rfilt, log))
         else:
             log('No test triple to rank (every one is in-sample).')
+    if getattr(flags, 'type_constrained', False):
+        # each answer among the entities of its type (the sampler's type set, not the --min_mentions pools);
+        # no confidence gate, nothing written to inference_results.tsv
+        type_of, csr_off, csr_ids = type_tables(data.entity_count, data.id_to_type)
+        eng.set_types(type_of, csr_off, csr_ids)
+        traw, tfilt = eval_link_prediction_type_constrained(eng, data.test, data.known, precision=precision)
+        log('\nType-constrained link prediction:')
+        if traw:
+            result = dict(result or {}, typed=score_mrr(traw, tfilt, log))
+        else:
+            log('No test triple to rank (every one is in-sample).')
+        if k:
+            value = np.tanh if getattr(flags, 'score_variant', 'complex') != 'complex' else None
+            path = os.path.join(flags.output_dir, 'predictions_typed.tsv')
+            n = predict_top_k(eng, data.test, data.known, data.relation_count, data.entity_count, k, path,
+                              precision=precision, value=value, type_of=type_of)
+            log('Wrote {} type-constrained predictions to {}'.format(n, path))
     return result
 
 
@@ -852,6 +899,12 @@ def build_parser():
                              '--predict_top_k, also write the K best new relations of every (head, tail) pair of the '
                              'test file to predictions.tsv.  Writes nothing to inference_results.tsv; --infer_gate '
                              'does not apply to it.')
+    parser.add_argument('--type_constrained', action='store_true',
+                        help='With --infer: also rank every test triple\'s tail and head among the entities of its own '
+                             'type (the types of entity_metadata.tsv the corruption sampler uses) and log that block\'s '
+                             'MRR / Hits; with --predict_top_k, also write the K best new entities of the answer\'s type '
+                             'for every (known pair, answer type) of the test file to predictions_typed.tsv.  No '
+                             'confidence gate; the all-entity outputs are unchanged.')
     parser.add_argument('--nearest_neighbors', type=int, default=0,
                         help='With --infer: write the K entity rows most similar (cosine of the embeddings) to every '
                              'entity of the test file, and the K relation rows most similar to every relation of it, '

@@ -457,6 +457,38 @@ HOLE_API int hole_neighbors(hole_ctx* ctx, const float* table, int64_t ent_begin
                             const int64_t* filter_off, const int32_t* filter_ids,
                             int32_t* ids_out, float* sim_out, void* stream);
 
+/* ---- type-constrained ranking and top-k: each query against the entities of one type only, the candidate set
+ * training draws its negatives from (hole_corrupt) and the reference's per-type candidate pools.
+ * Candidate set of query q: the rows csr_ids[csr_off[tau_q] .. csr_off[tau_q + 1]) of one type tau_q, in the type
+ * tables of hole_corrupt (type_of int32[n_rows], csr_off int64[n_types + 1], csr_ids int32[.], ids ASCENDING within a
+ * type: the tie order rests on it).  There is no ent_begin / ent_end range: the whole table is the candidate pool.
+ *   hole_rank_typed:  tau_q = type_of[true id] (t for HOLE_SIDE_TAIL, h for HOLE_SIDE_HEAD); the true id must be
+ *                     a row of its type.
+ *   hole_topk_typed:  tau_q = query_type[q], which the caller guarantees lies in [0, n_types).
+ * Sides: HOLE_SIDE_TAIL and HOLE_SIDE_HEAD only (BOTH and RELATION return HOLE_ERR_ARG).  Both score modes (the
+ * query packers are hole_rank's) and both precisions.  Limits and errors as hole_rank / hole_topk: dim <= 640 (bf16)
+ * / 320 (bf16x3) else HOLE_ERR_UNSUPPORTED, 1 <= k <= 128 else HOLE_ERR_ARG, HOLE_ERR_ALLOC when the workspace
+ * does not fit (split Q).  A refused call launches nothing, writes nothing and leaves the context usable.
+ * Results are hole_rank's and hole_topk's restricted to the type, and are WRITTEN (not accumulated):
+ *   raw_before[q]  = #{j of type tau_q : (s_j, j) < (s_true, true)}
+ *   filt_before[q] = raw_before[q] minus the filtered candidates among them (filter_off int64[Q+1] / filter_ids,
+ *                    may be NULL, global ids ascending within a slice; ids of other types are ignored)
+ *   true_score_out[q] = s_true from the same contraction (the diagonal pass)
+ *   ids_out [Q, k] / scores_out [Q, k]: the first k candidates of the type by (score, id), skipping the filter
+ *                    slice, rescored in fp32; padded with (-1, +inf) when the type has fewer than k left.
+ * Operand cache: like hole_neighbors, a typed call packs its own candidate operand (in type order) and drops a
+ * hole_rank_prepare'd one.  Row-sharded tables: gather the table first (gather_embeddings()).
+ * Cost: the contraction covers only the (query, candidate) tile pairs of each type; the device plan that groups
+ * the queries by type and lists the work items costs a few small launches and no host round trip. */
+HOLE_API int hole_rank_typed(hole_ctx* ctx, const float* table, const int32_t* queries, int64_t Q, int side,
+                             int precision, const int32_t* type_of, const int64_t* csr_off, const int32_t* csr_ids,
+                             int64_t n_types, const int64_t* filter_off, const int32_t* filter_ids,
+                             float* true_score_out, int32_t* raw_before, int32_t* filt_before, void* stream);
+HOLE_API int hole_topk_typed(hole_ctx* ctx, const float* table, const int32_t* queries, const int32_t* query_type,
+                             int64_t Q, int side, int precision, int k, const int64_t* csr_off,
+                             const int32_t* csr_ids, int64_t n_types, const int64_t* filter_off,
+                             const int32_t* filter_ids, int32_t* ids_out, float* scores_out, void* stream);
+
 /* Test hook: copy the bf16 operands the last hole_rank call packed (device to device).
  * cand_out [n_pad, K] / query_out [q_pad, K] may be NULL to query the shapes only. */
 HOLE_API int hole_rank_debug_operands(hole_ctx* ctx, void* cand_out, void* query_out,
